@@ -48,6 +48,7 @@ N_TRAIN, D_IN, B_PER_GPU = 4096, 16, 32
 N_PRED, D_PRED = 2000, 8
 FP64_PEAK_FALLBACK_TFLOPS = 37.19     # tools/ub_fp64.cu on this pool's B200 (profiles/r01_ub_fp64_peaks.json)
 HBM_PEAK_FALLBACK_GBS = 6552.0
+DUMP_PRED_POINTS = 1 << 18            # grid points whose posterior mean / variance --dump-outputs keeps (6 MB with their indices)
 
 
 def synth(n, d, seed=0):
@@ -114,6 +115,13 @@ def write_emulator_files(workdir, X, y, name, mucm="F", fix_nugget="T", alt_nugg
         f.write("beliefs %s_beliefs\ninputs %s_input\noutputs %s_output\ntv_config 10 0 0\ndelta_bounds [ ]\nsigma_bounds [ ]\n"
                 "nugget_bounds [ ]\ntries %d\nconstraints %s\n" % (name, name, name, tries, constraints))
     return name + "_config"
+
+
+def dump_outputs(outdir, arrays):
+    """Write every array as <outdir>/<name>.npy in float64, so that two builds can be compared output for output."""
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 @contextlib.contextmanager
@@ -307,7 +315,8 @@ def run_reference(args):
     """The reference's own algorithm for the metric's path on the host cores: every timed step is ONE real
     loglikelihood_gp4ml evaluation (value + gradient) at the full n = 4096, d = 16 -- a 1/32 sample of the B200 arm's
     step of 32 guesses, nothing extrapolated.  Warm-up steps run the same code at n = 1024 (they only have to spin
-    the BLAS pool up).  Timed steps stop early when the wall-clock budget is reached; `steps` is what was measured."""
+    the BLAS pool up).  --steps timed steps run unless --ref-budget caps the run's wall-clock time; `steps` is what was
+    measured."""
     if int(os.environ.get("RANK", "0")) != 0:
         return
     t_begin = time.perf_counter()
@@ -327,11 +336,11 @@ def run_reference(args):
         times = []
         for it in range(K):
             spent = time.perf_counter() - t_begin
-            if times and spent + 1.1 * max(times) > args.ref_budget:
+            if args.ref_budget is not None and times and spent + 1.1 * max(times) > args.ref_budget:
                 break
             times.append(cpu_llh_eval(X, y, H, thetas[it % B_PER_GPU] + 1e-3 * it))
         spent = time.perf_counter() - t_begin
-        if spent + 1.2 * max(times) < args.ref_budget + 60:      # one full-size MUCM evaluation when it still fits
+        if args.ref_budget is None or spent + 1.2 * max(times) < args.ref_budget + 60:      # one full-size MUCM evaluation when it fits
             t_mucm = cpu_llh_eval(X, y, H, thetas[0], mucm=True)
     v = len(times) / float(sum(times))
     extra_cpu["llh_n4096_d16"] = {"gp4ml_s_per_eval": [round(t, 3) for t in times], "gp4ml_s_per_eval_median": float(np.median(times)),
@@ -548,6 +557,17 @@ def run_b200(args):
     barrier()
     ms = e0.elapsed_time(e1)
     launches = dev.launches - l0
+    # what the last timed step returned, taken before the passes below reuse the buffers: every rank's block of guesses,
+    # gathered in guess order
+    dumped = None
+    if args.dump_outputs:
+        mine = torch.cat([llh_d[:, None], grad_d, sig_d[:, None], st_d.double()[:, None]], dim=1)
+        blocks = [mine]
+        if world > 1:
+            blocks = [torch.empty_like(mine) for _ in range(world)]
+            dist.all_gather(blocks, mine)
+        step = torch.cat(blocks).cpu().numpy()
+        dumped = {"llh": step[:, 0], "grad": step[:, 1:p + 1], "sigma_hat": step[:, p + 1], "status": step[:, p + 2]}
     t = torch.tensor([ms], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -633,6 +653,11 @@ def run_b200(args):
         p1.record(pstream)
         barrier()
         pred_launches = devp.launches - lp0
+        if dumped is not None and m:      # a fixed sample of the shard's points (flat grid indices kept beside the values)
+            pick = np.sort(np.random.default_rng(0).choice(m, size=min(m, DUMP_PRED_POINTS), replace=False))
+            pick_d = torch.from_numpy(pick).cuda()
+            dumped.update(posterior_index=start + pick, posterior_mean=mean_d[0, pick_d].cpu().numpy(),
+                          posterior_var=var_d[0, pick_d].cpu().numpy())
         pms = torch.tensor([p0.elapsed_time(p1)], dtype=torch.float64, device="cuda")
         if world > 1:
             dist.all_reduce(pms, op=dist.ReduceOp.MAX)
@@ -885,6 +910,8 @@ def run_b200(args):
                     line["extra"]["cpu"] = cpu_other_legs()
                 except Exception as ex:
                     line["extra"]["cpu"] = {"error": repr(ex)}
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(line), file=RESULT_OUT, flush=True)
     if world > 1:
         dist.barrier()
@@ -911,12 +938,20 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline legs")
     ap.add_argument("--no-extra", action="store_true", help="skip the config 2 / 3-as-optimisation / 5 legs")
     ap.add_argument("--no-noisefit", action="store_true", help="skip the noise-fit leg of config 5")
-    ap.add_argument("--ref-budget", type=float, default=300.0,
-                    help="wall-clock budget (s) of the --impl reference run: full-size evaluations are timed until it is reached "
-                         "(about six at 41 s each on 16 cores; their spread is under 2 %)")
+    ap.add_argument("--ref-budget", type=float, default=None,
+                    help="optional wall-clock cap (s) of the --impl reference run; when given it overrides --steps: timed full-size "
+                         "evaluations (about 41 s each on 16 host cores) stop before the cap is passed")
     ap.add_argument("--streams", type=int, default=8, help="concurrent sub-batch streams of gpe_llh_grad_batch")
     ap.add_argument("--grid-points", type=float, default=1e8, help="size of the prediction grid (config 4: 1e8)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (llh, grad, sigma_hat, status of every guess of the step, all "
+                         "ranks gathered in guess order) and the posterior mean / variance of a fixed sample of %d grid points with "
+                         "their flat indices (under N > 1: of rank 0's shard) as DIR/<name>.npy (float64)" % DUMP_PRED_POINTS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)
