@@ -103,6 +103,7 @@ class Beliefs:
     """Beliefs file (reference :102-213) and the writer of updated beliefs files (:217-250)."""
 
     REQUIRED = ("active", "output", "basis_str", "basis_inf", "beta", "delta", "sigma", "nugget", "fix_nugget", "mucm")
+    KERNELS = ("gaussian", "matern52")
 
     def __init__(self, beliefs_file):
         self.beliefs_file = beliefs_file
@@ -152,6 +153,10 @@ class Beliefs:
         self.mucm = words("mucm")[0]
         if self.mucm == "T" and self.alt_nugget == "T":
             _die("WARNING: mucm T cannot be used with alt_nugget T")
+        # covariance family: absent means the reference's Gaussian kernel, so every existing file keeps its meaning
+        self.kernel = words("kernel")[0] if "kernel" in b else "gaussian"
+        if self.kernel not in self.KERNELS:
+            _die("WARNING: kernel should be one of %s" % " ".join(self.KERNELS))
         self.input_minmax = eval(b["input_minmax"]) if "input_minmax" in b else []
 
     def final_beliefs(self, E, final=False):
@@ -175,6 +180,7 @@ class Beliefs:
             "fix_nugget " + str(self.fix_nugget),
             "alt_nugget " + str(self.alt_nugget),
             "mucm " + str(self.mucm),
+        ] + (["kernel " + self.kernel] if self.kernel != "gaussian" else []) + [
             "input_minmax " + str(E.all_data.input_minmax),
         ]
         try:
@@ -484,13 +490,14 @@ class Data:
         """The handle holding this data set on the GPU (created and re-uploaded on demand)."""
         if self._dev is None:
             self._dev = _lib.Device(_lib.default_device_index())
-        fp = self._fingerprint()
+        fp = (self.K.family,) + self._fingerprint()
         if fp != self._loaded:
             y = np.zeros(self.inputs.shape[0]) if self.outputs is None else self.outputs
             r = self._r_made if np.ndim(self._r_made) else None
             self._dev.set_training(self.inputs, y, self.H, r)
             if self.basis.poly is not None:
                 self._dev.set_basis(self.basis.basis_inf, self.basis.poly)
+            self._dev.set_kernel(self.K.family)
             self._loaded = fp
             self._fit_key = None
         return self._dev
@@ -499,7 +506,7 @@ class Data:
         """Factor the training matrix for the current hyper-parameters (cached): returns
         (device, optimal beta, analytic MUCM sigma)."""
         dev = self.device()
-        key = (tuple(np.asarray(self.K.d, dtype=float)), float(self.K.n), float(self.par.sigma), self.kind,
+        key = (tuple(np.asarray(self.K.d, dtype=float)), float(self.K.n), float(self.par.sigma), self.kind, self.K.family,
                None if beta is None else tuple(np.asarray(beta, dtype=float)), float(r_div))
         if key != self._fit_key:
             bopt, sig, st = dev.fit_state(self.K.d, self.K.n, self.par.sigma, self.kind, beta=beta, r_div=r_div)

@@ -1,8 +1,10 @@
 """Covariance kernels with the reference's interface (gp_emu_uqsa/_emulatorkernels.py):
 ``kernel`` -- (1-nugget)*exp(-sum((x_i-x_j)/delta)^2), diagonal 1 -- and ``kernel_alt_nug`` --
-exp(..), diagonal 1+nugget^2.  Every matrix is produced by the CUDA kernels behind the C-ABI
-(K1 ``cov_build_kernel`` / ``xcov_kernel``); the classes only carry the hyper-parameters and
-the reference's side effects (``self.A``)."""
+exp(..), diagonal 1+nugget^2.  ``kernel_matern52`` / ``kernel_matern52_alt_nug`` are the same two
+forms with the Matern 5/2 correlation R = (1 + sqrt5 r + 5 D/3) exp(-sqrt5 r), r = sqrt(D), in place of
+exp(-D), D = sum((x_i-x_j)/delta)^2 (beliefs key ``kernel matern52``).  Every matrix is produced by the
+CUDA kernels behind the C-ABI (K1 ``cov_build_kernel`` / ``xcov_kernel``); the classes only carry the
+hyper-parameters, the covariance family and the reference's side effects (``self.A``)."""
 import numpy as np
 
 from . import _lib
@@ -11,8 +13,9 @@ np.set_printoptions(precision=6)
 np.set_printoptions(suppress=True)
 
 
-class _GaussianKernel:
+class _Kernel:
     kind = 0
+    family = _lib.KERNEL_GAUSSIAN
 
     def __init__(self, dim, par):
         self.d = par.delta
@@ -39,14 +42,14 @@ class _GaussianKernel:
         return np.exp(hp / 2.0)
 
     # -- dense matrices for arbitrary point sets: one-off device calls on the scratch handle ----
-    @staticmethod
-    def _loaded_scratch(X):
+    def _loaded_scratch(self, X):
         X = np.ascontiguousarray(X, dtype=float)
         if X.ndim == 1:
             X = X.reshape(-1, 1)
         dev = _lib.scratch_device()
         n = X.shape[0]
         dev.set_training(X, np.zeros(n), np.ones((n, 1)))
+        dev.set_kernel(self.family)          # the scratch handle is shared by every kernel object
         return dev, X
 
     def var(self, X, predict=True):
@@ -76,9 +79,19 @@ class _GaussianKernel:
         return dev.cov_grad(self.d, self.n, self.kind, -1, s2)
 
 
-class kernel(_GaussianKernel):
+class kernel(_Kernel):
     kind = 0
 
 
-class kernel_alt_nug(_GaussianKernel):
+class kernel_alt_nug(_Kernel):
     kind = 1
+
+
+class kernel_matern52(_Kernel):
+    kind = 0
+    family = _lib.KERNEL_MATERN52
+
+
+class kernel_matern52_alt_nug(_Kernel):
+    kind = 1
+    family = _lib.KERNEL_MATERN52

@@ -12,6 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libgpe_b200.so")
 
 MODE_MUCM, MODE_ALT_NUGGET, MODE_NUGGET_FREE = 1, 2, 4
+KERNEL_GAUSSIAN, KERNEL_MATERN52 = 0, 1
 KM_FULL, KM_LE_J, KM_GE_J, KM_LE_I, KM_GE_I = 0, 1, 2, 3, 4
 
 _dp = C.c_void_p
@@ -42,6 +43,7 @@ def load():
         "gpe_get_stream": (p, [p]),
         "gpe_set_streams": (i, [p, i]),
         "gpe_set_async": (i, [p, i]),
+        "gpe_set_kernel": (i, [p, i]),
         "gpe_synchronize": (i, [p]),
         "gpe_profile_enable": (i, [p, i]),
         "gpe_profile_read": (i, [p, p, p, i]),
@@ -74,7 +76,7 @@ def load():
 
 
 EXPORTS = ["gpe_version", "gpe_create", "gpe_destroy", "gpe_last_error", "gpe_launch_count",
-           "gpe_get_stream", "gpe_set_streams", "gpe_set_async", "gpe_synchronize", "gpe_profile_enable", "gpe_profile_read",
+           "gpe_get_stream", "gpe_set_streams", "gpe_set_async", "gpe_set_kernel", "gpe_synchronize", "gpe_profile_enable", "gpe_profile_read",
            "gpe_set_training", "gpe_set_basis", "gpe_cov_build", "gpe_cov_grad", "gpe_cross_cov", "gpe_llh_grad_batch",
            "gpe_fit_state", "gpe_predict", "gpe_predict_grid", "gpe_predict_fullcov", "gpe_implausibility", "gpe_predict_implaus",
            "gpe_solve", "gpe_sens_contract", "gpe_sens_main_effect", "gpe_potrf", "gpe_pdist_argmin",
@@ -165,6 +167,10 @@ class Device:
     def set_streams(self, nstreams):
         """Number of concurrent sub-batch streams of llh_grad_batch (1 = serial launches)."""
         self._ck(self.L.gpe_set_streams(self.h, int(nstreams)))
+
+    def set_kernel(self, family):
+        """Covariance family of every later call (KERNEL_GAUSSIAN / KERNEL_MATERN52); a change drops the fit state."""
+        self._ck(self.L.gpe_set_kernel(self.h, int(family)))
 
     def set_async(self, on=True):
         """Calls whose inputs and outputs are all device tensors return once enqueued; ``synchronize()`` waits."""

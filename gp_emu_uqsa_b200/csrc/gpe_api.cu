@@ -316,7 +316,8 @@ static int llh_grad_fused(gpe_handle* h, int B) {
         mode = e ? atoi(e) : 2;
     }
     h->grad_use_e = false;
-    if (!gemm_is_big(h->npad, h->npad, 1, B)) return 0;
+    // Matérn: the stand-alone reduction recomputes R and G (the LAUUM epilogue and the E copy are Gaussian-only)
+    if (h->family != FAMILY_GAUSSIAN || !gemm_is_big(h->npad, h->npad, 1, B)) return 0;
     if (h->oz_nmod > 0 && h->npad >= h->oz_min && h->npad % OZ_BN == 0) {   // LAUUM on the INT8 route, A^-1 stored: the stand-alone
         static const int use_e = [] { const char* e = getenv("GPE_GRAD_E"); return e ? atoi(e) : 1; }();   // reduction reads the
         h->grad_use_e = use_e != 0;                                          // covariance build's copy of exp(-D)
@@ -389,7 +390,7 @@ int gpe_factor_and_reduce(gpe_handle* h, const SubBatch& sb, int mode, int with_
         ProfScope ps(h, gpe_handle::CAT_GRAD, st);
         launch_grad_partial(h->X, h->r, h->n, h->d, np, h->winv + (size_t)b0 * h->d, Ab, sM, U, h->q + 1,
                             h->gpart + (size_t)b0 * grad_ntiles(np) * grad_nvals(h->d), B, st,
-                            h->grad_use_e ? h->Ex + (size_t)b0 * sM : nullptr);
+                            h->grad_use_e ? h->Ex + (size_t)b0 * sM : nullptr, h->family);
     }
     h->launches++;
     return 0;
@@ -503,6 +504,22 @@ int gpe_set_streams(gpe_handle* h, int nstreams) {
     return 0;
 }
 
+int gpe_set_kernel(gpe_handle* h, int family) {
+    if (!h) return -2;
+    if (family != GPE_KERNEL_GAUSSIAN && family != GPE_KERNEL_MATERN52) return h->fail_msg("unknown kernel family");
+    if (family == h->family) return 0;
+    CK(cudaSetDevice(h->device));
+    CK(cudaStreamSynchronize(h->st));
+    // the fit state and the captured likelihood graphs (keyed on batch and mode only) belong to the old kernel; a new
+    // fit generation makes the prediction product re-make its residue planes of L^-1
+    h->family = family;
+    h->fitted = false;
+    h->fAinv_valid = false;
+    h->fit_gen++;
+    h->drop_graphs();
+    return 0;
+}
+
 int gpe_set_async(gpe_handle* h, int on) {
     if (!h) return -2;
     h->async = on != 0;
@@ -612,7 +629,7 @@ int gpe_cov_build(gpe_handle* h, const double* delta, double nugget, int kind, i
     std::vector<double> dl(h->d);
     CK(cudaMemcpy(dl.data(), delta, sizeof(double) * h->d, cudaMemcpyDefault));
     if ((rc = gpe_upload_single_par(h, dl.data(), nugget, kind, predict, s2))) return rc;
-    CK(launch_cov_build(h->X, h->r, h->n, h->d, h->npad, h->par, h->winv, h->A, 0, 1, 1, h->st));
+    CK(launch_cov_build(h->X, h->r, h->n, h->d, h->npad, h->par, h->winv, h->A, 0, 1, 1, h->st, 0, 0, nullptr, h->family));
     h->launches++;
     size_t nn = (size_t)h->n * h->n;
     double* dst = A_out;
@@ -638,6 +655,7 @@ int gpe_cov_grad(gpe_handle* h, const double* delta, double nugget, int kind, in
     ItemPar ip;
     host_item_par(ip, nugget, kind, 1, 1.0, 1.0);
     // grad_delta_A: s2 (1-nu) Delta^2 E  (alt: s2 Delta^2 E);  grad_nugget_A (kernel): -1/2 nu s2 E
+    // (Matérn: G in place of E in grad_delta_A, R in place of E in grad_nugget_A)
     ip.offs = (which >= 0) ? s2 * ip.c : -0.5 * nugget * s2;
     std::vector<double> w(h->d);
     for (int k = 0; k < h->d; k++) w[k] = 1.0 / dl[k];
@@ -654,7 +672,8 @@ int gpe_cov_grad(gpe_handle* h, const double* delta, double nugget, int kind, in
         CK(cudaMemcpy(G_out, host.data(), nn * sizeof(double), cudaMemcpyDefault));
         return 0;
     }
-    CK(launch_cov_build(h->X, h->r, h->n, h->d, h->npad, h->par, h->winv, h->A, 0, 1, 1, h->st, which >= 0 ? 1 : 2, which));
+    CK(launch_cov_build(h->X, h->r, h->n, h->d, h->npad, h->par, h->winv, h->A, 0, 1, 1, h->st, which >= 0 ? 1 : 2, which,
+                        nullptr, h->family));
     launch_unpad_sym(h->A, h->npad, h->n, dst, 0, h->st);
     h->launches += 2;
     if (!dev) CK(cudaMemcpyAsync(G_out, dst, nn * sizeof(double), cudaMemcpyDeviceToHost, h->st));
@@ -706,7 +725,7 @@ static int enqueue_llh_chunk(gpe_handle* h, int Bs, int p, int mode, double fixe
             ProfScope ps(h, gpe_handle::CAT_COV, sb.st);
             CK(launch_cov_build(h->X, h->r, h->n, h->d, h->npad, h->par + sb.b0, h->winv + (size_t)sb.b0 * h->d,
                                 h->A + (size_t)sb.b0 * sM, sM, sb.B, 0, sb.st, 0, 0,
-                                (h->grad_fused || h->grad_use_e) ? h->Ex + (size_t)sb.b0 * sM : nullptr));
+                                (h->grad_fused || h->grad_use_e) ? h->Ex + (size_t)sb.b0 * sM : nullptr, h->family));
         }
         h->launches++;
         if ((rc = gpe_factor_and_reduce(h, sb, mode, 1, nullptr, nullptr))) return rc;

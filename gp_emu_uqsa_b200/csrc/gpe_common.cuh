@@ -112,6 +112,22 @@ __device__ __forceinline__ double gpe_exp(double x) {
     return q * __hiloint2double((k1 + 1023) << 20, 0) * __hiloint2double((k2 + 1023) << 20, 0);
 }
 
+// ---- Matérn 5/2 from the scaled squared distance D = sum_k ((x_ik - x_jk) / delta_k)^2, r = sqrt(D) ----------------------
+// R = (1 + sqrt5 r + 5D/3) exp(-sqrt5 r) is the correlation; G = (5/6)(1 + sqrt5 r) exp(-sqrt5 r) is its derivative factor,
+// dR/dtheta_k = G Delta_k^2 for delta_k = exp(theta_k / 2).  One exponential serves both; sqrt is the IEEE one.
+constexpr int FAMILY_GAUSSIAN = 0, FAMILY_MATERN52 = 1;
+__device__ __forceinline__ double gpe_matern52(double D, double& G) {
+    const double s5r = 2.23606797749978969641 * __dsqrt_rn(D);
+    const double e = gpe_exp(-s5r);
+    const double p = 1.0 + s5r;
+    G = (5.0 / 6.0) * p * e;
+    return fma(D, 5.0 / 3.0, p) * e;
+}
+__device__ __forceinline__ double gpe_matern52(double D) {
+    double G;
+    return gpe_matern52(D, G);   // (G is dead code here)
+}
+
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

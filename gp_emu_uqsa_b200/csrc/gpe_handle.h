@@ -58,6 +58,7 @@ struct gpe_handle {
     int n = 0, d = 0, q = 0, npad = 0, nleaf = 0;
     double *X = nullptr, *y = nullptr, *H = nullptr, *r = nullptr, *HY = nullptr;
     bool has_basis = false;
+    int family = gpe::FAMILY_GAUSSIAN;   // covariance function of every call (gpe_set_kernel)
     int basis_idx[gpe::NR] = {0}, basis_pow[gpe::NR] = {0};
 
     // batched likelihood workspace

@@ -60,8 +60,10 @@ __device__ __forceinline__ void tri_decode(int t, int& ti, int& tj) {
 
 // GMODE 0: covariance (the hot path: no G registers, no spills under the 80-register cap of 3 CTAs/SM);
 // 1: d(s2 A)/d theta_delta[gdim] (grad_delta_A); 2: kernel grad_nugget_A (off-diagonal only; the alt-nugget form
-// is a pure diagonal and is assembled by the caller)
-template <int GMODE>
+// is a pure diagonal and is assembled by the caller).
+// FAM: FAMILY_GAUSSIAN (E = exp(-D) is both the entry and the derivative factor) or FAMILY_MATERN52 (entry R(D); GMODE 1
+// uses the derivative factor G(D) in its place; no E copy)
+template <int GMODE, int FAM>
 __global__ void __launch_bounds__(256, 3) cov_build_kernel(const double* __restrict__ X, const double* __restrict__ r,
                                                         int n, int d, int npad, const ItemPar* __restrict__ par,
                                                         const double* __restrict__ winv, double* __restrict__ A,
@@ -114,7 +116,11 @@ __global__ void __launch_bounds__(256, 3) cov_build_kernel(const double* __restr
 #pragma unroll
     for (int a = 0; a < 4; a++)
 #pragma unroll
-        for (int c = 0; c < 4; c++) D[a][c] = gpe_exp(-D[a][c]);
+        for (int c = 0; c < 4; c++) {
+            if constexpr (FAM == FAMILY_GAUSSIAN) D[a][c] = gpe_exp(-D[a][c]);
+            else if constexpr (GMODE == 1) gpe_matern52(D[a][c], D[a][c]);
+            else D[a][c] = gpe_matern52(D[a][c]);
+        }
     double* Ab = A + (size_t)b * sA;
 #pragma unroll
     for (int a = 0; a < 4; a++) {
@@ -135,7 +141,7 @@ __global__ void __launch_bounds__(256, 3) cov_build_kernel(const double* __restr
                 v[e] = val;
             }
             *reinterpret_cast<double2*>(&Ab[(size_t)gi * npad + gj0]) = make_double2(v[0], v[1]);
-            if constexpr (GMODE == 0) {
+            if constexpr (GMODE == 0 && FAM == FAMILY_GAUSSIAN) {
                 if (Eout != nullptr)
                     *reinterpret_cast<double2*>(&Eout[(size_t)b * sA + (size_t)gi * npad + gj0]) = make_double2(D[a][2 * h], D[a][2 * h + 1]);
             }
@@ -143,25 +149,34 @@ __global__ void __launch_bounds__(256, 3) cov_build_kernel(const double* __restr
     }
 }
 
-cudaError_t launch_cov_build(const double* X, const double* r, int n, int d, int npad, const ItemPar* par,
-                             const double* winv, double* A, long long sA, int B, int full, cudaStream_t st, int gmode, int gdim,
-                             double* Eout) {
-    const int nt = npad / CT;
-    dim3 grid = full ? dim3(nt, nt, B) : dim3(nt * (nt + 1) / 2, 1, B);
-    size_t smem = (size_t)d * (CT + CT + 2) * sizeof(double);
+template <int FAM>
+static cudaError_t launch_cov_build_fam(const double* X, const double* r, int n, int d, int npad, const ItemPar* par,
+                                       const double* winv, double* A, long long sA, dim3 grid, size_t smem, int full,
+                                       cudaStream_t st, int gmode, int gdim, double* Eout) {
     static SmemOptIn opt0, opt1, opt2;
     cudaError_t e;
     if (gmode == 0) {
-        if ((e = opt0.ensure(cov_build_kernel<0>, smem)) != cudaSuccess) return e;
-        cov_build_kernel<0><<<grid, 256, smem, st>>>(X, r, n, d, npad, par, winv, A, sA, full, gdim, Eout);
+        if ((e = opt0.ensure(cov_build_kernel<0, FAM>, smem)) != cudaSuccess) return e;
+        cov_build_kernel<0, FAM><<<grid, 256, smem, st>>>(X, r, n, d, npad, par, winv, A, sA, full, gdim, Eout);
     } else if (gmode == 1) {
-        if ((e = opt1.ensure(cov_build_kernel<1>, smem)) != cudaSuccess) return e;
-        cov_build_kernel<1><<<grid, 256, smem, st>>>(X, r, n, d, npad, par, winv, A, sA, full, gdim, nullptr);
+        if ((e = opt1.ensure(cov_build_kernel<1, FAM>, smem)) != cudaSuccess) return e;
+        cov_build_kernel<1, FAM><<<grid, 256, smem, st>>>(X, r, n, d, npad, par, winv, A, sA, full, gdim, nullptr);
     } else {
-        if ((e = opt2.ensure(cov_build_kernel<2>, smem)) != cudaSuccess) return e;
-        cov_build_kernel<2><<<grid, 256, smem, st>>>(X, r, n, d, npad, par, winv, A, sA, full, gdim, nullptr);
+        if ((e = opt2.ensure(cov_build_kernel<2, FAM>, smem)) != cudaSuccess) return e;
+        cov_build_kernel<2, FAM><<<grid, 256, smem, st>>>(X, r, n, d, npad, par, winv, A, sA, full, gdim, nullptr);
     }
     return cudaGetLastError();
+}
+
+cudaError_t launch_cov_build(const double* X, const double* r, int n, int d, int npad, const ItemPar* par,
+                             const double* winv, double* A, long long sA, int B, int full, cudaStream_t st, int gmode, int gdim,
+                             double* Eout, int family) {
+    const int nt = npad / CT;
+    dim3 grid = full ? dim3(nt, nt, B) : dim3(nt * (nt + 1) / 2, 1, B);
+    size_t smem = (size_t)d * (CT + CT + 2) * sizeof(double);
+    if (family == FAMILY_MATERN52)
+        return launch_cov_build_fam<FAMILY_MATERN52>(X, r, n, d, npad, par, winv, A, sA, grid, smem, full, st, gmode, gdim, nullptr);
+    return launch_cov_build_fam<FAMILY_GAUSSIAN>(X, r, n, d, npad, par, winv, A, sA, grid, smem, full, st, gmode, gdim, Eout);
 }
 
 __global__ void unpad_sym_kernel(const double* __restrict__ A, int npad, int n, double* __restrict__ out, int mirror) {
@@ -860,7 +875,8 @@ constexpr int GD = 16;  // dims accumulated per register pass
 
 // USE_E: E = exp(-D) is read from the copy the covariance build kept (8 B per entry from an idle HBM) instead of being
 // recomputed (2d + 22 FP64 instructions per entry on the pipe this kernel is bound by).
-template <bool USE_E>
+// FAM == FAMILY_MATERN52 (recompute path only): t holds 2 W G for the d delta sums and sE collects 2 W R directly.
+template <bool USE_E, int FAM>
 __global__ void __launch_bounds__(256, 2) grad_partial_kernel(const double* __restrict__ X, const double* __restrict__ r,
                                                            int n, int d, int npad, const double* __restrict__ winv,
                                                            const double* __restrict__ Ainv, long long sAinv,
@@ -961,10 +977,12 @@ __global__ void __launch_bounds__(256, 2) grad_partial_kernel(const double* __re
                         D[a][c] = fma(df, df, D[a][c]);
                     }
             }
+            if constexpr (FAM == FAMILY_GAUSSIAN) {
 #pragma unroll
-            for (int a = 0; a < 4; a++)
+                for (int a = 0; a < 4; a++)
 #pragma unroll
-                for (int c = 0; c < 4; c++) D[a][c] = gpe_exp(-D[a][c]);      // 16 interleaved chains, no branches
+                    for (int c = 0; c < 4; c++) D[a][c] = gpe_exp(-D[a][c]);      // 16 interleaved chains, no branches
+            }
         }
 #pragma unroll
         for (int a = 0; a < 4; a++) {
@@ -977,18 +995,33 @@ __global__ void __launch_bounds__(256, 2) grad_partial_kernel(const double* __re
                     int gj = gj0 + e;
                     double wv = dot[a][2 * h + e];
                     double tv = 0.0;
-                    // A^-1 is valid on and below the diagonal only (LAUUM computes lower fragments):
-                    // every off-diagonal pair is taken once from the lower triangle with weight 2
-                    if (gi < n && gj < n) {
-                        if (gi == gj) {
-                            sD += wv;
-                            if (r != nullptr) sDr = fma(wv, r[gi], sDr);
-                        } else if (gi > gj) {
-                            tv = 2.0 * wv * D[a][2 * h + e];
+                    if constexpr (FAM == FAMILY_GAUSSIAN) {
+                        // A^-1 is valid on and below the diagonal only (LAUUM computes lower fragments):
+                        // every off-diagonal pair is taken once from the lower triangle with weight 2
+                        if (gi < n && gj < n) {
+                            if (gi == gj) {
+                                sD += wv;
+                                if (r != nullptr) sDr = fma(wv, r[gi], sDr);
+                            } else if (gi > gj) {
+                                tv = 2.0 * wv * D[a][2 * h + e];
+                            }
                         }
+                        sE += tv;
+                    } else {
+                        double g, sv = 0.0;
+                        const double rv = gpe_matern52(D[a][2 * h + e], g);     // unconditional: the chains interleave
+                        if (gi < n && gj < n) {
+                            if (gi == gj) {
+                                sD += wv;
+                                if (r != nullptr) sDr = fma(wv, r[gi], sDr);
+                            } else if (gi > gj) {
+                                tv = 2.0 * wv * g;
+                                sv = 2.0 * wv * rv;
+                            }
+                        }
+                        sE += sv;
                     }
                     t[a][2 * h + e] = tv;
-                    sE += tv;
                 }
             }
         }
@@ -1038,16 +1071,20 @@ __global__ void __launch_bounds__(256, 2) grad_partial_kernel(const double* __re
 
 void launch_grad_partial(const double* X, const double* r, int n, int d, int npad, const double* winv,
                          const double* Ainv, long long sAinv, const double* U, int nu, double* part,
-                         int B, cudaStream_t st, const double* E) {
+                         int B, cudaStream_t st, const double* E, int family) {
     int nt = npad / CT;
     size_t smem = ((size_t)(d + nu) * (CT + CT + 2) + 8 * (size_t)(d + 3)) * sizeof(double);
-    static SmemOptIn optin, optin_e;
-    if (E != nullptr) {         // (same layout and item stride as A^-1)
-        optin_e.ensure(grad_partial_kernel<true>, smem);
-        grad_partial_kernel<true><<<dim3(nt * (nt + 1) / 2, 1, B), 256, smem, st>>>(X, r, n, d, npad, winv, Ainv, sAinv, U, nu, part, E);
+    static SmemOptIn optin, optin_e, optin_m;
+    const dim3 grid(nt * (nt + 1) / 2, 1, B);
+    if (family == FAMILY_MATERN52) {      // always recomputed: the covariance build keeps no copy of R or G
+        optin_m.ensure(grad_partial_kernel<false, FAMILY_MATERN52>, smem);
+        grad_partial_kernel<false, FAMILY_MATERN52><<<grid, 256, smem, st>>>(X, r, n, d, npad, winv, Ainv, sAinv, U, nu, part, nullptr);
+    } else if (E != nullptr) {         // (same layout and item stride as A^-1)
+        optin_e.ensure(grad_partial_kernel<true, FAMILY_GAUSSIAN>, smem);
+        grad_partial_kernel<true, FAMILY_GAUSSIAN><<<grid, 256, smem, st>>>(X, r, n, d, npad, winv, Ainv, sAinv, U, nu, part, E);
     } else {
-        optin.ensure(grad_partial_kernel<false>, smem);
-        grad_partial_kernel<false><<<dim3(nt * (nt + 1) / 2, 1, B), 256, smem, st>>>(X, r, n, d, npad, winv, Ainv, sAinv, U, nu, part, nullptr);
+        optin.ensure(grad_partial_kernel<false, FAMILY_GAUSSIAN>, smem);
+        grad_partial_kernel<false, FAMILY_GAUSSIAN><<<grid, 256, smem, st>>>(X, r, n, d, npad, winv, Ainv, sAinv, U, nu, part, nullptr);
     }
 }
 

@@ -35,7 +35,8 @@ void launch_prep_theta(const double* theta, int B, int p, int d, int mode, doubl
 // the factorisation overwrites A, the fused gradient epilogue reads this copy instead of recomputing the exponentials.
 cudaError_t launch_cov_build(const double* X, const double* r, int n, int d, int npad, const ItemPar* par,
                              const double* winv, double* A, long long sA, int B, int full, cudaStream_t st,
-                             int gmode = 0, int gdim = 0, double* Eout = nullptr);
+                             int gmode = 0, int gdim = 0, double* Eout = nullptr, int family = FAMILY_GAUSSIAN);
+// (family FAMILY_MATERN52: the entries are R(D) -- G(D) Delta^2 for gmode 1 -- and Eout is ignored)
 
 // copy the n x n top-left of a padded matrix into a dense [n,n] output, mirroring the lower triangle
 void launch_unpad_sym(const double* A, int npad, int n, double* out, int mirror, cudaStream_t st);
@@ -60,10 +61,10 @@ void launch_llh_finalize(const double* Wy, const double* GP, const double* logde
                          int n, int q, int npad, int mode, ItemPar* par, ItemOut* out, double* beta,
                          double* Z, int* status, int B, const double* beta_override, double* Kout, cudaStream_t st);
 
-// K1g: per-tile partial sums of  W_ij E_ij Delta_k^2, W_ij E_ij, W_ii, W_ii r_i.
+// K1g: per-tile partial sums of  W_ij E_ij Delta_k^2, W_ij E_ij, W_ii, W_ii r_i  (Matérn: W_ij G_ij Delta_k^2, W_ij R_ij, ..).
 void launch_grad_partial(const double* X, const double* r, int n, int d, int npad, const double* winv,
                          const double* Ainv, long long sAinv, const double* U, int nu, double* part,
-                         int B, cudaStream_t st, const double* E = nullptr);
+                         int B, cudaStream_t st, const double* E = nullptr, int family = FAMILY_GAUSSIAN);
 void launch_grad_finalize(const double* part, int ntile, int n, int d, int npad, int p, int mode, const ItemPar* par,
                           const ItemOut* out, const int* status, double* llh, double* grad,
                           double* sigma_hat, int B, cudaStream_t st);

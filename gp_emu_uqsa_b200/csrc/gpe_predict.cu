@@ -65,8 +65,9 @@ __global__ void grid_points_kernel(GridDesc g, long long start, long long count,
     }
 }
 
-// K1x: C[k][j] = c * exp(-sum_dim ((x_k - p_j)/delta)^2) for a chunk of mc points.
+// K1x: C[k][j] = c * exp(-sum_dim ((x_k - p_j)/delta)^2) for a chunk of mc points (FAMILY_MATERN52: c * R(sum_dim ..)).
 // CTA = 64 training rows x 128 points, 256 threads, each thread 8 rows x 4 points.
+template <int FAM>
 __global__ void __launch_bounds__(256, 3) xcov_kernel(const double* __restrict__ Xs /*[d][npad]*/, const double* __restrict__ P /*[mc][d]*/,
                                                    const double* __restrict__ winv, int n, int d, int npad, int mc, long long count,
                                                    double cscale, double* __restrict__ Cm, int ldc) {
@@ -108,11 +109,16 @@ __global__ void __launch_bounds__(256, 3) xcov_kernel(const double* __restrict__
 #pragma unroll
     for (int a = 0; a < 8; a++)
 #pragma unroll
-        for (int c = 0; c < 4; c++) D[a][c] = gpe_exp(-D[a][c]);      // straight-line: the chains interleave
+        for (int c = 0; c < 4; c++)      // straight-line: the chains interleave
+            if constexpr (FAM == FAMILY_GAUSSIAN) D[a][c] = gpe_exp(-D[a][c]);
 #pragma unroll
     for (int a = 0; a < 8; a++) {
         int gk = k0 + ty + 8 * a;
         bool live = gk < n;
+        if constexpr (FAM == FAMILY_MATERN52) {      // one row's four chains at a time: 32 at once would spill
+#pragma unroll
+            for (int c = 0; c < 4; c++) D[a][c] = gpe_matern52(D[a][c]);
+        }
 #pragma unroll
         for (int hh = 0; hh < 2; hh++) {
             int gj = j0 + 64 * hh + 2 * tx;
@@ -138,6 +144,9 @@ __global__ void __launch_bounds__(256, 3) xcov_kernel(const double* __restrict__
 // the TRMM needs.)  Each factor carries its own rounding, so an entry differs from exp(-sum) in the last few ulps --
 // the same size as the rounding of the summed exponent in the direct form; parity with the reference is checked on the
 // grid path itself (tests/test_gpu_fullsize.py).
+// The Matérn kernel does not factorise, but its argument D is still a sum over the dimensions: for FAMILY_MATERN52 the
+// table holds the one-dimensional terms df^2, the slow and fast parts are added instead of multiplied, and R(D) is
+// applied once per entry.
 constexpr int GS_MAXNF = 7;      // fast dimensions (levels >= 2 => at most 7 for a product >= 128)
 struct GridSep {
     int d, ks, nf;               // slow dimensions [0, ks), fast dimensions [ks, d)
@@ -147,6 +156,7 @@ struct GridSep {
     int ptiles;                  // 128-point tiles per CTA (<= pfast / 128: at most two slow combinations per CTA)
 };
 
+template <int FAM>
 __global__ void grid_table_kernel(const double* __restrict__ Xs, const double* __restrict__ winv, GridDesc g, GridSep sp, int npad,
                                   int ltot, double* __restrict__ T) {
     const long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x;
@@ -157,16 +167,17 @@ __global__ void grid_table_kernel(const double* __restrict__ Xs, const double* _
     const int l = trow - sp.toff[k];
     const double pt = (g.lo[k] + ((double)l + 0.5) * g.step[k]) * winv[k];      // the coordinate grid_points_kernel gives, scaled
     const double df = Xs[(size_t)k * npad + i] - pt;
-    T[idx] = gpe_exp(-(df * df));
+    if constexpr (FAM == FAMILY_GAUSSIAN) T[idx] = gpe_exp(-(df * df));
+    else T[idx] = df * df;
 }
 
-template <int NF>
+template <int NF, int FAM>
 __global__ void __launch_bounds__(256) xcov_grid_kernel(const double* __restrict__ T, GridSep sp, int n, int npad, int mc,
                                                         long long start, long long count, double cscale,
                                                         double* __restrict__ Cm, int ldc) {
     constexpr int ROWS = 128;
     extern __shared__ __align__(16) double sm[];
-    double* Ps = sm;                    // [2][ROWS]  cscale * product of the slow factors, per slow combination
+    double* Ps = sm;                    // [2][ROWS]  cscale * product of the slow factors (Matérn: sum of the slow terms)
     double* Tf = sm + 2 * ROWS;         // fast factors: block kf holds [ROWS][levels + 1]
     __shared__ int sdig[2][MAXD];
     const int tid = threadIdx.x, k0 = blockIdx.y * ROWS;
@@ -182,8 +193,12 @@ __global__ void __launch_bounds__(256) xcov_grid_kernel(const double* __restrict
     __syncthreads();
     {
         const int c = tid >> 7, row = tid & (ROWS - 1);
-        double prod = cscale;
-        for (int k = 0; k < sp.ks; k++) prod *= T[(size_t)(sp.toff[k] + sdig[c][k]) * npad + k0 + row];
+        double prod = (FAM == FAMILY_GAUSSIAN) ? cscale : 0.0;
+        for (int k = 0; k < sp.ks; k++) {
+            const double tv = T[(size_t)(sp.toff[k] + sdig[c][k]) * npad + k0 + row];
+            if constexpr (FAM == FAMILY_GAUSSIAN) prod *= tv;
+            else prod += tv;
+        }
         Ps[c * ROWS + row] = prod;
     }
 #pragma unroll
@@ -225,7 +240,12 @@ __global__ void __launch_bounds__(256) xcov_grid_kernel(const double* __restrict
             for (int q4 = 0; q4 < 4; q4++) {
                 double x = Ps[combo[q4] * ROWS + row];
 #pragma unroll
-                for (int kf = 0; kf < NF; kf++) x *= Tf[off[q4][kf] + row * (sp.levels[sp.ks + kf] + 1)];
+                for (int kf = 0; kf < NF; kf++) {
+                    const double tv = Tf[off[q4][kf] + row * (sp.levels[sp.ks + kf] + 1)];
+                    if constexpr (FAM == FAMILY_GAUSSIAN) x *= tv;
+                    else x += tv;
+                }
+                if constexpr (FAM == FAMILY_MATERN52) x = cscale * gpe_matern52(x);
                 v[q4] = (live && livep[q4]) ? x : 0.0;
             }
             double* cp = Cm + (size_t)(k0 + row) * ldc + j0 + 2 * tx;
@@ -261,26 +281,27 @@ static bool plan_grid_sep(const GridDesc& g, GridSep& sp, size_t& smem, int& lto
     return smem <= 96 * 1024 && ltot <= 4096;
 }
 
-template <int NF>
+template <int NF, int FAM>
 static cudaError_t launch_xcov_grid_nf(const double* T, const GridSep& sp, int n, int npad, int mc, long long start, long long count,
                                        double cscale, double* Cm, size_t smem, cudaStream_t st) {
     static SmemOptIn optin;
-    if (cudaError_t e = optin.ensure(xcov_grid_kernel<NF>, smem); e != cudaSuccess) return e;
+    if (cudaError_t e = optin.ensure(xcov_grid_kernel<NF, FAM>, smem); e != cudaSuccess) return e;
     const int per = sp.ptiles * 128;
-    xcov_grid_kernel<NF><<<dim3((mc + per - 1) / per, npad / 128), 256, smem, st>>>(T, sp, n, npad, mc, start, count, cscale, Cm, mc);
+    xcov_grid_kernel<NF, FAM><<<dim3((mc + per - 1) / per, npad / 128), 256, smem, st>>>(T, sp, n, npad, mc, start, count, cscale, Cm, mc);
     return cudaGetLastError();
 }
 
+template <int FAM>
 static cudaError_t launch_xcov_grid(const double* T, const GridSep& sp, int n, int npad, int mc, long long start, long long count,
                                     double cscale, double* Cm, size_t smem, cudaStream_t st) {
     switch (sp.nf) {
-        case 1: return launch_xcov_grid_nf<1>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
-        case 2: return launch_xcov_grid_nf<2>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
-        case 3: return launch_xcov_grid_nf<3>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
-        case 4: return launch_xcov_grid_nf<4>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
-        case 5: return launch_xcov_grid_nf<5>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
-        case 6: return launch_xcov_grid_nf<6>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
-        case 7: return launch_xcov_grid_nf<7>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
+        case 1: return launch_xcov_grid_nf<1, FAM>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
+        case 2: return launch_xcov_grid_nf<2, FAM>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
+        case 3: return launch_xcov_grid_nf<3, FAM>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
+        case 4: return launch_xcov_grid_nf<4, FAM>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
+        case 5: return launch_xcov_grid_nf<5, FAM>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
+        case 6: return launch_xcov_grid_nf<6, FAM>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
+        case 7: return launch_xcov_grid_nf<7, FAM>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
         default: return cudaErrorInvalidValue;
     }
 }
@@ -292,10 +313,26 @@ struct GridXcov {        // what predict_chunk needs to build a chunk's cross-co
     long long start;     // flat index of the chunk's first point
 };
 
-// d >= 32 needs more than 48 KB for the two k-major tiles
-static SmemOptIn& xcov_optin() {
-    static SmemOptIn o;
-    return o;
+static cudaError_t launch_xcov_grid(int family, const double* T, const GridSep& sp, int n, int npad, int mc, long long start,
+                                    long long count, double cscale, double* Cm, size_t smem, cudaStream_t st) {
+    if (family == FAMILY_MATERN52) return launch_xcov_grid<FAMILY_MATERN52>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
+    return launch_xcov_grid<FAMILY_GAUSSIAN>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
+}
+
+// C [n rows of npad, ldc] = cscale * K(training, P) for the mc points P [mc, d] (columns >= count zero)
+template <int FAM>
+static cudaError_t launch_xcov_fam(const double* Xs, const double* P, const double* winv, int n, int d, int npad, int mc,
+                                   long long count, double cscale, double* Cm, int ldc, cudaStream_t st) {
+    static SmemOptIn optin;      // d >= 32 needs more than 48 KB for the two k-major tiles
+    const size_t smem = (size_t)d * (64 + 130) * sizeof(double);
+    if (cudaError_t e = optin.ensure(xcov_kernel<FAM>, smem); e != cudaSuccess) return e;
+    xcov_kernel<FAM><<<dim3(mc / 128, npad / 64), 256, smem, st>>>(Xs, P, winv, n, d, npad, mc, count, cscale, Cm, ldc);
+    return cudaGetLastError();
+}
+static cudaError_t launch_xcov(int family, const double* Xs, const double* P, const double* winv, int n, int d, int npad, int mc,
+                               long long count, double cscale, double* Cm, int ldc, cudaStream_t st) {
+    if (family == FAMILY_MATERN52) return launch_xcov_fam<FAMILY_MATERN52>(Xs, P, winv, n, d, npad, mc, count, cscale, Cm, ldc, st);
+    return launch_xcov_fam<FAMILY_GAUSSIAN>(Xs, P, winv, n, d, npad, mc, count, cscale, Cm, ldc, st);
 }
 
 // Implausibility folded into the prediction of one emulator (history_match.py:96-132): instead of mean / variance the
@@ -509,6 +546,7 @@ __global__ void __launch_bounds__(256) implaus_kernel(const double* __restrict__
 }
 
 // full posterior covariance assembly: V = sigma^2 (A* - Z^T Z + G^T G)
+template <int FAM>
 __global__ void fullcov_finalize_kernel(const double* __restrict__ ZtZ, int mp, const double* __restrict__ aux, int ld,
                                         const double* __restrict__ P, const double* __restrict__ Hs, BasisDesc bd, int d,
                                         const double* __restrict__ winv, const double* __restrict__ Kf, double sigma2,
@@ -542,7 +580,8 @@ __global__ void fullcov_finalize_kernel(const double* __restrict__ ZtZ, int mp, 
         double df = P[(size_t)i * d + k] * winv[k] - P[(size_t)j * d + k] * winv[k];
         D = fma(df, df, D);
     }
-    double prior = (i == j) ? (astar + (r_new ? r_new[i] : 0.0)) : cscale * gpe_exp(-D);
+    double prior = (i == j) ? (astar + (r_new ? r_new[i] : 0.0))
+                            : cscale * (FAM == FAMILY_MATERN52 ? gpe_matern52(D) : gpe_exp(-D));
     double gg = 0.0;
     for (int a = 0; a < q; a++) gg = fma(Gbuf[(size_t)a * mp + i], Gbuf[(size_t)a * mp + j], gg);
     V[idx] = sigma2 * (prior - ZtZ[(size_t)i * mp + j] + gg);
@@ -585,15 +624,10 @@ long long default_chunk(gpe_handle* h) {
 int predict_chunk(gpe_handle* h, gpe_handle::PredSlot& sl, cudaStream_t st, const double* P_dev, const double* Hs_dev,
                   long long count, int mc, double* mean_dev, double* var_dev, const GridXcov* gx = nullptr, const ImpFuse* imp = nullptr) {
     const int np = h->npad;
-    size_t smem = (size_t)h->d * (64 + 130) * sizeof(double);
     {
         ProfScope ps(h, gpe_handle::CAT_COV, st);
-        if (gx != nullptr) {
-            CK(launch_xcov_grid(gx->T, gx->sp, h->n, np, mc, gx->start, count, h->fit_c, sl.C, gx->smem, st));
-        } else {
-            CK(xcov_optin().ensure(xcov_kernel, smem));
-            xcov_kernel<<<dim3(mc / 128, np / 64), 256, smem, st>>>(h->fXs, P_dev, h->fwinv, h->n, h->d, np, mc, count, h->fit_c, sl.C, mc);
-        }
+        if (gx != nullptr) CK(launch_xcov_grid(h->family, gx->T, gx->sp, h->n, np, mc, gx->start, count, h->fit_c, sl.C, gx->smem, st));
+        else CK(launch_xcov(h->family, h->fXs, P_dev, h->fwinv, h->n, h->d, np, mc, count, h->fit_c, sl.C, mc, st));
     }
     h->launches++;
     int rc;
@@ -624,7 +658,7 @@ int predict_chunk(gpe_handle* h, gpe_handle::PredSlot& sl, cudaStream_t st, cons
                 mp = np;
                 h->oz_reuse_a = true;
                 h->oz_a_tag = h->fit_gen;
-                // every entry of the slab is c exp(-D) in [0, c]: one scale for all points, no pass over the slab for its maxima.
+                // every entry of the slab is c exp(-D) or c R(D), in [0, c]: one scale for all points, no pass over the slab for its maxima.
                 // (A point far from every training input then keeps fewer significant bits of its tiny column -- its variance
                 // is the prior's to the same absolute accuracy, which is what the subtraction prior - |Z|^2 needs.)
                 static const int fixed_env = [] { const char* e = getenv("GPE_PRED_FIXED_SCALE"); return e ? atoi(e) : 1; }();
@@ -679,7 +713,7 @@ int gpe_fit_state(gpe_handle* h, const double* delta, double nugget, double sigm
         CK(cudaMemcpyAsync(h->fbeta, bin.data(), sizeof(double) * NR, cudaMemcpyHostToDevice, h->st));
         bov = h->fbeta;
     }
-    CK(launch_cov_build(h->X, h->r, h->n, h->d, np, h->par, h->winv, h->A, 0, 1, 0, h->st));
+    CK(launch_cov_build(h->X, h->r, h->n, h->d, np, h->par, h->winv, h->A, 0, 1, 0, h->st, 0, 0, nullptr, h->family));
     h->launches++;
     CK(cudaMemsetAsync(h->fK, 0, sizeof(double) * NR * NR, h->st));
     CK(cudaMemsetAsync(h->status, 0, sizeof(int), h->st));
@@ -741,7 +775,10 @@ static int predict_common(gpe_handle* h, const double* Xs, const double* Hs, con
             double* T = nullptr;
             CK(t_tab.get(&T, (size_t)ltot * h->npad));
             const long long tot = (long long)ltot * h->npad;
-            grid_table_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, h->st>>>(h->fXs, h->fwinv, *grid, gx.sp, h->npad, ltot, T);
+            if (h->family == FAMILY_MATERN52)
+                grid_table_kernel<FAMILY_MATERN52><<<(unsigned)((tot + 255) / 256), 256, 0, h->st>>>(h->fXs, h->fwinv, *grid, gx.sp, h->npad, ltot, T);
+            else
+                grid_table_kernel<FAMILY_GAUSSIAN><<<(unsigned)((tot + 255) / 256), 256, 0, h->st>>>(h->fXs, h->fwinv, *grid, gx.sp, h->npad, ltot, T);
             h->launches++;
             gx.T = T;
             use_sep = true;
@@ -913,9 +950,7 @@ int gpe_cross_cov(gpe_handle* h, const double* delta, double nugget, int kind, c
     CK(cudaMemsetAsync(P, 0, sizeof(double) * (size_t)mc * d, h->st));
     CK(cudaMemcpyAsync(P, Xs, sizeof(double) * (size_t)m * d, cudaMemcpyDefault, h->st));
     scale_train_kernel<<<(d * np + 255) / 256, 256, 0, h->st>>>(h->X, wd, h->n, d, np, xs);
-    size_t smem = (size_t)d * (64 + 130) * sizeof(double);
-    xcov_optin().ensure(xcov_kernel, smem);
-    xcov_kernel<<<dim3(mc / 128, np / 64), 256, smem, h->st>>>(xs, P, wd, h->n, d, np, mc, m, kind ? 1.0 : 1.0 - nugget, Cm, mc);
+    CK(launch_xcov(h->family, xs, P, wd, h->n, d, np, mc, m, kind ? 1.0 : 1.0 - nugget, Cm, mc, h->st));
     h->launches += 2;
     bool dev = gpe_is_device_ptr(C_out);
     CK(cudaMemcpy2DAsync(C_out, sizeof(double) * m, Cm, sizeof(double) * mc, sizeof(double) * m, h->n,
@@ -956,9 +991,7 @@ int gpe_predict_fullcov(gpe_handle* h, const double* Xs, const double* Hs, int m
         CK(t_rn.get(&rn, (size_t)m));
         CK(cudaMemcpyAsync(rn, r_new, sizeof(double) * m, cudaMemcpyDefault, h->st));
     }
-    size_t smem = (size_t)d * (64 + 130) * sizeof(double);
-    xcov_optin().ensure(xcov_kernel, smem);
-    xcov_kernel<<<dim3(mp / 128, np / 64), 256, smem, h->st>>>(h->fXs, P, h->fwinv, h->n, d, np, mp, m, h->fit_c, Cm, mp);
+    CK(launch_xcov(h->family, h->fXs, P, h->fwinv, h->n, d, np, mp, m, h->fit_c, Cm, mp, h->st));
     h->launches++;
     int rc = 0;
     if (!rc) rc = gpe_run_gemm(h, h->fE, Cm, aux, NR, mp, mp, 0, 0, 0, NR, mp, np, 1.0, 0, KM_FULL, 0, 1, 2, EPI_STORE);
@@ -970,11 +1003,11 @@ int gpe_predict_fullcov(gpe_handle* h, const double* Xs, const double* Hs, int m
         // mean via the diagonal finalize (var == nullptr)
         predict_finalize_kernel<false><<<(m + 127) / 128, 128, 0, h->st>>>(nullptr, 0, aux, mp, P, Hd, bd, d, h->fK, h->fbeta, s2,
                                                                             h->fit_astar, m, md, nullptr, ImpFuse{});
-        fullcov_finalize_kernel<<<(m + 127) / 128, 128, 0, h->st>>>(ZtZ, mp, aux, mp, P, Hd, bd, d, h->fwinv, h->fK, s2, h->fit_c,
-                                                                     h->fit_astar, rn, m, G, Vd, 0);
+        auto fin = h->family == FAMILY_MATERN52 ? fullcov_finalize_kernel<FAMILY_MATERN52> : fullcov_finalize_kernel<FAMILY_GAUSSIAN>;
+        fin<<<(m + 127) / 128, 128, 0, h->st>>>(ZtZ, mp, aux, mp, P, Hd, bd, d, h->fwinv, h->fK, s2, h->fit_c, h->fit_astar, rn, m, G, Vd, 0);
         size_t tot = (size_t)m * m;
-        fullcov_finalize_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, h->st>>>(ZtZ, mp, aux, mp, P, Hd, bd, d, h->fwinv, h->fK, s2,
-                                                                                   h->fit_c, h->fit_astar, rn, m, G, Vd, 1);
+        fin<<<(unsigned)((tot + 255) / 256), 256, 0, h->st>>>(ZtZ, mp, aux, mp, P, Hd, bd, d, h->fwinv, h->fK, s2, h->fit_c, h->fit_astar,
+                                                            rn, m, G, Vd, 1);
         h->launches += 3;
         CK(cudaMemcpyAsync(mean, md, sizeof(double) * m, cudaMemcpyDefault, h->st));
         CK(cudaMemcpyAsync(V, Vd, sizeof(double) * (size_t)m * m, cudaMemcpyDefault, h->st));

@@ -273,6 +273,7 @@ int gpe_solve(gpe_handle* h, const double* Bm, int k, double* out) {
 int gpe_sens_contract(gpe_handle* h, const double* gamma, const double* acoef, const double* mvec, double scale,
                       const double* V, int nv, double* trace_out, double* M_out) {
     if (!h || !gamma || !acoef || !mvec || !V || nv < 1 || nv > NR) return h ? h->fail_msg("bad argument (nv <= 32)") : -2;
+    if (h->family != FAMILY_GAUSSIAN) return h->fail_msg("sensitivity integrals need the Gaussian kernel");
     if (!h->fitted) return h->fail_msg("gpe_fit_state has not succeeded on this handle");
     NvtxRange nvtx("gpe_sens_contract");
     CK(cudaSetDevice(h->device));
@@ -328,6 +329,7 @@ int gpe_sens_main_effect(gpe_handle* h, const double* t1, const double* t2, cons
                          double* out) {
     if (!h || !h->n || !t1 || !t2 || !cdiag || !mvec || !evec || !which || !xw || !out || nwhich < 1 || points < 1)
         return h ? h->fail_msg("bad argument / no training set") : -2;
+    if (h->family != FAMILY_GAUSSIAN) return h->fail_msg("sensitivity integrals need the Gaussian kernel");
     NvtxRange nvtx("gpe_sens_main_effect");
     CK(cudaSetDevice(h->device));
     const int n = h->n, d = h->d;

@@ -22,11 +22,14 @@ def setup(config_file, datashuffle=True, scaleinputs=True):
     basis = _emuc.Basis(beliefs)
     tv_conf = _emuc.TV_config(*(config.tv_config))
     all_data = _emuc.All_Data(config.inputs, config.outputs, tv_conf, beliefs, par, datashuffle, scaleinputs)
+    if beliefs.kernel == "matern52":
+        print("\n*** Using Matern 5/2 kernel ***")
     if beliefs.alt_nugget != 'T':
-        K = _emuk.kernel(all_data.x_full[0].size, par)
+        cls = _emuk.kernel_matern52 if beliefs.kernel == "matern52" else _emuk.kernel
     else:
         print("\n*** Using alternative nugget ***")
-        K = _emuk.kernel_alt_nug(all_data.x_full[0].size, par)
+        cls = _emuk.kernel_matern52_alt_nug if beliefs.kernel == "matern52" else _emuk.kernel_alt_nug
+    K = cls(all_data.x_full[0].size, par)
     (x_T, y_T) = all_data.choose_T()
     (x_V, y_V) = all_data.choose_V()
     training = _emuc.Data(x_T, y_T, basis, par, beliefs, K)

@@ -28,6 +28,10 @@ def setup(emul, m, v, case="case2"):
     else:
         print("Only case2 of MUCM's U & S analysis is implemented. Return None.")
         return None
+    if emul.K.family != 0:
+        print("The sensitivity integrals need the Gaussian kernel; this emulator uses "
+              "the Matern 5/2 kernel. Return None.")
+        return None
     return Sensitivity(emul, _np.array(m), _np.array(v))
 
 

@@ -18,7 +18,10 @@
  *    no-op that touches no output, so an empty rank of a partitioned job needs no special case;
  *  - one handle per device per process; a handle is not thread-safe; calls are synchronous
  *    with respect to the returned host-visible results;
- *  - there is NO CPU fallback: every entry point fails if no sm_100 device is present.
+ *  - there is NO CPU fallback: every entry point fails if no sm_100 device is present;
+ *  - the covariance function is the reference's Gaussian exp(-sum((x_i-x_j)/delta)^2) unless
+ *    gpe_set_kernel selects the Matern 5/2 family for the handle (everything else -- nugget forms,
+ *    mode bits, likelihoods, posterior formulas -- is shared by both families).
  */
 #ifndef GPE_B200_H
 #define GPE_B200_H
@@ -33,6 +36,13 @@ typedef struct gpe_handle gpe_handle;
 #define GPE_MODE_MUCM 1        /* beliefs.mucm == 'T'      (loglikelihood_mucm)              */
 #define GPE_MODE_ALT_NUGGET 2  /* beliefs.alt_nugget == 'T' (kernel_alt_nug)                  */
 #define GPE_MODE_NUGGET_FREE 4 /* beliefs.fix_nugget == 'F' (nugget is an optimised parameter) */
+
+/* covariance families for gpe_set_kernel.  With D_ij = sum_k ((x_ik - x_jk) / delta_k)^2 and r = sqrt(D):
+ * GAUSSIAN  exp(-D) (the reference's kernel / kernel_alt_nug);
+ * MATERN52  (1 + sqrt5 r + 5D/3) exp(-sqrt5 r), Matérn with smoothness 5/2 in the same scaled distance.
+ * The nugget / alt-nugget forms (argument `kind` below) and the diagonals are the same for both. */
+#define GPE_KERNEL_GAUSSIAN 0
+#define GPE_KERNEL_MATERN52 1
 
 int gpe_version(void);
 int gpe_create(int device, gpe_handle** out);
@@ -54,6 +64,12 @@ int gpe_set_streams(gpe_handle* h, int nstreams);
  * calls with a host pointer stay synchronous.  gpe_synchronize waits for the handle's stream.  This is what lets one
  * host thread keep several handles busy (the emulators of a history-matching job, history_match.py:96-118) or order
  * its own kernels after a call with events on gpe_get_stream. */
+/* Covariance family of the emulator this handle holds (GPE_KERNEL_*; Gaussian by default).  It applies to
+ * gpe_cov_build, gpe_cov_grad, gpe_cross_cov, gpe_llh_grad_batch, gpe_fit_state, gpe_predict* and gpe_predict_implaus.
+ * A change clears the fit state (gpe_fit_state must run again) and the captured likelihood graphs.  With MATERN52,
+ * gpe_sens_contract and gpe_sens_main_effect fail: their closed-form integrals exist for the Gaussian only. */
+int gpe_set_kernel(gpe_handle* h, int family);
+
 int gpe_set_async(gpe_handle* h, int on);
 int gpe_synchronize(gpe_handle* h);
 
