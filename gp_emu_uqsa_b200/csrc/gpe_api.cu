@@ -226,10 +226,8 @@ int gpe_run_gemm(gpe_handle* h, const double* A, const double* B, double* C, int
 // 128x128 diagonal leaves are factored by a panel kernel.  2n^3/3 flops, 5 launches per node.
 int gpe_handle::ensure_side(int g) {
     if (side_st[g][0]) return 0;
-    int prio_least = 0, prio_greatest = 0;
-    cudaDeviceGetStreamPriorityRange(&prio_least, &prio_greatest);
     for (int k = 0; k < MAX_DEPTH; k++) {
-        if (cudaStreamCreateWithPriority(&side_st[g][k], cudaStreamNonBlocking, prio_least) != cudaSuccess) return -1;
+        if (cudaStreamCreateWithFlags(&side_st[g][k], cudaStreamNonBlocking) != cudaSuccess) return -1;
         cudaEventCreateWithFlags(&ev_sf[g][k], cudaEventDisableTiming);
         cudaEventCreateWithFlags(&ev_sj[g][k], cudaEventDisableTiming);
     }
@@ -244,9 +242,8 @@ static int potrf_inv_rec(gpe_handle* h, const FactorWs& ws, const SubBatch& sb, 
     double* Lb = ws.Li + (size_t)sb.b0 * sM;
     if (m == NB) {
         {
-            cudaStream_t st = sb.stream(true);
-            ProfScope ps(h, gpe_handle::CAT_LEAF, st);
-            launch_leaf(Ab, Lb, ld, sM, sM, off, ws.logdet_part + (size_t)sb.b0 * ws.nleaf, ws.nleaf, ws.status + sb.b0, B, st,
+            ProfScope ps(h, gpe_handle::CAT_LEAF, sb.st);
+            launch_leaf(Ab, Lb, ld, sM, sM, off, ws.logdet_part + (size_t)sb.b0 * ws.nleaf, ws.nleaf, ws.status + sb.b0, B, sb.st,
                         want_L ? Sb : nullptr);
         }
         h->launches++;
@@ -263,7 +260,7 @@ static int potrf_inv_rec(gpe_handle* h, const FactorWs& ws, const SubBatch& sb, 
     double* Li22 = Lb + (size_t)(off + m1) * ld + off + m1;
     double* Li21 = Lb + (size_t)(off + m1) * ld + off;
     // L21 = A21 * Linv11^T           (NT, Linv11 lower: k <= j)
-    if ((rc = run_gemm(h, sb.stream(!gemm_is_big(m2, m1, 0, B)), A21, Li11, S21, ld, ld, ld, sM, sM, sM, m2, m1, m1, 1.0, 0, KM_LE_J, 0, B, 0))) return rc;
+    if ((rc = run_gemm(h, sb.st, A21, Li11, S21, ld, ld, ld, sM, sM, sM, m2, m1, m1, 1.0, 0, KM_LE_J, 0, B, 0))) return rc;
     // T = L21 * Linv11  (NN, Linv11 lower: k >= j) -> dead A21 block.  It needs only L21 and Linv11, not the
     // factorisation of A22: with side streams it is launched now, beside the SYRK and the whole A22 sub-recursion
     // (whose leaves and small levels cannot fill the machine), and joined before the last product of the node.
@@ -273,58 +270,49 @@ static int potrf_inv_rec(gpe_handle* h, const FactorWs& ws, const SubBatch& sb, 
     const bool fork = !oz_node && sb.side != nullptr && depth < gpe_handle::MAX_DEPTH;
     if (fork) {
         cudaStream_t side = sb.side[depth];
-        cudaEventRecord(sb.ef[depth], sb.current());
+        cudaEventRecord(sb.ef[depth], sb.st);
         cudaStreamWaitEvent(side, sb.ef[depth], 0);
         if ((rc = run_gemm(h, side, S21, Li11, A21, ld, ld, ld, sM, sM, sM, m2, m1, m1, 1.0, 0, KM_GE_J, 0, B, 1))) return rc;
         cudaEventRecord(sb.ej[depth], side);
     }
     // A22 -= L21 * L21^T             (SYRK, lower tiles)
-    if ((rc = run_gemm(h, sb.stream(!gemm_is_big(m2, m2, 1, B)), S21, S21, A22, ld, ld, ld, sM, sM, sM, m2, m2, m1, -1.0, 1, KM_FULL, 1, B, 0))) return rc;
+    if ((rc = run_gemm(h, sb.st, S21, S21, A22, ld, ld, ld, sM, sM, sM, m2, m2, m1, -1.0, 1, KM_FULL, 1, B, 0))) return rc;
     if (oz_node) {
         h->oz_reuse_a = true;
-        if ((rc = run_gemm(h, sb.current(), S21, Li11, A21, ld, ld, ld, sM, sM, sM, m2, m1, m1, 1.0, 0, KM_GE_J, 0, B, 1))) return rc;
+        if ((rc = run_gemm(h, sb.st, S21, Li11, A21, ld, ld, ld, sM, sM, sM, m2, m1, m1, 1.0, 0, KM_GE_J, 0, B, 1))) return rc;
     }
     if ((rc = potrf_inv_rec(h, ws, sb, off + m1, m2, want_L, depth + 1))) return rc;
     if (fork) {
-        cudaStreamWaitEvent(sb.current(), sb.ej[depth], 0);
+        cudaStreamWaitEvent(sb.st, sb.ej[depth], 0);
     } else if (!oz_node) {
-        if ((rc = run_gemm(h, sb.stream(!gemm_is_big(m2, m1, 0, B)), S21, Li11, A21, ld, ld, ld, sM, sM, sM, m2, m1, m1, 1.0, 0, KM_GE_J, 0, B, 1))) return rc;
+        if ((rc = run_gemm(h, sb.st, S21, Li11, A21, ld, ld, ld, sM, sM, sM, m2, m1, m1, 1.0, 0, KM_GE_J, 0, B, 1))) return rc;
     }
     // Linv21 = -Linv22 * T           (NN, Linv22 lower: k <= i)
-    if ((rc = run_gemm(h, sb.stream(!gemm_is_big(m2, m1, 0, B)), Li22, A21, Li21, ld, ld, ld, sM, sM, sM, m2, m1, m2, -1.0, 0, KM_LE_I, 0, B, 1))) return rc;
+    if ((rc = run_gemm(h, sb.st, Li22, A21, Li21, ld, ld, ld, sM, sM, sM, m2, m1, m2, -1.0, 0, KM_LE_I, 0, B, 1))) return rc;
     return 0;
 }
 int gpe_potrf_inv(gpe_handle* h, const FactorWs& ws, const SubBatch& sb, int want_L) { return potrf_inv_rec(h, ws, sb, 0, ws.npad, want_L); }
 
 static FactorWs handle_ws(gpe_handle* h) { return FactorWs{h->A, h->S, h->Li, h->npad, h->nleaf, h->logdet_part, h->status}; }
 
-// How the gradient reduction of a chunk is done (GPE_FUSED_GRAD = 0 | 1 | 2; all routes sum the same terms, results agree
-// to rounding).
-//   0: A^-1 by the generic LAUUM GEMM, stored, then the stand-alone reduction kernel that recomputes E and U.U^T
-//      (round 1; still used for launches too small for 128x128 tiles).
-//   1: LAUUM with the columns of U in its k loop stores W = A^-1 - U U^T; a light kernel reduces W against the
-//      covariance build's copy of E.
-//   2 (default when 128x128 tiles fill the machine): the reduction in LAUUM's epilogue (gpe_lauum_grad.cu); nothing
+// How the gradient reduction of a chunk is done (both routes sum the same terms, results agree to rounding).
+//   classic (false): A^-1 by the generic LAUUM GEMM, stored, then the stand-alone reduction kernel that recomputes E and
+//      U.U^T (round 1; still used for launches too small for 128x128 tiles, inputs too wide for the fused epilogue's shared
+//      memory, the Matérn family and the INT8 route).
+//   fused (true, when 128x128 tiles fill the machine): the reduction in LAUUM's epilogue (gpe_lauum_grad.cu); nothing
 //      of size n x n is written after the factorisation.
-// Measured on one B200 in one call, n = 4096, d = 16, 32 items, 8 streams, graph replay: 75.41 / 75.79 / 75.38 ms per step
-// for routes 0 / 1 / 2, 73.9 ms with the reduction switched off altogether.  The reduction is scalar FP64 work on the pipe
-// the DMMAs use: fusing moves it, it does not remove it (DESIGN.md section 8).
-static int llh_grad_fused(gpe_handle* h, int B) {
-    static int mode = -1;
-    if (mode < 0) {
-        const char* e = getenv("GPE_FUSED_GRAD");
-        mode = e ? atoi(e) : 2;
-    }
+// Measured on one B200 in one call, n = 4096, d = 16, 32 items, 8 streams, graph replay: 75.41 / 75.38 ms per step
+// for the classic / fused route, 73.9 ms with the reduction switched off altogether.  The reduction is scalar FP64 work on
+// the pipe the DMMAs use: fusing moves it, it does not remove it (DESIGN.md section 8).
+static bool llh_grad_fused(gpe_handle* h, int B) {
     h->grad_use_e = false;
     // Matérn: the stand-alone reduction recomputes R and G (the LAUUM epilogue and the E copy are Gaussian-only)
-    if (h->family != FAMILY_GAUSSIAN || !gemm_is_big(h->npad, h->npad, 1, B)) return 0;
+    if (h->family != FAMILY_GAUSSIAN || !gemm_is_big(h->npad, h->npad, 1, B)) return false;
     if (h->oz_nmod > 0 && h->npad >= h->oz_min && h->npad % OZ_BN == 0) {   // LAUUM on the INT8 route, A^-1 stored: the stand-alone
-        static const int use_e = [] { const char* e = getenv("GPE_GRAD_E"); return e ? atoi(e) : 1; }();   // reduction reads the
-        h->grad_use_e = use_e != 0;                                          // covariance build's copy of exp(-D)
-        return 0;
+        h->grad_use_e = true;                                                // reduction reads the covariance build's copy of exp(-D)
+        return false;
     }
-    if (mode == 2 && !lauum_grad_supported(h->d)) return 1;
-    return mode;
+    return lauum_grad_supported(h->d);
 }
 
 // Everything after the covariance build for the items of `sb`, already described by h->par / h->winv.
@@ -332,7 +320,7 @@ static int llh_grad_fused(gpe_handle* h, int B) {
 int gpe_factor_and_reduce(gpe_handle* h, const SubBatch& sb, int mode, int with_grad, const double* beta_override, double* Kout) {
     const int np = h->npad, ld = np, B = sb.B, b0 = sb.b0;
     const long long sM = (long long)np * np, sP = (long long)np * NR;
-    cudaStream_t st;
+    const cudaStream_t st = sb.st;
     const int nslab = (np + GRAM_SLAB - 1) / GRAM_SLAB;
     double* Ab = h->A + (size_t)b0 * sM;
     double* Lb = h->Li + (size_t)b0 * sM;
@@ -341,7 +329,6 @@ int gpe_factor_and_reduce(gpe_handle* h, const SubBatch& sb, int mode, int with_
     int rc;
     if ((rc = potrf_inv_rec(h, handle_ws(h), sb, 0, np, 0))) return rc;
     // Wy = Linv [H | y]
-    st = sb.stream(true);
     if ((rc = run_gemm(h, st, Lb, h->HY, Wy, ld, NR, NR, sM, 0, sP, np, NR, np, 1.0, 0, KM_LE_I, 0, B, 1))) return rc;
     {
         ProfScope ps(h, gpe_handle::CAT_OTHER, st);
@@ -353,8 +340,7 @@ int gpe_factor_and_reduce(gpe_handle* h, const SubBatch& sb, int mode, int with_
     // U = Linv^T Z = [A^-1 H K^-T | sqrt(f) A^-1 (y - H beta)]
     if ((rc = run_gemm(h, st, Lb, Z, U, ld, NR, NR, sM, sP, sP, np, NR, np, 1.0, 0, KM_GE_I, 0, B, 2))) return rc;
     if (!with_grad) return 0;
-    st = sb.stream(false);
-    if (h->grad_fused == 2) {
+    if (h->grad_fused) {
         // LAUUM with the gradient reduction in its epilogue: W = A^-1 - U U^T never leaves the CTA that computed it
         // (gpe_lauum_grad.cu).  Wy and Z are dead by now and hold U^T and -U^T.
         ProfScope ps(h, gpe_handle::CAT_LAUUM, st);
@@ -363,23 +349,6 @@ int gpe_factor_and_reduce(gpe_handle* h, const SubBatch& sb, int mode, int with_
                                           h->gpart + (size_t)b0 * lauum_grad_ntiles(np) * grad_nvals(h->d), B, st);
         h->launches += 2;
         if (e != cudaSuccess) return h->fail("launch_lauum_grad", e);
-        return 0;
-    }
-    if (h->grad_fused == 1) {
-        // split route (default for machine-filling launches): the same LAUUM launch stores W = A^-1 - U U^T (the columns of
-        // U ride along in its k loop) into the dead A buffer; a light reduction kernel combines it with the E copy
-        {
-            ProfScope ps(h, gpe_handle::CAT_LAUUM, st);
-            cudaError_t e = launch_lauum_grad(Lb, sM, np, h->n, h->d, h->q + 1, U, Wy, Z, h->X, h->r, h->winv + (size_t)b0 * h->d,
-                                              nullptr, 0, nullptr, B, st, Ab);
-            h->launches += 2;
-            if (e != cudaSuccess) return h->fail("launch_lauum_grad (store W)", e);
-        }
-        ProfScope ps(h, gpe_handle::CAT_GRAD, st);
-        cudaError_t e = launch_grad_partial_we(h->X, h->r, h->n, h->d, np, h->winv + (size_t)b0 * h->d, Ab, h->Ex + (size_t)b0 * sM, sM,
-                                               h->gpart + (size_t)b0 * grad_ntiles(np) * grad_nvals(h->d), B, st);
-        h->launches++;
-        if (e != cudaSuccess) return h->fail("launch_grad_partial_we", e);
         return 0;
     }
     // small launches (64x64 tiles) and very wide inputs: A^-1 = Linv^T Linv (lower tiles) into the dead A buffer, then
@@ -435,19 +404,9 @@ int gpe_create(int device, gpe_handle** out) {
     h->device = device;
     h->sms = prop.multiProcessorCount;
     if (cudaStreamCreateWithFlags(&h->st, cudaStreamNonBlocking) != cudaSuccess) { delete h; return -3; }
-    int prio_least = 0, prio_greatest = 0;
-    cudaDeviceGetStreamPriorityRange(&prio_least, &prio_greatest);
-    if (const char* e = getenv("GPE_PRIO")) h->use_prio = e[0] != '0';
-    // GPE_SUB_ASYM=1 (experiment): the even sub-batch streams get the highest priority, so that one group runs at full speed and
-    // the other fills the gaps its tensor-bound kernels leave, instead of both drifting through the same phases
-    const bool asym = [] { const char* e = getenv("GPE_SUB_ASYM"); return e && e[0] != '0'; }();
     for (int s = 0; s < gpe_handle::MAX_SUB; s++) {
-        cudaStreamCreateWithPriority(&h->sub_st[s], cudaStreamNonBlocking, (asym && s % 2 == 0) ? prio_greatest : prio_least);
+        cudaStreamCreateWithFlags(&h->sub_st[s], cudaStreamNonBlocking);
         cudaEventCreateWithFlags(&h->ev_join[s], cudaEventDisableTiming);
-        if (h->use_prio) {          // the optional high-priority twin streams (experiment knob, DESIGN.md section 8)
-            cudaStreamCreateWithPriority(&h->sub_hi[s], cudaStreamNonBlocking, prio_greatest);
-            cudaEventCreateWithFlags(&h->ev_sw[s], cudaEventDisableTiming);
-        }
     }
     cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming);
     {   // keep freed temporaries cached in the device's default pool instead of returning them to the driver
@@ -465,7 +424,6 @@ int gpe_create(int device, gpe_handle** out) {
     if (const char* e = getenv("GPE_OZAKI_STREAMS")) h->oz_nsub = std::max(1, std::min((int)gpe_handle::MAX_SUB, atoi(e)));
     if (const char* e = getenv("GPE_STREAMS")) h->nsub = std::max(1, std::min((int)gpe_handle::MAX_SUB, atoi(e)));
     if (const char* e = getenv("GPE_GRAPHS")) h->use_graphs = e[0] != '0';
-    if (const char* e = getenv("GPE_SIDE")) h->use_side = e[0] != '0';
     *out = h;
     return 0;
 }
@@ -477,9 +435,7 @@ int gpe_destroy(gpe_handle* h) {
     h->free_training();
     for (int s = 0; s < gpe_handle::MAX_SUB; s++) {
         if (h->sub_st[s]) { cudaStreamSynchronize(h->sub_st[s]); cudaStreamDestroy(h->sub_st[s]); }
-        if (h->sub_hi[s]) { cudaStreamSynchronize(h->sub_hi[s]); cudaStreamDestroy(h->sub_hi[s]); }
         if (h->ev_join[s]) cudaEventDestroy(h->ev_join[s]);
-        if (h->ev_sw[s]) cudaEventDestroy(h->ev_sw[s]);
     }
     for (int s = 0; s < gpe_handle::MAX_SUB; s++)
         for (int k = 0; k < gpe_handle::MAX_DEPTH; k++) {
@@ -715,8 +671,7 @@ static int enqueue_llh_chunk(gpe_handle* h, int Bs, int p, int mode, double fixe
         sb.b0 = (int)((long long)Bs * g / ns);
         sb.B = (int)((long long)Bs * (g + 1) / ns) - sb.b0;
         sb.st = ns > 1 ? h->sub_st[g] : h->st;
-        if (ns > 1 && h->use_prio) { sb.hi = h->sub_hi[g]; sb.ev = h->ev_sw[g]; }
-        if (h->nsub > 1 && h->use_side) {      // also for a single group (small batches): intra-item overlap only
+        if (h->nsub > 1) {      // also for a single group (small batches): intra-item overlap only
             if (h->ensure_side(g)) return h->fail_msg("could not create side streams");
             sb.side = h->side_st[g]; sb.ef = h->ev_sf[g]; sb.ej = h->ev_sj[g];
         }
@@ -730,13 +685,13 @@ static int enqueue_llh_chunk(gpe_handle* h, int Bs, int p, int mode, double fixe
         h->launches++;
         if ((rc = gpe_factor_and_reduce(h, sb, mode, 1, nullptr, nullptr))) return rc;
         if (ns > 1) {
-            CK(cudaEventRecord(h->ev_join[g], sb.stream(false)));
+            CK(cudaEventRecord(h->ev_join[g], sb.st));
             CK(cudaStreamWaitEvent(h->st, h->ev_join[g], 0));
         }
     }
     {
         ProfScope ps(h, gpe_handle::CAT_OTHER);
-        launch_grad_finalize(h->gpart, h->grad_fused == 2 ? lauum_grad_ntiles(h->npad) : grad_ntiles(h->npad), h->n, h->d, h->npad, p, mode,
+        launch_grad_finalize(h->gpart, h->grad_fused ? lauum_grad_ntiles(h->npad) : grad_ntiles(h->npad), h->n, h->d, h->npad, p, mode,
                              h->par, h->out, h->status, h->llh_d, h->grad_d,
                              h->sig_d, Bs, h->st);
     }

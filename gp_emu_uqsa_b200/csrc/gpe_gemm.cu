@@ -1,30 +1,7 @@
 // Dispatch for the batched DMMA GEMM family (see gpe_gemm.cuh).
 #include "gpe_gemm.cuh"
 
-#include <cstdlib>
-
 namespace gpe {
-
-// GPE_GEMM_WS=0 selects the single-role (block-barrier) 128x128 kernel, kept for A/B measurements.
-static bool use_ws() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("GPE_GEMM_WS");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v == 1;
-}
-
-// The two-CTAs-per-SM 128x64 kernel for the machine-filling launches of the factorisation (see gpe_gemm.cuh): a
-// consistent +0.6 % on the n = 4096 step in same-box A/B runs (75.01 -> 74.53 ms, 74.81 -> 74.42 ms).  GPE_WS2=0 switches it off.
-static bool use_ws2() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("GPE_WS2");
-        v = e ? atoi(e) : 1;
-    }
-    return v == 1;
-}
 
 template <bool A_KC, bool B_KC>
 static cudaError_t dispatch_tiles(const GemmP& p, int epi, cudaStream_t st) {
@@ -46,15 +23,15 @@ static cudaError_t dispatch_tiles(const GemmP& p, int epi, cudaStream_t st) {
     if (p.lower) t128 = t128 / 2 + (p.M / 128) * p.batch / 2;
     bool big = (p.M % 128 == 0) && (p.N % 128 == 0) && (t128 >= 120);
     if (epi == EPI_SUMSQ) {
-        // column norms are accumulated per 128-row tile: the partial buffer is sized for BM = 128
-        if (use_ws2() && p.M % 128 == 0) return launch_gemm_ws2<A_KC, B_KC, EPI_SUMSQ>(p, st);
-        if (p.M % 128 && !use_ws()) return cudaErrorInvalidValue;      // the ragged last row tile exists in the ws kernel only
-        return use_ws() ? launch_gemm_ws<A_KC, B_KC, EPI_SUMSQ>(p, st)
-                        : launch_gemm_cfg<128, 128, 2, 4, A_KC, B_KC, EPI_SUMSQ>(p, st);
+        // column norms are accumulated per 128-row tile: the partial buffer is sized for BM = 128.  The ragged last row
+        // tile exists in the one-CTA kernel only.
+        if (p.M % 128 == 0) return launch_gemm_ws2<A_KC, B_KC, EPI_SUMSQ>(p, st);
+        return launch_gemm_ws<A_KC, B_KC, EPI_SUMSQ>(p, st);
     }
-    if (big && use_ws2()) return launch_gemm_ws2<A_KC, B_KC, EPI_STORE>(p, st);
-    if (big) return use_ws() ? launch_gemm_ws<A_KC, B_KC, EPI_STORE>(p, st)
-                             : launch_gemm_cfg<128, 128, 2, 4, A_KC, B_KC, EPI_STORE>(p, st);
+    // the two-CTAs-per-SM 128x64 kernel for the machine-filling launches of the factorisation (see gpe_gemm.cuh): a
+    // consistent +0.6 % on the n = 4096 step over the one-CTA 128x128 kernel in same-box A/B runs (75.01 -> 74.53 ms,
+    // 74.81 -> 74.42 ms)
+    if (big) return launch_gemm_ws2<A_KC, B_KC, EPI_STORE>(p, st);
     // latency regime (one or two guesses at n <= 2000): 64x64 tiles would occupy under half of the SMs
     long long t64 = (long long)(p.M / 64) * (p.N / 64) * p.batch;
     if (p.lower) t64 = t64 / 2 + (p.M / 64) * p.batch / 2;

@@ -503,12 +503,7 @@ inline cudaError_t launch_gemm_ws_shape(const GemmP& p, cudaStream_t st) {
 // row-triangular launches (k <= i, k >= i) get the 4x2 warp grid, everything else the 2x4 grid
 template <bool A_KC, bool B_KC, int EPI>
 inline cudaError_t launch_gemm_ws(const GemmP& p, cudaStream_t st) {
-    static int force2 = -1;
-    if (force2 < 0) {
-        const char* e = getenv("GPE_WS_SHAPE");
-        force2 = (e && e[0] == '2') ? 1 : 0;
-    }
-    if (!force2 && (p.kmode == KM_LE_I || p.kmode == KM_GE_I)) return launch_gemm_ws_shape<A_KC, B_KC, EPI, 4>(p, st);
+    if (p.kmode == KM_LE_I || p.kmode == KM_GE_I) return launch_gemm_ws_shape<A_KC, B_KC, EPI, 4>(p, st);
     return launch_gemm_ws_shape<A_KC, B_KC, EPI, 2>(p, st);
 }
 
@@ -720,7 +715,8 @@ inline cudaError_t launch_gemm_ws2(const GemmP& p, cudaStream_t st) {
 }
 
 // Layout ids: 0 = (A_KC,B_KC) "NT", 1 = (A_KC,!B_KC) "NN", 2 = (!A_KC,!B_KC) "TN".
-// Tile choice: 128x128 when that still fills the machine, else 64x64; N == 32 panels use 128x32.
+// Tile choice: 128x64 tiles, two CTAs per SM, when 128x128 tiles still fill the machine, else 64x64 (or 32x32);
+// N == 32 panels use 128x32.  Column norms (EPI_SUMSQ) take the 128x64 kernel, or the 128x128 one for a ragged M.
 cudaError_t launch_gemm(const GemmP& p, int layout, int epi, cudaStream_t st);
 
 }  // namespace gpe

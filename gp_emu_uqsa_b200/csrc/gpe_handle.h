@@ -33,17 +33,14 @@ struct gpe_handle {
     // levels overlap the other groups' large DMMA GEMMs
     enum { MAX_SUB = 16 };
     int nsub = 8;
-    cudaStream_t sub_st[MAX_SUB] = {nullptr};      // low priority: the large DMMA GEMMs, covariance build, gradient reduction
-    cudaStream_t sub_hi[MAX_SUB] = {nullptr};      // high priority: leaf panels, small recursion levels, skinny panels
-    cudaEvent_t ev_fork = nullptr, ev_join[MAX_SUB] = {nullptr}, ev_sw[MAX_SUB] = {nullptr};
-    bool use_prio = false;
+    cudaStream_t sub_st[MAX_SUB] = {nullptr};
+    cudaEvent_t ev_fork = nullptr, ev_join[MAX_SUB] = {nullptr};
     // side streams, one per (group, recursion depth): the product T = L21 L11^-1 of a node does not depend on
     // the factorisation of its A22 block, so it runs beside that whole sub-recursion (gpe_api.cu:potrf_inv_rec)
     enum { MAX_DEPTH = 10 };
-    bool use_side = true;
     cudaStream_t side_st[MAX_SUB][MAX_DEPTH] = {{nullptr}};
     cudaEvent_t ev_sf[MAX_SUB][MAX_DEPTH] = {{nullptr}}, ev_sj[MAX_SUB][MAX_DEPTH] = {{nullptr}};
-    int ensure_side(int g);     // measured neutral on B200 (DESIGN.md section 8): off unless GPE_PRIO=1
+    int ensure_side(int g);     // creates the side streams of group g on first use
 
     // CUDA graphs of the likelihood step: the launch sequence of a (batch size, mode) pair is
     // captured the third time it is seen and replayed afterwards (one cudaGraphLaunch instead of
@@ -63,9 +60,9 @@ struct gpe_handle {
 
     // batched likelihood workspace
     int Bcap = 0;
-    bool Bcap_final = false;
+    bool Bcap_final = false;     // the workspace already has the largest size obtainable (env cap or device memory)
     bool grad_use_e = false;     // classic route with the covariance build's copy of exp(-D) (INT8 route)
-    int grad_fused = 0;          // gradient route of the current chunk (gpe_api.cu:llh_grad_fused): 0 classic, 1 split W/E, 2 epilogue     // the workspace already has the largest size obtainable (env cap or device memory)
+    bool grad_fused = false;     // gradient route of the current chunk (gpe_api.cu:llh_grad_fused): LAUUM epilogue or classic
     double *A = nullptr, *S = nullptr, *Li = nullptr;        // [Bcap][npad][npad]
     double* Ex = nullptr;                                    // [Bcap][npad][npad] exp(-D) kept by the covariance build for the fused gradient epilogue
     double *Wy = nullptr, *Z = nullptr, *U = nullptr;        // [Bcap][npad][NR]
@@ -116,28 +113,13 @@ struct ProfScope {
     ~ProfScope() { h->prof_end(cat, e0, s); }
 };
 
-// items [b0, b0 + B) of the batch workspace.  A group owns a low-priority stream `st` for its large
-// kernels and (optionally) a high-priority stream `hi` for its latency-bound small ones: the block
-// scheduler hands freed SMs to high-priority grids first, so one group's leaf panels and small
-// recursion levels run inside another group's big GEMM instead of waiting for its tail.  `stream(small)`
-// returns the stream for the next launch and orders it after everything the group has enqueued so far.
+// items [b0, b0 + B) of the batch workspace.  A group launches in order on its stream `st`; only the
+// products T = L21 L11^-1 of the recursion go to its side streams.
 struct SubBatch {
     int b0, B;
     cudaStream_t st;
-    cudaStream_t hi = nullptr;
-    cudaEvent_t ev = nullptr;
-    mutable bool on_hi = false;
     cudaStream_t* side = nullptr;      // [MAX_DEPTH] side streams of this group (nullptr: everything in order on st)
     cudaEvent_t *ef = nullptr, *ej = nullptr;
-    cudaStream_t stream(bool small) const {
-        if (!hi || small == on_hi) return on_hi ? hi : st;
-        cudaStream_t from = on_hi ? hi : st, to = small ? hi : st;
-        cudaEventRecord(ev, from);
-        cudaStreamWaitEvent(to, ev, 0);
-        on_hi = small;
-        return to;
-    }
-    cudaStream_t current() const { return on_hi ? hi : st; }
 };
 
 // Stream-ordered temporary device buffer (cudaMallocAsync / cudaFreeAsync on the handle's stream): released

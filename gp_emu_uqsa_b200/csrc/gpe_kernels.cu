@@ -226,121 +226,10 @@ void launch_unpad_lower(const double* src, int npad, int n, double* dst, int bat
 }
 
 // =========================================================================== K2 leaf
-// One CTA (1024 threads = 128 groups of 8 lanes) factors a 128x128 SPD block held in shared
-// memory and inverts its Cholesky factor.  Left-looking Cholesky: group i owns row i; at column
-// j it forms a_ij - sum_k l_ik l_jk *and* (redundantly) the pivot a_jj - sum_k l_jk^2, so a single
-// barrier per column suffices.  The inverse is a forward substitution per column (group j owns
-// column j of L^-1, stored transposed in the unused upper triangle), which needs no block barrier.
-constexpr int LS = NB + 1;
-
-__global__ void __launch_bounds__(1024, 1) leaf_potrf_trtri_kernel(const double* __restrict__ A, double* __restrict__ Linv,
-                                                                    int ld, long long sA, long long sL, int off,
-                                                                    double* __restrict__ logdet_part, int nleaf,
-                                                                    int* __restrict__ status, double* __restrict__ Lfac) {
-    extern __shared__ __align__(16) double S[];  // [NB][LS] + dinv[NB]
-    double* dinv = S + NB * LS;
-    const int b = blockIdx.x, tid = threadIdx.x;
-    const double* Ab = A + (size_t)b * sA + (size_t)off * ld + off;
-    for (int e = tid; e < NB * NB; e += 1024) {
-        int i = e >> 7, j = e & (NB - 1);
-        S[i * LS + j] = (j <= i) ? Ab[(size_t)i * ld + j] : 0.0;
-    }
-    __syncthreads();
-    const int g = tid >> 3, sub = tid & 7;
-    double logsum = 0.0;
-    int bad_at = 0;
-    for (int j = 0; j < NB; j++) {
-        double s = 0.0, pv = 0.0;
-        if (g >= j) {
-            const double* rj = S + j * LS;
-            const double* ri = S + g * LS;
-            for (int k = sub; k < j; k += 8) {
-                double ljk = rj[k];
-                s = fma(ri[k], ljk, s);
-                pv = fma(ljk, ljk, pv);
-            }
-        }
-#pragma unroll
-        for (int o = 1; o < 8; o <<= 1) {
-            s += __shfl_xor_sync(0xffffffffu, s, o);
-            pv += __shfl_xor_sync(0xffffffffu, pv, o);
-        }
-        if (g >= j) {
-            double piv = S[j * LS + j] - pv;
-            if (!(piv > 0.0)) {  // LAPACK dpotrf: ajj <= 0 or NaN -> info = j+1
-                if (bad_at == 0) bad_at = off + j + 1;
-                piv = 1.0;
-            }
-            double ljj = sqrt(piv);
-            if (g == j) {
-                if (sub == 0) {
-                    dinv[j] = 1.0 / ljj;
-                    logsum += log(ljj);
-                }
-            } else if (sub == 0) {
-                S[g * LS + j] = (S[g * LS + j] - s) / ljj;
-            }
-        }
-        __syncthreads();
-    }
-    // logsum lives in lane sub==0 of each group g (its own diagonal): block-reduce it.
-    {
-        __shared__ double red[32];
-        double v = (sub == 0) ? logsum : 0.0;
-        double tot = block_sum(v, red);
-        if (tid == 0) logdet_part[(size_t)b * nleaf + off / NB] = 2.0 * tot;
-        int bad = bad_at ? bad_at : 0x7fffffff;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) bad = min(bad, __shfl_xor_sync(0xffffffffu, bad, o));
-        if ((tid & 31) == 0 && bad != 0x7fffffff) {
-            int old = atomicCAS(&status[b], 0, bad);
-            while (old != 0 && old > bad) {
-                int prev = atomicCAS(&status[b], old, bad);
-                if (prev == old) break;
-                old = prev;
-            }
-        }
-    }
-    __syncthreads();
-    // ---- inverse: column j of X = L^-1 ; X[i][j] (i > j) stored at S[j][i]
-    {
-        const int j = g;
-        double* xcol = S + j * LS;  // entries k > j
-        const int jw = (tid >> 5) * 4;   // smallest column owned by this warp: keeps the loop warp-uniform
-        for (int i = jw + 1; i < NB; i++) {
-            const double* li = S + i * LS;
-            double s = 0.0;
-            if (i > j) {
-                for (int k = j + sub; k < i; k += 8) {   // k = j term uses the diagonal inverse
-                    double xk = (k == j) ? dinv[j] : xcol[k];
-                    s = fma(li[k], xk, s);
-                }
-            }
-#pragma unroll
-            for (int o = 1; o < 8; o <<= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-            if (sub == 0 && i > j) xcol[i] = -s * dinv[i];
-            __syncwarp();
-        }
-    }
-    __syncthreads();
-    double* Lb = Linv + (size_t)b * sL + (size_t)off * ld + off;
-    for (int e = tid; e < NB * NB; e += 1024) {
-        int i = e >> 7, j = e & (NB - 1);
-        double v = (j < i) ? S[j * LS + i] : ((j == i) ? dinv[i] : 0.0);
-        Lb[(size_t)i * ld + j] = v;
-    }
-    if (Lfac != nullptr) {   // the Cholesky factor of this block (np.linalg.cholesky consumers)
-        double* Fb = Lfac + (size_t)b * sL + (size_t)off * ld + off;
-        for (int e = tid; e < NB * NB; e += 1024) {
-            int i = e >> 7, j = e & (NB - 1);
-            Fb[(size_t)i * ld + j] = (j < i) ? S[i * LS + j] : ((j == i) ? 1.0 / dinv[i] : 0.0);
-        }
-    }
-}
-
+// One CTA factors a 128x128 SPD block held in shared memory and inverts its Cholesky factor.
 // ---- v3 leaf: blocked, barrier-light, O(n^3) parts on the FP64 tensor pipe -------------------------
-// The v1 kernel above spends one block barrier, one FP64 sqrt and one FP64 divide per column on a
-// 1024-thread CTA (238 us per launch of 128x128 blocks, the longest latency chain of an evaluation).
+// The v1 kernel (left-looking, one column per step) spent one block barrier, one FP64 sqrt and one FP64 divide
+// per column on a 1024-thread CTA (238 us per launch of 128x128 blocks, the longest latency chain of an evaluation).
 // v3 keeps the block in shared memory and works in 8-wide panels:
 //   potrf  (16 panels): (1) the 8x8 diagonal block is factored by ONE warp in registers -- lane i owns
 //          row i, pivots and columns travel by shuffles, 1/sqrt(pivot) comes from rsqrt() so there is
@@ -652,26 +541,12 @@ __global__ void __launch_bounds__(LT, 1) leaf_potrf_trtri_v3_kernel(const double
     LEAF_TICK(8);
 }
 
-// GPE_LEAF=1 selects the v1 leaf (kept for A/B measurements); default is v3.
-static int leaf_version() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("GPE_LEAF");
-        v = (e && atoi(e) == 1) ? 1 : 3;
-    }
-    return v;
-}
-
 void launch_leaf(const double* A, double* Linv, int ld, long long sA, long long sL, int off,
                  double* logdet_part, int nleaf, int* status, int B, cudaStream_t st, double* Lfac) {
-    static SmemOptIn opt1, opt3;
-    const size_t smem1 = (size_t)(NB * LS + NB) * sizeof(double);
+    static SmemOptIn opt3;
     const size_t smem3 = (size_t)(NB * L3 + T3MAX + 2 * NB) * sizeof(double);
-    opt1.ensure(leaf_potrf_trtri_kernel, smem1);
     opt3.ensure(leaf_potrf_trtri_v3_kernel, smem3);
-    const int v = leaf_version();
-    if (v == 1) leaf_potrf_trtri_kernel<<<B, 1024, smem1, st>>>(A, Linv, ld, sA, sL, off, logdet_part, nleaf, status, Lfac);
-    else leaf_potrf_trtri_v3_kernel<<<B, LT, smem3, st>>>(A, Linv, ld, sA, sL, off, logdet_part, nleaf, status, Lfac);
+    leaf_potrf_trtri_v3_kernel<<<B, LT, smem3, st>>>(A, Linv, ld, sA, sL, off, logdet_part, nleaf, status, Lfac);
 }
 
 // =========================================================================== K3 pieces
@@ -1086,113 +961,6 @@ void launch_grad_partial(const double* X, const double* r, int n, int d, int npa
         optin.ensure(grad_partial_kernel<false, FAMILY_GAUSSIAN>, smem);
         grad_partial_kernel<false, FAMILY_GAUSSIAN><<<grid, 256, smem, st>>>(X, r, n, d, npad, winv, Ainv, sAinv, U, nu, part, nullptr);
     }
-}
-
-
-// ---- light gradient reduction: W and E are given ---------------------------------------------------------------
-// The LAUUM launch of the likelihood path (gpe_lauum_grad.cu) appends the columns of U to its k loop, so what it stores
-// is already W = A^-1 - U U^T; the covariance build keeps a copy of E = exp(-D).  What is left per entry is
-// t = 2 W E and the d weighted sums of Delta_k^2: 3 + 3d FP64 instructions instead of 2 nu + 5d + 22 (exp) + 3 --
-// 51 instead of 125 at d = 16, nu = 18 -- for 16 bytes read per entry from an otherwise idle HBM.
-__global__ void __launch_bounds__(256, 3) grad_partial_we_kernel(const double* __restrict__ X, const double* __restrict__ r,
-                                                              int n, int d, int npad, const double* __restrict__ winv,
-                                                              const double* __restrict__ W, const double* __restrict__ E,
-                                                              long long sM, double* __restrict__ part) {
-    int ti, tj;
-    tri_decode(blockIdx.x, ti, tj);
-    const int b = blockIdx.z;
-    extern __shared__ __align__(16) double sm[];
-    double* Xi = sm;                                // [d][64]
-    double* Xj = Xi + (size_t)d * CT;               // [d][66]
-    double* red = Xj + (size_t)d * (CT + 2);        // [8][d+3]
-    const int tid = threadIdx.x;
-    const int ty = tid >> 4, tx = tid & 15;
-    // the two matrix tiles first: their latency hides behind the input-tile fill
-    const double* Wb = W + (size_t)b * sM;
-    const double* Eb = E + (size_t)b * sM;
-    double2 wv[4][2], ev[4][2];
-#pragma unroll
-    for (int a = 0; a < 4; a++)
-#pragma unroll
-        for (int h = 0; h < 2; h++) {
-            const size_t off = (size_t)(ti * CT + ty + 16 * a) * npad + tj * CT + 32 * h + 2 * tx;
-            wv[a][h] = __ldg(reinterpret_cast<const double2*>(Wb + off));
-            ev[a][h] = __ldg(reinterpret_cast<const double2*>(Eb + off));
-        }
-    const double* w = winv + (size_t)b * d;
-    {
-        const int row = tid >> 2, gi = ti * CT + row, gj = tj * CT + row;
-        for (int k = tid & 3; k < d; k += 4) {
-            Xi[k * CT + row] = (gi < n) ? X[(size_t)gi * d + k] * w[k] : 0.0;
-            Xj[k * (CT + 2) + row] = (gj < n) ? X[(size_t)gj * d + k] * w[k] : 0.0;
-        }
-    }
-    __syncthreads();
-    double t[4][4];
-    double sE = 0.0, sD = 0.0, sDr = 0.0;
-#pragma unroll
-    for (int a = 0; a < 4; a++) {
-        const int gi = ti * CT + ty + 16 * a;
-#pragma unroll
-        for (int h = 0; h < 2; h++) {
-            const int gj0 = tj * CT + 32 * h + 2 * tx;
-#pragma unroll
-            for (int e = 0; e < 2; e++) {
-                const int gj = gj0 + e;
-                const double wvv = e ? wv[a][h].y : wv[a][h].x, evv = e ? ev[a][h].y : ev[a][h].x;
-                double tv = 2.0 * wvv * evv;
-                // W and E are valid on and below the diagonal only: every off-diagonal pair is taken once, with weight 2
-                const bool below = gi < n && gj < gi;
-                if (gi == gj && gi < n) {
-                    sD += wvv;
-                    if (r != nullptr) sDr = fma(wvv, r[gi], sDr);
-                }
-                tv = below ? tv : 0.0;
-                t[a][2 * h + e] = tv;
-                sE += tv;
-            }
-        }
-    }
-    const int nv = d + 3;
-    const int warp = tid >> 5, lane = tid & 31;
-    double* pout = part + ((size_t)b * gridDim.x + blockIdx.x) * nv;
-    sE = warp_sum(sE); sD = warp_sum(sD); sDr = warp_sum(sDr);
-    if (lane == 0) { red[warp * nv + d] = sE; red[warp * nv + d + 1] = sD; red[warp * nv + d + 2] = sDr; }
-    for (int k = 0; k < d; k++) {
-        double xi[4], xj[4];
-#pragma unroll
-        for (int a = 0; a < 4; a++) xi[a] = Xi[k * CT + ty + 16 * a];
-        const double2 v0 = *reinterpret_cast<const double2*>(&Xj[k * (CT + 2) + 2 * tx]);
-        const double2 v1 = *reinterpret_cast<const double2*>(&Xj[k * (CT + 2) + 32 + 2 * tx]);
-        xj[0] = v0.x; xj[1] = v0.y; xj[2] = v1.x; xj[3] = v1.y;
-        double g[4] = {0.0, 0.0, 0.0, 0.0};
-#pragma unroll
-        for (int a = 0; a < 4; a++)
-#pragma unroll
-            for (int c = 0; c < 4; c++) {
-                const double df = xi[a] - xj[c];
-                g[c] = fma(t[a][c] * df, df, g[c]);
-            }
-        const double gs = warp_sum((g[0] + g[1]) + (g[2] + g[3]));
-        if (lane == 0) red[warp * nv + k] = gs;
-    }
-    __syncthreads();
-    for (int v = tid; v < nv; v += 256) {
-        double s = 0.0;
-#pragma unroll
-        for (int wv2 = 0; wv2 < 8; wv2++) s += red[wv2 * nv + v];
-        pout[v] = s;
-    }
-}
-
-cudaError_t launch_grad_partial_we(const double* X, const double* r, int n, int d, int npad, const double* winv, const double* W,
-                                   const double* E, long long sM, double* part, int B, cudaStream_t st) {
-    const int nt = npad / CT;
-    const size_t smem = ((size_t)d * (CT + CT + 2) + 8 * (size_t)(d + 3)) * sizeof(double);
-    static SmemOptIn optin;
-    if (cudaError_t e = optin.ensure(grad_partial_we_kernel, smem); e != cudaSuccess) return e;
-    grad_partial_we_kernel<<<dim3(nt * (nt + 1) / 2, 1, B), 256, smem, st>>>(X, r, n, d, npad, winv, W, E, sM, part);
-    return cudaGetLastError();
 }
 
 // Sum the tile partials in a fixed order and apply the per-parameter prefactors

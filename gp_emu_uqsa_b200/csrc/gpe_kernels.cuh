@@ -76,11 +76,7 @@ bool lauum_grad_supported(int d);
 int lauum_grad_ntiles(int npad);
 cudaError_t launch_lauum_grad(const double* Li, long long sL, int np, int n, int d, int nu, const double* U, double* Ut, double* nUt,
                               const double* X, const double* r, const double* winv, const double* E, long long sE, double* part,
-                              int B, cudaStream_t st, double* Wout = nullptr);
-// Wout != nullptr: the same launch with a plain store epilogue -- the lower 128x128 tiles of W = A^-1 - U U^T go to Wout
-// (strides as Li) and the reduction is left to launch_grad_partial_we.
-cudaError_t launch_grad_partial_we(const double* X, const double* r, int n, int d, int npad, const double* winv, const double* W,
-                                   const double* E, long long sM, double* part, int B, cudaStream_t st);
+                              int B, cudaStream_t st);
 
 inline int grad_ntiles(int npad) { int t = npad / 64; return t * (t + 1) / 2; }
 inline int grad_nvals(int d) { return d + 3; }

@@ -41,8 +41,6 @@ struct LauumGradP {
     long long sE;
     double* part;          // [B][ntile][d + 3]
     int ntile;
-    double* Wout;          // non-null: store the W tile (strides sL / np) and leave the reduction to another kernel
-    int order;             // tile order: 0 lower-triangle rows, 1 the generic kernel's column groups (GPE_LG_ORDER)
 };
 
 constexpr int LG_LDX = 128 + 4;     // row stride of the k-major X tiles in the epilogue
@@ -66,20 +64,8 @@ __global__ void __launch_bounds__(WS_THREADS, 1) lauum_grad_kernel(LauumGradP p)
     // lower-triangle tiles, row by row: tile t = ti (ti + 1) / 2 + tj.  Row ti has the k range [ti * 128, np):
     // the launch starts on its longest tiles and ends on its shortest
     int ti, tj;
-    if (p.order == 0) {
-        tri_decode_lg((int)blockIdx.x, ti, tj);
-    } else {
-        // the generic kernel's order for row-triangular launches: column blocks in groups of 16, rows ascending inside a group
-        const int T = p.np / BM, id = (int)blockIdx.x;
-        const int full = (T / WS_COLGROUP) * WS_COLGROUP * T;
-        int g0, gsz, r;
-        if (id < full) { g0 = (id / (WS_COLGROUP * T)) * WS_COLGROUP; gsz = WS_COLGROUP; r = id % (WS_COLGROUP * T); }
-        else { g0 = (T / WS_COLGROUP) * WS_COLGROUP; gsz = T - g0; r = id - full; }
-        ti = r / gsz;
-        tj = g0 + (r - ti * gsz);
-        if (ti < tj) return;
-    }
-    const int tile_id = ti * (ti + 1) / 2 + tj;
+    tri_decode_lg((int)blockIdx.x, ti, tj);
+    const int tile_id = (int)blockIdx.x;
     const int b = blockIdx.z;
     const int m0 = ti * BM, n0 = tj * BN;
     const int kbeg = m0;
@@ -119,7 +105,7 @@ __global__ void __launch_bounds__(WS_THREADS, 1) lauum_grad_kernel(LauumGradP p)
             cp_async_mbar_arrive_noinc(&full_bar[s]);
             // the epilogue reads this tile's 128 x 128 block of E (written by the covariance build a whole factorisation
             // ago: it comes from HBM).  Ask L2 for it while the consumers still have a few k-tiles to go.
-            if (p.Wout == nullptr && (kt == KT - GEMM_STAGES - 4 || (KT < GEMM_STAGES + 5 && kt == 0))) {
+            if (kt == KT - GEMM_STAGES - 4 || (KT < GEMM_STAGES + 5 && kt == 0)) {
                 const double* Eg = p.E + (size_t)b * p.sE + (size_t)m0 * p.np + n0;
 #pragma unroll 4
                 for (int q = 0; q < 32; q++) {                 // 128 rows x 8 lines of 128 bytes
@@ -191,15 +177,6 @@ __global__ void __launch_bounds__(WS_THREADS, 1) lauum_grad_kernel(LauumGradP p)
         if (lane == 0) mbar_arrive(&empty_bar[s]);
     }
 
-    if (p.Wout != nullptr) {                         // split route: W = A^-1 - U U^T to global memory, 16-byte stores
-        double* Cg = p.Wout + (size_t)b * p.sL + (size_t)(m0 + wm0 + fr) * p.np + n0 + wn0 + 2 * fc;
-#pragma unroll
-        for (int i = 0; i < FM; i++)
-#pragma unroll
-            for (int j = 0; j < FN; j++)
-                *reinterpret_cast<double2*>(Cg + (size_t)(8 * i) * p.np + 8 * j) = make_double2(acc[i][j][0], acc[i][j][1]);
-        return;
-    }
     // ===== epilogue: acc = W tile.  The pipeline stages are free: stage the E tile and the scaled input tiles there. =====
     const int d = p.d, n = p.n;
     named_bar_sync(2, WS_CONSUMERS * 32);           // every consumer is past its last stage read
@@ -355,264 +332,6 @@ __global__ void __launch_bounds__(WS_THREADS, 1) lauum_grad_kernel(LauumGradP p)
 }
 
 
-// ------------------------------------------------------------------------------------------------------------------
-// Two CTAs per SM: the same kernel on 128x64 tiles with 4 math warps (4x1 grid, warp tile 32x64 as above) + 1 producer warp
-// and 3 stages.  The epilogue of one CTA -- barrier, E-tile and X-tile loads, the scalar FP64 passes -- then overlaps the
-// other CTA's DMMA main loop instead of leaving the tensor pipe idle (one-CTA kernel: 0.9 ms of waits per 32-item launch), and
-// the idle warps of diagonal tiles give their pipe slots to the neighbour.  Shared memory: max(3 stages = 77 KB, epilogue =
-// E tile 70 KB + X tiles (d = 16: 26 KB)) per CTA.
-constexpr int LG2_CONS = 4;
-constexpr int LG2_THREADS = (LG2_CONS + 1) * 32;
-constexpr int LG2_STAGES = 3;
-constexpr int LG2_LDE = 64 + 4;        // row stride of the 128 x 64 E tile and of the k-major X_j tile
-
-__global__ void __launch_bounds__(LG2_THREADS, 2) lauum_grad64_kernel(LauumGradP p) {
-    constexpr int BM = 128, BN = 64, FM = 4, FN = 8;               // per warp: 32 rows x 64 columns
-    constexpr int A_EL = TileShape<BM, false>::ELEMS, B_EL = TileShape<BN, false>::ELEMS;
-    constexpr int A_LD = TileShape<BM, false>::LD, B_LD = TileShape<BN, false>::LD;
-    extern __shared__ __align__(16) double smem[];
-    __shared__ __align__(8) uint64_t full_bar[LG2_STAGES], empty_bar[LG2_STAGES];
-
-    // lower-triangle tiles in 64-column units, row by row: row ti holds tj = 0 .. 2 ti + 1; tile id t = ti (ti + 1) + tj
-    int ti, tj;
-    {
-        const int t = (int)blockIdx.x;
-        int r = (int)((sqrtf(4.0f * (float)t + 1.0f) - 1.0f) * 0.5f);
-        while ((r + 1) * (r + 2) <= t) r++;
-        while (r * (r + 1) > t) r--;
-        ti = r;
-        tj = t - r * (r + 1);
-    }
-    const int b = blockIdx.z;
-    const int m0 = ti * BM, n0 = tj * BN;
-    const int kbeg = m0;
-    const int KT0 = (p.np - kbeg) / GEMM_BK, KT = KT0 + p.ku;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-
-    if (tid == 0) {
-#pragma unroll
-        for (int s = 0; s < LG2_STAGES; s++) {
-            mbar_init(&full_bar[s], 32);
-            mbar_init(&empty_bar[s], LG2_CONS);
-        }
-    }
-    __syncthreads();
-
-    double* As = smem;
-    double* Bs = smem + LG2_STAGES * A_EL;
-
-    if (warp == LG2_CONS) {
-        const double* Lb = p.Li + (size_t)b * p.sL;
-        const double* Ag = Lb + (size_t)kbeg * p.np + m0;
-        const double* Bg = Lb + (size_t)kbeg * p.np + n0;
-        const double* Au = p.nUt + (size_t)b * p.sU + m0;
-        const double* Bu = p.Ut + (size_t)b * p.sU + n0;
-        const size_t kstep = (size_t)GEMM_BK * p.np;
-        for (int kt = 0; kt < KT; kt++) {
-            const int s = kt % LG2_STAGES;
-            if (kt >= LG2_STAGES) mbar_wait(&empty_bar[s], ((kt / LG2_STAGES) - 1) & 1);
-            if (kt < KT0) {
-                load_tile_warp<BM, false>(As + s * A_EL, Ag + kt * kstep, p.np, lane);
-                load_tile_warp<BN, false>(Bs + s * B_EL, Bg + kt * kstep, p.np, lane);
-            } else {
-                load_tile_warp<BM, false>(As + s * A_EL, Au + (kt - KT0) * kstep, p.np, lane);
-                load_tile_warp<BN, false>(Bs + s * B_EL, Bu + (kt - KT0) * kstep, p.np, lane);
-            }
-            cp_async_mbar_arrive_noinc(&full_bar[s]);
-            if (p.Wout == nullptr && (kt == KT - LG2_STAGES - 4 || (KT < LG2_STAGES + 5 && kt == 0))) {
-                const double* Eg = p.E + (size_t)b * p.sE + (size_t)m0 * p.np + n0;
-#pragma unroll 4
-                for (int q = 0; q < 16; q++) {                 // 128 rows x 4 lines of 128 bytes
-                    const int li = q * 32 + lane;
-                    asm volatile("prefetch.global.L2 [%0];" ::"l"(Eg + (size_t)(li >> 2) * p.np + (li & 3) * 16));
-                }
-            }
-        }
-        cp_async_wait<0>();
-        return;
-    }
-
-    const int wm0 = warp * 32;
-    const int fr = lane >> 2, fc = lane & 3;
-    const int wk_lo = wm0 / GEMM_BK;
-    double acc[FM][FN][2];
-#pragma unroll
-    for (int i = 0; i < FM; i++)
-#pragma unroll
-        for (int j = 0; j < FN; j++) acc[i][j][0] = acc[i][j][1] = 0.0;
-    const int a_off = fc * A_LD + wm0 + fr;
-    const int b_off = fc * B_LD + fr;
-    constexpr int a_kk = 4 * A_LD, b_kk = 4 * B_LD;
-    // fragment columns that touch the lower triangle: all of them below the diagonal band; on it, a warp whose rows end
-    // before the tile's columns begin has nothing to do, one whose rows end inside the left half needs that half only
-    int jn = FN;
-    {
-        const int row_end = m0 + wm0 + 32;            // one past the warp's last row
-        if (row_end <= n0) jn = 0;
-        else if (row_end <= n0 + 32) jn = FN / 2;
-    }
-    for (int kt = 0; kt < KT; kt++) {
-        const int s = kt % LG2_STAGES;
-        mbar_wait(&full_bar[s], (kt / LG2_STAGES) & 1);
-        const double* at = As + s * A_EL + a_off;
-        const double* bt = Bs + s * B_EL + b_off;
-        if (kt >= wk_lo) {
-            if (jn == FN) {
-#pragma unroll
-                for (int kk = 0; kk < GEMM_BK / 4; kk++) {
-                    double af[FM], bf[FN];
-#pragma unroll
-                    for (int i = 0; i < FM; i++) af[i] = at[kk * a_kk + i * 8];
-#pragma unroll
-                    for (int j = 0; j < FN; j++) bf[j] = bt[kk * b_kk + j * 8];
-#pragma unroll
-                    for (int i = 0; i < FM; i++)
-#pragma unroll
-                        for (int j = 0; j < FN; j++) dmma884(acc[i][j][0], acc[i][j][1], af[i], bf[j]);
-                }
-            } else if (jn == FN / 2) {
-#pragma unroll
-                for (int kk = 0; kk < GEMM_BK / 4; kk++) {
-                    double af[FM], bf[FN / 2];
-#pragma unroll
-                    for (int i = 0; i < FM; i++) af[i] = at[kk * a_kk + i * 8];
-#pragma unroll
-                    for (int j = 0; j < FN / 2; j++) bf[j] = bt[kk * b_kk + j * 8];
-#pragma unroll
-                    for (int i = 0; i < FM; i++)
-#pragma unroll
-                        for (int j = 0; j < FN / 2; j++) dmma884(acc[i][j][0], acc[i][j][1], af[i], bf[j]);
-                }
-            }
-        }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&empty_bar[s]);
-    }
-
-    if (p.Wout != nullptr) {
-        double* Cg = p.Wout + (size_t)b * p.sL + (size_t)(m0 + wm0 + fr) * p.np + n0 + 2 * fc;
-#pragma unroll
-        for (int i = 0; i < FM; i++)
-#pragma unroll
-            for (int j = 0; j < FN; j++)
-                *reinterpret_cast<double2*>(Cg + (size_t)(8 * i) * p.np + 8 * j) = make_double2(acc[i][j][0], acc[i][j][1]);
-        return;
-    }
-    // ===== epilogue (as in the one-CTA kernel, 128 threads) =====
-    const int d = p.d, n = p.n;
-    named_bar_sync(2, LG2_CONS * 32);
-    double* Es = smem;                              // [128][LG2_LDE]; later the per-lane partial sums [d][128]
-    double* Xi = Es + (128 * LG2_LDE > 128 * d ? 128 * LG2_LDE : 128 * d);   // [d][LG_LDX]
-    double* Xj = Xi + (size_t)d * LG_LDX;           // [d][LG2_LDE]
-    double* red = Xj + (size_t)d * LG2_LDE;         // [4][3]
-    {
-        const double* src = p.E + (size_t)b * p.sE + (size_t)(m0 + (tid >> 5)) * p.np + n0 + 2 * (tid & 31);
-        double* dst = Es + (tid >> 5) * LG2_LDE + 2 * (tid & 31);
-        const size_t sstep = (size_t)4 * p.np;
-#pragma unroll 4
-        for (int it = 0; it < 32; it++) {
-            cp_async16(dst, src);
-            src += sstep;
-            dst += 4 * LG2_LDE;
-        }
-        cp_async_commit();
-        const double* __restrict__ w = p.winv + (size_t)b * d;
-        const double* __restrict__ Xg = p.X;
-        const int gi = m0 + tid, gj = n0 + tid;
-        for (int k = 0; k < d; k++) {
-            const double wk = __ldg(w + k);
-            Xi[k * LG_LDX + tid] = (gi < n) ? __ldg(Xg + (size_t)gi * d + k) * wk : 0.0;
-            if (tid < BN) Xj[k * LG2_LDE + tid] = (gj < n) ? __ldg(Xg + (size_t)gj * d + k) * wk : 0.0;
-        }
-        cp_async_wait<0>();
-    }
-    named_bar_sync(2, LG2_CONS * 32);
-
-    const int row0 = wm0 + fr, col0 = 2 * fc;
-    double sE = 0.0, sD = 0.0, sDr = 0.0;
-    if (n0 + BN <= m0 && m0 + BM <= n) {            // strictly below the diagonal band and inside the matrix
-#pragma unroll
-        for (int j = 0; j < FN; j++)
-#pragma unroll
-            for (int i = 0; i < FM; i++) {
-                const double2 ev = *reinterpret_cast<const double2*>(Es + (row0 + 8 * i) * LG2_LDE + col0 + 8 * j);
-                const double t0 = 2.0 * acc[i][j][0] * ev.x, t1 = 2.0 * acc[i][j][1] * ev.y;
-                acc[i][j][0] = t0;
-                acc[i][j][1] = t1;
-                sE += t0 + t1;
-            }
-    } else {
-#pragma unroll
-        for (int j = 0; j < FN; j++)
-#pragma unroll
-            for (int i = 0; i < FM; i++) {
-                const int gi = m0 + row0 + 8 * i;
-                const double2 ev = *reinterpret_cast<const double2*>(Es + (row0 + 8 * i) * LG2_LDE + col0 + 8 * j);
-#pragma unroll
-                for (int e = 0; e < 2; e++) {
-                    const int gj = n0 + col0 + 8 * j + e;
-                    const double wv = acc[i][j][e];
-                    double tv = 2.0 * wv * (e ? ev.y : ev.x);
-                    const bool below = gi < n && gj < gi;       // each pair once, from below; selected, not multiplied by 0
-                    if (gi == gj && gi < n) {
-                        sD += wv;
-                        if (p.r != nullptr) sDr = fma(wv, p.r[gi], sDr);
-                    }
-                    tv = below ? tv : 0.0;
-                    acc[i][j][e] = tv;
-                    sE += tv;
-                }
-            }
-    }
-    sE = warp_sum(sE); sD = warp_sum(sD); sDr = warp_sum(sDr);
-    if (lane == 0) { red[warp * 3] = sE; red[warp * 3 + 1] = sD; red[warp * 3 + 2] = sDr; }
-    named_bar_sync(2, LG2_CONS * 32);               // the E tile is consumed: its memory now takes the partial sums
-    double* gpart = Es;                             // [d][128]
-    for (int k = 0; k < d; k++) {
-        double xi[FM];
-#pragma unroll
-        for (int i = 0; i < FM; i++) xi[i] = Xi[k * LG_LDX + row0 + 8 * i];
-        double g[2][2] = {{0.0, 0.0}, {0.0, 0.0}};
-#pragma unroll
-        for (int j = 0; j < FN; j++) {
-            const double2 xj = *reinterpret_cast<const double2*>(Xj + k * LG2_LDE + col0 + 8 * j);
-#pragma unroll
-            for (int i = 0; i < FM; i++) {
-                const double d0 = xi[i] - xj.x, d1 = xi[i] - xj.y;
-                g[i & 1][0] = fma(acc[i][j][0] * d0, d0, g[i & 1][0]);
-                g[i & 1][1] = fma(acc[i][j][1] * d1, d1, g[i & 1][1]);
-            }
-        }
-        gpart[k * 128 + tid] = (g[0][0] + g[0][1]) + (g[1][0] + g[1][1]);
-    }
-    named_bar_sync(2, LG2_CONS * 32);
-    const int nv = d + 3;
-    double* pout = p.part + ((size_t)b * p.ntile + blockIdx.x) * nv;
-    for (int k0 = 0; k0 < d; k0 += 16) {            // dimension k: 8 threads add 16 lane partials each, then an 8-lane butterfly
-        const int k = k0 + (tid >> 3), part = tid & 7;
-        double sacc = 0.0;
-        if (k < d) {
-#pragma unroll
-            for (int q = 0; q < 16; q++) sacc += gpart[k * 128 + part * 16 + q];
-        }
-#pragma unroll
-        for (int o = 4; o > 0; o >>= 1) sacc += __shfl_xor_sync(0xffffffffu, sacc, o);
-        if (k < d && part == 0) pout[k] = sacc;
-    }
-    if (tid < 3) {
-        double sacc = 0.0;
-#pragma unroll
-        for (int w = 0; w < LG2_CONS; w++) sacc += red[w * 3 + tid];
-        pout[d + tid] = sacc;
-    }
-}
-
-static size_t lauum_grad64_smem(int d) {
-    const size_t stages = (size_t)LG2_STAGES * (TileShape<128, false>::ELEMS + TileShape<64, false>::ELEMS) * sizeof(double);
-    const size_t epi = ((size_t)std::max(128 * LG2_LDE, 128 * d) + (size_t)d * LG_LDX + (size_t)d * LG2_LDE + 4 * 3) * sizeof(double);
-    return std::max(stages, epi);
-}
-
 // -U^T and U^T, k-major: Ut[b][c][i] = U[b][i][c]
 __global__ void __launch_bounds__(256) ut_kernel(const double* __restrict__ U, int np, double* __restrict__ Ut, double* __restrict__ nUt) {
     __shared__ double T[32][NR + 1];
@@ -639,52 +358,26 @@ bool lauum_grad_supported(int d) { return lauum_grad_smem(d) <= 227 * 1024; }
 
 cudaError_t launch_lauum_grad(const double* Li, long long sL, int np, int n, int d, int nu, const double* U, double* Ut, double* nUt,
                               const double* X, const double* r, const double* winv, const double* E, long long sE, double* part,
-                              int B, cudaStream_t st, double* Wout) {
-    if (np % 128 || (Wout == nullptr && !lauum_grad_supported(d))) return cudaErrorInvalidValue;
+                              int B, cudaStream_t st) {
+    if (np % 128 || !lauum_grad_supported(d)) return cudaErrorInvalidValue;
     ut_kernel<<<dim3(np / 32, B), 256, 0, st>>>(U, np, Ut, nUt);
     LauumGradP p;
     p.Li = Li; p.sL = sL; p.np = np; p.n = n; p.d = d;
     p.ku = (nu + GEMM_BK - 1) / GEMM_BK;
     p.Ut = Ut; p.nUt = nUt; p.sU = (long long)NR * np;
-    p.X = X; p.r = r; p.winv = winv; p.E = E; p.sE = sE; p.part = part; p.Wout = Wout;
+    p.X = X; p.r = r; p.winv = winv; p.E = E; p.sE = sE; p.part = part;
     const int T = np / 128;
     p.ntile = T * (T + 1) / 2;
-    static int order = -1, wide64 = -1;
-    if (order < 0) {
-        const char* e = getenv("GPE_LG_ORDER");
-        order = e ? atoi(e) : 0;
-        e = getenv("GPE_LG64");                       // two-CTAs-per-SM 128x64 variant (A/B knob)
-        wide64 = e ? atoi(e) : 0;
-    }
-    p.order = order;
-    if (wide64 && 2 * lauum_grad64_smem(d) <= 220 * 1024) {
-        const size_t smem = lauum_grad64_smem(d);
-        static SmemOptIn optin64;
-        if (cudaError_t e = optin64.ensure(lauum_grad64_kernel, smem); e != cudaSuccess) return e;
-        static bool carve = false;
-        if (!carve) {
-            cudaFuncSetAttribute(lauum_grad64_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-            carve = true;
-        }
-        p.ntile = T * (T + 1);
-        lauum_grad64_kernel<<<dim3(p.ntile, 1, B), LG2_THREADS, smem, st>>>(p);
-        return cudaGetLastError();
-    }
-    const size_t smem = Wout ? gemm_smem_bytes<128, 128, false, false>() : lauum_grad_smem(d);
+    const size_t smem = lauum_grad_smem(d);
     static SmemOptIn optin;
     if (cudaError_t e = optin.ensure(lauum_grad_kernel, smem); e != cudaSuccess) return e;
-    lauum_grad_kernel<<<dim3(order ? T * T : p.ntile, 1, B), WS_THREADS, smem, st>>>(p);
+    lauum_grad_kernel<<<dim3(p.ntile, 1, B), WS_THREADS, smem, st>>>(p);
     return cudaGetLastError();
 }
 
 int lauum_grad_ntiles(int npad) {
     const int T = npad / 128;
-    static int wide64 = -1;
-    if (wide64 < 0) {
-        const char* e = getenv("GPE_LG64");
-        wide64 = e ? atoi(e) : 0;
-    }
-    return wide64 ? T * (T + 1) : T * (T + 1) / 2;       // partial rows per item: one per 128x64 or per 128x128 lower tile
+    return T * (T + 1) / 2;       // partial rows per item: one per 128x128 lower tile
 }
 
 }  // namespace gpe

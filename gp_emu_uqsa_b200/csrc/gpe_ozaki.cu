@@ -814,10 +814,6 @@ __global__ void __launch_bounds__(256, 2) oz_combine_rowsumsq_kernel(const uint8
 
 // ---------------------------------------------------------------------------------------------- host side
 void OzWs::release() {
-    if (hi) cudaStreamDestroy(hi);
-    if (ev_a) cudaEventDestroy(ev_a);
-    if (ev_b) cudaEventDestroy(ev_b);
-    hi = nullptr; ev_a = ev_b = nullptr;
     cudaFree(PA); cudaFree(PB); cudaFree(PD); cudaFree(sA); cudaFree(sB);
     PA = PB = PD = nullptr; sA = sB = nullptr;
     capA = capB = capD = capS = 0;
@@ -839,8 +835,7 @@ bool oz_supported(const GemmP& p, int epi) {
 }
 
 bool oz_sumsq_swapped(const GemmP& p, int epi) {
-    static const int swap_env = [] { const char* e = getenv("GPE_OZAKI_SUMSQ_SWAP"); return e ? atoi(e) : 1; }();
-    return swap_env && epi == EPI_SUMSQ && p.kmode == KM_LE_I && p.M % OZ_BN == 0 && p.N % OZ_BM == 0 && p.N % OZ_RS_ROWS == 0;
+    return epi == EPI_SUMSQ && p.kmode == KM_LE_I && p.M % OZ_BN == 0 && p.N % OZ_BM == 0 && p.N % OZ_RS_ROWS == 0;
 }
 
 static bool same_operand(const GemmP& p, int layout) {
@@ -943,19 +938,13 @@ cudaError_t oz_gemm(const GemmP& p, int layout, int epi, int nmod, OzWs& ws, cud
     const bool a_kc = layout != 2, b_kc = layout == 0;
     // column norms of Z = A B with A lower triangular (prediction): run as Z^T = B^T A^T, the triangular factor on the column side
     const bool swap = oz_sumsq_swapped(p, epi);
-    // cluster size of the residue GEMM: row-triangular products (k <= i, k >= i) pay for a larger cluster with a coarser k
-    // range per unit
-    // pairs by default: quadruples cut the L2 -> SM traffic further (24 instead of 32 KB per k block) but only 33 of them are
-    // resident at once (132 of the 148 SMs: the GPCs' SM counts are not multiples of four) and row-triangular operands are then
-    // converted and read in 512-row granules; same-box A/B at n = 4096, 32 items: 44.4-44.9 (pairs) against 45.4-45.9 ms per step
-    static const int cl_env = [] { const char* e = getenv("GPE_OZAKI_CLUSTER"); return e ? atoi(e) : 2; }();
-    static const int cl_env_i = [] { const char* e = getenv("GPE_OZAKI_CLUSTER_I"); return e ? atoi(e) : 4; }();
-    static const int cl_env_s = [] { const char* e = getenv("GPE_OZAKI_CLUSTER_SUMSQ"); return e ? atoi(e) : 2; }();
-    // (the prediction product -- one item, 65 536 columns, k <= i -- measured 13.6 Mpred/s with pairs against 13.35 with quadruples)
-    const int cl_want = swap ? cl_env : (epi == EPI_SUMSQ ? std::min(cl_env, cl_env_s)
-                                         : ((p.kmode == KM_LE_I || p.kmode == KM_GE_I) ? std::min(cl_env, cl_env_i) : cl_env));
+    // cluster size of the residue GEMM: pairs wherever the row tiles pair up.  Quadruples cut the L2 -> SM traffic further (24
+    // instead of 32 KB per k block) but only 33 of them are resident at once (132 of the 148 SMs: the GPCs' SM counts are not
+    // multiples of four) and row-triangular operands are then converted and read in 512-row granules; same-box A/B at n = 4096,
+    // 32 items: 44.4-44.9 (pairs) against 45.4-45.9 ms per step; the prediction product (one item, 65 536 columns, k <= i)
+    // 13.6 Mpred/s with pairs against 13.35 with quadruples
     const int tiles_m = (swap ? p.N : p.M) / OZ_BM;
-    const int CL = (cl_want >= 4 && tiles_m % 4 == 0) ? 4 : ((cl_want >= 2 && tiles_m % 2 == 0) ? 2 : 1);
+    const int CL = tiles_m % 2 == 0 ? 2 : 1;
     // k ranges of triangular operands (zero blocks are neither converted nor read): granule = rows of the GEMM's work unit
     const int gA = swap ? OZ_BN : std::max(OZ_BM * CL, same ? OZ_BN : 0);
     const int triA = p.kmode == KM_LE_I ? gA : (p.kmode == KM_GE_I ? -gA : 0);
@@ -977,23 +966,7 @@ cudaError_t oz_gemm(const GemmP& p, int layout, int epi, int nmod, OzWs& ws, cud
         sBp = ws.sB;
     }
     hook(0, false, st);
-    // residue GEMM.  GPE_OZAKI_HI=1 (experiment, off): launch it on a high-priority twin stream so that its CTAs take freed SM
-    // resources ahead of another stream's queued conversion / CRT CTAs -- measured neutral under graph replay (37.59 ms per step
-    // both ways), worse with eager launches (41.2 against 38.5 ms), +2 % on the grid prediction
-    static const int hi_env = [] { const char* e = getenv("GPE_OZAKI_HI"); return e ? atoi(e) : 0; }();
-    cudaStream_t gst = st;
-    if (hi_env && hook.fn == nullptr) {
-        if (!ws.hi) {
-            int lo_p = 0, hi_p = 0;
-            cudaDeviceGetStreamPriorityRange(&lo_p, &hi_p);
-            if ((e = cudaStreamCreateWithPriority(&ws.hi, cudaStreamNonBlocking, hi_p)) != cudaSuccess) return e;
-            if ((e = cudaEventCreateWithFlags(&ws.ev_a, cudaEventDisableTiming)) != cudaSuccess) return e;
-            if ((e = cudaEventCreateWithFlags(&ws.ev_b, cudaEventDisableTiming)) != cudaSuccess) return e;
-        }
-        gst = ws.hi;
-        if ((e = cudaEventRecord(ws.ev_a, st)) != cudaSuccess) return e;
-        if ((e = cudaStreamWaitEvent(gst, ws.ev_a, 0)) != cudaSuccess) return e;
-    }
+    // residue GEMM
     hook(1, true, st);
     CUtensorMap tmA, tmB;
     const int nbp = p.batch * nmod;
@@ -1010,8 +983,7 @@ cudaError_t oz_gemm(const GemmP& p, int layout, int epi, int nmod, OzWs& ws, cud
         if ((e = make_map(&tmB, PBp, p.K, p.N, nbp, OZ_BN / CL)) != cudaSuccess) return e;
     }
     g.K = p.K; g.nmod = nmod; g.nbp = nbp; g.lower = p.lower;
-    static const int nmajor_env = [] { const char* e = getenv("GPE_OZAKI_NMAJOR"); return e ? atoi(e) : 1; }();
-    g.nmajor = (nmajor_env && !p.lower && (swap || (p.kmode == KM_LE_I && g.tiles_n > 2 * (g.tiles_m / CL)))) ? 1 : 0;
+    g.nmajor = (!p.lower && (swap || (p.kmode == KM_LE_I && g.tiles_n > 2 * (g.tiles_m / CL)))) ? 1 : 0;
     const int units_m = g.tiles_m / CL;
     if (p.lower) {
         int T = 0;
@@ -1027,41 +999,32 @@ cudaError_t oz_gemm(const GemmP& p, int layout, int epi, int nmod, OzWs& ws, cud
         static SmemOptIn optin;
         if ((e = optin.ensure(oz_gemm_kernel<1>, OZ_SMEM)) != cudaSuccess) return e;
         const int grid = (int)std::min<long long>(NUM_SMS, total);
-        oz_gemm_kernel<1><<<grid, OZ_THREADS, OZ_SMEM, gst>>>(tmA, tmB, g);
+        oz_gemm_kernel<1><<<grid, OZ_THREADS, OZ_SMEM, st>>>(tmA, tmB, g);
     } else {
-        static SmemOptIn optin2, optin4;
-        if (CL == 2) e = optin2.ensure(oz_gemm_kernel<2>, OZ_SMEM);
-        else e = optin4.ensure(oz_gemm_kernel<4>, OZ_SMEM);
-        if (e != cudaSuccess) return e;
+        static SmemOptIn optin2;
+        if ((e = optin2.ensure(oz_gemm_kernel<2>, OZ_SMEM)) != cudaSuccess) return e;
         cudaLaunchConfig_t cfg = {};
         cudaLaunchAttribute attr[1];
         attr[0].id = cudaLaunchAttributeClusterDimension;
         attr[0].val.clusterDim.x = CL; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-        cfg.blockDim = dim3(OZ_THREADS); cfg.dynamicSmemBytes = OZ_SMEM; cfg.stream = gst; cfg.attrs = attr; cfg.numAttrs = 1;
-        static int max_clusters[16][5] = {{0}};
+        cfg.blockDim = dim3(OZ_THREADS); cfg.dynamicSmemBytes = OZ_SMEM; cfg.stream = st; cfg.attrs = attr; cfg.numAttrs = 1;
+        static int max_clusters[16] = {0};
         int dev = 0;
         cudaGetDevice(&dev);
-        int& mc = max_clusters[dev & 15][CL];
+        int& mc = max_clusters[dev & 15];
         if (!mc) {       // clusters that are resident at once: a persistent grid must not exceed them
             cfg.gridDim = dim3(NUM_SMS / CL * CL);
             int n = 0;
-            cudaError_t qe = CL == 2 ? cudaOccupancyMaxActiveClusters(&n, oz_gemm_kernel<2>, &cfg)
-                                     : cudaOccupancyMaxActiveClusters(&n, oz_gemm_kernel<4>, &cfg);
+            cudaError_t qe = cudaOccupancyMaxActiveClusters(&n, oz_gemm_kernel<2>, &cfg);
             if (qe != cudaSuccess || n < 1) n = NUM_SMS / CL - 4;
             mc = std::min(n, NUM_SMS / CL);
             if (getenv("GPE_OZAKI_VERBOSE")) fprintf(stderr, "oz_gemm: cluster %d, %d clusters resident\n", CL, mc);
         }
         const int ncl = (int)std::min<long long>(mc, total);
         cfg.gridDim = dim3(CL * ncl);
-        if (CL == 2) e = cudaLaunchKernelEx(&cfg, oz_gemm_kernel<2>, tmA, tmB, g);
-        else e = cudaLaunchKernelEx(&cfg, oz_gemm_kernel<4>, tmA, tmB, g);
-        if (e != cudaSuccess) return e;
+        if ((e = cudaLaunchKernelEx(&cfg, oz_gemm_kernel<2>, tmA, tmB, g)) != cudaSuccess) return e;
     }
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
-    if (gst != st) {
-        if ((e = cudaEventRecord(ws.ev_b, gst)) != cudaSuccess) return e;
-        if ((e = cudaStreamWaitEvent(st, ws.ev_b, 0)) != cudaSuccess) return e;
-    }
     hook(1, false, st);
     // CRT + scale + store
     hook(2, true, st);

@@ -14,7 +14,8 @@
 // K 2^(1-bits); bits = 63 (nmod = 18), 59-60 (17), 56 (16).  The reference arithmetic this replaces is NumPy's float64
 // matmul / LAPACK inside np.linalg.cholesky and solve (_emulatoroptimise.py:313-335, 425-441); the parity bar (llh 1e-10,
 // gradient 1e-9 against the real reference at n = 4096) is what decides nmod.  oracle/ozaki2_oracle.py restates the
-// arithmetic limb for limb.  Off unless GPE_OZAKI=<nmod> is set; DMMA stays the default path.
+// arithmetic limb for limb.  The default (nmod = 16) for products of 1024 and more in every dimension (GPE_OZAKI_MIN);
+// GPE_OZAKI=<nmod> sets the number of moduli, GPE_OZAKI=0 keeps every product on DMMA.
 #pragma once
 #include "gpe_gemm.cuh"
 
@@ -42,10 +43,6 @@ struct OzWs {
     bool have_a = false;
     double b_bound = 0.0;        // set before a call: |B| <= b_bound everywhere, so operand B takes one scale and its maxima are not
                                  // searched (holds for that call only)
-    // high-priority twin of the stream this scratch belongs to: the residue GEMM is launched there (between two events), so that
-    // its CTAs take freed SM resources ahead of the queued CTAs of another stream's conversion / CRT launches
-    cudaStream_t hi = nullptr;
-    cudaEvent_t ev_a = nullptr, ev_b = nullptr;
     bool grew = false;           // set when a buffer was reallocated: captured graphs that used the old one are stale
     void release();
 };

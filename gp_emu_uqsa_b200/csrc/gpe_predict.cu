@@ -641,12 +641,7 @@ int predict_chunk(gpe_handle* h, gpe_handle::PredSlot& sl, cudaStream_t st, cons
     int ntile = 0;
     if (var_dev != nullptr || imp != nullptr) {
         // column norms of Z = Linv C    (NN, Linv lower: k <= i), reduced in the epilogue
-        static int ragged = -1;
-        if (ragged < 0) {
-            const char* e = getenv("GPE_PRED_RAGGED");
-            ragged = (e && e[0] == '0') ? 0 : 1;
-        }
-        int mp = ragged ? kp : np;
+        int mp = kp;
         // INT8 tensor-core route (gpe_ozaki.cuh) for chunks it supports: the residue planes of L^-1 are made once per fit and
         // stream (the tag is the generation of the fit state), the padded size is used (rows >= n of Z are zero)
         bool one_row = false;
@@ -661,8 +656,7 @@ int predict_chunk(gpe_handle* h, gpe_handle::PredSlot& sl, cudaStream_t st, cons
                 // every entry of the slab is c exp(-D) or c R(D), in [0, c]: one scale for all points, no pass over the slab for its maxima.
                 // (A point far from every training input then keeps fewer significant bits of its tiny column -- its variance
                 // is the prior's to the same absolute accuracy, which is what the subtraction prior - |Z|^2 needs.)
-                static const int fixed_env = [] { const char* e = getenv("GPE_PRED_FIXED_SCALE"); return e ? atoi(e) : 1; }();
-                if (fixed_env) h->oz_b_bound = h->fit_c;
+                h->oz_b_bound = h->fit_c;
                 one_row = oz_sumsq_swapped(p, EPI_SUMSQ);
             }
         }

@@ -9,11 +9,6 @@ pred() { timeout 300 python tools/perf_pred.py 2000 8 4194304 2>&1 | tail -n 1; 
 echo "--- default";                       llh; pred
 echo "--- FP64 DMMA everywhere";          GPE_OZAKI=0 llh; GPE_OZAKI=0 pred
 echo "--- 14 moduli";                     GPE_OZAKI=14 llh; GPE_OZAKI=14 pred
-echo "--- four-CTA clusters";             GPE_OZAKI_CLUSTER=4 llh; GPE_OZAKI_CLUSTER=4 pred
 echo "--- INT8 from 512 up";              GPE_OZAKI_MIN=512 llh
 echo "--- one / four sub-batch groups";   GPE_OZAKI_STREAMS=1 llh; GPE_OZAKI_STREAMS=4 llh
-echo "--- asymmetric stream priorities";  GPE_SUB_ASYM=1 llh
-echo "--- gradient: exp recomputed";      GPE_GRAD_E=0 llh
-echo "--- prediction: L^-1 on the row side / old unit order / searched maxima"
-GPE_OZAKI_SUMSQ_SWAP=0 pred; GPE_OZAKI_NMAJOR=0 GPE_OZAKI_SUMSQ_SWAP=0 pred; GPE_PRED_FIXED_SCALE=0 pred
 echo "--- default";                       llh; pred

@@ -1,5 +1,5 @@
 """Leaf kernel timing (development aid): batched 128x128 Cholesky+inverse through gpe_potrf with the
-per-category CUDA-event profile.  GPE_LEAF=1 selects the v1 kernel."""
+per-category CUDA-event profile."""
 import os, sys
 import numpy as np
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
@@ -15,4 +15,4 @@ for _ in range(5):
 pr = dev.profile_read()
 ms, cnt = pr["potrf_leaf"]
 err = np.abs(Li[0] @ np.linalg.cholesky(A[0]) - np.eye(128)).max()
-print("GPE_LEAF=%s: leaf %.1f us per launch (%d launches), |Linv L - I| = %.2e" % (os.environ.get("GPE_LEAF", "3"), ms / cnt * 1e3, cnt, err))
+print("leaf %.1f us per launch (%d launches), |Linv L - I| = %.2e" % (ms / cnt * 1e3, cnt, err))
