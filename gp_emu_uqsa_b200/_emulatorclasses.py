@@ -104,6 +104,7 @@ class Beliefs:
 
     REQUIRED = ("active", "output", "basis_str", "basis_inf", "beta", "delta", "sigma", "nugget", "fix_nugget", "mucm")
     KERNELS = ("gaussian", "matern52")
+    OBJECTIVES = ("llh", "loo")
 
     def __init__(self, beliefs_file):
         self.beliefs_file = beliefs_file
@@ -157,6 +158,10 @@ class Beliefs:
         self.kernel = words("kernel")[0] if "kernel" in b else "gaussian"
         if self.kernel not in self.KERNELS:
             _die("WARNING: kernel should be one of %s" % " ".join(self.KERNELS))
+        # training objective: absent means maximum likelihood; loo minimises the leave-one-out cross-validation objective
+        self.objective = words("objective")[0] if "objective" in b else "llh"
+        if self.objective not in self.OBJECTIVES:
+            _die("WARNING: objective should be one of %s" % " ".join(self.OBJECTIVES))
         self.input_minmax = eval(b["input_minmax"]) if "input_minmax" in b else []
 
     def final_beliefs(self, E, final=False):
@@ -180,7 +185,8 @@ class Beliefs:
             "fix_nugget " + str(self.fix_nugget),
             "alt_nugget " + str(self.alt_nugget),
             "mucm " + str(self.mucm),
-        ] + (["kernel " + self.kernel] if self.kernel != "gaussian" else []) + [
+        ] + (["kernel " + self.kernel] if self.kernel != "gaussian" else []) + (
+            ["objective loo"] if self.objective == "loo" else []) + [
             "input_minmax " + str(E.all_data.input_minmax),
         ]
         try:

@@ -90,6 +90,8 @@ class Optimize:
             m |= _lib.MODE_ALT_NUGGET
         if self.beliefs.fix_nugget == "F":
             m |= _lib.MODE_NUGGET_FREE
+        if getattr(self.beliefs, "objective", "llh") == "loo":
+            m |= _lib.MODE_LOO
         return m
 
     def standard_constraint(self, bounds):
@@ -171,13 +173,16 @@ class Optimize:
         self.last_table = pack                     # rows [ok, fun, theta...] per guess, in guess order
         K.n = fixed_n if self.beliefs.fix_nugget != "F" else K.n
 
-        # sigma for the printed lines (mucm): one more batched evaluation at the optima
+        # sigma for the printed lines (mucm): one more batched evaluation at the optima (with the LOO objective its sigma_hat
+        # is the profiled LOO sigma, which also becomes the emulator's sigma below)
         okrows = np.nonzero(pack[:, 0] == 1.0)[0]
         sig_print = {}
         if mucm and okrows.size:
             _, _, ok2, sig = self._eval_batch(pack[okrows, 2:])
             sig_print = {int(c): float(s) for c, s, o in zip(okrows, sig, ok2) if o}
 
+        loo = self._mode() & _lib.MODE_LOO
+        label = "loo" if loo else "llh"
         first_try, best_min, best_x, best_C = True, 10000000.0, None, -1
         for C in range(numguesses):
             if pack[C, 0] != 1.0:
@@ -190,7 +195,7 @@ class Optimize:
             if mucm and C in sig_print:
                 self.par.sigma = sig_print[C]
                 sig_str = "  sig: " + str(np.around(self.par.sigma, decimals=4))
-            print("  hp: ", np.around(K.untransform(x), decimals=4), " llh: ", -1.0 * np.around(fun, decimals=4), sig_str)
+            print("  hp: ", np.around(K.untransform(x), decimals=4), " %s: " % label, -1.0 * np.around(fun, decimals=4), sig_str)
             if fun < best_min or first_try:
                 best_min, best_x, first_try, best_C = fun, K.untransform(x), False, C
         print("********")
@@ -200,7 +205,10 @@ class Optimize:
         if mucm:
             K.set_params(best_x)
             self.par.delta, self.par.nugget = K.d, K.n
-            self.sigma_analytic_mucm(best_x)
+            if loo:
+                self.par.sigma = sig_print.get(best_C, self.par.sigma)
+            else:
+                self.sigma_analytic_mucm(best_x)
         else:
             K.set_params(best_x[:-1])
             self.par.delta, self.par.nugget = K.d, K.n

@@ -11,7 +11,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libgpe_b200.so")
 
-MODE_MUCM, MODE_ALT_NUGGET, MODE_NUGGET_FREE = 1, 2, 4
+MODE_MUCM, MODE_ALT_NUGGET, MODE_NUGGET_FREE, MODE_LOO = 1, 2, 4, 8
 KERNEL_GAUSSIAN, KERNEL_MATERN52 = 0, 1
 KM_FULL, KM_LE_J, KM_GE_J, KM_LE_I, KM_GE_I = 0, 1, 2, 3, 4
 
@@ -54,6 +54,7 @@ def load():
         "gpe_cross_cov": (i, [p, p, d, i, p, i, p]),
         "gpe_llh_grad_batch": (i, [p, p, i, i, i, d, p, p, p, p]),
         "gpe_fit_state": (i, [p, p, d, d, i, d, p, p, p, p]),
+        "gpe_loo": (i, [p, p, p]),
         "gpe_predict": (i, [p, p, p, ll, p, p]),
         "gpe_predict_grid": (i, [p, p, p, p, ll, ll, p, p]),
         "gpe_predict_fullcov": (i, [p, p, p, i, p, p, p]),
@@ -78,7 +79,7 @@ def load():
 EXPORTS = ["gpe_version", "gpe_create", "gpe_destroy", "gpe_last_error", "gpe_launch_count",
            "gpe_get_stream", "gpe_set_streams", "gpe_set_async", "gpe_set_kernel", "gpe_synchronize", "gpe_profile_enable", "gpe_profile_read",
            "gpe_set_training", "gpe_set_basis", "gpe_cov_build", "gpe_cov_grad", "gpe_cross_cov", "gpe_llh_grad_batch",
-           "gpe_fit_state", "gpe_predict", "gpe_predict_grid", "gpe_predict_fullcov", "gpe_implausibility", "gpe_predict_implaus",
+           "gpe_fit_state", "gpe_loo", "gpe_predict", "gpe_predict_grid", "gpe_predict_fullcov", "gpe_implausibility", "gpe_predict_implaus",
            "gpe_solve", "gpe_sens_contract", "gpe_sens_main_effect", "gpe_potrf", "gpe_pdist_argmin",
            "gpe_dbg_gemm", "gpe_dbg_gemm_oz", "gpe_dbg_potrf_inv", "gpe_dbg_int8_products"]
 
@@ -251,6 +252,13 @@ class Device:
         self._ck(self.L.gpe_fit_state(self.h, _ptr(delta), float(nugget), float(sigma), int(kind), float(r_div), _ptr(beta_in),
                                       _ptr(beta_out), C.addressof(sig), C.addressof(st)))
         return beta_out, float(sig.value), int(st.value)
+
+    def loo(self, out=None):
+        """Leave-one-out (mean [n], var [n]) of the training points for the state fit_state left (beta re-estimated
+        on the n - 1 other points; NaN where P_ii <= 0).  ``out``: a (mean, var) pair of torch CUDA tensors to fill."""
+        mean, var = (np.empty(self.n), np.empty(self.n)) if out is None else out
+        self._ck(self.L.gpe_loo(self.h, _ptr(mean), _ptr(var)))
+        return mean, var
 
     def predict(self, Xs, Hs=None, want_var=True, out=None):
         host = isinstance(Xs, np.ndarray) or not hasattr(Xs, "data_ptr")

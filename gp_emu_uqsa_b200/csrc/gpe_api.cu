@@ -315,6 +315,35 @@ static bool llh_grad_fused(gpe_handle* h, int B) {
     return lauum_grad_supported(h->d);
 }
 
+// LOO weight matrix of a GPE_MODE_LOO chunk (gpe_loo.cu): A^-1 (lower tiles, in A) -> W = F F^T - 1/2 [(P c) alpha^T +
+// alpha (P c)^T] (lower tiles, in A), which the gradient reduction then contracts with every dA/dtheta like A^-1 - U U^T.
+// F = P diag(sqrt w) goes to the dead S buffer, the LOO panel V to the dead Wy, P c = F V to the dead Z: no n x n buffer is
+// added.  F F^T is the one extra O(n^3) product (n^3 flops per item); it takes the INT8 route or DMMA like every other.
+static int loo_weights(gpe_handle* h, const SubBatch& sb, int mode) {
+    const int np = h->npad, ld = np, B = sb.B, b0 = sb.b0;
+    const long long sM = (long long)np * np, sP = (long long)np * NR;
+    const cudaStream_t st = sb.st;
+    double* Ab = h->A + (size_t)b0 * sM;
+    double* Sb = h->S + (size_t)b0 * sM;
+    double *V = h->Wy + (size_t)b0 * sP, *Pc = h->Z + (size_t)b0 * sP, *U = h->U + (size_t)b0 * sP;
+    int rc;
+    {
+        ProfScope ps(h, gpe_handle::CAT_OTHER, st);
+        launch_loo_stats(Ab, sM, U, h->n, h->q, np, mode, h->par + b0, h->out + b0, V, h->status + b0, B, st);
+        launch_loo_f(Ab, sM, U, V, h->n, h->q, np, Sb, B, st);
+    }
+    h->launches += 2;
+    // P c = F (c / sqrt w)   (NN, skinny)
+    if ((rc = run_gemm(h, st, Sb, V, Pc, ld, NR, NR, sM, sP, sP, np, NR, np, 1.0, 0, KM_FULL, 0, B, 1))) return rc;
+    {
+        ProfScope ps(h, gpe_handle::CAT_OTHER, st);
+        launch_loo_rank2(Pc, V, np, Ab, sM, B, st);
+    }
+    h->launches++;
+    // W += F F^T   (NT, lower tiles)
+    return run_gemm(h, st, Sb, Sb, Ab, ld, ld, ld, sM, sM, sM, np, np, np, 1.0, 1, KM_FULL, 1, B, 0);
+}
+
 // Everything after the covariance build for the items of `sb`, already described by h->par / h->winv.
 // with_grad = 0 stops after the GLS/likelihood scalars (fit_state path).
 int gpe_factor_and_reduce(gpe_handle* h, const SubBatch& sb, int mode, int with_grad, const double* beta_override, double* Kout) {
@@ -355,9 +384,12 @@ int gpe_factor_and_reduce(gpe_handle* h, const SubBatch& sb, int mode, int with_
     // the stand-alone reduction kernel
     if ((rc = run_gemm(h, st, Lb, Lb, Ab, ld, ld, ld, sM, sM, sM, np, np, np, 1.0, 0, KM_GE_I, 1, B, 2, EPI_STORE,
                        gpe_handle::CAT_LAUUM))) return rc;
+    // LOO: the weight matrix replaces A^-1 and carries the whole of W, so no column of U is subtracted
+    const bool loo = mode & GPE_MODE_LOO;
+    if (loo && (rc = loo_weights(h, sb, mode))) return rc;
     {
         ProfScope ps(h, gpe_handle::CAT_GRAD, st);
-        launch_grad_partial(h->X, h->r, h->n, h->d, np, h->winv + (size_t)b0 * h->d, Ab, sM, U, h->q + 1,
+        launch_grad_partial(h->X, h->r, h->n, h->d, np, h->winv + (size_t)b0 * h->d, Ab, sM, U, loo ? 0 : h->q + 1,
                             h->gpart + (size_t)b0 * grad_ntiles(np) * grad_nvals(h->d), B, st,
                             h->grad_use_e ? h->Ex + (size_t)b0 * sM : nullptr, h->family);
     }
@@ -663,8 +695,10 @@ static int enqueue_llh_chunk(gpe_handle* h, int Bs, int p, int mode, double fixe
     int ns = h->npad < (capturing ? group_npad_graph : group_npad) ? 1 : std::max(1, std::min(h->nsub, Bs / 2));
     if (oz_takes(h, h->npad / 2, h->npad / 2, h->npad / 2)) ns = std::min(ns, h->oz_nsub);   // the top level runs on the INT8 route
     // one decision for the whole chunk (every group writes the same partial layout): the smallest group must still
-    // fill the machine with 128x128 tiles
-    h->grad_fused = llh_grad_fused(h, Bs / ns);
+    // fill the machine with 128x128 tiles.  A LOO chunk always takes the classic route: its weight matrix is built from
+    // the stored A^-1.
+    const bool loo = mode & GPE_MODE_LOO;
+    h->grad_fused = llh_grad_fused(h, Bs / ns) && !loo;
     if (ns > 1) CK(cudaEventRecord(h->ev_fork, h->st));
     for (int g = 0; g < ns; g++) {
         SubBatch sb;
@@ -689,7 +723,10 @@ static int enqueue_llh_chunk(gpe_handle* h, int Bs, int p, int mode, double fixe
             CK(cudaStreamWaitEvent(h->st, h->ev_join[g], 0));
         }
     }
-    {
+    if (loo) {
+        ProfScope ps(h, gpe_handle::CAT_OTHER);
+        launch_loo_finalize(h->gpart, grad_ntiles(h->npad), h->d, p, mode, h->par, h->out, h->llh_d, h->grad_d, h->sig_d, Bs, h->st);
+    } else {
         ProfScope ps(h, gpe_handle::CAT_OTHER);
         launch_grad_finalize(h->gpart, h->grad_fused ? lauum_grad_ntiles(h->npad) : grad_ntiles(h->npad), h->n, h->d, h->npad, p, mode,
                              h->par, h->out, h->status, h->llh_d, h->grad_d,

@@ -76,6 +76,7 @@ struct gpe_handle {
     bool fitted = false;
     int fit_kind = 0;
     double fit_nugget = 0, fit_sigma = 1, fit_c = 1, fit_astar = 1;
+    double fit_dbeta[gpe::NR] = {0};     // GLS beta minus the beta the state was fitted with (gpe_loo re-estimates beta)
     double *fLi = nullptr;       // [npad][npad]  L^-1 of the training matrix
     double *fE = nullptr;        // [npad][NR]    U = [A^-1 H K^-T | A^-1 (y - H beta)]
     double *fK = nullptr;        // [NR][NR]      Cholesky factor of Q = H^T A^-1 H (host-filled)

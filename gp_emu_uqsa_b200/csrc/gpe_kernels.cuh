@@ -78,6 +78,16 @@ cudaError_t launch_lauum_grad(const double* Li, long long sL, int np, int n, int
                               const double* X, const double* r, const double* winv, const double* E, long long sE, double* part,
                               int B, cudaStream_t st);
 
+// Leave-one-out objective of a GPE_MODE_LOO chunk (gpe_loo.cu).  V [B][npad][NR] is the item's LOO panel (columns:
+// c / sqrt w, alpha, sqrt w); F [B][npad][npad] = P diag(sqrt w); Pc [B][npad][NR] = F V (P c in column 0).
+void launch_loo_stats(const double* Ainv, long long sA, const double* U, int n, int q, int npad, int mode, ItemPar* par, ItemOut* out,
+                      double* V, int* status, int B, cudaStream_t st);
+void launch_loo_f(const double* Ainv, long long sA, const double* U, const double* V, int n, int q, int npad, double* F, int B,
+                  cudaStream_t st);
+void launch_loo_rank2(const double* Pc, const double* V, int npad, double* C, long long sC, int B, cudaStream_t st);
+void launch_loo_finalize(const double* part, int ntile, int d, int p, int mode, const ItemPar* par, const ItemOut* out,
+                         double* llh, double* grad, double* sigma_hat, int B, cudaStream_t st);
+
 inline int grad_ntiles(int npad) { int t = npad / 64; return t * (t + 1) / 2; }
 inline int grad_nvals(int d) { return d + 3; }
 

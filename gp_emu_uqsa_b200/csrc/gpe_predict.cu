@@ -728,6 +728,7 @@ int gpe_fit_state(gpe_handle* h, const double* delta, double nugget, double sigm
     CK(cudaStreamSynchronize(h->st));
     CK(cudaGetLastError());
     h->fit_kind = kind; h->fit_nugget = nugget; h->fit_sigma = sigma;
+    for (int a = 0; a < NR; a++) h->fit_dbeta[a] = beta_in ? bopt[a] - bin[a] : 0.0;
     h->fit_c = kind ? 1.0 : (1.0 - nugget);
     h->fit_astar = kind ? (1.0 + nugget * nugget) : 1.0;
     h->fitted = (st == 0);

@@ -10,7 +10,7 @@ from . import _emulatoroptimise as _emuo
 from . import _emulatorplotting as _emup
 from . import _lib
 
-__all__ = ["setup", "train", "plot", "posterior", "posterior_sample", "posterior_diag"]
+__all__ = ["setup", "train", "plot", "posterior", "posterior_sample", "posterior_diag", "loo"]
 
 
 def setup(config_file, datashuffle=True, scaleinputs=True):
@@ -158,3 +158,14 @@ def posterior_sample(E, x, predict=True):
     Lf = _lib.scratch_device().cholesky(p.var)
     u = _np.random.randn(x[:, 0].size)
     return p.mean + Lf.dot(u)
+
+
+def loo(E):
+    """Leave-one-out cross-validation of the trained emulator on its own training points, with no simulator run held
+    out: (mean [n], var [n]), the predictive of each training output from the other n - 1 points (beta re-estimated
+    by GLS, sigma and the other hyper-parameters as trained).  Standardised LOO errors are
+    ``(E.training.outputs - mean) / sqrt(var)``; for a well-calibrated emulator they look like draws from N(0, 1)."""
+    dev, _, _, st = E.training.fit(beta=E.par.beta, r_div=E.training._A_args[0])
+    if st != 0:
+        raise _lib.GpeError("training covariance matrix is not positive definite")
+    return dev.loo()

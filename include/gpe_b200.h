@@ -36,6 +36,7 @@ typedef struct gpe_handle gpe_handle;
 #define GPE_MODE_MUCM 1        /* beliefs.mucm == 'T'      (loglikelihood_mucm)              */
 #define GPE_MODE_ALT_NUGGET 2  /* beliefs.alt_nugget == 'T' (kernel_alt_nug)                  */
 #define GPE_MODE_NUGGET_FREE 4 /* beliefs.fix_nugget == 'F' (nugget is an optimised parameter) */
+#define GPE_MODE_LOO 8         /* beliefs.objective == 'loo': gpe_llh_grad_batch returns the leave-one-out objective */
 
 /* covariance families for gpe_set_kernel.  With D_ij = sum_k ((x_ik - x_jk) / delta_k)^2 and r = sqrt(D):
  * GAUSSIAN  exp(-D) (the reference's kernel / kernel_alt_nug);
@@ -112,7 +113,16 @@ int gpe_cross_cov(gpe_handle* h, const double* delta, double nugget, int kind,
  * for B transformed parameter vectors at once (the multistart batch of Optimize.optimal,
  * :227-247).  theta [B,p] with p = d (+1 nugget) (+1 sigma), ordered [delta.., nugget?, sigma?].
  * Outputs: llh [B] (the minimised value), grad [B,p], sigma_hat [B] (mucm: analytic sigma,
- * :324-327; gp4ml: sigma from theta), status [B]. */
+ * :324-327; gp4ml: sigma from theta), status [B].
+ * With GPE_MODE_LOO in mode the minimised value is the leave-one-out (LOO) cross-validation objective instead (the other
+ * bits and p keep their meaning; DESIGN.md section 9c).  With A the matrix the likelihood of the same mode factors,
+ * P = A^-1 - A^-1 H (H^T A^-1 H)^-1 H^T A^-1 and alpha = P y, the LOO predictive of y_i with beta re-estimated by GLS on
+ * the other n - 1 points has residual alpha_i / P_ii and variance s^2 / P_ii, and
+ *   llh = 1/2 sum_i [ log(2 pi s^2 / P_ii) + alpha_i^2 / (s^2 P_ii) ],  grad = its exact gradient,
+ * s^2 = 1 in gp4ml mode (sigma^2 is inside A; sigma_hat = sigma from theta), s^2 = (1/n) sum_i alpha_i^2 / P_ii in MUCM mode
+ * (sigma_hat = s).  status: as for the likelihood, plus 2 npad + i + 1 (npad = n rounded up to a multiple of 128) when
+ * P_ii <= 0 for some point i (first such i; e.g. a point the mean basis fits exactly); such an item returns llh = +inf.
+ * A LOO step costs about twice a likelihood step: one more n x n x n product per item. */
 int gpe_llh_grad_batch(gpe_handle* h, const double* theta, int B, int p, int mode,
                        double fixed_nugget, double* llh, double* grad, double* sigma_hat,
                        int* status);
@@ -177,6 +187,12 @@ int gpe_predict_implaus(gpe_handle* h, const double* Xs, const double* Hs, const
                         int first, int last, double* Itop, double cm, long long cell_pts, long long first_index,
                         long long ncell, unsigned char* keep, unsigned long long* count_lt, double* cell_min,
                         unsigned long long* cell_count);
+
+/* Leave-one-out predictions of the training points for the matrix gpe_fit_state last factored, with its sigma:
+ * mean [n] = y_i - alpha_i / P_ii and var [n] = sigma^2 / P_ii (P and alpha as for GPE_MODE_LOO above).  beta is
+ * re-estimated by GLS on the n - 1 remaining points whatever beta_in gpe_fit_state was given.  Standardised LOO errors are
+ * (y - mean) / sqrt(var).  A point with P_ii <= 0 gets NaN in both.  Outputs host or device. */
+int gpe_loo(gpe_handle* h, double* mean, double* var);
 
 /* out [n,k] = A^-1 Bm [n,k] for the training matrix factored by gpe_fit_state -- the
  * np.linalg.solve(self.A, .) call sites of the sensitivity code
