@@ -136,37 +136,28 @@ int gpe_ensure_batch_ws(gpe_handle* h, int B) {
 }
 
 // ------------------------------------------------------------------------------------- GEMM helper
-// does launch_gemm pick the warp-specialised 128x128 kernel with a machine-filling grid? (mirrors dispatch_tiles)
-static bool gemm_is_big(int M, int N, int lower, int batch) {
-    if (M % 128 || N % 128 || M == 32 || N == 32) return false;
-    long long t128 = (long long)(M / 128) * (N / 128) * batch;
-    if (lower) t128 = t128 / 2 + (M / 128) * batch / 2;
-    return t128 >= 120;
+// The INT8 route rule: does product p take the INT8 tensor-core route (gpe_ozaki.cuh) by its shape?
+static bool int8_rule(const gpe_handle* h, const GemmP& p, int epi) {
+    return h->oz_nmod > 0 && p.M >= h->oz_min && p.N >= h->oz_min && p.K >= h->oz_min && oz_supported(p, epi);
 }
 
-static bool oz_takes(const gpe_handle* h, int M, int N, int K) {
-    return h->oz_nmod > 0 && M >= h->oz_min && N >= h->oz_min && K >= h->oz_min && M % OZ_BM == 0 && N % OZ_BN == 0 && K % OZ_BK == 0;
+bool gpe_int8_route(gpe_handle* h, cudaStream_t st, const GemmP& p, int layout, int epi) {
+    if (!int8_rule(h, p, epi)) return false;
+    // scratch is per stream; growing it is not allowed inside a capture, and every shape has been seen eagerly at least twice
+    // before its graph is captured
+    OzWs& ws = h->oz_ws[st];
+    const cudaError_t e = oz_reserve(ws, p, layout, h->oz_nmod);
+    if (ws.grew) { ws.grew = false; h->graphs_stale = true; }
+    if (e == cudaSuccess) return true;
+    // out of memory (a prediction chunk over a very large training set): the product runs on DMMA.  The failed cudaMalloc is the
+    // last runtime error at this point, so clearing it drops nothing else.
+    cudaGetLastError();
+    return false;
 }
 
-static int run_gemm(gpe_handle* h, cudaStream_t st, const double* A, const double* B, double* C, int lda, int ldb, int ldc,
-                    long long sA, long long sB, long long sC, int M, int N, int K, double alpha, int acc,
-                    int kmode, int lower, int batch, int layout, int epi = EPI_STORE, int cat = -1) {
-    GemmP p;
-    p.A = A; p.B = B; p.C = C; p.lda = lda; p.ldb = ldb; p.ldc = ldc; p.sA = sA; p.sB = sB; p.sC = sC;
-    p.M = M; p.N = N; p.K = K; p.alpha = alpha; p.accumulate = acc; p.kmode = kmode; p.lower = lower; p.batch = batch;
-    bool big = (M % 128 == 0 || epi == EPI_SUMSQ) && (N % 128 == 0) && N != 32 && M != 32;
+int gpe_gemm_routed(gpe_handle* h, cudaStream_t st, const GemmP& p, int layout, int epi, bool int8, const OzHint& hint, int cat) {
     cudaError_t e;
-    const bool reuse_a = h->oz_reuse_a;      // a request holds for one product only, whichever route it takes
-    const unsigned long long a_tag = h->oz_a_tag;
-    const double b_bound = h->oz_b_bound;
-    h->oz_reuse_a = false;
-    h->oz_a_tag = 0;
-    h->oz_b_bound = 0.0;
-    if (h->oz_nmod > 0 && M >= h->oz_min && N >= h->oz_min && K >= h->oz_min && oz_supported(p, epi)) {
-        // INT8 tensor-core route (gpe_ozaki.cuh): scratch is per stream; growing it is not allowed inside a capture, and
-        // every shape has been seen eagerly at least twice before its graph is captured
-        OzWs& ws = h->oz_ws[st];
-        ws.b_bound = b_bound;
+    if (int8) {
         struct HookCtx { gpe_handle* h; cudaEvent_t e0[3]; } hc{h, {nullptr, nullptr, nullptr}};
         OzHook hook;
         if (h->prof_on) {       // per-phase event pairs: residue conversion, residue GEMM, CRT
@@ -178,16 +169,13 @@ static int run_gemm(gpe_handle* h, cudaStream_t st, const double* A, const doubl
                 else x->h->prof_end(pc, x->e0[phase], s);
             };
         }
-        e = oz_gemm(p, layout, epi, h->oz_nmod, ws, st, reuse_a, a_tag, hook);
+        e = oz_gemm(p, layout, epi, h->oz_nmod, h->oz_ws[st], st, hint, hook);
         h->launches += 4;
         h->oz_calls++;
-        if (ws.grew) {          // (never during a capture: a shape is captured after it has run eagerly twice)
-            ws.grew = false;
-            h->graphs_stale = true;
-        }
         if (e != cudaSuccess) return h->fail("oz_gemm", e);
         return 0;
     }
+    const bool big = (p.M % 128 == 0 || epi == EPI_SUMSQ) && (p.N % 128 == 0) && p.N != 32 && p.M != 32;
     {
         ProfScope ps(h, cat >= 0 ? cat : (big ? gpe_handle::CAT_GEMM_BIG : gpe_handle::CAT_GEMM_SMALL), st);
         e = launch_gemm(p, layout, epi, st);
@@ -195,29 +183,6 @@ static int run_gemm(gpe_handle* h, cudaStream_t st, const double* A, const doubl
     h->launches++;
     if (e != cudaSuccess) return h->fail("launch_gemm", e);
     return 0;
-}
-// Can the INT8 route hold the scratch of product `p` on stream `st`?  Grows the scratch if it must; on an allocation failure the
-// error is cleared and the caller stays on the DMMA route (a prediction chunk over a very large training set).
-bool gpe_oz_reserve(gpe_handle* h, cudaStream_t st, const GemmP& p) {
-    OzWs& ws = h->oz_ws[st];
-    bool grew = false;
-    const cudaError_t e = oz_reserve(ws, p, h->oz_nmod, grew, false);
-    if (grew) { ws.have_a = false; ws.grew = true; }
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        return false;
-    }
-    return true;
-}
-int gpe_run_gemm_on(gpe_handle* h, cudaStream_t st, const double* A, const double* B, double* C, int lda, int ldb, int ldc,
-                    long long sA, long long sB, long long sC, int M, int N, int K, double alpha, int acc,
-                    int kmode, int lower, int batch, int layout, int epi) {
-    return run_gemm(h, st, A, B, C, lda, ldb, ldc, sA, sB, sC, M, N, K, alpha, acc, kmode, lower, batch, layout, epi);
-}
-int gpe_run_gemm(gpe_handle* h, const double* A, const double* B, double* C, int lda, int ldb, int ldc,
-                 long long sA, long long sB, long long sC, int M, int N, int K, double alpha, int acc,
-                 int kmode, int lower, int batch, int layout, int epi) {
-    return run_gemm(h, h->st, A, B, C, lda, ldb, ldc, sA, sB, sC, M, N, K, alpha, acc, kmode, lower, batch, layout, epi);
 }
 
 // Recursive Cholesky + triangular inverse of the diagonal block [off, off+m) of every item:
@@ -234,85 +199,115 @@ int gpe_handle::ensure_side(int g) {
     return 0;
 }
 
-static int potrf_inv_rec(gpe_handle* h, const FactorWs& ws, const SubBatch& sb, int off, int m, int want_L, int depth = 0) {
+// The four products of the recursion node [off, off + m) over the items of sb; its first half is [off, off + m1).
+struct NodeProducts {
+    int m1;
+    GemmP l21, t, syrk, li21;
+};
+static NodeProducts node_products(const FactorWs& ws, const SubBatch& sb, int off, int m) {
     const int ld = ws.npad, B = sb.B;
     const long long sM = (long long)ws.npad * ws.npad;
+    const int nb = m / NB;
+    const int m1 = ((nb + 1) / 2) * NB, m2 = m - m1;
     double* Ab = ws.A + (size_t)sb.b0 * sM;
     double* Sb = ws.S + (size_t)sb.b0 * sM;
     double* Lb = ws.Li + (size_t)sb.b0 * sM;
-    if (m == NB) {
-        {
-            ProfScope ps(h, gpe_handle::CAT_LEAF, sb.st);
-            launch_leaf(Ab, Lb, ld, sM, sM, off, ws.logdet_part + (size_t)sb.b0 * ws.nleaf, ws.nleaf, ws.status + sb.b0, B, sb.st,
-                        want_L ? Sb : nullptr);
-        }
-        h->launches++;
-        return 0;
-    }
-    const int nb = m / NB;
-    const int m1 = ((nb + 1) / 2) * NB, m2 = m - m1;
-    int rc;
-    if ((rc = potrf_inv_rec(h, ws, sb, off, m1, want_L, depth + 1))) return rc;
     double* A21 = Ab + (size_t)(off + m1) * ld + off;
     double* A22 = Ab + (size_t)(off + m1) * ld + off + m1;
     double* S21 = Sb + (size_t)(off + m1) * ld + off;
     double* Li11 = Lb + (size_t)off * ld + off;
     double* Li22 = Lb + (size_t)(off + m1) * ld + off + m1;
     double* Li21 = Lb + (size_t)(off + m1) * ld + off;
-    // L21 = A21 * Linv11^T           (NT, Linv11 lower: k <= j)
-    if ((rc = run_gemm(h, sb.st, A21, Li11, S21, ld, ld, ld, sM, sM, sM, m2, m1, m1, 1.0, 0, KM_LE_J, 0, B, 0))) return rc;
-    // T = L21 * Linv11  (NN, Linv11 lower: k >= j) -> dead A21 block.  It needs only L21 and Linv11, not the
-    // factorisation of A22: with side streams it is launched now, beside the SYRK and the whole A22 sub-recursion
-    // (whose leaves and small levels cannot fill the machine), and joined before the last product of the node.
-    // On the INT8 route the node's products run in order on one stream: L21 is converted to residues once, for the SYRK, and
-    // the planes serve T = L21 Linv11 right after it.
-    const bool oz_node = oz_takes(h, m2, m1, m1) && oz_takes(h, m2, m2, m1);
-    const bool fork = !oz_node && sb.side != nullptr && depth < gpe_handle::MAX_DEPTH;
+    return NodeProducts{
+        m1,
+        // L21 = A21 * Linv11^T           (NT, Linv11 lower: k <= j)
+        {.A = A21, .B = Li11, .C = S21, .lda = ld, .ldb = ld, .ldc = ld, .sA = sM, .sB = sM, .sC = sM, .M = m2, .N = m1, .K = m1,
+         .kmode = KM_LE_J, .batch = B},
+        // T = L21 * Linv11               (NN, Linv11 lower: k >= j) -> dead A21 block
+        {.A = S21, .B = Li11, .C = A21, .lda = ld, .ldb = ld, .ldc = ld, .sA = sM, .sB = sM, .sC = sM, .M = m2, .N = m1, .K = m1,
+         .kmode = KM_GE_J, .batch = B},
+        // A22 -= L21 * L21^T             (NT, SYRK, lower tiles)
+        {.A = S21, .B = S21, .C = A22, .lda = ld, .ldb = ld, .ldc = ld, .sA = sM, .sB = sM, .sC = sM, .M = m2, .N = m2, .K = m1,
+         .alpha = -1.0, .accumulate = 1, .lower = 1, .batch = B},
+        // Linv21 = -Linv22 * T           (NN, Linv22 lower: k <= i)
+        {.A = Li22, .B = A21, .C = Li21, .lda = ld, .ldb = ld, .ldc = ld, .sA = sM, .sB = sM, .sC = sM, .M = m2, .N = m1, .K = m2,
+         .alpha = -1.0, .kmode = KM_LE_I, .batch = B},
+    };
+}
+
+// On the INT8 route the node's products run in order on one stream: L21 is converted to residues once, for the SYRK, and the
+// planes serve T = L21 Linv11 right after it.
+static bool int8_node(const gpe_handle* h, const NodeProducts& nd) {
+    return int8_rule(h, nd.syrk, EPI_STORE) && int8_rule(h, nd.t, EPI_STORE);
+}
+
+static int potrf_inv_rec(gpe_handle* h, const FactorWs& ws, const SubBatch& sb, int off, int m, int want_L, int depth = 0) {
+    const int ld = ws.npad, B = sb.B;
+    const long long sM = (long long)ws.npad * ws.npad;
+    if (m == NB) {
+        {
+            ProfScope ps(h, gpe_handle::CAT_LEAF, sb.st);
+            launch_leaf(ws.A + (size_t)sb.b0 * sM, ws.Li + (size_t)sb.b0 * sM, ld, sM, sM, off, ws.logdet_part + (size_t)sb.b0 * ws.nleaf,
+                        ws.nleaf, ws.status + sb.b0, B, sb.st, want_L ? ws.S + (size_t)sb.b0 * sM : nullptr);
+        }
+        h->launches++;
+        return 0;
+    }
+    const NodeProducts nd = node_products(ws, sb, off, m);
+    int rc;
+    if ((rc = potrf_inv_rec(h, ws, sb, off, nd.m1, want_L, depth + 1))) return rc;
+    if ((rc = gpe_gemm(h, sb.st, nd.l21, GEMM_NT))) return rc;
+    // T needs only L21 and Linv11, not the factorisation of A22: with side streams it is launched now, beside the SYRK and the
+    // whole A22 sub-recursion (whose leaves and small levels cannot fill the machine), and joined before the last product.
+    const bool int8 = int8_node(h, nd);
+    const bool fork = !int8 && sb.side != nullptr && depth < gpe_handle::MAX_DEPTH;
     if (fork) {
         cudaStream_t side = sb.side[depth];
         cudaEventRecord(sb.ef[depth], sb.st);
         cudaStreamWaitEvent(side, sb.ef[depth], 0);
-        if ((rc = run_gemm(h, side, S21, Li11, A21, ld, ld, ld, sM, sM, sM, m2, m1, m1, 1.0, 0, KM_GE_J, 0, B, 1))) return rc;
+        if ((rc = gpe_gemm(h, side, nd.t, GEMM_NN))) return rc;
         cudaEventRecord(sb.ej[depth], side);
     }
-    // A22 -= L21 * L21^T             (SYRK, lower tiles)
-    if ((rc = run_gemm(h, sb.st, S21, S21, A22, ld, ld, ld, sM, sM, sM, m2, m2, m1, -1.0, 1, KM_FULL, 1, B, 0))) return rc;
-    if (oz_node) {
-        h->oz_reuse_a = true;
-        if ((rc = run_gemm(h, sb.st, S21, Li11, A21, ld, ld, ld, sM, sM, sM, m2, m1, m1, 1.0, 0, KM_GE_J, 0, B, 1))) return rc;
-    }
-    if ((rc = potrf_inv_rec(h, ws, sb, off + m1, m2, want_L, depth + 1))) return rc;
+    if ((rc = gpe_gemm(h, sb.st, nd.syrk, GEMM_NT))) return rc;
+    if (int8 && (rc = gpe_gemm(h, sb.st, nd.t, GEMM_NN, EPI_STORE, OzHint{.reuse_a = true}))) return rc;
+    if ((rc = potrf_inv_rec(h, ws, sb, off + nd.m1, m - nd.m1, want_L, depth + 1))) return rc;
     if (fork) {
         cudaStreamWaitEvent(sb.st, sb.ej[depth], 0);
-    } else if (!oz_node) {
-        if ((rc = run_gemm(h, sb.st, S21, Li11, A21, ld, ld, ld, sM, sM, sM, m2, m1, m1, 1.0, 0, KM_GE_J, 0, B, 1))) return rc;
+    } else if (!int8) {
+        if ((rc = gpe_gemm(h, sb.st, nd.t, GEMM_NN))) return rc;
     }
-    // Linv21 = -Linv22 * T           (NN, Linv22 lower: k <= i)
-    if ((rc = run_gemm(h, sb.st, Li22, A21, Li21, ld, ld, ld, sM, sM, sM, m2, m1, m2, -1.0, 0, KM_LE_I, 0, B, 1))) return rc;
-    return 0;
+    return gpe_gemm(h, sb.st, nd.li21, GEMM_NN);
 }
 int gpe_potrf_inv(gpe_handle* h, const FactorWs& ws, const SubBatch& sb, int want_L) { return potrf_inv_rec(h, ws, sb, 0, ws.npad, want_L); }
 
 static FactorWs handle_ws(gpe_handle* h) { return FactorWs{h->A, h->S, h->Li, h->npad, h->nleaf, h->logdet_part, h->status}; }
 
-// How the gradient reduction of a chunk is done (both routes sum the same terms, results agree to rounding).
-//   classic (false): A^-1 by the generic LAUUM GEMM, stored, then the stand-alone reduction kernel that recomputes E and
-//      U.U^T (round 1; still used for launches too small for 128x128 tiles, inputs too wide for the fused epilogue's shared
-//      memory, the Matérn family and the INT8 route).
-//   fused (true, when 128x128 tiles fill the machine): the reduction in LAUUM's epilogue (gpe_lauum_grad.cu); nothing
-//      of size n x n is written after the factorisation.
+// A^-1 = Linv^T Linv (lower tiles) of the items [b0, b0 + B) into their dead A buffers: LAUUM of the classic gradient route
+static GemmP lauum_product(const gpe_handle* h, int b0, int B) {
+    const int np = h->npad;
+    const long long sM = (long long)np * np;
+    const double* Lb = h->Li + (size_t)b0 * sM;
+    return GemmP{.A = Lb, .B = Lb, .C = h->A + (size_t)b0 * sM, .lda = np, .ldb = np, .ldc = np, .sA = sM, .sB = sM, .sC = sM,
+                 .M = np, .N = np, .K = np, .kmode = KM_GE_I, .lower = 1, .batch = B};
+}
+
+// How the gradient reduction of a likelihood chunk whose smallest group has B items is done (both routes sum the same terms,
+// results agree to rounding; one decision for the whole chunk: every group writes the same partial layout).
+//   classic: A^-1 by the generic LAUUM GEMM, stored, then the stand-alone reduction kernel that recomputes E and U.U^T (round 1;
+//      still used for launches too small to fill the machine with 128x128 tiles, inputs too wide for the fused epilogue's shared
+//      memory, the Matérn family and LOO, whose weight matrix is built from the stored A^-1).  With LAUUM on the INT8 route the
+//      reduction reads the covariance build's copy of exp(-D) instead (classic with E).
+//   fused: the reduction in LAUUM's epilogue (gpe_lauum_grad.cu); nothing of size n x n is written after the factorisation.
 // Measured on one B200 in one call, n = 4096, d = 16, 32 items, 8 streams, graph replay: 75.41 / 75.38 ms per step
 // for the classic / fused route, 73.9 ms with the reduction switched off altogether.  The reduction is scalar FP64 work on
 // the pipe the DMMAs use: fusing moves it, it does not remove it (DESIGN.md section 8).
-static bool llh_grad_fused(gpe_handle* h, int B) {
-    h->grad_use_e = false;
+static GradRoute grad_route(const gpe_handle* h, int mode, int B) {
+    const GemmP lauum = lauum_product(h, 0, B);
     // Matérn: the stand-alone reduction recomputes R and G (the LAUUM epilogue and the E copy are Gaussian-only)
-    if (h->family != FAMILY_GAUSSIAN || !gemm_is_big(h->npad, h->npad, 1, B)) return false;
-    if (h->oz_nmod > 0 && h->npad >= h->oz_min && h->npad % OZ_BN == 0) {   // LAUUM on the INT8 route, A^-1 stored: the stand-alone
-        h->grad_use_e = true;                                                // reduction reads the covariance build's copy of exp(-D)
-        return false;
-    }
-    return lauum_grad_supported(h->d);
+    if (h->family != FAMILY_GAUSSIAN || !gemm_fills_machine(lauum)) return GRAD_CLASSIC;
+    if (int8_rule(h, lauum, EPI_STORE)) return GRAD_CLASSIC_E;
+    if ((mode & GPE_MODE_LOO) || !lauum_grad_supported(h->d)) return GRAD_CLASSIC;
+    return GRAD_FUSED;
 }
 
 // LOO weight matrix of a GPE_MODE_LOO chunk (gpe_loo.cu): A^-1 (lower tiles, in A) -> W = F F^T - 1/2 [(P c) alpha^T +
@@ -333,20 +328,22 @@ static int loo_weights(gpe_handle* h, const SubBatch& sb, int mode) {
         launch_loo_f(Ab, sM, U, V, h->n, h->q, np, Sb, B, st);
     }
     h->launches += 2;
-    // P c = F (c / sqrt w)   (NN, skinny)
-    if ((rc = run_gemm(h, st, Sb, V, Pc, ld, NR, NR, sM, sP, sP, np, NR, np, 1.0, 0, KM_FULL, 0, B, 1))) return rc;
+    // P c = F (c / sqrt w)   (skinny)
+    if ((rc = gpe_gemm(h, st, {.A = Sb, .B = V, .C = Pc, .lda = ld, .ldb = NR, .ldc = NR, .sA = sM, .sB = sP, .sC = sP, .M = np, .N = NR,
+                               .K = np, .batch = B}, GEMM_NN))) return rc;
     {
         ProfScope ps(h, gpe_handle::CAT_OTHER, st);
         launch_loo_rank2(Pc, V, np, Ab, sM, B, st);
     }
     h->launches++;
-    // W += F F^T   (NT, lower tiles)
-    return run_gemm(h, st, Sb, Sb, Ab, ld, ld, ld, sM, sM, sM, np, np, np, 1.0, 1, KM_FULL, 1, B, 0);
+    // W += F F^T   (lower tiles)
+    return gpe_gemm(h, st, {.A = Sb, .B = Sb, .C = Ab, .lda = ld, .ldb = ld, .ldc = ld, .sA = sM, .sB = sM, .sC = sM, .M = np, .N = np,
+                            .K = np, .accumulate = 1, .lower = 1, .batch = B}, GEMM_NT);
 }
 
 // Everything after the covariance build for the items of `sb`, already described by h->par / h->winv.
-// with_grad = 0 stops after the GLS/likelihood scalars (fit_state path).
-int gpe_factor_and_reduce(gpe_handle* h, const SubBatch& sb, int mode, int with_grad, const double* beta_override, double* Kout) {
+// GRAD_NONE stops after the GLS/likelihood scalars (fit_state path).
+int gpe_factor_and_reduce(gpe_handle* h, const SubBatch& sb, int mode, GradRoute grad, const double* beta_override, double* Kout) {
     const int np = h->npad, ld = np, B = sb.B, b0 = sb.b0;
     const long long sM = (long long)np * np, sP = (long long)np * NR;
     const cudaStream_t st = sb.st;
@@ -358,7 +355,8 @@ int gpe_factor_and_reduce(gpe_handle* h, const SubBatch& sb, int mode, int with_
     int rc;
     if ((rc = potrf_inv_rec(h, handle_ws(h), sb, 0, np, 0))) return rc;
     // Wy = Linv [H | y]
-    if ((rc = run_gemm(h, st, Lb, h->HY, Wy, ld, NR, NR, sM, 0, sP, np, NR, np, 1.0, 0, KM_LE_I, 0, B, 1))) return rc;
+    if ((rc = gpe_gemm(h, st, {.A = Lb, .B = h->HY, .C = Wy, .lda = ld, .ldb = NR, .ldc = NR, .sA = sM, .sC = sP, .M = np, .N = NR,
+                               .K = np, .kmode = KM_LE_I, .batch = B}, GEMM_NN))) return rc;
     {
         ProfScope ps(h, gpe_handle::CAT_OTHER, st);
         launch_gram(Wy, np, B, GP, st);
@@ -367,9 +365,10 @@ int gpe_factor_and_reduce(gpe_handle* h, const SubBatch& sb, int mode, int with_
     }
     h->launches += 2;
     // U = Linv^T Z = [A^-1 H K^-T | sqrt(f) A^-1 (y - H beta)]
-    if ((rc = run_gemm(h, st, Lb, Z, U, ld, NR, NR, sM, sP, sP, np, NR, np, 1.0, 0, KM_GE_I, 0, B, 2))) return rc;
-    if (!with_grad) return 0;
-    if (h->grad_fused) {
+    if ((rc = gpe_gemm(h, st, {.A = Lb, .B = Z, .C = U, .lda = ld, .ldb = NR, .ldc = NR, .sA = sM, .sB = sP, .sC = sP, .M = np, .N = NR,
+                               .K = np, .kmode = KM_GE_I, .batch = B}, GEMM_TN))) return rc;
+    if (grad == GRAD_NONE) return 0;
+    if (grad == GRAD_FUSED) {
         // LAUUM with the gradient reduction in its epilogue: W = A^-1 - U U^T never leaves the CTA that computed it
         // (gpe_lauum_grad.cu).  Wy and Z are dead by now and hold U^T and -U^T.
         ProfScope ps(h, gpe_handle::CAT_LAUUM, st);
@@ -380,10 +379,8 @@ int gpe_factor_and_reduce(gpe_handle* h, const SubBatch& sb, int mode, int with_
         if (e != cudaSuccess) return h->fail("launch_lauum_grad", e);
         return 0;
     }
-    // small launches (64x64 tiles) and very wide inputs: A^-1 = Linv^T Linv (lower tiles) into the dead A buffer, then
-    // the stand-alone reduction kernel
-    if ((rc = run_gemm(h, st, Lb, Lb, Ab, ld, ld, ld, sM, sM, sM, np, np, np, 1.0, 0, KM_GE_I, 1, B, 2, EPI_STORE,
-                       gpe_handle::CAT_LAUUM))) return rc;
+    // classic route: A^-1 into the dead A buffer, then the stand-alone reduction kernel
+    if ((rc = gpe_gemm(h, st, lauum_product(h, b0, B), GEMM_TN, EPI_STORE, OzHint(), gpe_handle::CAT_LAUUM))) return rc;
     // LOO: the weight matrix replaces A^-1 and carries the whole of W, so no column of U is subtracted
     const bool loo = mode & GPE_MODE_LOO;
     if (loo && (rc = loo_weights(h, sb, mode))) return rc;
@@ -391,7 +388,7 @@ int gpe_factor_and_reduce(gpe_handle* h, const SubBatch& sb, int mode, int with_
         ProfScope ps(h, gpe_handle::CAT_GRAD, st);
         launch_grad_partial(h->X, h->r, h->n, h->d, np, h->winv + (size_t)b0 * h->d, Ab, sM, U, loo ? 0 : h->q + 1,
                             h->gpart + (size_t)b0 * grad_ntiles(np) * grad_nvals(h->d), B, st,
-                            h->grad_use_e ? h->Ex + (size_t)b0 * sM : nullptr, h->family);
+                            grad == GRAD_CLASSIC_E ? h->Ex + (size_t)b0 * sM : nullptr, h->family);
     }
     h->launches++;
     return 0;
@@ -693,12 +690,9 @@ static int enqueue_llh_chunk(gpe_handle* h, int Bs, int p, int mode, double fixe
         group_npad_graph = e ? atoi(e) : 512;
     }
     int ns = h->npad < (capturing ? group_npad_graph : group_npad) ? 1 : std::max(1, std::min(h->nsub, Bs / 2));
-    if (oz_takes(h, h->npad / 2, h->npad / 2, h->npad / 2)) ns = std::min(ns, h->oz_nsub);   // the top level runs on the INT8 route
-    // one decision for the whole chunk (every group writes the same partial layout): the smallest group must still
-    // fill the machine with 128x128 tiles.  A LOO chunk always takes the classic route: its weight matrix is built from
-    // the stored A^-1.
-    const bool loo = mode & GPE_MODE_LOO;
-    h->grad_fused = llh_grad_fused(h, Bs / ns) && !loo;
+    if (int8_node(h, node_products(handle_ws(h), SubBatch{0, Bs, h->st}, 0, h->npad)))    // the top level runs on the INT8 route
+        ns = std::min(ns, h->oz_nsub);
+    const GradRoute grad = grad_route(h, mode, Bs / ns);
     if (ns > 1) CK(cudaEventRecord(h->ev_fork, h->st));
     for (int g = 0; g < ns; g++) {
         SubBatch sb;
@@ -714,21 +708,21 @@ static int enqueue_llh_chunk(gpe_handle* h, int Bs, int p, int mode, double fixe
             ProfScope ps(h, gpe_handle::CAT_COV, sb.st);
             CK(launch_cov_build(h->X, h->r, h->n, h->d, h->npad, h->par + sb.b0, h->winv + (size_t)sb.b0 * h->d,
                                 h->A + (size_t)sb.b0 * sM, sM, sb.B, 0, sb.st, 0, 0,
-                                (h->grad_fused || h->grad_use_e) ? h->Ex + (size_t)sb.b0 * sM : nullptr, h->family));
+                                (grad == GRAD_FUSED || grad == GRAD_CLASSIC_E) ? h->Ex + (size_t)sb.b0 * sM : nullptr, h->family));
         }
         h->launches++;
-        if ((rc = gpe_factor_and_reduce(h, sb, mode, 1, nullptr, nullptr))) return rc;
+        if ((rc = gpe_factor_and_reduce(h, sb, mode, grad, nullptr, nullptr))) return rc;
         if (ns > 1) {
             CK(cudaEventRecord(h->ev_join[g], sb.st));
             CK(cudaStreamWaitEvent(h->st, h->ev_join[g], 0));
         }
     }
-    if (loo) {
+    if (mode & GPE_MODE_LOO) {
         ProfScope ps(h, gpe_handle::CAT_OTHER);
         launch_loo_finalize(h->gpart, grad_ntiles(h->npad), h->d, p, mode, h->par, h->out, h->llh_d, h->grad_d, h->sig_d, Bs, h->st);
     } else {
         ProfScope ps(h, gpe_handle::CAT_OTHER);
-        launch_grad_finalize(h->gpart, h->grad_fused ? lauum_grad_ntiles(h->npad) : grad_ntiles(h->npad), h->n, h->d, h->npad, p, mode,
+        launch_grad_finalize(h->gpart, grad == GRAD_FUSED ? lauum_grad_ntiles(h->npad) : grad_ntiles(h->npad), h->n, h->d, h->npad, p, mode,
                              h->par, h->out, h->status, h->llh_d, h->grad_d,
                              h->sig_d, Bs, h->st);
     }
@@ -808,7 +802,8 @@ int gpe_dbg_gemm(gpe_handle* h, const double* A, const double* B, double* C, int
                  int kmode, int lower, int batch, int layout) {
     if (!h) return -2;
     CK(cudaSetDevice(h->device));
-    int rc = run_gemm(h, h->st, A, B, C, lda, ldb, ldc, sA, sB, sC, M, N, K, alpha, accumulate, kmode, lower, batch, layout);
+    int rc = gpe_gemm(h, h->st, {.A = A, .B = B, .C = C, .lda = lda, .ldb = ldb, .ldc = ldc, .sA = sA, .sB = sB, .sC = sC, .M = M, .N = N,
+                                 .K = K, .alpha = alpha, .accumulate = accumulate, .kmode = kmode, .lower = lower, .batch = batch}, layout);
     if (rc) return rc;
     CK(cudaStreamSynchronize(h->st));
     return 0;
@@ -820,15 +815,14 @@ int gpe_dbg_gemm_oz(gpe_handle* h, const double* A, const double* B, double* C, 
                     unsigned char* planesB, unsigned char* planesD, int* sexpA, int* sexpB) {
     if (!h) return -2;
     CK(cudaSetDevice(h->device));
-    GemmP p;
-    p.A = A; p.B = B; p.C = C; p.lda = lda; p.ldb = ldb; p.ldc = ldc; p.sA = sA; p.sB = sB; p.sC = sC;
-    p.M = M; p.N = N; p.K = K; p.alpha = alpha; p.accumulate = accumulate; p.kmode = kmode; p.lower = lower; p.batch = batch;
+    const GemmP p{.A = A, .B = B, .C = C, .lda = lda, .ldb = ldb, .ldc = ldc, .sA = sA, .sB = sB, .sC = sC, .M = M, .N = N, .K = K,
+                  .alpha = alpha, .accumulate = accumulate, .kmode = kmode, .lower = lower, .batch = batch};
     if (!oz_supported(p, EPI_STORE)) return h->fail_msg("gpe_dbg_gemm_oz: shape not supported by the INT8 route");
     OzWs& ws = h->oz_ws[h->st];
     cudaError_t e = oz_gemm(p, layout, EPI_STORE, nmod, ws, h->st);
     if (e != cudaSuccess) return h->fail("oz_gemm", e);
     CK(cudaStreamSynchronize(h->st));
-    const bool same = (A == B && lda == ldb && sA == sB && M == N && layout != 1);
+    const bool same = (A == B && lda == ldb && sA == sB && M == N && layout != GEMM_NN);
     const size_t nA = (size_t)batch * nmod * M * K, nB = (size_t)batch * nmod * N * K, nD = (size_t)batch * nmod * M * N;
     if (planesA) CK(cudaMemcpy(planesA, ws.PA, nA, cudaMemcpyDefault));
     if (planesB) CK(cudaMemcpy(planesB, same ? ws.PA : ws.PB, nB, cudaMemcpyDefault));

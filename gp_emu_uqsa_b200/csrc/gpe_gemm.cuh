@@ -30,18 +30,25 @@ enum Epi : int {
     EPI_SUMSQ = 1,  // part[b][ti][col] = sum_rows acc^2   (column norms of Z = L^-1 C)
 };
 
+// How the operands of launch_gemm are stored: A [M][K] or, transposed, [K][M]; B [N][K] or, not transposed, [K][N].
+enum Layout : int {
+    GEMM_NT = 0,  // C = A B^T   (A [M][K], B [N][K]: both K-contiguous)
+    GEMM_NN = 1,  // C = A B     (A [M][K], B [K][N])
+    GEMM_TN = 2,  // C = A^T B   (A [K][M], B [K][N])
+};
+
 struct GemmP {
     const double* A;
     const double* B;
     double* C;          // EPI_SUMSQ: partial buffer [batch][tiles_m][N]
     int lda, ldb, ldc;  // leading dimensions (elements)
-    long long sA, sB, sC;  // batch strides (elements)
+    long long sA = 0, sB = 0, sC = 0;  // batch strides (elements)
     int M, N, K;
-    double alpha;
-    int accumulate;  // 1: C += alpha*acc
-    int kmode;
-    int lower;  // 1: skip tiles strictly above the diagonal (square C)
-    int batch;
+    double alpha = 1.0;
+    int accumulate = 0;  // 1: C += alpha*acc
+    int kmode = KM_FULL;
+    int lower = 0;  // 1: skip tiles strictly above the diagonal (square C)
+    int batch = 1;
 };
 
 constexpr int GEMM_BK = 16;
@@ -714,9 +721,11 @@ inline cudaError_t launch_gemm_ws2(const GemmP& p, cudaStream_t st) {
     return launch_gemm_ws2_shape<A_KC, B_KC, EPI, 2>(p, st);
 }
 
-// Layout ids: 0 = (A_KC,B_KC) "NT", 1 = (A_KC,!B_KC) "NN", 2 = (!A_KC,!B_KC) "TN".
+// Layouts: GEMM_NT = (A_KC,B_KC), GEMM_NN = (A_KC,!B_KC), GEMM_TN = (!A_KC,!B_KC).
 // Tile choice: 128x64 tiles, two CTAs per SM, when 128x128 tiles still fill the machine, else 64x64 (or 32x32);
 // N == 32 panels use 128x32.  Column norms (EPI_SUMSQ) take the 128x64 kernel, or the 128x128 one for a ragged M.
 cudaError_t launch_gemm(const GemmP& p, int layout, int epi, cudaStream_t st);
+// does an EPI_STORE product take the two-CTAs-per-SM kernel, i.e. do 128x128 tiles fill the machine?
+bool gemm_fills_machine(const GemmP& p);
 
 }  // namespace gpe

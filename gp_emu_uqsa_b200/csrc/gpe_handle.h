@@ -61,8 +61,6 @@ struct gpe_handle {
     // batched likelihood workspace
     int Bcap = 0;
     bool Bcap_final = false;     // the workspace already has the largest size obtainable (env cap or device memory)
-    bool grad_use_e = false;     // classic route with the covariance build's copy of exp(-D) (INT8 route)
-    bool grad_fused = false;     // gradient route of the current chunk (gpe_api.cu:llh_grad_fused): LAUUM epilogue or classic
     double *A = nullptr, *S = nullptr, *Li = nullptr;        // [Bcap][npad][npad]
     double* Ex = nullptr;                                    // [Bcap][npad][npad] exp(-D) kept by the covariance build for the fused gradient epilogue
     double *Wy = nullptr, *Z = nullptr, *U = nullptr;        // [Bcap][npad][NR]
@@ -97,9 +95,7 @@ struct gpe_handle {
     int oz_nmod = 16, oz_min = 1024, oz_nsub = 2;
     std::map<cudaStream_t, gpe::OzWs> oz_ws;
     long long oz_calls = 0;
-    unsigned long long oz_a_tag = 0, fit_gen = 0;   // tag of operand A for the next product; generation of the fit state
-    double oz_b_bound = 0.0;     // the next product's operand B is bounded by this in magnitude (0: unknown; one product only)
-    bool oz_reuse_a = false;     // the next product may use the residue planes of operand A left by the previous one
+    unsigned long long fit_gen = 0;   // generation of the fit state (tags the prediction product's residue planes of L^-1)
 
     int fail(const char* what, cudaError_t e);
     int fail_msg(const char* what);
@@ -161,12 +157,21 @@ struct NvtxRange {
 bool gpe_is_device_ptr(const void* p);
 int gpe_ensure_batch_ws(gpe_handle* h, int B);
 int gpe_potrf_inv(gpe_handle* h, const FactorWs& ws, const SubBatch& sb, int want_L);
-int gpe_factor_and_reduce(gpe_handle* h, const SubBatch& sb, int mode, int with_grad, const double* beta_override, double* Kout);
+// How the likelihood gradient of a chunk is reduced (gpe_api.cu:grad_route): not at all (fit state), in the LAUUM epilogue, or by
+// the stand-alone reduction kernel after A^-1 is stored, recomputing exp(-D) or reading the covariance build's copy of it.
+enum GradRoute { GRAD_NONE, GRAD_FUSED, GRAD_CLASSIC, GRAD_CLASSIC_E };
+int gpe_factor_and_reduce(gpe_handle* h, const SubBatch& sb, int mode, GradRoute grad, const double* beta_override, double* Kout);
 int gpe_upload_single_par(gpe_handle* h, const double* delta, double nugget, int kind, int predict, double s2_for_r);
-bool gpe_oz_reserve(gpe_handle* h, cudaStream_t st, const gpe::GemmP& p);
-int gpe_run_gemm_on(gpe_handle* h, cudaStream_t st, const double* A, const double* B, double* C, int lda, int ldb, int ldc,
-                    long long sA, long long sB, long long sC, int M, int N, int K, double alpha, int acc,
-                    int kmode, int lower, int batch, int layout, int epi);
-int gpe_run_gemm(gpe_handle* h, const double* A, const double* B, double* C, int lda, int ldb, int ldc,
-                 long long sA, long long sB, long long sC, int M, int N, int K, double alpha, int acc,
-                 int kmode, int lower, int batch, int layout, int epi);
+// Does product p take the INT8 route on stream st?  Yes when its shape does (route on, every dimension >= oz_min, supported) and
+// the stream's residue scratch can hold it; the scratch is grown here, and on an allocation failure the error is cleared and the
+// product stays on DMMA.
+bool gpe_int8_route(gpe_handle* h, cudaStream_t st, const gpe::GemmP& p, int layout, int epi);
+// C = alpha op(A) op(B) (+ C) on the route int8 names, which a caller that plans around the route (the prediction chunk) has
+// taken from gpe_int8_route, once.  cat: profile category of a DMMA launch (-1: by shape).
+int gpe_gemm_routed(gpe_handle* h, cudaStream_t st, const gpe::GemmP& p, int layout, int epi, bool int8, const gpe::OzHint& hint,
+                    int cat = -1);
+// Every other dense product: the same on the route gpe_int8_route picks.
+inline int gpe_gemm(gpe_handle* h, cudaStream_t st, const gpe::GemmP& p, int layout, int epi = gpe::EPI_STORE,
+                    const gpe::OzHint& hint = gpe::OzHint(), int cat = -1) {
+    return gpe_gemm_routed(h, st, p, layout, epi, gpe_int8_route(h, st, p, layout, epi), hint, cat);
+}

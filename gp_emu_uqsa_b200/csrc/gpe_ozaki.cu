@@ -839,16 +839,17 @@ bool oz_sumsq_swapped(const GemmP& p, int epi) {
 }
 
 static bool same_operand(const GemmP& p, int layout) {
-    return p.A == p.B && p.lda == p.ldb && p.sA == p.sB && p.M == p.N && layout != 1;
+    return p.A == p.B && p.lda == p.ldb && p.sA == p.sB && p.M == p.N && layout != GEMM_NN;
 }
 
-cudaError_t oz_reserve(OzWs& ws, const GemmP& p, int nmod, bool& grew, bool same) {
-    grew = false;
+cudaError_t oz_reserve(OzWs& ws, const GemmP& p, int layout, int nmod) {
+    const bool same = same_operand(p, layout);
     const size_t needA = (size_t)p.batch * nmod * p.M * p.K, needB = same ? 0 : (size_t)p.batch * nmod * p.N * p.K;
     const size_t needD = (size_t)p.batch * nmod * p.M * p.N, needS = (size_t)p.batch * (size_t)(p.M > p.N ? p.M : p.N);
+    auto grown = [&]() { ws.have_a = false; ws.grew = true; };
     auto grow = [&](uint8_t*& ptr, size_t& cap, size_t need) -> cudaError_t {
         if (need <= cap) return cudaSuccess;
-        grew = true;
+        grown();
         if (ptr) cudaFree(ptr);
         ptr = nullptr;
         cap = 0;
@@ -861,7 +862,7 @@ cudaError_t oz_reserve(OzWs& ws, const GemmP& p, int nmod, bool& grew, bool same
     if ((e = grow(ws.PB, ws.capB, needB)) != cudaSuccess) return e;
     if ((e = grow(ws.PD, ws.capD, needD)) != cudaSuccess) return e;
     if (needS > ws.capS) {
-        grew = true;
+        grown();
         cudaFree(ws.sA); cudaFree(ws.sB);
         ws.sA = ws.sB = nullptr;
         ws.capS = 0;
@@ -916,8 +917,7 @@ static cudaError_t launch_convert(bool kc, const double* src, int ld, long long 
     return cudaGetLastError();
 }
 
-cudaError_t oz_gemm(const GemmP& p, int layout, int epi, int nmod, OzWs& ws, cudaStream_t st, bool reuse_a, unsigned long long a_tag,
-                    const OzHook& hook) {
+cudaError_t oz_gemm(const GemmP& p, int layout, int epi, int nmod, OzWs& ws, cudaStream_t st, const OzHint& hint, const OzHook& hook) {
     if (nmod < 2 || nmod > OZ_MAXMOD || !oz_supported(p, epi)) return cudaErrorInvalidValue;
     cudaError_t e;
     if ((e = upload_const()) != cudaSuccess) return e;
@@ -929,13 +929,10 @@ cudaError_t oz_gemm(const GemmP& p, int layout, int epi, int nmod, OzWs& ws, cud
         std::lock_guard<std::mutex> lk(crt_mu);
         if (!have_crt[nmod]) { crt[nmod] = make_crt(nmod); have_crt[nmod] = true; }
     }
-    bool grew;
     const bool same = same_operand(p, layout);
-    struct BoundReset { OzWs& w; ~BoundReset() { w.b_bound = 0.0; } } bound_reset{ws};
-    if ((e = oz_reserve(ws, p, nmod, grew, same)) != cudaSuccess) return e;
-    if (grew) { ws.have_a = false; ws.grew = true; }
+    if ((e = oz_reserve(ws, p, layout, nmod)) != cudaSuccess) return e;
     const int bits = oz_operand_bits(nmod, p.K);
-    const bool a_kc = layout != 2, b_kc = layout == 0;
+    const bool a_kc = layout != GEMM_TN, b_kc = layout == GEMM_NT;
     // column norms of Z = A B with A lower triangular (prediction): run as Z^T = B^T A^T, the triangular factor on the column side
     const bool swap = oz_sumsq_swapped(p, epi);
     // cluster size of the residue GEMM: pairs wherever the row tiles pair up.  Quadruples cut the L2 -> SM traffic further (24
@@ -951,17 +948,17 @@ cudaError_t oz_gemm(const GemmP& p, int layout, int epi, int nmod, OzWs& ws, cud
     const int triB = p.kmode == KM_LE_J ? OZ_BN : (p.kmode == KM_GE_J ? -OZ_BN : 0);
     hook(0, true, st);
     const OzWs::Key keyA{p.A, p.lda, p.sA, p.M, p.K, p.batch, nmod, bits, triA, a_kc ? 1 : 0};
-    if (!(reuse_a && ws.have_a && ws.key_a == keyA && ws.tag_a == a_tag)) {
+    if (!(hint.reuse_a && ws.have_a && ws.key_a == keyA && ws.tag_a == hint.a_tag)) {
         if ((e = launch_convert(a_kc, p.A, p.lda, p.sA, p.M, p.K, nmod, bits, triA, ws.PA, ws.sA, p.batch, st)) != cudaSuccess) return e;
     }
     ws.key_a = keyA;
-    ws.tag_a = a_tag;
+    ws.tag_a = hint.a_tag;
     ws.have_a = true;
     const uint8_t* PBp = ws.PA;
     const int* sBp = ws.sA;
     if (!same) {
-        const double b_bound = ws.b_bound;      // one-shot: the caller's bound on |B| (0: none)
-        if ((e = launch_convert(b_kc, p.B, p.ldb, p.sB, p.N, p.K, nmod, bits, triB, ws.PB, ws.sB, p.batch, st, b_bound)) != cudaSuccess) return e;
+        if ((e = launch_convert(b_kc, p.B, p.ldb, p.sB, p.N, p.K, nmod, bits, triB, ws.PB, ws.sB, p.batch, st, hint.b_bound)) != cudaSuccess)
+            return e;
         PBp = ws.PB;
         sBp = ws.sB;
     }

@@ -41,10 +41,17 @@ struct OzWs {
     Key key_a{};
     unsigned long long tag_a = 0; // caller's generation of the source (0: none)
     bool have_a = false;
-    double b_bound = 0.0;        // set before a call: |B| <= b_bound everywhere, so operand B takes one scale and its maxima are not
-                                 // searched (holds for that call only)
     bool grew = false;           // set when a buffer was reallocated: captured graphs that used the old one are stale
     void release();
+};
+
+// What the caller of one product knows about its operands (all zero: nothing).
+struct OzHint {
+    // the planes of operand A left on this stream by the previous product may be used again if they describe the same operand
+    // and carry the same tag (the caller vouches that the source has not changed)
+    bool reuse_a = false;
+    unsigned long long a_tag = 0;
+    double b_bound = 0.0;        // |B| <= b_bound everywhere: operand B takes one scale and its maxima are not searched
 };
 
 bool oz_supported(const GemmP& p, int epi);
@@ -60,12 +67,11 @@ struct OzHook {
 // column norms (EPI_SUMSQ, k <= i) evaluated with the roles swapped -- Z^T = B^T A^T, row norms: the output is then ONE row of
 // partial sums, C[0 .. N), instead of M / 128 rows
 bool oz_sumsq_swapped(const GemmP& p, int epi);
-// makes sure `ws` can hold the planes of `p` (allocates: must not be called during stream capture when it has to grow)
-cudaError_t oz_reserve(OzWs& ws, const GemmP& p, int nmod, bool& grew, bool same_operand);
+// makes sure `ws` can hold the planes of `p` (allocates: must not be called during stream capture when it has to grow); a
+// reallocation sets ws.grew and forgets the planes of operand A
+cudaError_t oz_reserve(OzWs& ws, const GemmP& p, int layout, int nmod);
 // C = alpha op(A) op(B) (+ C), same meaning of every field of p, of `layout` and of `epi` as launch_gemm (EPI_SUMSQ: batch 1).
-// reuse_a: the planes of operand A left on this stream by the previous call may be used again if they describe the same
-// operand and carry the same caller tag (the caller vouches that the source has not changed)
-cudaError_t oz_gemm(const GemmP& p, int layout, int epi, int nmod, OzWs& ws, cudaStream_t st, bool reuse_a = false,
-                    unsigned long long a_tag = 0, const OzHook& hook = OzHook());
+cudaError_t oz_gemm(const GemmP& p, int layout, int epi, int nmod, OzWs& ws, cudaStream_t st, const OzHint& hint = OzHint(),
+                    const OzHook& hook = OzHook());
 
 }  // namespace gpe

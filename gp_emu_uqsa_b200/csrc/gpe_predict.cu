@@ -637,31 +637,28 @@ int predict_chunk(gpe_handle* h, gpe_handle::PredSlot& sl, cudaStream_t st, cons
     // triangular product has 80 live rows, not 128)
     const int kp = std::min(np, (h->n + GEMM_BK - 1) / GEMM_BK * GEMM_BK);
     const int maux = (h->q + 1 <= 16) ? 16 : NR;
-    if ((rc = gpe_run_gemm_on(h, st, h->fE, sl.C, sl.Aux, NR, mc, mc, 0, 0, 0, maux, mc, kp, 1.0, 0, KM_FULL, 0, 1, 2, EPI_STORE))) return rc;
+    if ((rc = gpe_gemm(h, st, {.A = h->fE, .B = sl.C, .C = sl.Aux, .lda = NR, .ldb = mc, .ldc = mc, .M = maux, .N = mc, .K = kp}, GEMM_TN)))
+        return rc;
     int ntile = 0;
     if (var_dev != nullptr || imp != nullptr) {
-        // column norms of Z = Linv C    (NN, Linv lower: k <= i), reduced in the epilogue
-        int mp = kp;
-        // INT8 tensor-core route (gpe_ozaki.cuh) for chunks it supports: the residue planes of L^-1 are made once per fit and
-        // stream (the tag is the generation of the fit state), the padded size is used (rows >= n of Z are zero)
+        // column norms of Z = Linv C    (Linv lower: k <= i), reduced in the epilogue
+        GemmP z{.A = h->fLi, .B = sl.C, .C = sl.Part, .lda = np, .ldb = mc, .ldc = mc, .M = np, .N = mc, .K = np, .kmode = KM_LE_I};
+        OzHint hint;
         bool one_row = false;
-        if (h->oz_nmod > 0 && np >= h->oz_min && mc >= h->oz_min) {
-            GemmP p;
-            p.A = h->fLi; p.B = sl.C; p.C = sl.Part; p.lda = np; p.ldb = mc; p.ldc = mc; p.sA = p.sB = p.sC = 0;
-            p.M = np; p.N = mc; p.K = np; p.alpha = 1.0; p.accumulate = 0; p.kmode = KM_LE_I; p.lower = 0; p.batch = 1;
-            if (oz_supported(p, EPI_SUMSQ) && gpe_oz_reserve(h, st, p)) {
-                mp = np;
-                h->oz_reuse_a = true;
-                h->oz_a_tag = h->fit_gen;
-                // every entry of the slab is c exp(-D) or c R(D), in [0, c]: one scale for all points, no pass over the slab for its maxima.
-                // (A point far from every training input then keeps fewer significant bits of its tiny column -- its variance
-                // is the prior's to the same absolute accuracy, which is what the subtraction prior - |Z|^2 needs.)
-                h->oz_b_bound = h->fit_c;
-                one_row = oz_sumsq_swapped(p, EPI_SUMSQ);
-            }
+        const bool int8 = gpe_int8_route(h, st, z, GEMM_NN, EPI_SUMSQ);      // decided once: the plan below is the route taken
+        if (int8) {
+            // INT8 tensor-core route (gpe_ozaki.cuh): the residue planes of L^-1 are made once per fit and stream (the tag is the
+            // generation of the fit state), the padded size is used (rows >= n of Z are zero).  Every entry of the slab is
+            // c exp(-D) or c R(D), in [0, c]: one scale for all points, no pass over the slab for its maxima.  (A point far from
+            // every training input then keeps fewer significant bits of its tiny column -- its variance is the prior's to the same
+            // absolute accuracy, which is what the subtraction prior - |Z|^2 needs.)
+            hint = OzHint{.reuse_a = true, .a_tag = h->fit_gen, .b_bound = h->fit_c};
+            one_row = oz_sumsq_swapped(z, EPI_SUMSQ);
+        } else {
+            z.M = z.K = kp;
         }
-        if ((rc = gpe_run_gemm_on(h, st, h->fLi, sl.C, sl.Part, np, mc, mc, 0, 0, 0, mp, mc, mp, 1.0, 0, KM_LE_I, 0, 1, 1, EPI_SUMSQ))) return rc;
-        ntile = one_row ? 1 : (mp + 127) / 128;
+        if ((rc = gpe_gemm_routed(h, st, z, GEMM_NN, EPI_SUMSQ, int8, hint))) return rc;
+        ntile = one_row ? 1 : (z.M + 127) / 128;
     }
     {
         ProfScope ps(h, gpe_handle::CAT_OTHER, st);
@@ -712,7 +709,7 @@ int gpe_fit_state(gpe_handle* h, const double* delta, double nugget, double sigm
     CK(cudaMemsetAsync(h->fK, 0, sizeof(double) * NR * NR, h->st));
     CK(cudaMemsetAsync(h->status, 0, sizeof(int), h->st));
     SubBatch sb{0, 1, h->st};
-    if ((rc = gpe_factor_and_reduce(h, sb, 0, 0, bov, h->fK))) return rc;
+    if ((rc = gpe_factor_and_reduce(h, sb, 0, GRAD_NONE, bov, h->fK))) return rc;
     CK(cudaMemcpyAsync(h->fLi, h->Li, (size_t)np * np * sizeof(double), cudaMemcpyDeviceToDevice, h->st));
     CK(cudaMemcpyAsync(h->fE, h->U, (size_t)np * NR * sizeof(double), cudaMemcpyDeviceToDevice, h->st));
     CK(cudaMemcpyAsync(h->fwinv, h->winv, (size_t)h->d * sizeof(double), cudaMemcpyDeviceToDevice, h->st));
@@ -989,9 +986,11 @@ int gpe_predict_fullcov(gpe_handle* h, const double* Xs, const double* Hs, int m
     CK(launch_xcov(h->family, h->fXs, P, h->fwinv, h->n, d, np, mp, m, h->fit_c, Cm, mp, h->st));
     h->launches++;
     int rc = 0;
-    if (!rc) rc = gpe_run_gemm(h, h->fE, Cm, aux, NR, mp, mp, 0, 0, 0, NR, mp, np, 1.0, 0, KM_FULL, 0, 1, 2, EPI_STORE);
-    if (!rc) rc = gpe_run_gemm(h, h->fLi, Cm, Zm, np, mp, mp, 0, 0, 0, np, mp, np, 1.0, 0, KM_LE_I, 0, 1, 1, EPI_STORE);
-    if (!rc) rc = gpe_run_gemm(h, Zm, Zm, ZtZ, mp, mp, mp, 0, 0, 0, mp, mp, np, 1.0, 0, KM_FULL, 0, 1, 2, EPI_STORE);
+    if (!rc) rc = gpe_gemm(h, h->st, {.A = h->fE, .B = Cm, .C = aux, .lda = NR, .ldb = mp, .ldc = mp, .M = NR, .N = mp, .K = np}, GEMM_TN);
+    if (!rc)
+        rc = gpe_gemm(h, h->st, {.A = h->fLi, .B = Cm, .C = Zm, .lda = np, .ldb = mp, .ldc = mp, .M = np, .N = mp, .K = np, .kmode = KM_LE_I},
+                      GEMM_NN);
+    if (!rc) rc = gpe_gemm(h, h->st, {.A = Zm, .B = Zm, .C = ZtZ, .lda = mp, .ldb = mp, .ldc = mp, .M = mp, .N = mp, .K = np}, GEMM_TN);
     if (!rc) {
         BasisDesc bd = basis_of(h);
         double s2 = h->fit_sigma * h->fit_sigma;

@@ -222,7 +222,8 @@ int ensure_ainv(gpe_handle* h) {
     const int np = h->npad;
     if (!h->fAinv) CK(cudaMalloc((void**)&h->fAinv, (size_t)np * np * sizeof(double)));
     // LAUUM: A^-1 = Linv^T Linv, lower 128-tiles
-    int rc = gpe_run_gemm(h, h->fLi, h->fLi, h->fAinv, np, np, np, 0, 0, 0, np, np, np, 1.0, 0, KM_GE_I, 1, 1, 2, EPI_STORE);
+    int rc = gpe_gemm(h, h->st, {.A = h->fLi, .B = h->fLi, .C = h->fAinv, .lda = np, .ldb = np, .ldc = np, .M = np, .N = np, .K = np,
+                                 .kmode = KM_GE_I, .lower = 1}, GEMM_TN);
     if (rc) return rc;
     h->fAinv_valid = true;
     return 0;
@@ -255,8 +256,11 @@ int gpe_solve(gpe_handle* h, const double* Bm, int k, double* out) {
         pack_panel_kernel<<<(np * NR + 255) / 256, 256, 0, h->st>>>(src, n, kc, np, p0);
         h->launches++;
         // p1 = Linv p0 ; p2 = Linv^T p1   (A^-1 = L^-T L^-1)
-        rc = gpe_run_gemm(h, h->fLi, p0, p1, np, NR, NR, 0, 0, 0, np, NR, np, 1.0, 0, KM_LE_I, 0, 1, 1, EPI_STORE);
-        if (!rc) rc = gpe_run_gemm(h, h->fLi, p1, p2, np, NR, NR, 0, 0, 0, np, NR, np, 1.0, 0, KM_GE_I, 0, 1, 2, EPI_STORE);
+        rc = gpe_gemm(h, h->st, {.A = h->fLi, .B = p0, .C = p1, .lda = np, .ldb = NR, .ldc = NR, .M = np, .N = NR, .K = np, .kmode = KM_LE_I},
+                      GEMM_NN);
+        if (!rc)
+            rc = gpe_gemm(h, h->st, {.A = h->fLi, .B = p1, .C = p2, .lda = np, .ldb = NR, .ldc = NR, .M = np, .N = NR, .K = np, .kmode = KM_GE_I},
+                          GEMM_TN);
         if (rc) break;
         unpack_panel_kernel<<<(n * kc + 255) / 256, 256, 0, h->st>>>(p2, n, kc, dst);
         h->launches++;
@@ -304,7 +308,7 @@ int gpe_sens_contract(gpe_handle* h, const double* gamma, const double* acoef, c
     sens_pw_kernel<<<dim3(nt, nt), 256, smem, h->st>>>(h->X, n, d, np, coef, coef + d, coef + 2 * d, scale, h->fAinv, h->S, tpart);
     h->launches += 2;
     // Y = P Vp   (P dense [np,np] row-major; rows/cols >= n are zero because u = 0 there)
-    rc = gpe_run_gemm(h, h->S, Vp, Yp, np, NR, NR, 0, 0, 0, np, NR, np, 1.0, 0, KM_FULL, 0, 1, 1, EPI_STORE);
+    rc = gpe_gemm(h, h->st, {.A = h->S, .B = Vp, .C = Yp, .lda = np, .ldb = NR, .ldc = NR, .M = np, .N = NR, .K = np}, GEMM_NN);
     if (!rc) {
         sens_reduce_kernel<<<1, 1024, 0, h->st>>>(tpart, ntile, Vp, Yp, np, outd);
         h->launches++;
