@@ -44,11 +44,6 @@ void gpe_handle::prof_end(int cat, cudaEvent_t e0, cudaStream_t s) {
     cudaEventRecord(e1, s);
     prof_recs.push_back({cat, e0, e1});
 }
-#define CK(call)                                                   \
-    do {                                                           \
-        cudaError_t e__ = (call);                                  \
-        if (e__ != cudaSuccess) return h->fail(#call, e__);        \
-    } while (0)
 
 bool gpe_is_device_ptr(const void* p) {
     cudaPointerAttributes a;
@@ -57,16 +52,6 @@ bool gpe_is_device_ptr(const void* p) {
         return false;
     }
     return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
-}
-
-template <class T>
-static cudaError_t dev_alloc(T** p, size_t count) {
-    return cudaMalloc((void**)p, std::max<size_t>(count, 1) * sizeof(T));
-}
-template <class T>
-static void dev_free(T*& p) {
-    if (p) cudaFree(p);
-    p = nullptr;
 }
 
 void gpe_handle::drop_graphs() {
@@ -403,14 +388,34 @@ static void host_item_par(ItemPar& ip, double nugget, int kind, int predict, dou
     ip.s2A = s2A; ip.nugget = nugget; ip.sigma = std::sqrt(s2A); ip.pad_ = 0.0;
 }
 
-int gpe_upload_single_par(gpe_handle* h, const double* delta, double nugget, int kind, int predict, double s2_for_r) {
+int gpe_upload_single_par(gpe_handle* h, const double* delta, double nugget, int kind, int predict, double s2_for_r, std::optional<double> offs) {
     ItemPar ip;
     host_item_par(ip, nugget, kind, predict, s2_for_r, 1.0);
-    std::vector<double> w(h->d);
-    for (int k = 0; k < h->d; k++) w[k] = 1.0 / delta[k];
+    if (offs) ip.offs = *offs;
+    std::vector<double> w;
+    CK(read_small(w, delta, h->d));
+    for (double& v : w) v = 1.0 / v;
     CK(cudaMemcpyAsync(h->par, &ip, sizeof ip, cudaMemcpyHostToDevice, h->st));
     CK(cudaMemcpyAsync(h->winv, w.data(), sizeof(double) * h->d, cudaMemcpyHostToDevice, h->st));
     CK(cudaStreamSynchronize(h->st));   // host vectors go out of scope
+    return 0;
+}
+
+// The covariance matrix of the training inputs (build 0), or its derivative by delta_which (1) or the nugget (2), into out [n,n]
+static int cov_dense(gpe_handle* h, const double* delta, double nugget, int kind, int predict, double s2_for_r,
+                     std::optional<double> offs, int build, int which, double* out) {
+    int rc;
+    if ((rc = gpe_ensure_batch_ws(h, 1))) return rc;
+    if ((rc = gpe_upload_single_par(h, delta, nugget, kind, predict, s2_for_r, offs))) return rc;
+    DevOut<double> o(h);
+    // a host matrix is staged through the batch workspace's scratch S, which is already n x n or larger: no temporary
+    CK(o.stage(out, (size_t)h->n * h->n, h->S));
+    CK(launch_cov_build(h->X, h->r, h->n, h->d, h->npad, h->par, h->winv, h->A, 0, 1, 1, h->st, build, which, nullptr, h->family));
+    launch_unpad_sym(h->A, h->npad, h->n, o.p, 0, h->st);
+    h->launches += 2;
+    CK(o.flush());
+    CK(cudaStreamSynchronize(h->st));
+    CK(cudaGetLastError());
     return 0;
 }
 
@@ -609,23 +614,7 @@ int gpe_cov_build(gpe_handle* h, const double* delta, double nugget, int kind, i
     if (!h || !h->n || !delta || !A_out) return h ? h->fail_msg("bad argument / no training set") : -2;
     NvtxRange nvtx("gpe_cov_build");
     CK(cudaSetDevice(h->device));
-    int rc;
-    if ((rc = gpe_ensure_batch_ws(h, 1))) return rc;
-    std::vector<double> dl(h->d);
-    CK(cudaMemcpy(dl.data(), delta, sizeof(double) * h->d, cudaMemcpyDefault));
-    if ((rc = gpe_upload_single_par(h, dl.data(), nugget, kind, predict, s2))) return rc;
-    CK(launch_cov_build(h->X, h->r, h->n, h->d, h->npad, h->par, h->winv, h->A, 0, 1, 1, h->st, 0, 0, nullptr, h->family));
-    h->launches++;
-    size_t nn = (size_t)h->n * h->n;
-    double* dst = A_out;
-    bool dev = gpe_is_device_ptr(A_out);
-    if (!dev) dst = h->S;   // stage through scratch
-    launch_unpad_sym(h->A, h->npad, h->n, dst, 0, h->st);
-    h->launches++;
-    if (!dev) CK(cudaMemcpyAsync(A_out, dst, nn * sizeof(double), cudaMemcpyDeviceToHost, h->st));
-    CK(cudaStreamSynchronize(h->st));
-    CK(cudaGetLastError());
-    return 0;
+    return cov_dense(h, delta, nugget, kind, predict, s2, std::nullopt, 0, 0, A_out);
 }
 
 int gpe_cov_grad(gpe_handle* h, const double* delta, double nugget, int kind, int which, double s2, double* G_out) {
@@ -633,38 +622,17 @@ int gpe_cov_grad(gpe_handle* h, const double* delta, double nugget, int kind, in
     if (which < -1 || which >= h->d) return h->fail_msg("which must be a delta index or -1 (nugget)");
     NvtxRange nvtx("gpe_cov_grad");
     CK(cudaSetDevice(h->device));
-    int rc;
-    if ((rc = gpe_ensure_batch_ws(h, 1))) return rc;
-    std::vector<double> dl(h->d);
-    CK(cudaMemcpy(dl.data(), delta, sizeof(double) * h->d, cudaMemcpyDefault));
-    ItemPar ip;
-    host_item_par(ip, nugget, kind, 1, 1.0, 1.0);
-    // grad_delta_A: s2 (1-nu) Delta^2 E  (alt: s2 Delta^2 E);  grad_nugget_A (kernel): -1/2 nu s2 E
-    // (Matérn: G in place of E in grad_delta_A, R in place of E in grad_nugget_A)
-    ip.offs = (which >= 0) ? s2 * ip.c : -0.5 * nugget * s2;
-    std::vector<double> w(h->d);
-    for (int k = 0; k < h->d; k++) w[k] = 1.0 / dl[k];
-    CK(cudaMemcpyAsync(h->par, &ip, sizeof ip, cudaMemcpyHostToDevice, h->st));
-    CK(cudaMemcpyAsync(h->winv, w.data(), sizeof(double) * h->d, cudaMemcpyHostToDevice, h->st));
-    CK(cudaStreamSynchronize(h->st));
-    size_t nn = (size_t)h->n * h->n;
-    bool dev = gpe_is_device_ptr(G_out);
-    double* dst = dev ? G_out : h->S;
     if (which == -1 && kind == 1) {
         // kernel_alt_nug.grad_nugget_A: diag(nu^2 s2)
-        std::vector<double> host(nn, 0.0);
+        std::vector<double> host((size_t)h->n * h->n, 0.0);
         for (int i = 0; i < h->n; i++) host[(size_t)i * h->n + i] = nugget * nugget * s2;
-        CK(cudaMemcpy(G_out, host.data(), nn * sizeof(double), cudaMemcpyDefault));
+        CK(cudaMemcpy(G_out, host.data(), host.size() * sizeof(double), cudaMemcpyDefault));
         return 0;
     }
-    CK(launch_cov_build(h->X, h->r, h->n, h->d, h->npad, h->par, h->winv, h->A, 0, 1, 1, h->st, which >= 0 ? 1 : 2, which,
-                        nullptr, h->family));
-    launch_unpad_sym(h->A, h->npad, h->n, dst, 0, h->st);
-    h->launches += 2;
-    if (!dev) CK(cudaMemcpyAsync(G_out, dst, nn * sizeof(double), cudaMemcpyDeviceToHost, h->st));
-    CK(cudaStreamSynchronize(h->st));
-    CK(cudaGetLastError());
-    return 0;
+    // grad_delta_A: s2 (1-nu) Delta^2 E  (alt: s2 Delta^2 E);  grad_nugget_A (kernel): -1/2 nu s2 E
+    // (Matérn: G in place of E in grad_delta_A, R in place of E in grad_nugget_A)
+    const double offs = (which >= 0) ? s2 * (kind ? 1.0 : 1.0 - nugget) : -0.5 * nugget * s2;
+    return cov_dense(h, delta, nugget, kind, 1, 1.0, offs, which >= 0 ? 1 : 2, which, G_out);
 }
 
 // Device work of one resident sub-batch: theta_d -> (llh_d, grad_d, sig_d, status).  Everything is

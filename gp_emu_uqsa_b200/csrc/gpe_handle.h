@@ -1,5 +1,6 @@
 // Internal handle layout shared by the C-ABI translation units.
 #pragma once
+#include <optional>
 #include <string>
 #include <vector>
 
@@ -119,6 +120,26 @@ struct SubBatch {
     cudaEvent_t *ef = nullptr, *ej = nullptr;
 };
 
+// Return h->fail from the enclosing entry point when a CUDA call fails (needs `gpe_handle* h` in scope).
+#define CK(call)                                                   \
+    do {                                                           \
+        cudaError_t e__ = (call);                                  \
+        if (e__ != cudaSuccess) return h->fail(#call, e__);        \
+    } while (0)
+
+// Device buffers the handle keeps between calls
+template <class T>
+inline cudaError_t dev_alloc(T** p, size_t count) {
+    return cudaMalloc((void**)p, (count ? count : 1) * sizeof(T));
+}
+template <class T>
+inline void dev_free(T*& p) {
+    if (p) cudaFree(p);
+    p = nullptr;
+}
+
+bool gpe_is_device_ptr(const void* p);
+
 // Stream-ordered temporary device buffer (cudaMallocAsync / cudaFreeAsync on the handle's stream): released
 // on every exit path of the entry point that owns it, after the work already enqueued on that stream; the
 // device's default memory pool keeps the memory cached between calls (release threshold set in gpe_create),
@@ -138,6 +159,53 @@ struct TmpDev {
     }
 };
 
+// A caller's input array of `count` elements (host or device memory: each buffer is looked at on its own) as a device pointer
+// `p`: the caller's own pointer when it is device memory, else a stream-ordered copy into a temporary.  Null stays null.
+template <class T>
+struct DevIn {
+    TmpDev tmp;
+    const T* p = nullptr;
+    explicit DevIn(gpe_handle* h) : tmp(h) {}
+    cudaError_t stage(const T* src, size_t count) {
+        p = src;
+        if (!src || gpe_is_device_ptr(src)) return cudaSuccess;
+        T* d;
+        const cudaError_t e = tmp.get(&d, count);
+        p = d;
+        return e != cudaSuccess ? e : cudaMemcpyAsync(d, src, count * sizeof(T), cudaMemcpyHostToDevice, tmp.st);
+    }
+};
+
+// A caller's output array of `count` elements as a device pointer `p` to write through: the caller's own pointer when it is
+// device memory, else `scratch` (a device buffer of at least count elements) if given, else a temporary; flush() enqueues
+// the copy back to host memory after the writes.  A null pointer leaves p null and flush() a no-op (optional outputs).
+template <class T>
+struct DevOut {
+    TmpDev tmp;
+    T* dst = nullptr;
+    T* p = nullptr;
+    size_t count = 0;
+    explicit DevOut(gpe_handle* h) : tmp(h) {}
+    cudaError_t stage(T* out, size_t n, T* scratch = nullptr) {
+        p = out;
+        if (!out || gpe_is_device_ptr(out)) return cudaSuccess;
+        dst = out;
+        count = n;
+        if (scratch) { p = scratch; return cudaSuccess; }
+        return tmp.get(&p, n);
+    }
+    cudaError_t flush() {
+        return (dst && count) ? cudaMemcpyAsync(dst, p, count * sizeof(T), cudaMemcpyDeviceToHost, tmp.st) : cudaSuccess;
+    }
+};
+
+// Appends `count` elements of a short caller array (host or device memory) to the host vector v.
+template <class T>
+inline cudaError_t read_small(std::vector<T>& v, const T* p, size_t count) {
+    v.resize(v.size() + count);
+    return cudaMemcpy(v.data() + v.size() - count, p, count * sizeof(T), cudaMemcpyDefault);
+}
+
 // The buffers one batched recursive factorisation works on (items are addressed through SubBatch::b0):
 // A [B][npad][npad] in (identity padded), overwritten; S scratch (ends up holding the Cholesky factor when asked
 // for); Li <- L^-1 (upper blocks must be zero on entry); logdet_part [B][nleaf]; status [B].
@@ -154,14 +222,14 @@ struct NvtxRange {
     ~NvtxRange();
 };
 
-bool gpe_is_device_ptr(const void* p);
 int gpe_ensure_batch_ws(gpe_handle* h, int B);
 int gpe_potrf_inv(gpe_handle* h, const FactorWs& ws, const SubBatch& sb, int want_L);
 // How the likelihood gradient of a chunk is reduced (gpe_api.cu:grad_route): not at all (fit state), in the LAUUM epilogue, or by
 // the stand-alone reduction kernel after A^-1 is stored, recomputing exp(-D) or reading the covariance build's copy of it.
 enum GradRoute { GRAD_NONE, GRAD_FUSED, GRAD_CLASSIC, GRAD_CLASSIC_E };
 int gpe_factor_and_reduce(gpe_handle* h, const SubBatch& sb, int mode, GradRoute grad, const double* beta_override, double* Kout);
-int gpe_upload_single_par(gpe_handle* h, const double* delta, double nugget, int kind, int predict, double s2_for_r);
+// One item's parameters into h->par / h->winv from the caller's delta [d] (host or device); offs replaces ItemPar::offs.
+int gpe_upload_single_par(gpe_handle* h, const double* delta, double nugget, int kind, int predict, double s2_for_r, std::optional<double> offs = {});
 // Does product p take the INT8 route on stream st?  Yes when its shape does (route on, every dimension >= oz_min, supported) and
 // the stream's residue scratch can hold it; the scratch is grown here, and on an allocation failure the error is cleared and the
 // product stays on DMMA.

@@ -246,36 +246,28 @@ __global__ void __launch_bounds__(128) loo_fit_kernel(const double* __restrict__
 
 using namespace gpe;
 
-#define CK(call)                                                   \
-    do {                                                           \
-        cudaError_t e__ = (call);                                  \
-        if (e__ != cudaSuccess) return h->fail(#call, e__);        \
-    } while (0)
-
 extern "C" int gpe_loo(gpe_handle* h, double* mean, double* var) {
     if (!h || !mean || !var) return h ? h->fail_msg("bad argument") : -2;
     if (!h->fitted) return h->fail_msg("gpe_fit_state has not succeeded on this handle");
     NvtxRange nvtx("gpe_loo");
     CK(cudaSetDevice(h->device));
     const int n = h->n, q = h->q;
-    std::vector<double> K((size_t)NR * NR);
-    CK(cudaMemcpy(K.data(), h->fK, sizeof(double) * NR * NR, cudaMemcpyDeviceToHost));
+    std::vector<double> K;
+    CK(read_small(K, h->fK, (size_t)NR * NR));
     LooShift sh{};
     for (int a = 0; a < q; a++)
         for (int k = a; k < q; k++) sh.t[a] += K[(size_t)k * NR + a] * h->fit_dbeta[k];
-    const bool m_dev = gpe_is_device_ptr(mean), v_dev = gpe_is_device_ptr(var);
-    double *md = mean, *vd = var;
-    TmpDev t_m(h), t_v(h);
-    if (!m_dev) CK(t_m.get(&md, (size_t)n));
-    if (!v_dev) CK(t_v.get(&vd, (size_t)n));
+    DevOut<double> md(h), vd(h);
+    CK(md.stage(mean, (size_t)n));
+    CK(vd.stage(var, (size_t)n));
     {
         ProfScope ps(h, gpe_handle::CAT_OTHER, h->st);
-        loo_fit_kernel<<<(n + 127) / 128, 128, 0, h->st>>>(h->fLi, h->fE, h->y, n, q, h->npad, sh, h->fit_sigma * h->fit_sigma, md, vd);
+        loo_fit_kernel<<<(n + 127) / 128, 128, 0, h->st>>>(h->fLi, h->fE, h->y, n, q, h->npad, sh, h->fit_sigma * h->fit_sigma, md.p, vd.p);
     }
     h->launches++;
     CK(cudaGetLastError());
-    if (!m_dev) CK(cudaMemcpyAsync(mean, md, sizeof(double) * n, cudaMemcpyDeviceToHost, h->st));
-    if (!v_dev) CK(cudaMemcpyAsync(var, vd, sizeof(double) * n, cudaMemcpyDeviceToHost, h->st));
+    CK(md.flush());
+    CK(vd.flush());
     CK(cudaStreamSynchronize(h->st));
     return 0;
 }

@@ -16,17 +16,10 @@
 
 using namespace gpe;
 
-#define CK(call)                                                   \
-    do {                                                           \
-        cudaError_t e__ = (call);                                  \
-        if (e__ != cudaSuccess) return h->fail(#call, e__);        \
-    } while (0)
-
 void gpe_handle::free_fit() {
-    auto fr = [](double*& p) { if (p) cudaFree(p); p = nullptr; };
-    fr(fLi); fr(fE); fr(fK); fr(fbeta); fr(fwinv); fr(fXs); fr(fAinv);
+    dev_free(fLi); dev_free(fE); dev_free(fK); dev_free(fbeta); dev_free(fwinv); dev_free(fXs); dev_free(fAinv);
     fAinv_valid = false;
-    for (auto& sl : ps) { fr(sl.C); fr(sl.Part); fr(sl.Aux); fr(sl.X); fr(sl.H); fr(sl.Mean); fr(sl.Var); }
+    for (auto& sl : ps) { dev_free(sl.C); dev_free(sl.Part); dev_free(sl.Aux); dev_free(sl.X); dev_free(sl.H); dev_free(sl.Mean); dev_free(sl.Var); }
     pchunk = 0;
     fitted = false;
 }
@@ -589,18 +582,17 @@ __global__ void fullcov_finalize_kernel(const double* __restrict__ ZtZ, int mp, 
 
 int ensure_predict_ws(gpe_handle* h, long long mc) {
     if (mc <= h->pchunk) return 0;
-    auto fr = [](double*& p) { if (p) cudaFree(p); p = nullptr; };
     h->pchunk = 0;
     size_t ntile = h->npad / 128;
     for (auto& sl : h->ps) {
-        fr(sl.C); fr(sl.Part); fr(sl.Aux); fr(sl.X); fr(sl.H); fr(sl.Mean); fr(sl.Var);
-        CK(cudaMalloc((void**)&sl.C, (size_t)h->npad * mc * sizeof(double)));
-        CK(cudaMalloc((void**)&sl.Part, ntile * mc * sizeof(double)));
-        CK(cudaMalloc((void**)&sl.Aux, (size_t)NR * mc * sizeof(double)));
-        CK(cudaMalloc((void**)&sl.X, (size_t)mc * h->d * sizeof(double)));
-        CK(cudaMalloc((void**)&sl.H, (size_t)mc * NR * sizeof(double)));
-        CK(cudaMalloc((void**)&sl.Mean, (size_t)mc * sizeof(double)));
-        CK(cudaMalloc((void**)&sl.Var, (size_t)mc * sizeof(double)));
+        dev_free(sl.C); dev_free(sl.Part); dev_free(sl.Aux); dev_free(sl.X); dev_free(sl.H); dev_free(sl.Mean); dev_free(sl.Var);
+        CK(dev_alloc(&sl.C, (size_t)h->npad * mc));
+        CK(dev_alloc(&sl.Part, ntile * mc));
+        CK(dev_alloc(&sl.Aux, (size_t)NR * mc));
+        CK(dev_alloc(&sl.X, (size_t)mc * h->d));
+        CK(dev_alloc(&sl.H, (size_t)mc * NR));
+        CK(dev_alloc(&sl.Mean, (size_t)mc));
+        CK(dev_alloc(&sl.Var, (size_t)mc));
     }
     h->pchunk = mc;
     return 0;
@@ -675,6 +667,58 @@ int predict_chunk(gpe_handle* h, gpe_handle::PredSlot& sl, cudaStream_t st, cons
     return 0;
 }
 
+// The tensor grid of gpe_predict_grid / gpe_predict_implaus from the caller's levels, lo, hi [d] (host memory)
+int make_grid(gpe_handle* h, const int* levels, const double* lo, const double* hi, GridDesc& g) {
+    if (h->d > MAXD) return h->fail_msg("grid prediction supports d <= 64");
+    g.d = h->d;
+    for (int k = 0; k < h->d; k++) {
+        g.levels[k] = levels[k];
+        g.lo[k] = lo[k];
+        g.step[k] = (hi[k] - lo[k]) / (double)levels[k];
+    }
+    return 0;
+}
+
+// The cell arguments of the implausibility entry points; m = 0 skips the check that ncell covers the cells of m points.
+int check_cells(gpe_handle* h, long long cell_pts, long long first_index, long long ncell, long long m) {
+    if (cell_pts < 0 || first_index < 0 || ncell < 0) return h->fail_msg("cell_pts, first_index and ncell must be non-negative");
+    if (cell_pts > 0 && m > 0 && (first_index + m - 1) / cell_pts - first_index / cell_pts + 1 > ncell)
+        return h->fail_msg("the points span more cells than ncell");
+    return 0;
+}
+
+// The implausibility reductions over a call's points: count_lt [maxno] and, with cells, cell_min [ncell][maxno] (bits of I >= 0,
+// which order like the value) and cell_count; finish() copies them to the caller's outputs (host, device or NULL) and waits.
+struct ImpAccum {
+    gpe_handle* h;
+    int maxno;
+    long long ncell;        // 0 without cells (cell_pts == 0)
+    unsigned long long *count_lt = nullptr, *cell_min = nullptr, *cell_count = nullptr;
+    TmpDev t_cnt, t_cmin, t_ccnt;
+    ImpAccum(gpe_handle* h_, int maxno_, long long cell_pts, long long ncell_)
+        : h(h_), maxno(maxno_), ncell(cell_pts > 0 ? ncell_ : 0), t_cnt(h_), t_cmin(h_), t_ccnt(h_) {}
+    int init() {
+        CK(t_cnt.get(&count_lt, (size_t)maxno));
+        CK(cudaMemsetAsync(count_lt, 0, sizeof(unsigned long long) * maxno, h->st));
+        if (ncell > 0) {
+            CK(t_cmin.get(&cell_min, (size_t)ncell * maxno));
+            CK(t_ccnt.get(&cell_count, (size_t)ncell * maxno));
+            // 0x7f in every byte is a large positive double: the minimum of a cell that holds no point of the call is +huge
+            CK(cudaMemsetAsync(cell_min, 0x7f, sizeof(unsigned long long) * ncell * maxno, h->st));
+            CK(cudaMemsetAsync(cell_count, 0, sizeof(unsigned long long) * ncell * maxno, h->st));
+        }
+        return 0;
+    }
+    int finish(unsigned long long* count_out, double* min_out, unsigned long long* cnt_out) {
+        if (count_out) CK(cudaMemcpyAsync(count_out, count_lt, sizeof(unsigned long long) * maxno, cudaMemcpyDefault, h->st));
+        if (ncell > 0 && min_out) CK(cudaMemcpyAsync(min_out, cell_min, sizeof(double) * ncell * maxno, cudaMemcpyDefault, h->st));
+        if (ncell > 0 && cnt_out) CK(cudaMemcpyAsync(cnt_out, cell_count, sizeof(unsigned long long) * ncell * maxno, cudaMemcpyDefault, h->st));
+        CK(cudaStreamSynchronize(h->st));
+        CK(cudaGetLastError());
+        return 0;
+    }
+};
+
 }  // namespace
 
 extern "C" {
@@ -687,20 +731,20 @@ int gpe_fit_state(gpe_handle* h, const double* delta, double nugget, double sigm
     int rc;
     if ((rc = gpe_ensure_batch_ws(h, 1))) return rc;
     const int np = h->npad, q = h->q;
-    std::vector<double> dl(h->d), bin(NR, 0.0);
-    CK(cudaMemcpy(dl.data(), delta, sizeof(double) * h->d, cudaMemcpyDefault));
-    if ((rc = gpe_upload_single_par(h, dl.data(), nugget, kind, 1, r_div > 0 ? r_div : 1.0))) return rc;
+    if ((rc = gpe_upload_single_par(h, delta, nugget, kind, 1, r_div > 0 ? r_div : 1.0))) return rc;
     if (!h->fLi) {
-        CK(cudaMalloc((void**)&h->fLi, (size_t)np * np * sizeof(double)));
-        CK(cudaMalloc((void**)&h->fE, (size_t)np * NR * sizeof(double)));
-        CK(cudaMalloc((void**)&h->fK, (size_t)NR * NR * sizeof(double)));
-        CK(cudaMalloc((void**)&h->fbeta, (size_t)NR * sizeof(double)));
-        CK(cudaMalloc((void**)&h->fwinv, (size_t)h->d * sizeof(double)));
-        CK(cudaMalloc((void**)&h->fXs, (size_t)h->d * np * sizeof(double)));
+        CK(dev_alloc(&h->fLi, (size_t)np * np));
+        CK(dev_alloc(&h->fE, (size_t)np * NR));
+        CK(dev_alloc(&h->fK, (size_t)NR * NR));
+        CK(dev_alloc(&h->fbeta, (size_t)NR));
+        CK(dev_alloc(&h->fwinv, (size_t)h->d));
+        CK(dev_alloc(&h->fXs, (size_t)h->d * np));
     }
+    std::vector<double> bin;
     double* bov = nullptr;
     if (beta_in) {
-        CK(cudaMemcpy(bin.data(), beta_in, sizeof(double) * q, cudaMemcpyDefault));
+        CK(read_small(bin, beta_in, q));
+        bin.resize(NR, 0.0);
         CK(cudaMemcpyAsync(h->fbeta, bin.data(), sizeof(double) * NR, cudaMemcpyHostToDevice, h->st));
         bov = h->fbeta;
     }
@@ -844,14 +888,8 @@ int gpe_predict_grid(gpe_handle* h, const int* levels, const double* lo, const d
                      long long count, double* mean, double* var) {
     if (h && count == 0) return 0;                               // empty shard of the grid
     if (!h || !levels || !lo || !hi || !mean || count < 1) return h ? h->fail_msg("bad argument") : -2;
-    if (h->d > MAXD) return h->fail_msg("grid prediction supports d <= 64");
     GridDesc g;
-    g.d = h->d;
-    for (int k = 0; k < h->d; k++) {
-        g.levels[k] = levels[k];
-        g.lo[k] = lo[k];
-        g.step[k] = (hi[k] - lo[k]) / (double)levels[k];
-    }
+    if (int rc = make_grid(h, levels, lo, hi, g)) return rc;
     return predict_common(h, nullptr, nullptr, &g, start, count, mean, var);
 }
 
@@ -863,63 +901,38 @@ int gpe_predict_implaus(gpe_handle* h, const double* Xs, const double* Hs, const
     if (!h || m < 0 || (!Xs && (!levels || !lo || !hi)) || maxno < 1 || maxno > MAXEM) return h ? h->fail_msg("bad argument") : -2;
     if (!Itop && !(first && last)) return h->fail_msg("Itop is needed to carry the list from one emulator to the next");
     if (Itop && !gpe_is_device_ptr(Itop)) return h->fail_msg("Itop must be device memory");
-    if (cell_pts < 0 || first_index < 0 || ncell < 0) return h->fail_msg("cell_pts, first_index and ncell must be non-negative");
-    if (cell_pts == 0) ncell = 0;
-    if (last && cell_pts > 0 && m > 0 && (first_index + m - 1) / cell_pts - first_index / cell_pts + 1 > ncell)
-        return h->fail_msg("the points span more cells than ncell");
+    int rc;
+    if ((rc = check_cells(h, cell_pts, first_index, ncell, last ? m : 0))) return rc;
     NvtxRange nvtx("gpe_predict_implaus");
     CK(cudaSetDevice(h->device));
     ImpFuse ic{};
     ic.z = z; ic.ve = var_extra; ic.cm = cm; ic.maxno = maxno; ic.first = first != 0; ic.last = last != 0;
     ic.store_top = Itop != nullptr;
     ic.first_index = first_index; ic.cell_pts = last ? cell_pts : 0; ic.cell_base = cell_pts > 0 ? first_index / cell_pts : 0;
-    double* top_tmp = nullptr;
-    unsigned char* kd = nullptr;
-    unsigned long long *cnt = nullptr, *cmin = nullptr, *ccnt = nullptr;
-    TmpDev t_top(h), t_k(h), t_cnt(h), t_cmin(h), t_ccnt(h);
-    if (!Itop) CK(t_top.get(&top_tmp, (size_t)std::max<long long>(m, 1) * maxno));      // first == last: a one-emulator job
-    ic.Itop = Itop ? Itop : top_tmp;
-    const bool k_dev = keep && gpe_is_device_ptr(keep);
+    TmpDev t_top(h);
+    ic.Itop = Itop;
+    if (!Itop) CK(t_top.get(&ic.Itop, (size_t)std::max<long long>(m, 1) * maxno));      // first == last: a one-emulator job
+    DevOut<unsigned char> ko(h);
+    ImpAccum acc(h, maxno, cell_pts, ncell);
     if (last) {
-        if (keep) { if (k_dev) kd = keep; else CK(t_k.get(&kd, (size_t)std::max<long long>(m, 1))); }
-        ic.keep = kd;
-        CK(t_cnt.get(&cnt, (size_t)maxno));
-        CK(cudaMemsetAsync(cnt, 0, sizeof(unsigned long long) * maxno, h->st));
-        ic.count_lt = cnt;
-        if (ncell > 0) {
-            CK(t_cmin.get(&cmin, (size_t)ncell * maxno));
-            CK(t_ccnt.get(&ccnt, (size_t)ncell * maxno));
-            CK(cudaMemsetAsync(cmin, 0x7f, sizeof(unsigned long long) * ncell * maxno, h->st));
-            CK(cudaMemsetAsync(ccnt, 0, sizeof(unsigned long long) * ncell * maxno, h->st));
-            ic.cell_min_bits = cmin; ic.cell_count = ccnt;
-        }
+        CK(ko.stage(keep, (size_t)m));
+        if ((rc = acc.init())) return rc;
+        ic.keep = ko.p;
+        ic.count_lt = acc.count_lt; ic.cell_min_bits = acc.cell_min; ic.cell_count = acc.cell_count;
     }
-    int rc = 0;
     if (m > 0) {
         if (Xs) {
             rc = predict_common(h, Xs, Hs, nullptr, 0, m, nullptr, nullptr, &ic);
         } else {
-            if (h->d > MAXD) return h->fail_msg("grid prediction supports d <= 64");
             GridDesc g;
-            g.d = h->d;
-            for (int k = 0; k < h->d; k++) {
-                g.levels[k] = levels[k];
-                g.lo[k] = lo[k];
-                g.step[k] = (hi[k] - lo[k]) / (double)levels[k];
-            }
+            if ((rc = make_grid(h, levels, lo, hi, g))) return rc;
             rc = predict_common(h, nullptr, nullptr, &g, start, m, nullptr, nullptr, &ic);
         }
         if (rc) return rc;
     }
-    if (last) {
-        if (keep && !k_dev && m > 0) CK(cudaMemcpyAsync(keep, kd, (size_t)m, cudaMemcpyDeviceToHost, h->st));
-        if (count_lt) CK(cudaMemcpyAsync(count_lt, cnt, sizeof(unsigned long long) * maxno, cudaMemcpyDefault, h->st));
-        if (ncell > 0 && cell_min) CK(cudaMemcpyAsync(cell_min, cmin, sizeof(double) * ncell * maxno, cudaMemcpyDefault, h->st));
-        if (ncell > 0 && cell_count) CK(cudaMemcpyAsync(cell_count, ccnt, sizeof(unsigned long long) * ncell * maxno, cudaMemcpyDefault, h->st));
-        CK(cudaStreamSynchronize(h->st));
-        CK(cudaGetLastError());
-    }
-    return 0;
+    if (!last) return 0;
+    CK(ko.flush());
+    return acc.finish(count_lt, cell_min, cell_count);
 }
 
 int gpe_cross_cov(gpe_handle* h, const double* delta, double nugget, int kind, const double* Xs, int m, double* C_out) {
@@ -929,9 +942,9 @@ int gpe_cross_cov(gpe_handle* h, const double* delta, double nugget, int kind, c
     CK(cudaSetDevice(h->device));
     const int np = h->npad, d = h->d;
     int mc = (m + 127) / 128 * 128;
-    std::vector<double> w(d), dl(d);
-    CK(cudaMemcpy(dl.data(), delta, sizeof(double) * d, cudaMemcpyDefault));
-    for (int k = 0; k < d; k++) w[k] = 1.0 / dl[k];
+    std::vector<double> w;
+    CK(read_small(w, delta, d));
+    for (double& v : w) v = 1.0 / v;
     double *wd = nullptr, *xs = nullptr, *P = nullptr, *Cm = nullptr;
     TmpDev t_wd(h), t_xs(h), t_P(h), t_Cm(h);
     CK(t_wd.get(&wd, (size_t)d));
@@ -962,27 +975,22 @@ int gpe_predict_fullcov(gpe_handle* h, const double* Xs, const double* Hs, int m
     CK(cudaSetDevice(h->device));
     const int np = h->npad, d = h->d, q = h->q;
     const int mp = (m + 127) / 128 * 128;
-    double *P = nullptr, *Hd = nullptr, *Cm = nullptr, *Zm = nullptr, *ZtZ = nullptr, *aux = nullptr, *G = nullptr, *rn = nullptr,
-           *md = nullptr, *Vd = nullptr;
-    TmpDev t_P(h), t_Cm(h), t_Zm(h), t_ZtZ(h), t_aux(h), t_G(h), t_md(h), t_Vd(h), t_Hd(h), t_rn(h);
+    double *P = nullptr, *Cm = nullptr, *Zm = nullptr, *ZtZ = nullptr, *aux = nullptr, *G = nullptr;
+    TmpDev t_P(h), t_Cm(h), t_Zm(h), t_ZtZ(h), t_aux(h), t_G(h);
+    DevIn<double> Hd(h), rn(h);
+    DevOut<double> md(h), Vd(h);
     CK(t_P.get(&P, (size_t)mp * d));
     CK(t_Cm.get(&Cm, (size_t)np * mp));
     CK(t_Zm.get(&Zm, (size_t)np * mp));
     CK(t_ZtZ.get(&ZtZ, (size_t)mp * mp));
     CK(t_aux.get(&aux, (size_t)NR * mp));
     CK(t_G.get(&G, (size_t)NR * mp));
-    CK(t_md.get(&md, (size_t)mp));
-    CK(t_Vd.get(&Vd, (size_t)m * m));
+    CK(md.stage(mean, (size_t)m));
+    CK(Vd.stage(V, (size_t)m * m));
     CK(cudaMemsetAsync(P, 0, sizeof(double) * (size_t)mp * d, h->st));
     CK(cudaMemcpyAsync(P, Xs, sizeof(double) * (size_t)m * d, cudaMemcpyDefault, h->st));
-    if (Hs) {
-        CK(t_Hd.get(&Hd, (size_t)m * q));
-        CK(cudaMemcpyAsync(Hd, Hs, sizeof(double) * (size_t)m * q, cudaMemcpyDefault, h->st));
-    }
-    if (r_new) {
-        CK(t_rn.get(&rn, (size_t)m));
-        CK(cudaMemcpyAsync(rn, r_new, sizeof(double) * m, cudaMemcpyDefault, h->st));
-    }
+    CK(Hd.stage(Hs, (size_t)m * q));
+    CK(rn.stage(r_new, (size_t)m));
     CK(launch_xcov(h->family, h->fXs, P, h->fwinv, h->n, d, np, mp, m, h->fit_c, Cm, mp, h->st));
     h->launches++;
     int rc = 0;
@@ -995,16 +1003,16 @@ int gpe_predict_fullcov(gpe_handle* h, const double* Xs, const double* Hs, int m
         BasisDesc bd = basis_of(h);
         double s2 = h->fit_sigma * h->fit_sigma;
         // mean via the diagonal finalize (var == nullptr)
-        predict_finalize_kernel<false><<<(m + 127) / 128, 128, 0, h->st>>>(nullptr, 0, aux, mp, P, Hd, bd, d, h->fK, h->fbeta, s2,
-                                                                            h->fit_astar, m, md, nullptr, ImpFuse{});
+        predict_finalize_kernel<false><<<(m + 127) / 128, 128, 0, h->st>>>(nullptr, 0, aux, mp, P, Hd.p, bd, d, h->fK, h->fbeta, s2,
+                                                                            h->fit_astar, m, md.p, nullptr, ImpFuse{});
         auto fin = h->family == FAMILY_MATERN52 ? fullcov_finalize_kernel<FAMILY_MATERN52> : fullcov_finalize_kernel<FAMILY_GAUSSIAN>;
-        fin<<<(m + 127) / 128, 128, 0, h->st>>>(ZtZ, mp, aux, mp, P, Hd, bd, d, h->fwinv, h->fK, s2, h->fit_c, h->fit_astar, rn, m, G, Vd, 0);
+        fin<<<(m + 127) / 128, 128, 0, h->st>>>(ZtZ, mp, aux, mp, P, Hd.p, bd, d, h->fwinv, h->fK, s2, h->fit_c, h->fit_astar, rn.p, m, G, Vd.p, 0);
         size_t tot = (size_t)m * m;
-        fin<<<(unsigned)((tot + 255) / 256), 256, 0, h->st>>>(ZtZ, mp, aux, mp, P, Hd, bd, d, h->fwinv, h->fK, s2, h->fit_c, h->fit_astar,
-                                                            rn, m, G, Vd, 1);
+        fin<<<(unsigned)((tot + 255) / 256), 256, 0, h->st>>>(ZtZ, mp, aux, mp, P, Hd.p, bd, d, h->fwinv, h->fK, s2, h->fit_c, h->fit_astar,
+                                                            rn.p, m, G, Vd.p, 1);
         h->launches += 3;
-        CK(cudaMemcpyAsync(mean, md, sizeof(double) * m, cudaMemcpyDefault, h->st));
-        CK(cudaMemcpyAsync(V, Vd, sizeof(double) * (size_t)m * m, cudaMemcpyDefault, h->st));
+        CK(md.flush());
+        CK(Vd.flush());
     }
     CK(cudaStreamSynchronize(h->st));
     if (rc) return rc;
@@ -1018,54 +1026,32 @@ int gpe_implausibility(gpe_handle* h, const double* mean, const double* var, int
                        unsigned long long* cell_count) {
     if (!h || !z || !var_extra || n_emul < 1 || m < 0 || (m > 0 && (!mean || !var))) return h ? h->fail_msg("bad argument") : -2;
     if (n_emul > MAXEM || maxno < 1 || maxno > n_emul) return h->fail_msg("need 1 <= maxno <= n_emul <= 16");
-    if (cell_pts < 0 || first_index < 0 || ncell < 0) return h->fail_msg("cell_pts, first_index and ncell must be non-negative");
-    if (cell_pts == 0) ncell = 0;
-    if (cell_pts > 0 && m > 0 && (first_index + m - 1) / cell_pts - first_index / cell_pts + 1 > ncell)
-        return h->fail_msg("the points span more cells than ncell");
+    if (int rc = check_cells(h, cell_pts, first_index, ncell, m)) return rc;
     NvtxRange nvtx("gpe_implausibility");
     CK(cudaSetDevice(h->device));
     ImpDesc ds;
     ds.n_emul = n_emul; ds.maxno = maxno; ds.cm = cm;
-    std::vector<double> zz(n_emul), vv(n_emul);
-    CK(cudaMemcpy(zz.data(), z, sizeof(double) * n_emul, cudaMemcpyDefault));
-    CK(cudaMemcpy(vv.data(), var_extra, sizeof(double) * n_emul, cudaMemcpyDefault));
+    std::vector<double> zz, vv;
+    CK(read_small(zz, z, n_emul));
+    CK(read_small(vv, var_extra, n_emul));
     for (int o = 0; o < n_emul; o++) { ds.z[o] = zz[o]; ds.ve[o] = vv[o]; }
-    const bool in_dev = gpe_is_device_ptr(mean);
-    const double *md = mean, *vd = var;
-    double *mtmp = nullptr, *vtmp = nullptr, *Id = nullptr;
-    unsigned char* kd = nullptr;
-    unsigned long long *cnt = nullptr, *cmin = nullptr, *ccnt = nullptr;
-    TmpDev t_m(h), t_v(h), t_I(h), t_k(h), t_cnt(h), t_cmin(h), t_ccnt(h);
-    if (!in_dev) {
-        CK(t_m.get(&mtmp, (size_t)n_emul * m));
-        CK(t_v.get(&vtmp, (size_t)n_emul * m));
-        CK(cudaMemcpyAsync(mtmp, mean, sizeof(double) * (size_t)n_emul * m, cudaMemcpyHostToDevice, h->st));
-        CK(cudaMemcpyAsync(vtmp, var, sizeof(double) * (size_t)n_emul * m, cudaMemcpyHostToDevice, h->st));
-        md = mtmp; vd = vtmp;
-    }
-    const bool I_dev = Imax && gpe_is_device_ptr(Imax), k_dev = keep && gpe_is_device_ptr(keep);
-    if (Imax) { if (I_dev) Id = Imax; else CK(t_I.get(&Id, (size_t)m * maxno)); }
-    if (keep) { if (k_dev) kd = keep; else CK(t_k.get(&kd, (size_t)m)); }
-    CK(t_cnt.get(&cnt, (size_t)maxno));
-    CK(cudaMemsetAsync(cnt, 0, sizeof(unsigned long long) * maxno, h->st));
-    if (ncell > 0) {
-        CK(t_cmin.get(&cmin, (size_t)ncell * maxno));
-        CK(t_ccnt.get(&ccnt, (size_t)ncell * maxno));
-        CK(cudaMemsetAsync(cmin, 0x7f, sizeof(unsigned long long) * ncell * maxno, h->st));   // large positive double
-        CK(cudaMemsetAsync(ccnt, 0, sizeof(unsigned long long) * ncell * maxno, h->st));
-    }
+    DevIn<double> md(h), vd(h);
+    DevOut<double> Io(h);
+    DevOut<unsigned char> ko(h);
+    ImpAccum acc(h, maxno, cell_pts, ncell);
+    CK(md.stage(mean, (size_t)n_emul * m));
+    CK(vd.stage(var, (size_t)n_emul * m));
+    CK(Io.stage(Imax, (size_t)m * maxno));
+    CK(ko.stage(keep, (size_t)m));
+    if (int rc = acc.init()) return rc;
     if (m > 0) {                                                 // m == 0: zero counts, +huge cell minima
-        implaus_kernel<<<(unsigned)((m + 255) / 256), 256, 0, h->st>>>(md, vd, m, ds, ncell > 0 ? cell_pts : 0, first_index, Id, kd, cnt, cmin, ccnt);
+        implaus_kernel<<<(unsigned)((m + 255) / 256), 256, 0, h->st>>>(md.p, vd.p, m, ds, acc.ncell > 0 ? cell_pts : 0, first_index, Io.p, ko.p,
+                                                                       acc.count_lt, acc.cell_min, acc.cell_count);
         h->launches++;
     }
-    if (Imax && !I_dev && m > 0) CK(cudaMemcpyAsync(Imax, Id, sizeof(double) * (size_t)m * maxno, cudaMemcpyDeviceToHost, h->st));
-    if (keep && !k_dev && m > 0) CK(cudaMemcpyAsync(keep, kd, (size_t)m, cudaMemcpyDeviceToHost, h->st));
-    if (count_lt) CK(cudaMemcpyAsync(count_lt, cnt, sizeof(unsigned long long) * maxno, cudaMemcpyDefault, h->st));
-    if (ncell > 0 && cell_min) CK(cudaMemcpyAsync(cell_min, cmin, sizeof(double) * ncell * maxno, cudaMemcpyDefault, h->st));
-    if (ncell > 0 && cell_count) CK(cudaMemcpyAsync(cell_count, ccnt, sizeof(unsigned long long) * ncell * maxno, cudaMemcpyDefault, h->st));
-    CK(cudaStreamSynchronize(h->st));
-    CK(cudaGetLastError());
-    return 0;
+    CK(Io.flush());
+    CK(ko.flush());
+    return acc.finish(count_lt, cell_min, cell_count);
 }
 
 }  // extern "C"

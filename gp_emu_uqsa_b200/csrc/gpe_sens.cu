@@ -18,12 +18,6 @@
 
 using namespace gpe;
 
-#define CK(call)                                                   \
-    do {                                                           \
-        cudaError_t e__ = (call);                                  \
-        if (e__ != cudaSuccess) return h->fail(#call, e__);        \
-    } while (0)
-
 namespace {
 
 constexpr int ST = 64;   // tile edge
@@ -220,7 +214,7 @@ __global__ void __launch_bounds__(256) pdist_argmin_kernel(const double* __restr
 int ensure_ainv(gpe_handle* h) {
     if (h->fAinv_valid) return 0;
     const int np = h->npad;
-    if (!h->fAinv) CK(cudaMalloc((void**)&h->fAinv, (size_t)np * np * sizeof(double)));
+    if (!h->fAinv) CK(dev_alloc(&h->fAinv, (size_t)np * np));
     // LAUUM: A^-1 = Linv^T Linv, lower 128-tiles
     int rc = gpe_gemm(h, h->st, {.A = h->fLi, .B = h->fLi, .C = h->fAinv, .lda = np, .ldb = np, .ldc = np, .M = np, .N = np, .K = np,
                                  .kmode = KM_GE_I, .lower = 1}, GEMM_TN);
@@ -285,11 +279,11 @@ int gpe_sens_contract(gpe_handle* h, const double* gamma, const double* acoef, c
     int rc;
     if ((rc = gpe_ensure_batch_ws(h, 1))) return rc;     // h->S: scratch for P
     if ((rc = ensure_ainv(h))) return rc;
-    std::vector<double> g(d), hostbuf(3 * d);
-    CK(cudaMemcpy(g.data(), gamma, sizeof(double) * d, cudaMemcpyDefault));
-    for (int k = 0; k < d; k++) hostbuf[k] = std::sqrt(g[k]);
-    CK(cudaMemcpy(hostbuf.data() + d, acoef, sizeof(double) * d, cudaMemcpyDefault));
-    CK(cudaMemcpy(hostbuf.data() + 2 * d, mvec, sizeof(double) * d, cudaMemcpyDefault));
+    std::vector<double> hostbuf;        // [sqrt(gamma) | acoef | mvec]
+    CK(read_small(hostbuf, gamma, d));
+    for (double& g : hostbuf) g = std::sqrt(g);
+    CK(read_small(hostbuf, acoef, d));
+    CK(read_small(hostbuf, mvec, d));
     const int nt = np / ST, ntile = nt * (nt + 1) / 2;
     double *coef = nullptr, *tpart = nullptr, *Vsrc = nullptr, *Vp = nullptr, *Yp = nullptr, *outd = nullptr;
     TmpDev t_coef(h), t_tpart(h), t_Vsrc(h), t_Vp(h), t_Yp(h), t_outd(h);
@@ -337,15 +331,15 @@ int gpe_sens_main_effect(gpe_handle* h, const double* t1, const double* t2, cons
     NvtxRange nvtx("gpe_sens_main_effect");
     CK(cudaSetDevice(h->device));
     const int n = h->n, d = h->d;
-    std::vector<double> hb(4 * d + n + (size_t)nwhich * points);
-    std::vector<int> wh(nwhich);
-    CK(cudaMemcpy(hb.data(), t1, sizeof(double) * d, cudaMemcpyDefault));
-    CK(cudaMemcpy(hb.data() + d, t2, sizeof(double) * d, cudaMemcpyDefault));
-    CK(cudaMemcpy(hb.data() + 2 * d, cdiag, sizeof(double) * d, cudaMemcpyDefault));
-    CK(cudaMemcpy(hb.data() + 3 * d, mvec, sizeof(double) * d, cudaMemcpyDefault));
-    CK(cudaMemcpy(hb.data() + 4 * d, evec, sizeof(double) * n, cudaMemcpyDefault));
-    CK(cudaMemcpy(hb.data() + 4 * d + n, xw, sizeof(double) * (size_t)nwhich * points, cudaMemcpyDefault));
-    CK(cudaMemcpy(wh.data(), which, sizeof(int) * nwhich, cudaMemcpyDefault));
+    std::vector<double> hb;             // [t1 | t2 | cdiag | mvec | evec | xw]
+    std::vector<int> wh;
+    CK(read_small(hb, t1, d));
+    CK(read_small(hb, t2, d));
+    CK(read_small(hb, cdiag, d));
+    CK(read_small(hb, mvec, d));
+    CK(read_small(hb, evec, n));
+    CK(read_small(hb, xw, (size_t)nwhich * points));
+    CK(read_small(wh, which, nwhich));
     for (int w = 0; w < nwhich; w++)
         if (wh[w] < 0 || wh[w] >= d) return h->fail_msg("input index out of range");
     double *db = nullptr, *od = nullptr;
@@ -372,23 +366,13 @@ int gpe_pdist_argmin(gpe_handle* h, const double* designs, int N, int n, int dim
     NvtxRange nvtx("gpe_pdist_argmin");
     CK(cudaSetDevice(h->device));
     const int P = n + ne, nblk = (P - 1 + PD_ROWS - 1) / PD_ROWS;
-    double *dd = nullptr, *de = nullptr;
     PdBest* dp = nullptr;
-    TmpDev t_d(h), t_e(h), t_p(h);
-    const double* dsrc = designs;
-    if (!gpe_is_device_ptr(designs)) {
-        CK(t_d.get(&dd, (size_t)N * n * dim));
-        CK(cudaMemcpyAsync(dd, designs, sizeof(double) * (size_t)N * n * dim, cudaMemcpyHostToDevice, h->st));
-        dsrc = dd;
-    }
-    const double* esrc = extra;
-    if (ne > 0 && !gpe_is_device_ptr(extra)) {
-        CK(t_e.get(&de, (size_t)ne * dim));
-        CK(cudaMemcpyAsync(de, extra, sizeof(double) * (size_t)ne * dim, cudaMemcpyHostToDevice, h->st));
-        esrc = de;
-    }
+    TmpDev t_p(h);
+    DevIn<double> ds(h), es(h);
+    CK(ds.stage(designs, (size_t)N * n * dim));
+    CK(es.stage(ne > 0 ? extra : nullptr, (size_t)ne * dim));
     CK(t_p.get(&dp, (size_t)N * nblk));
-    pdist_argmin_kernel<<<dim3(nblk, N), 256, 0, h->st>>>(dsrc, n, dim, esrc, ne, dp);
+    pdist_argmin_kernel<<<dim3(nblk, N), 256, 0, h->st>>>(ds.p, n, dim, es.p, ne, dp);
     h->launches++;
     std::vector<PdBest> part((size_t)N * nblk);
     CK(cudaMemcpyAsync(part.data(), dp, sizeof(PdBest) * part.size(), cudaMemcpyDeviceToHost, h->st));
