@@ -328,21 +328,103 @@ static cudaError_t launch_xcov(int family, const double* Xs, const double* P, co
     return launch_xcov_fam<FAMILY_GAUSSIAN>(Xs, P, winv, n, d, npad, mc, count, cscale, Cm, ldc, st);
 }
 
-// Implausibility folded into the prediction of one emulator (history_match.py:96-132): instead of mean / variance the
-// per-point list of the maxno largest implausibilities over the emulators seen so far, Itop [m][maxno] ascending, is
-// updated; the last emulator's pass also produces the keep mask, the counts and the cell statistics, so neither the
-// means / variances nor (unless asked for) the final list ever travel through HBM.
+// K5 implausibility I = |mean - z| / sqrt(var + var_extra) of a point against each emulator's observation z, the per-point
+// ascending list of the maxno largest I over the emulators (history_match.py:96-132) and, on the finished lists, the keep mask,
+// the counts and the cell statistics.  Two routes share the update and the reduction below, so they give bit-identical results:
+// gpe_implausibility (implaus_kernel) on given mean / variance arrays, and gpe_predict_implaus, which folds the update into the
+// prediction of one emulator (predict_finalize_kernel<true>: a running list Itop [m][maxno] instead of mean / variance) and the
+// reduction into the last emulator's pass, so neither the means / variances nor (unless asked for) the final list travel through HBM.
 constexpr int MAXEM = 16;
+
+// What the reduction adds into.  I >= 0, so the IEEE bit pattern orders like the value and the cell minima are integer atomics
+// (deterministic).  Cells are runs of cell_pts points of the global flat index; output cell 0 is the cell of the call's first point.
+struct ImpStats {
+    double cm;
+    int maxno;
+    long long cell_pts;                  // 0: no cell statistics
+    long long cell_base;                 // (call's first_index) / cell_pts
+    unsigned char* keep;                 // or null
+    unsigned long long *count_lt, *cell_min_bits, *cell_count;      // [maxno], [ncell][maxno]
+};
+
+__device__ __forceinline__ double implaus_value(double mean, double var, double z, double ve) {
+    const double dz = mean - z;
+    return sqrt(dz * dz / (var + ve));
+}
+
+// I into the ascending list of the maxno largest, top[maxno-1] the largest (np.sort(np.partition(I, -maxno)[-maxno:]), :129)
+__device__ __forceinline__ void top_insert(double (&top)[MAXEM], int maxno, double I) {
+    if (I > top[0]) {
+        top[0] = I;
+#pragma unroll
+        for (int k = 0; k < MAXEM - 1; k++) {
+            if (k + 1 < maxno && top[k] > top[k + 1]) {
+                double t = top[k];
+                top[k] = top[k + 1];
+                top[k + 1] = t;
+            }
+        }
+    }
+}
+
+// The reduction of a point's finished list; every lane of the warp calls it.  local: the point's index in keep, global: its flat index.
+// A warp's 32 consecutive points almost always sit in one cell: reduce in the warp first, one atomic per warp instead of one per point.
+__device__ __forceinline__ void imp_finish(const double (&top)[MAXEM], bool live, long long local, long long global, const ImpStats& s) {
+    if (live && s.keep != nullptr) s.keep[local] = (top[0] < s.cm) ? 1 : 0;
+    const long long cell = (s.cell_pts > 0 && live) ? global / s.cell_pts - s.cell_base : -1;
+    const long long cell0 = __shfl_sync(0xffffffffu, cell, 0);
+    const bool uniform = s.cell_pts > 0 && __all_sync(0xffffffffu, cell == cell0) && cell0 >= 0;
+    for (int k = 0; k < s.maxno; k++) {
+        const double vk = top[s.maxno - 1 - k];      // the k-th statistic refers to the (k+1)-th largest
+        const bool lt = live && (vk < s.cm);
+        const unsigned bal = __ballot_sync(0xffffffffu, lt);
+        if ((threadIdx.x & 31) == 0 && bal && s.count_lt != nullptr) atomicAdd(&s.count_lt[k], (unsigned long long)__popc(bal));
+        if (s.cell_pts <= 0) continue;
+        if (uniform) {
+            unsigned long long bits = (unsigned long long)__double_as_longlong(vk);
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                unsigned long long other = __shfl_xor_sync(0xffffffffu, bits, o);
+                bits = other < bits ? other : bits;
+            }
+            if ((threadIdx.x & 31) == 0) {
+                if (s.cell_min_bits != nullptr) atomicMin(&s.cell_min_bits[(size_t)cell0 * s.maxno + k], bits);
+                if (bal && s.cell_count != nullptr) atomicAdd(&s.cell_count[(size_t)cell0 * s.maxno + k], (unsigned long long)__popc(bal));
+            }
+        } else if (live) {
+            if (s.cell_min_bits != nullptr) atomicMin(&s.cell_min_bits[(size_t)cell * s.maxno + k], (unsigned long long)__double_as_longlong(vk));
+            if (lt && s.cell_count != nullptr) atomicAdd(&s.cell_count[(size_t)cell * s.maxno + k], 1ull);
+        }
+    }
+}
+
 struct ImpFuse {
-    double z, ve, cm;
-    int maxno, first, last;
+    double z, ve;
+    int first, last;
     double* Itop;                        // chunk's first point; in/out (out may be skipped on the last pass: store_top)
     int store_top;
-    long long cell_pts, first_index;     // global flat index of the chunk's first point (cells as in gpe_implausibility)
-    unsigned char* keep;                 // chunk's first point, or null
-    unsigned long long *count_lt, *cell_min_bits, *cell_count;      // [maxno], [ncell][maxno] (cell 0 = the cell of the call's first point)
-    long long cell_base;                 // index of that cell: (call's first_index) / cell_pts
+    long long first_index;               // global flat index of the chunk's first point
+    ImpStats st;                         // last pass (keep: the chunk's first point)
 };
+
+// h_a(x_j), the a-th mean basis function at point j: the caller's H* [m][q] when given, else the device polynomial basis
+__device__ __forceinline__ double basis_value(const double* __restrict__ Hs, int q, const double* __restrict__ P, int d,
+                                              const BasisDesc& bd, long long j, int a) {
+    if (Hs != nullptr) return Hs[(size_t)j * q + a];
+    if (a == 0) return 1.0;
+    const double x = P[(size_t)j * d + bd.idx[a]];
+    const int pw = bd.pw[a];
+    return (pw == 1) ? x : pow(x, (double)pw);
+}
+
+// Row a of the forward substitution kv = K^-1 h with the lower-triangular K (leading dimension LD), from kv[0:a] and h_a.
+// One row at a time: the callers use kv[a] as soon as it is ready.
+template <int LD>
+__device__ __forceinline__ double forward_subst_row(const double* K, const double (&kv)[NR], double h, int a) {
+    double s = h;
+    for (int k = 0; k < a; k++) s = fma(-K[a * LD + k], kv[k], s);
+    return s / K[a * LD + a];
+}
 
 // per point: mean, variance from the GEMM outputs
 template <bool IMP>
@@ -365,19 +447,7 @@ __global__ void __launch_bounds__(128) predict_finalize_kernel(const double* __r
     if (live) {
         double hv[NR];
 #pragma unroll
-        for (int a = 0; a < NR; a++) {
-            double v = 0.0;
-            if (a < q) {
-                if (Hs != nullptr) v = Hs[(size_t)j * q + a];
-                else if (a == 0) v = 1.0;
-                else {
-                    double x = P[(size_t)j * d + bd.idx[a]];
-                    int pw = bd.pw[a];
-                    v = (pw == 1) ? x : pow(x, (double)pw);
-                }
-            }
-            hv[a] = v;
-        }
+        for (int a = 0; a < NR; a++) hv[a] = (a < q) ? basis_value(Hs, q, P, d, bd, j, a) : 0.0;
         mu = aux[(size_t)q * ld + j];
 #pragma unroll
         for (int a = 0; a < NR; a++)
@@ -392,9 +462,7 @@ __global__ void __launch_bounds__(128) predict_finalize_kernel(const double* __r
 #pragma unroll
         for (int a = 0; a < NR; a++) {
             if (a < q) {
-                double s = hv[a];
-                for (int k = 0; k < a; k++) s = fma(-Ks[a][k], kv[k], s);
-                kv[a] = s / Ks[a][a];
+                kv[a] = forward_subst_row<NR + 1>(&Ks[0][0], kv, hv[a], a);
                 double g = kv[a] - aux[(size_t)a * ld + j];
                 gn = fma(g, g, gn);
             } else {
@@ -410,132 +478,41 @@ __global__ void __launch_bounds__(128) predict_finalize_kernel(const double* __r
         }
     }
     if (IMP) {
-        // this emulator's implausibility into the ascending top-maxno list (np.sort(np.partition(I, -maxno)[-maxno:]), :129)
+        // this emulator's implausibility into the running list; the last emulator's pass reduces the finished lists
+        const int maxno = imp.st.maxno;
         double top[MAXEM];
 #pragma unroll
         for (int k = 0; k < MAXEM; k++) top[k] = -1.0;
         if (live) {
             if (!imp.first)
-                for (int k = 0; k < imp.maxno; k++) top[k] = imp.Itop[(size_t)j * imp.maxno + k];
-            const double dz = mu - imp.z;
-            const double I = sqrt(dz * dz / (vj + imp.ve));
-            if (I > top[0]) {
-                top[0] = I;
-#pragma unroll
-                for (int k = 0; k < MAXEM - 1; k++) {
-                    if (k + 1 < imp.maxno && top[k] > top[k + 1]) {
-                        double t = top[k];
-                        top[k] = top[k + 1];
-                        top[k + 1] = t;
-                    }
-                }
-            }
+                for (int k = 0; k < maxno; k++) top[k] = imp.Itop[(size_t)j * maxno + k];
+            top_insert(top, maxno, implaus_value(mu, vj, imp.z, imp.ve));
             if (!imp.last || imp.store_top)
-                for (int k = 0; k < imp.maxno; k++) imp.Itop[(size_t)j * imp.maxno + k] = top[k];
+                for (int k = 0; k < maxno; k++) imp.Itop[(size_t)j * maxno + k] = top[k];
         }
         if (!imp.last) return;
-        // last emulator: the reductions of implaus_kernel on the finished list (warp-aggregated, integer atomics: deterministic)
-        if (live && imp.keep != nullptr) imp.keep[j] = (top[0] < imp.cm) ? 1 : 0;
-        const long long cell = (imp.cell_pts > 0 && live) ? (imp.first_index + j) / imp.cell_pts - imp.cell_base : -1;
-        const long long cell0 = __shfl_sync(0xffffffffu, cell, 0);
-        const bool uniform = imp.cell_pts > 0 && __all_sync(0xffffffffu, cell == cell0) && cell0 >= 0;
-        for (int k = 0; k < imp.maxno; k++) {
-            const double vk = top[imp.maxno - 1 - k];
-            const bool lt = live && (vk < imp.cm);
-            const unsigned bal = __ballot_sync(0xffffffffu, lt);
-            if ((threadIdx.x & 31) == 0 && bal && imp.count_lt != nullptr) atomicAdd(&imp.count_lt[k], (unsigned long long)__popc(bal));
-            if (imp.cell_pts <= 0) continue;
-            if (uniform) {
-                unsigned long long bits = (unsigned long long)__double_as_longlong(vk);
-#pragma unroll
-                for (int o = 16; o > 0; o >>= 1) {
-                    unsigned long long other = __shfl_xor_sync(0xffffffffu, bits, o);
-                    bits = other < bits ? other : bits;
-                }
-                if ((threadIdx.x & 31) == 0) {
-                    if (imp.cell_min_bits != nullptr) atomicMin(&imp.cell_min_bits[(size_t)cell0 * imp.maxno + k], bits);
-                    if (bal && imp.cell_count != nullptr) atomicAdd(&imp.cell_count[(size_t)cell0 * imp.maxno + k], (unsigned long long)__popc(bal));
-                }
-            } else if (live) {
-                if (imp.cell_min_bits != nullptr) atomicMin(&imp.cell_min_bits[(size_t)cell * imp.maxno + k], (unsigned long long)__double_as_longlong(vk));
-                if (lt && imp.cell_count != nullptr) atomicAdd(&imp.cell_count[(size_t)cell * imp.maxno + k], 1ull);
-            }
-        }
+        imp_finish(top, live, j, imp.first_index + j, imp.st);
     }
 }
 
-// K5: implausibility per point + reductions.  I >= 0, so the IEEE bit pattern orders like the value
-// and min-reductions can use integer atomics (deterministic).
 struct ImpDesc {
-    int n_emul, maxno;
+    int n_emul;
     double z[MAXEM], ve[MAXEM];
-    double cm;
 };
 
 __global__ void __launch_bounds__(256) implaus_kernel(const double* __restrict__ mean, const double* __restrict__ var, long long m,
-                                                      ImpDesc ds, long long cell_pts, long long first_index, double* __restrict__ Imax,
-                                                      unsigned char* __restrict__ keep, unsigned long long* __restrict__ count_lt,
-                                                      unsigned long long* __restrict__ cell_min_bits,
-                                                      unsigned long long* __restrict__ cell_count) {
-    long long r = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+                                                      ImpDesc ds, long long first_index, double* __restrict__ Imax, ImpStats st) {
+    const long long r = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     const bool live = r < m;
-    double top[MAXEM];   // ascending, top[maxno-1] is the largest
+    double top[MAXEM];
 #pragma unroll
     for (int k = 0; k < MAXEM; k++) top[k] = -1.0;
-    if (live) {
-        for (int o = 0; o < ds.n_emul; o++) {
-            double mu = mean[(size_t)o * m + r], v = var[(size_t)o * m + r];
-            double dz = mu - ds.z[o];
-            double I = sqrt(dz * dz / (v + ds.ve[o]));
-            // keep the maxno largest, ascending (np.sort(np.partition(I, -maxno)[-maxno:]))
-            if (I > top[0]) {
-                top[0] = I;
-#pragma unroll
-                for (int k = 0; k < MAXEM - 1; k++) {
-                    if (k + 1 < ds.maxno && top[k] > top[k + 1]) {
-                        double t = top[k];
-                        top[k] = top[k + 1];
-                        top[k + 1] = t;
-                    }
-                }
-            }
-        }
-    }
-    // outputs
-    for (int k = 0; k < ds.maxno; k++) {
-        double vk = top[k];
-        if (live && Imax != nullptr) Imax[(size_t)r * ds.maxno + k] = vk;
-    }
-    if (live && keep != nullptr) keep[r] = (top[0] < ds.cm) ? 1 : 0;
-    // cells are contiguous runs of cell_pts points, so a warp (32 consecutive points) almost always
-    // sits inside one cell: reduce in the warp first, one atomic per warp instead of one per point
-    // cells are runs of cell_pts points of the GLOBAL flat index first_index + r; the outputs start at the cell of point 0
-    const long long cell = (cell_pts > 0 && live) ? (first_index + r) / cell_pts - first_index / cell_pts : -1;
-    const long long cell0 = __shfl_sync(0xffffffffu, cell, 0);
-    const bool uniform = cell_pts > 0 && __all_sync(0xffffffffu, cell == cell0) && cell0 >= 0;
-    for (int k = 0; k < ds.maxno; k++) {
-        // k-th output statistic refers to the (k+1)-th largest: top[maxno-1-k]
-        double vk = top[ds.maxno - 1 - k];
-        bool lt = live && (vk < ds.cm);
-        unsigned bal = __ballot_sync(0xffffffffu, lt);
-        if ((threadIdx.x & 31) == 0 && bal && count_lt != nullptr) atomicAdd(&count_lt[k], (unsigned long long)__popc(bal));
-        if (cell_pts <= 0) continue;
-        if (uniform) {
-            unsigned long long bits = (unsigned long long)__double_as_longlong(vk);
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) {
-                unsigned long long other = __shfl_xor_sync(0xffffffffu, bits, o);
-                bits = other < bits ? other : bits;
-            }
-            if ((threadIdx.x & 31) == 0) {
-                if (cell_min_bits != nullptr) atomicMin(&cell_min_bits[(size_t)cell0 * ds.maxno + k], bits);
-                if (bal && cell_count != nullptr) atomicAdd(&cell_count[(size_t)cell0 * ds.maxno + k], (unsigned long long)__popc(bal));
-            }
-        } else if (live) {
-            if (cell_min_bits != nullptr) atomicMin(&cell_min_bits[(size_t)cell * ds.maxno + k], (unsigned long long)__double_as_longlong(vk));
-            if (lt && cell_count != nullptr) atomicAdd(&cell_count[(size_t)cell * ds.maxno + k], 1ull);
-        }
-    }
+    if (live)
+        for (int o = 0; o < ds.n_emul; o++)
+            top_insert(top, st.maxno, implaus_value(mean[(size_t)o * m + r], var[(size_t)o * m + r], ds.z[o], ds.ve[o]));
+    if (live && Imax != nullptr)
+        for (int k = 0; k < st.maxno; k++) Imax[(size_t)r * st.maxno + k] = top[k];
+    imp_finish(top, live, r, first_index + r, st);
 }
 
 // full posterior covariance assembly: V = sigma^2 (A* - Z^T Z + G^T G)
@@ -551,16 +528,7 @@ __global__ void fullcov_finalize_kernel(const double* __restrict__ ZtZ, int mp, 
         if (j >= m) return;
         double kv[NR];
         for (int a = 0; a < q; a++) {
-            double hvv;
-            if (Hs != nullptr) hvv = Hs[(size_t)j * q + a];
-            else if (a == 0) hvv = 1.0;
-            else {
-                double x = P[(size_t)j * d + bd.idx[a]];
-                hvv = (bd.pw[a] == 1) ? x : pow(x, (double)bd.pw[a]);
-            }
-            double s = hvv;
-            for (int k = 0; k < a; k++) s = fma(-Kf[a * NR + k], kv[k], s);
-            kv[a] = s / Kf[a * NR + a];
+            kv[a] = forward_subst_row<NR>(Kf, kv, basis_value(Hs, q, P, d, bd, j, a), a);
             Gbuf[(size_t)a * mp + j] = kv[a] - aux[(size_t)a * ld + j];
         }
         return;
@@ -688,15 +656,20 @@ int check_cells(gpe_handle* h, long long cell_pts, long long first_index, long l
 }
 
 // The implausibility reductions over a call's points: count_lt [maxno] and, with cells, cell_min [ncell][maxno] (bits of I >= 0,
-// which order like the value) and cell_count; finish() copies them to the caller's outputs (host, device or NULL) and waits.
+// which order like the value) and cell_count; stats() is what the kernels add into, finish() copies the sums to the caller's
+// outputs (host, device or NULL) and waits.
 struct ImpAccum {
     gpe_handle* h;
     int maxno;
-    long long ncell;        // 0 without cells (cell_pts == 0)
+    long long cell_pts, ncell;      // both 0 without cells
     unsigned long long *count_lt = nullptr, *cell_min = nullptr, *cell_count = nullptr;
     TmpDev t_cnt, t_cmin, t_ccnt;
-    ImpAccum(gpe_handle* h_, int maxno_, long long cell_pts, long long ncell_)
-        : h(h_), maxno(maxno_), ncell(cell_pts > 0 ? ncell_ : 0), t_cnt(h_), t_cmin(h_), t_ccnt(h_) {}
+    ImpAccum(gpe_handle* h_, int maxno_, long long cell_pts_, long long ncell_)
+        : h(h_), maxno(maxno_), cell_pts(ncell_ > 0 ? cell_pts_ : 0), ncell(cell_pts_ > 0 ? ncell_ : 0), t_cnt(h_), t_cmin(h_), t_ccnt(h_) {}
+    // first_index: global flat index of the call's first point; keep: the call's mask on the device, or null
+    ImpStats stats(double cm, long long first_index, unsigned char* keep) const {
+        return ImpStats{cm, maxno, cell_pts, cell_pts > 0 ? first_index / cell_pts : 0, keep, count_lt, cell_min, cell_count};
+    }
     int init() {
         CK(t_cnt.get(&count_lt, (size_t)maxno));
         CK(cudaMemsetAsync(count_lt, 0, sizeof(unsigned long long) * maxno, h->st));
@@ -857,8 +830,8 @@ static int predict_common(gpe_handle* h, const double* Xs, const double* Hs, con
         ImpFuse ic;
         if (imp_call) {          // this chunk's window of the per-point arrays
             ic = *imp_call;
-            ic.Itop += (size_t)s * ic.maxno;
-            if (ic.keep) ic.keep += s;
+            ic.Itop += (size_t)s * ic.st.maxno;
+            if (ic.st.keep) ic.st.keep += s;
             ic.first_index += s;
         }
         if ((rc = predict_chunk(h, sl, st, P, Hc, cnt, mc, mo, vo, use_sep ? &gx : nullptr, imp_call ? &ic : nullptr))) return rc;
@@ -905,21 +878,17 @@ int gpe_predict_implaus(gpe_handle* h, const double* Xs, const double* Hs, const
     if ((rc = check_cells(h, cell_pts, first_index, ncell, last ? m : 0))) return rc;
     NvtxRange nvtx("gpe_predict_implaus");
     CK(cudaSetDevice(h->device));
-    ImpFuse ic{};
-    ic.z = z; ic.ve = var_extra; ic.cm = cm; ic.maxno = maxno; ic.first = first != 0; ic.last = last != 0;
-    ic.store_top = Itop != nullptr;
-    ic.first_index = first_index; ic.cell_pts = last ? cell_pts : 0; ic.cell_base = cell_pts > 0 ? first_index / cell_pts : 0;
     TmpDev t_top(h);
-    ic.Itop = Itop;
-    if (!Itop) CK(t_top.get(&ic.Itop, (size_t)std::max<long long>(m, 1) * maxno));      // first == last: a one-emulator job
+    double* top = Itop;
+    if (!Itop) CK(t_top.get(&top, (size_t)std::max<long long>(m, 1) * maxno));      // first == last: a one-emulator job
     DevOut<unsigned char> ko(h);
     ImpAccum acc(h, maxno, cell_pts, ncell);
     if (last) {
         CK(ko.stage(keep, (size_t)m));
         if ((rc = acc.init())) return rc;
-        ic.keep = ko.p;
-        ic.count_lt = acc.count_lt; ic.cell_min_bits = acc.cell_min; ic.cell_count = acc.cell_count;
     }
+    const ImpFuse ic{.z = z, .ve = var_extra, .first = first != 0, .last = last != 0, .Itop = top, .store_top = Itop != nullptr,
+                     .first_index = first_index, .st = acc.stats(cm, first_index, ko.p)};
     if (m > 0) {
         if (Xs) {
             rc = predict_common(h, Xs, Hs, nullptr, 0, m, nullptr, nullptr, &ic);
@@ -1030,7 +999,7 @@ int gpe_implausibility(gpe_handle* h, const double* mean, const double* var, int
     NvtxRange nvtx("gpe_implausibility");
     CK(cudaSetDevice(h->device));
     ImpDesc ds;
-    ds.n_emul = n_emul; ds.maxno = maxno; ds.cm = cm;
+    ds.n_emul = n_emul;
     std::vector<double> zz, vv;
     CK(read_small(zz, z, n_emul));
     CK(read_small(vv, var_extra, n_emul));
@@ -1045,8 +1014,7 @@ int gpe_implausibility(gpe_handle* h, const double* mean, const double* var, int
     CK(ko.stage(keep, (size_t)m));
     if (int rc = acc.init()) return rc;
     if (m > 0) {                                                 // m == 0: zero counts, +huge cell minima
-        implaus_kernel<<<(unsigned)((m + 255) / 256), 256, 0, h->st>>>(md.p, vd.p, m, ds, acc.ncell > 0 ? cell_pts : 0, first_index, Io.p, ko.p,
-                                                                       acc.count_lt, acc.cell_min, acc.cell_count);
+        implaus_kernel<<<(unsigned)((m + 255) / 256), 256, 0, h->st>>>(md.p, vd.p, m, ds, first_index, Io.p, acc.stats(cm, first_index, ko.p));
         h->launches++;
     }
     CK(Io.flush());

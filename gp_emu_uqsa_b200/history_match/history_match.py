@@ -18,54 +18,6 @@ from ._hmutilfunctions import check_act, emulsetup, load_datafiles, make_sets, r
 __all__ = ["imp_plot", "imp_plot_recon", "nonimp_data", "new_wave_design"]
 
 
-def _device_buffers(n_emul, m):
-    import torch
-    dev = torch.device("cuda", _lib.default_device_index())
-    return (torch.empty((n_emul, m), dtype=torch.float64, device=dev), torch.empty((n_emul, m), dtype=torch.float64, device=dev))
-
-
-def _predict_all(emuls, zs, x, act_ref, active_fn):
-    """mean/var [n_emul, m] on device for the points x [m, num_inputs] (scaled, combined columns).
-    Emulators for which active_fn(E) is False contribute I = 0 (reference :93, :99-100): their slots
-    are filled with mean = z, var = 1."""
-    import torch
-    m = x.shape[0]
-    mean_d, var_d = _device_buffers(len(emuls), m)
-    busy = []
-    for o, E in enumerate(emuls):
-        if not active_fn(E):
-            mean_d[o].fill_(float(zs[o]))
-            var_d[o].fill_(1.0)
-            continue
-        cols = [act_ref[str(l)] for l in E.beliefs.active_index]
-        dev, _, _, st = E.training.fit(beta=E.par.beta, r_div=E.training._A_args[0])
-        if st != 0:
-            raise _lib.GpeError("training covariance matrix of emulator %d is not positive definite" % o)
-        xe = _np.ascontiguousarray(x[:, cols])
-        if E.basis.poly is not None:
-            # device-resident points + asynchronous handle: the emulators' predictions are enqueued back to back on
-            # their own streams and overlap; one wait per handle at the end
-            xd = torch.from_numpy(xe).to(mean_d.device)
-            dev.set_async(True)
-            dev.predict(xd, None, out=(mean_d[o], var_d[o]))
-            busy.append((dev, xd))
-        else:
-            dev.predict(xe, E.basis.design_matrix(xe), out=(mean_d[o], var_d[o]))
-    for dev, _ in busy:
-        dev.synchronize()
-        dev.set_async(False)
-    return mean_d, var_d
-
-
-def _implausibility(emuls, mean_d, var_d, zs, var_extra, cm, maxno, cell_pts=0, first_index=0):
-    dev = emuls[0].training.device()
-    import torch
-    keep = torch.empty(mean_d.shape[1], dtype=torch.uint8, device=mean_d.device)
-    _, _, count, cmin, ccnt = dev.implausibility(mean_d, var_d, zs, var_extra, cm, maxno=maxno, cell_pts=cell_pts,
-                                                  first_index=first_index, want_imax=False, out=(None, keep))
-    return keep, count, cmin, ccnt
-
-
 def _implausibility_fused(emuls, zs, var_extra, x, act_ref, active_fn, cm, maxno, cell_pts=0, first_index=0):
     """(keep, count, cell_min, cell_count) for the points x without the per-emulator mean / variance arrays: every active
     emulator's prediction folds its implausibility into the running top-``maxno`` list on the device
@@ -73,16 +25,20 @@ def _implausibility_fused(emuls, zs, var_extra, x, act_ref, active_fn, cm, maxno
     ``active_fn`` is False contribute I = 0 (reference :93, :99-100): they are entered as zeros in the initial list."""
     import torch
     active = [o for o, E in enumerate(emuls) if active_fn(E)]
-    if not active:
-        mean_d, var_d = _predict_all(emuls, zs, x, act_ref, active_fn)
-        return _implausibility(emuls, mean_d, var_d, zs, var_extra, cm, maxno, cell_pts=cell_pts, first_index=first_index)
     m = x.shape[0]
     tdev = torch.device("cuda", _lib.default_device_index())
+    keep = torch.empty(m, dtype=torch.uint8, device=tdev)
+    if not active:          # no prediction: every emulator enters with mean = z, var = 1, i.e. I = 0
+        mean = _np.repeat(_np.asarray(zs, dtype=_np.float64)[:, None], m, axis=1)
+        torch.cuda.current_stream(tdev).synchronize()      # the handle works on its own stream
+        _, _, count, cmin, ccnt = emuls[0].training.device().implausibility(mean, _np.ones_like(mean), zs, var_extra, cm, maxno=maxno,
+                                                                              cell_pts=cell_pts, first_index=first_index,
+                                                                              want_imax=False, out=(None, keep))
+        return keep, count, cmin, ccnt
     Itop = torch.full((m, maxno), -1.0, dtype=torch.float64, device=tdev)
     n_inactive = len(emuls) - len(active)
     if n_inactive:
         Itop[:, max(0, maxno - n_inactive):] = 0.0
-    keep = torch.empty(m, dtype=torch.uint8, device=tdev)
     torch.cuda.current_stream(tdev).synchronize()          # the handles work on their own streams
     res = None
     for pos, o in enumerate(active):
