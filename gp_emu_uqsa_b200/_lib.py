@@ -63,6 +63,7 @@ def load():
         "gpe_solve": (i, [p, p, i, p]),
         "gpe_sens_contract": (i, [p, p, p, p, d, p, i, p, p]),
         "gpe_sens_main_effect": (i, [p, p, p, p, p, p, d, p, i, p, i, p]),
+        "gpe_sens_sample": (i, [p, p, p, ll, p, i, d, p]),
         "gpe_dbg_gemm": (i, [p, p, p, p, i, i, i, ll, ll, ll, i, i, i, d, i, i, i, i, i]),
         "gpe_dbg_gemm_oz": (i, [p, p, p, p, i, i, i, ll, ll, ll, i, i, i, d, i, i, i, i, i, i, p, p, p, p, p]),
         "gpe_potrf": (i, [p, p, i, i, p, p, p, p]),
@@ -80,7 +81,7 @@ EXPORTS = ["gpe_version", "gpe_create", "gpe_destroy", "gpe_last_error", "gpe_la
            "gpe_get_stream", "gpe_set_streams", "gpe_set_async", "gpe_set_kernel", "gpe_synchronize", "gpe_profile_enable", "gpe_profile_read",
            "gpe_set_training", "gpe_set_basis", "gpe_cov_build", "gpe_cov_grad", "gpe_cross_cov", "gpe_llh_grad_batch",
            "gpe_fit_state", "gpe_loo", "gpe_predict", "gpe_predict_grid", "gpe_predict_fullcov", "gpe_implausibility", "gpe_predict_implaus",
-           "gpe_solve", "gpe_sens_contract", "gpe_sens_main_effect", "gpe_potrf", "gpe_pdist_argmin",
+           "gpe_solve", "gpe_sens_contract", "gpe_sens_main_effect", "gpe_sens_sample", "gpe_potrf", "gpe_pdist_argmin",
            "gpe_dbg_gemm", "gpe_dbg_gemm_oz", "gpe_dbg_potrf_inv", "gpe_dbg_int8_products"]
 
 
@@ -378,6 +379,19 @@ class Device:
         self._ck(self.L.gpe_sens_main_effect(self.h, _ptr(t1), _ptr(t2), _ptr(cdiag), _ptr(mvec), _ptr(evec), float(scale),
                                              _ptr(which), len(which), _ptr(xw), int(xw.shape[1]), _ptr(out)))
         return out
+
+    def sens_sample(self, XA, XB, which, shift=0.0, out=None):
+        """Pick-freeze sums of the sampled sensitivity terms (see gpe_sens_sample) for the samples XA, XB [M, d] (NumPy or
+        torch CUDA tensors) and the inputs ``which``: [2, 3 + 2 len(which)] = sums and sums of squares of
+        (t_E, t_V, t_EV, t_S[which], t_T[which]) over the M samples."""
+        if isinstance(XA, np.ndarray) or not hasattr(XA, "data_ptr"):
+            XA, XB = _f64(XA), _f64(XB)
+        if not hasattr(which, "data_ptr"):
+            which = np.ascontiguousarray(which, dtype=np.int32)
+        nw = int(which.numel()) if hasattr(which, "numel") else int(which.size)
+        sums = np.empty((2, 3 + 2 * nw)) if out is None else out
+        self._ck(self.L.gpe_sens_sample(self.h, _ptr(XA), _ptr(XB), int(XA.shape[0]), _ptr(which), nw, float(shift), _ptr(sums)))
+        return sums
 
     # ------------------------------------------------------------------ dense Cholesky
     def cholesky(self, A):

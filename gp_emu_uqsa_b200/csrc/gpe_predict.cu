@@ -692,6 +692,160 @@ struct ImpAccum {
     }
 };
 
+// K4s sampled sensitivity (gpe_sens_sample).  A chunk of Mc samples is evaluated as the (nw + 2) Mc explicit points
+// [A | B | AB_which[0] | ... ], Mc consecutive columns each; Z = L^-1 C of all of them is stored, and the posterior covariance of
+// a pair of columns is formed from their dot product in Z.
+constexpr int SS_MAXW = 16;
+constexpr int SS_PG = 4;         // inputs per CTA of the pair-dot pass: A and B are read once per four AB_P columns
+
+// P [(nw + 2) Mc][d]: column block 0 = A, 1 = B, 2 + k = A with input which[k] from B; samples >= cnt are zero rows
+__global__ void sens_compose_kernel(const double* __restrict__ XA, const double* __restrict__ XB, long long cnt, int Mc, int d,
+                                    const int* __restrict__ which, int nw, double* __restrict__ P) {
+    const long long j = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (j >= (long long)(nw + 2) * Mc) return;
+    const int b = (int)(j / Mc), i = (int)(j % Mc);
+    const int wk = b >= 2 ? which[b - 2] : -1;
+    for (int k = 0; k < d; k++) {
+        double v = 0.0;
+        if (i < cnt) v = (b == 1 || k == wk) ? XB[(size_t)i * d + k] : XA[(size_t)i * d + k];
+        P[j * d + k] = v;
+    }
+}
+
+// Tile partials of the pair dots over the rows [128 t, 128 t + 128) of Z (live rows < n):
+// part [t][3 + 3 nw][Mc] = |z_A|^2, |z_B|^2, z_A.z_B, then per input k |z_X|^2, z_B.z_X, z_A.z_X (X = AB_which[k]).
+// One thread per sample: consecutive threads read consecutive columns of Z.  CTA z handles inputs [4z, 4z + 4).
+__global__ void __launch_bounds__(128) sens_pairdot_kernel(const double* __restrict__ Z, int n, int Mc, int nw,
+                                                           double* __restrict__ part) {
+    const int i = blockIdx.x * 128 + threadIdx.x;
+    const int t = blockIdx.y, g0 = blockIdx.z * SS_PG;
+    const int ng = min(SS_PG, nw - g0), E = 3 + 3 * nw;
+    const size_t ld = (size_t)(nw + 2) * Mc;
+    const double* za = Z + i;
+    const double* zb = Z + Mc + i;
+    const double* zx = Z + (size_t)(2 + g0) * Mc + i;
+    double aa = 0.0, bb = 0.0, ab = 0.0, xx[SS_PG], bx[SS_PG], ax[SS_PG];
+#pragma unroll
+    for (int k = 0; k < SS_PG; k++) xx[k] = bx[k] = ax[k] = 0.0;
+    const int r1 = min(n, t * 128 + 128);
+#pragma unroll 2
+    for (int r = t * 128; r < r1; r++) {
+        const size_t o = (size_t)r * ld;
+        const double a = za[o], b = zb[o];
+        aa = fma(a, a, aa);
+        bb = fma(b, b, bb);
+        ab = fma(a, b, ab);
+#pragma unroll
+        for (int k = 0; k < SS_PG; k++) {
+            if (k < ng) {
+                const double x = zx[o + (size_t)k * Mc];
+                xx[k] = fma(x, x, xx[k]);
+                bx[k] = fma(b, x, bx[k]);
+                ax[k] = fma(a, x, ax[k]);
+            }
+        }
+    }
+    double* pp = part + (size_t)t * E * Mc + i;
+    if (blockIdx.z == 0) {
+        pp[0] = aa;
+        pp[(size_t)Mc] = bb;
+        pp[(size_t)2 * Mc] = ab;
+    }
+#pragma unroll
+    for (int k = 0; k < SS_PG; k++) {
+        if (k < ng) {
+            const size_t e = 3 + 3 * (size_t)(g0 + k);
+            pp[e * Mc] = xx[k];
+            pp[(e + 1) * Mc] = bx[k];
+            pp[(e + 2) * Mc] = ax[k];
+        }
+    }
+}
+
+// One thread per sample: the estimator terms (t_E, t_V, t_EV, t_S[k], t_T[k]) from the pair dots, the regression vectors
+// G [q][cols] (fullcov_finalize_kernel phase 0), the means and the prior of each pair; then the CTA's sums of the terms and of
+// their squares, each over its 128 samples in index order, into bpart [blk0 + CTA][2][3 + 2 nw].  Samples >= cnt add zero.
+template <int FAM>
+__global__ void __launch_bounds__(128) sens_sample_finalize_kernel(const double* __restrict__ part, int ntile, const double* __restrict__ aux,
+                                                                   const double* __restrict__ G, const double* __restrict__ P, BasisDesc bd,
+                                                                   int d, const double* __restrict__ winv, const double* __restrict__ beta,
+                                                                   const int* __restrict__ which, int nw, int Mc, long long cnt, double sigma2, double cscale,
+                                                                   double astar, double shift, double* __restrict__ bpart, long long blk0) {
+    extern __shared__ double terms[];        // [3 + 2 nw][128]
+    __shared__ double bs[NR];
+    const int q = bd.q, T = 3 + 2 * nw, E = 3 + 3 * nw;
+    const size_t cols = (size_t)(nw + 2) * Mc;
+    if (threadIdx.x < NR) bs[threadIdx.x] = beta[threadIdx.x];
+    __syncthreads();
+    const int i = blockIdx.x * 128 + threadIdx.x;
+    auto psum = [&](int e) {                 // tile partials in row-tile order
+        double s = 0.0;
+        for (int t = 0; t < ntile; t++) s += part[((size_t)t * E + e) * Mc + i];
+        return s;
+    };
+    auto mean = [&](size_t j) {              // as predict_finalize_kernel
+        double mu = aux[(size_t)q * cols + j];
+        for (int a = 0; a < q; a++) mu = fma(basis_value(nullptr, q, P, d, bd, (long long)j, a), bs[a], mu);
+        return mu;
+    };
+    auto gdot = [&](size_t x, size_t y) {
+        double s = 0.0;
+        for (int a = 0; a < q; a++) s = fma(G[(size_t)a * cols + x], G[(size_t)a * cols + y], s);
+        return s;
+    };
+    auto prior = [&](double D) { return cscale * (FAM == FAMILY_MATERN52 ? gpe_matern52(D) : gpe_exp(-D)); };
+    const size_t jA = i, jB = (size_t)Mc + i;
+    const double* pa = P + jA * d;
+    const double* pb = P + jB * d;
+    double Dab = 0.0;
+    for (int k = 0; k < d; k++) {
+        const double df = (pa[k] - pb[k]) * winv[k];
+        Dab = fma(df, df, Dab);
+    }
+    const double mA = mean(jA), mB = mean(jB);
+    const double vA = sigma2 * (astar - psum(0) + gdot(jA, jA)), vB = sigma2 * (astar - psum(1) + gdot(jB, jB));
+    const double cAB = sigma2 * (prior(Dab) - psum(2) + gdot(jA, jB));
+    double* col = terms + threadIdx.x;
+    col[0] = mA;
+    col[128] = cAB;
+    col[256] = 0.5 * ((mA - mB) * (mA - mB) + vA + vB - 2.0 * cAB);
+    for (int k = 0; k < nw; k++) {
+        const int w = which[k];
+        const size_t jX = (size_t)(2 + k) * Mc + i;
+        double Dbx = 0.0;                    // AB_w differs from B in every input but w, from A only in w
+        for (int kk = 0; kk < d; kk++) {
+            if (kk == w) continue;
+            const double df = (pa[kk] - pb[kk]) * winv[kk];
+            Dbx = fma(df, df, Dbx);
+        }
+        const double dfw = (pa[w] - pb[w]) * winv[w];
+        const double mX = mean(jX);
+        const double vX = sigma2 * (astar - psum(3 + 3 * k) + gdot(jX, jX));
+        const double cBX = sigma2 * (prior(Dbx) - psum(4 + 3 * k) + gdot(jB, jX));
+        const double cAX = sigma2 * (prior(dfw * dfw) - psum(5 + 3 * k) + gdot(jA, jX));
+        col[(3 + k) * 128] = (mB - shift) * (mX - mA) + cBX - cAB;
+        col[(3 + nw + k) * 128] = 0.5 * ((mA - mX) * (mA - mX) + vA + vX - 2.0 * cAX);
+    }
+    if (i >= cnt)
+        for (int t = 0; t < T; t++) col[t * 128] = 0.0;
+    __syncthreads();
+    for (int e = threadIdx.x; e < 2 * T; e += 128) {
+        const double* tv = terms + (e < T ? e : e - T) * 128;
+        double s = 0.0;
+        for (int r = 0; r < 128; r++) s = (e < T) ? s + tv[r] : fma(tv[r], tv[r], s);
+        bpart[(size_t)(blk0 + blockIdx.x) * 2 * T + e] = s;
+    }
+}
+
+// sums [w] = sum over the CTA partials bpart [nblk][w], in CTA order
+__global__ void sens_sample_reduce_kernel(const double* __restrict__ bpart, long long nblk, int w, double* __restrict__ sums) {
+    const int e = threadIdx.x;
+    if (e >= w) return;
+    double s = 0.0;
+    for (long long b = 0; b < nblk; b++) s += bpart[(size_t)b * w + e];
+    sums[e] = s;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1020,6 +1174,111 @@ int gpe_implausibility(gpe_handle* h, const double* mean, const double* var, int
     CK(Io.flush());
     CK(ko.flush());
     return acc.finish(count_lt, cell_min, cell_count);
+}
+
+int gpe_sens_sample(gpe_handle* h, const double* XA, const double* XB, long long M, const int* which, int nw, double shift,
+                    double* sums) {
+    if (h && M == 0) return 0;
+    if (!h || !XA || !XB || !which || !sums || M < 0) return h ? h->fail_msg("bad argument") : -2;
+    if (nw < 1 || nw > SS_MAXW) return h->fail_msg("gpe_sens_sample takes 1 <= nw <= 16 inputs");
+    if (!h->fitted) return h->fail_msg("gpe_fit_state has not succeeded on this handle");
+    if (!h->has_basis) return h->fail_msg("no H* given and no device basis set (gpe_set_basis)");
+    NvtxRange nvtx("gpe_sens_sample");
+    CK(cudaSetDevice(h->device));
+    std::vector<int> wv;
+    CK(read_small(wv, which, (size_t)nw));
+    for (int k = 0; k < nw; k++) {
+        if (wv[k] < 0 || wv[k] >= h->d) return h->fail_msg("which: every input must lie in [0, d)");
+        for (int k2 = 0; k2 < k; k2++)
+            if (wv[k2] == wv[k]) return h->fail_msg("which: the inputs must be distinct");
+    }
+    const int np = h->npad, d = h->d, q = h->q, nb = nw + 2, T = 3 + 2 * nw, E = 3 + 3 * nw;
+    // samples per chunk: a multiple of 256 (the INT8 route's column tile) with the chunk's nb Mc columns at most the prediction
+    // chunk, but never fewer than 256
+    const long long Mc = std::min<long long>(std::max<long long>(256, default_chunk(h) / nb / 256 * 256), (M + 255) / 256 * 256);
+    const int cols = (int)(nb * Mc);
+    const int ntile = (h->n + 127) / 128;
+    const long long nchunk = (M + Mc - 1) / Mc, nblk = nchunk * (Mc / 128);
+    int rc;
+    if ((rc = ensure_predict_ws(h, cols))) return rc;
+    DevIn<double> xa(h), xb(h);
+    DevIn<int> wd(h);
+    DevOut<double> so(h);
+    CK(xa.stage(XA, (size_t)M * d));
+    CK(xb.stage(XB, (size_t)M * d));
+    CK(wd.stage(which, (size_t)nw));
+    CK(so.stage(sums, (size_t)2 * T));
+    const bool two = nchunk > 1 && !h->prof_on;
+    TmpDev t_z[2] = {TmpDev(h), TmpDev(h)}, t_g[2] = {TmpDev(h), TmpDev(h)}, t_part[2] = {TmpDev(h), TmpDev(h)};
+    TmpDev t_bp(h);
+    double *Zs[2] = {nullptr, nullptr}, *Gs[2] = {nullptr, nullptr}, *Parts[2] = {nullptr, nullptr}, *bpart = nullptr;
+    for (int k = 0; k < (two ? 2 : 1); k++) {
+        CK(t_z[k].get(&Zs[k], (size_t)np * cols));
+        CK(t_g[k].get(&Gs[k], (size_t)q * cols));
+        CK(t_part[k].get(&Parts[k], (size_t)ntile * E * Mc));
+    }
+    CK(t_bp.get(&bpart, (size_t)nblk * 2 * T));
+    if (two) {
+        CK(cudaEventRecord(h->ev_fork, h->st));
+        for (int k = 0; k < 2; k++) CK(cudaStreamWaitEvent(h->sub_st[k], h->ev_fork, 0));
+    }
+    const BasisDesc bd = basis_of(h);
+    const double s2 = h->fit_sigma * h->fit_sigma;
+    const int kp = std::min(np, (h->n + GEMM_BK - 1) / GEMM_BK * GEMM_BK);
+    const int maux = (q + 1 <= 16) ? 16 : NR;
+    long long ci = 0;
+    for (long long s = 0; s < M; s += Mc, ci++) {
+        const int k = two ? (int)(ci & 1) : 0;
+        gpe_handle::PredSlot& sl = h->ps[k];
+        cudaStream_t st = two ? h->sub_st[k] : h->st;
+        const long long cnt = std::min(Mc, M - s);
+        {
+            ProfScope ps(h, gpe_handle::CAT_OTHER, st);
+            sens_compose_kernel<<<(unsigned)((cols + 127) / 128), 128, 0, st>>>(xa.p + (size_t)s * d, xb.p + (size_t)s * d, cnt, (int)Mc,
+                                                                               d, wd.p, nw, sl.X);
+        }
+        {
+            ProfScope ps(h, gpe_handle::CAT_COV, st);
+            CK(launch_xcov(h->family, h->fXs, sl.X, h->fwinv, h->n, d, np, cols, cols, h->fit_c, sl.C, cols, st));
+        }
+        h->launches += 2;
+        // aux = [A^-1 H K^-T | e]^T C, as in predict_chunk
+        if ((rc = gpe_gemm(h, st, {.A = h->fE, .B = sl.C, .C = sl.Aux, .lda = NR, .ldb = cols, .ldc = cols, .M = maux, .N = cols, .K = kp},
+                           GEMM_TN)))
+            return rc;
+        // Z = L^-1 C stored; on the INT8 route the residue planes of L^-1 are converted once per stream and fit state (the key
+        // differs from the prediction's swapped product) and every entry of C lies in [0, c]
+        GemmP z{.A = h->fLi, .B = sl.C, .C = Zs[k], .lda = np, .ldb = cols, .ldc = cols, .M = np, .N = cols, .K = np, .kmode = KM_LE_I};
+        const bool int8 = gpe_int8_route(h, st, z, GEMM_NN, EPI_STORE);
+        const OzHint hint = int8 ? OzHint{.reuse_a = true, .a_tag = h->fit_gen, .b_bound = h->fit_c} : OzHint();
+        if ((rc = gpe_gemm_routed(h, st, z, GEMM_NN, EPI_STORE, int8, hint))) return rc;
+        {
+            ProfScope ps(h, gpe_handle::CAT_OTHER, st);
+            sens_pairdot_kernel<<<dim3((unsigned)(Mc / 128), ntile, (nw + SS_PG - 1) / SS_PG), 128, 0, st>>>(Zs[k], h->n, (int)Mc, nw, Parts[k]);
+            fullcov_finalize_kernel<FAMILY_GAUSSIAN><<<(unsigned)((cols + 127) / 128), 128, 0, st>>>(
+                nullptr, cols, sl.Aux, cols, sl.X, nullptr, bd, d, h->fwinv, h->fK, s2, h->fit_c, h->fit_astar, nullptr, cols, Gs[k], nullptr, 0);
+            auto fin = h->family == FAMILY_MATERN52 ? sens_sample_finalize_kernel<FAMILY_MATERN52> : sens_sample_finalize_kernel<FAMILY_GAUSSIAN>;
+            fin<<<(unsigned)(Mc / 128), 128, (size_t)T * 128 * sizeof(double), st>>>(Parts[k], ntile, sl.Aux, Gs[k], sl.X, bd, d, h->fwinv,
+                                                                                      h->fbeta, wd.p, nw, (int)Mc, cnt, s2, h->fit_c, h->fit_astar,
+                                                                                      shift, bpart, ci * (Mc / 128));
+        }
+        h->launches += 3;
+    }
+    if (two) {
+        for (int k = 0; k < 2; k++) {
+            CK(cudaEventRecord(h->ev_join[k], h->sub_st[k]));
+            CK(cudaStreamWaitEvent(h->st, h->ev_join[k], 0));
+        }
+    }
+    {
+        ProfScope ps(h, gpe_handle::CAT_OTHER, h->st);
+        sens_sample_reduce_kernel<<<1, 128, 0, h->st>>>(bpart, nblk, 2 * T, so.p);
+    }
+    h->launches++;
+    CK(so.flush());
+    CK(cudaStreamSynchronize(h->st));
+    CK(cudaGetLastError());
+    return 0;
 }
 
 }  // extern "C"

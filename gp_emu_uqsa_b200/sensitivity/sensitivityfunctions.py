@@ -1,9 +1,10 @@
 """User-facing sensitivity functions (reference: gp_emu_uqsa/sensitivity/sensitivityfunctions.py)."""
 import numpy as _np
 
+from ._sampledsensitivity import SampledSensitivity
 from ._sensitivityclasses import Sensitivity
 
-__all__ = ["setup", "sense_table", "Sensitivity"]
+__all__ = ["setup", "setup_sampled", "sense_table", "Sensitivity", "SampledSensitivity"]
 
 
 def setup(emul, m, v, case="case2"):
@@ -33,6 +34,43 @@ def setup(emul, m, v, case="case2"):
               "the Matern 5/2 kernel. Return None.")
         return None
     return Sensitivity(emul, _np.array(m), _np.array(v))
+
+
+def setup_sampled(emul, m=None, v=None, bounds=None, samples=65536, seed=0):
+    """Return a SampledSensitivity instance (any covariance family, any polynomial mean) for independent inputs that are
+    either normal -- means ``m`` and variances ``v`` -- or uniform over ``bounds`` = [[lo, hi], ...], one entry per
+    active input in the units ``setup`` takes; ``samples`` (a power of two >= 256) Sobol points drawn with ``seed``.
+    None on bad arguments, with a message."""
+    print("\n*** Initialising SampledSensitivity class ***")
+    d = emul.training.inputs.shape[1]
+    normal = m is not None and v is not None
+    if (m is None) != (v is None) or normal == (bounds is not None):
+        print("ERROR: give either input means m and variances v, or uniform input bounds. Return None.")
+        return None
+    if normal:
+        ok = _np.shape(m) == (d,) and _np.shape(v) == (d,)
+        if not ok or not (_np.all(_np.isfinite(m)) and _np.all(_np.isfinite(v))):
+            print("Mean and Variance lists must both contain as many finite values "
+                  "as there are input dimensions. Return None.")
+            return None
+        if _np.any(_np.asarray(v, dtype=float) <= 0.0):
+            print("ERROR: input variances must be positive. Return None.")
+            return None
+    else:
+        if _np.shape(bounds) != (d, 2) or not _np.all(_np.isfinite(bounds)):
+            print("ERROR: bounds must hold one finite [lo, hi] pair per input dimension. Return None.")
+            return None
+        if _np.any(_np.asarray(bounds, dtype=float)[:, 0] >= _np.asarray(bounds, dtype=float)[:, 1]):
+            print("ERROR: every input range needs lo < hi. Return None.")
+            return None
+    if not isinstance(samples, (int, _np.integer)) or samples < 256 or samples & (samples - 1):
+        print("ERROR: samples must be a power of two of at least 256. Return None.")
+        return None
+    if emul.basis.poly is None:
+        print("The sampled sensitivity routines need a polynomial mean function "
+              "('1.0', 'x', 'x**k' terms). Return None.")
+        return None
+    return SampledSensitivity(emul, m=m, v=v, bounds=bounds, samples=int(samples), seed=seed)
 
 
 def sense_table(sense_list, inputNames=[], outputNames=[], rowHeight=6):

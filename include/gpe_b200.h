@@ -68,7 +68,8 @@ int gpe_set_streams(gpe_handle* h, int nstreams);
 /* Covariance family of the emulator this handle holds (GPE_KERNEL_*; Gaussian by default).  It applies to
  * gpe_cov_build, gpe_cov_grad, gpe_cross_cov, gpe_llh_grad_batch, gpe_fit_state, gpe_predict* and gpe_predict_implaus.
  * A change clears the fit state (gpe_fit_state must run again) and the captured likelihood graphs.  With MATERN52,
- * gpe_sens_contract and gpe_sens_main_effect fail: their closed-form integrals exist for the Gaussian only. */
+ * gpe_sens_contract and gpe_sens_main_effect fail: their closed-form integrals exist for the Gaussian only;
+ * gpe_sens_sample estimates the same quantities by sampling for both families. */
 int gpe_set_kernel(gpe_handle* h, int family);
 
 int gpe_set_async(gpe_handle* h, int on);
@@ -213,6 +214,25 @@ int gpe_sens_contract(gpe_handle* h, const double* gamma, const double* acoef, c
 int gpe_sens_main_effect(gpe_handle* h, const double* t1, const double* t2, const double* cdiag,
                          const double* mvec, const double* evec, double scale, const int* which,
                          int nwhich, const double* xw, int points, double* out);
+
+/* Sample-based uncertainty and sensitivity analysis on the posterior of the state gpe_fit_state factored (either family,
+ * every nugget form, sigma as given there); needs the device basis (gpe_set_basis).  A pick-freeze (Saltelli / Jansen)
+ * estimator: XA, XB [M,d] are two independent samples of the input distribution in the scaled training-input units, AB_P is
+ * XA with input P taken from XB, m / v the posterior mean / variance of gpe_predict and, for two distinct points,
+ * c(x,x') = sigma^2 [c R(D(x,x')) - z_x.z_x' + g_x.g_x'] with the off-diagonal prior (c = 1 - nugget or 1, z = L^-1 c_x,
+ * g = K^-1 h - (A^-1 H K^-T)^T c_x).  Per sample the terms are
+ *   t_E    = m(A)                                                    estimates E*[E f]
+ *   t_V    = c(A,B)                                                  Var*[E f]
+ *   t_EV   = (1/2) [(m(A) - m(B))^2 + v(A) + v(B) - 2 c(A,B)]        E*[Var f]
+ *   t_S[P] = (m(B) - shift)(m(AB_P) - m(A)) + c(B,AB_P) - c(A,B)     E*[V_P]     first-order variance of input P
+ *   t_T[P] = (1/2) [(m(A) - m(AB_P))^2 + v(A) + v(AB_P) - 2 c(A,AB_P)]  E*[V_T,P]  total-effect variance of input P
+ * (shift, e.g. the mean of the training outputs, lowers the variance of t_S and not its expectation).  which [nw]: 1 <= nw <= 16
+ * distinct inputs in [0, d).  sums [2][3 + 2 nw] (host or device): row 0 the sums over the M samples of
+ * (t_E, t_V, t_EV, t_S[which[0..nw)], t_T[which[0..nw)]), row 1 the sums of their squares.  Dividing by M gives the estimates.
+ * The result is the same bit for bit from call to call for the same samples and GPE_PRED_CHUNK; another chunk size only
+ * reorders the sums.  Cost: the posterior covariance of (nw + 2) M points, i.e. one prediction of that many points. */
+int gpe_sens_sample(gpe_handle* h, const double* XA, const double* XB, long long M, const int* which, int nw,
+                    double shift, double* sums);
 
 /* Maximin criterion of the optimised Latin hypercube (design_inputs/design_inputs.py:59-77):
  * argmin_out[k] = np.argmin(pdist(concat(designs[k], extra), 'sqeuclidean')) for N candidate designs
