@@ -127,6 +127,11 @@ __device__ __forceinline__ double gpe_matern52(double D) {
     double G;
     return gpe_matern52(D, G);   // (G is dead code here)
 }
+// Prior covariance c·k(D) of two distinct points at scaled squared distance D
+template <int FAM>
+__device__ __forceinline__ double cov_prior(double cscale, double D) {
+    return cscale * (FAM == FAMILY_MATERN52 ? gpe_matern52(D) : gpe_exp(-D));
+}
 
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll

@@ -3,11 +3,12 @@
 // (_emulatorclasses.py:607-631), kernel.covar (_emulatorkernels.py:75-79, :148-152),
 // history_match.py:121-136 / :237-250 / :317-329.
 //
-// Nothing of size m x m or n x m_total is ever materialised: points are processed in chunks;
+// Nothing of size m x m or n x m_total is ever materialised: points are processed in chunks (for_chunks);
 // per chunk the cross-covariance tile C [n, mc] is generated on device (optionally straight from
-// a flat grid index), Z = L^-1 C runs on the FP64 tensor pipe with the column norms |L^-1 c_j|^2
-// reduced in the GEMM epilogue, and a skinny product [A^-1 H K^-T | e]^T C gives the mean and the
-// regression-variance term.   v_j = sigma^2 (a*_jj - |L^-1 c_j|^2 + |K^-1 h_j - (Gm K^-T)^T c_j|^2).
+// a flat grid index) and a skinny product [A^-1 H K^-T | e]^T C gives the mean and the regression-variance
+// term (posterior_cross), and Z = L^-1 C runs with the column norms |L^-1 c_j|^2 reduced in the GEMM
+// epilogue (fit_z_product).   v_j = sigma^2 (a*_jj - |L^-1 c_j|^2 + |K^-1 h_j - (Gm K^-T)^T c_j|^2).
+// gpe_predict_fullcov and gpe_sens_sample build on the same steps.
 #include "gpe_handle.h"
 
 #include <algorithm>
@@ -541,8 +542,7 @@ __global__ void fullcov_finalize_kernel(const double* __restrict__ ZtZ, int mp, 
         double df = P[(size_t)i * d + k] * winv[k] - P[(size_t)j * d + k] * winv[k];
         D = fma(df, df, D);
     }
-    double prior = (i == j) ? (astar + (r_new ? r_new[i] : 0.0))
-                            : cscale * (FAM == FAMILY_MATERN52 ? gpe_matern52(D) : gpe_exp(-D));
+    double prior = (i == j) ? (astar + (r_new ? r_new[i] : 0.0)) : cov_prior<FAM>(cscale, D);
     double gg = 0.0;
     for (int a = 0; a < q; a++) gg = fma(Gbuf[(size_t)a * mp + i], Gbuf[(size_t)a * mp + j], gg);
     V[idx] = sigma2 * (prior - ZtZ[(size_t)i * mp + j] + gg);
@@ -579,47 +579,94 @@ long long default_chunk(gpe_handle* h) {
     return (c + 127) / 128 * 128;
 }
 
+// The fit state a posterior entry point works on; has_H: the caller gives H* for its points
+int check_fit(gpe_handle* h, bool has_H) {
+    if (!h->fitted) return h->fail_msg("gpe_fit_state has not succeeded on this handle");
+    if (!has_H && !h->has_basis) return h->fail_msg("no H* given and no device basis set (gpe_set_basis)");
+    return 0;
+}
+
+// The caller's points Xs [cnt][d] (host or device memory) into the device buffer P [mc][d], rows >= cnt zero
+cudaError_t stage_points(double* P, const double* Xs, long long cnt, int mc, int d, cudaStream_t st) {
+    if (cnt < mc)
+        if (cudaError_t e = cudaMemsetAsync(P, 0, (size_t)mc * d * sizeof(double), st); e != cudaSuccess) return e;
+    return cudaMemcpyAsync(P, Xs, (size_t)cnt * d * sizeof(double), cudaMemcpyDefault, st);
+}
+
+// Rows / columns >= n of the padded matrices are identity padding and the slab's rows >= n are zero: the DMMA products over the
+// slab need only the first n rounded up to the k-tile (n = 2000: 2000 instead of 2048 -- the last, heaviest row tile of the
+// triangular product has 80 live rows, not 128)
+int live_k(const gpe_handle* h) { return std::min(h->npad, (h->n + GEMM_BK - 1) / GEMM_BK * GEMM_BK); }
+
+// The slab C [npad][cols] = c K(training, points) of the points P [cols][d] or of the grid chunk gx (columns >= count zero), and
+// aux = [A^-1 H K^-T | e]^T C (TN, skinny: the q + 1 live columns of the panel padded to 16 or 32 rows)
+int posterior_cross(gpe_handle* h, cudaStream_t st, const double* P, const GridXcov* gx, int cols, long long count, double* C,
+                    double* aux) {
+    {
+        ProfScope ps(h, gpe_handle::CAT_COV, st);
+        if (gx != nullptr) CK(launch_xcov_grid(h->family, gx->T, gx->sp, h->n, h->npad, cols, gx->start, count, h->fit_c, C, gx->smem, st));
+        else CK(launch_xcov(h->family, h->fXs, P, h->fwinv, h->n, h->d, h->npad, cols, count, h->fit_c, C, cols, st));
+    }
+    h->launches++;
+    const int maux = (h->q + 1 <= 16) ? 16 : NR;
+    return gpe_gemm(h, st, {.A = h->fE, .B = C, .C = aux, .lda = NR, .ldb = cols, .ldc = cols, .M = maux, .N = cols, .K = live_k(h)},
+                    GEMM_TN);
+}
+
+// Z = L^-1 C of the fit state (L^-1 lower: k <= i), stored into out (EPI_STORE) or reduced to column norms in the epilogue, tile
+// partials out [*ntile][cols] (EPI_SUMSQ).  The route is decided once: the plan below is the route taken.
+int fit_z_product(gpe_handle* h, cudaStream_t st, const double* C, int cols, double* out, int epi, int* ntile = nullptr) {
+    const int np = h->npad;
+    GemmP z{.A = h->fLi, .B = C, .C = out, .lda = np, .ldb = cols, .ldc = cols, .M = np, .N = cols, .K = np, .kmode = KM_LE_I};
+    OzHint hint;
+    const bool int8 = gpe_int8_route(h, st, z, GEMM_NN, epi);
+    if (int8) {
+        // INT8 tensor-core route (gpe_ozaki.cuh): the residue planes of L^-1 are made once per fit, stream and layout (the tag is
+        // the generation of the fit state), the padded size is used (rows >= n of Z are zero).  Every entry of the slab is
+        // c exp(-D) or c R(D), in [0, c]: one scale for all points, no pass over the slab for its maxima.  (A point far from
+        // every training input then keeps fewer significant bits of its tiny column -- its variance is the prior's to the same
+        // absolute accuracy, which is what the subtraction prior - |Z|^2 needs.)
+        hint = OzHint{.reuse_a = true, .a_tag = h->fit_gen, .b_bound = h->fit_c};
+    } else if (epi == EPI_SUMSQ) {      // the ragged last row tile exists for the column norms only
+        z.M = z.K = live_k(h);
+    }
+    if (int rc = gpe_gemm_routed(h, st, z, GEMM_NN, epi, int8, hint)) return rc;
+    if (ntile != nullptr) *ntile = (int8 && oz_sumsq_swapped(z, epi)) ? 1 : (z.M + 127) / 128;
+    return 0;
+}
+
+// Chunks alternate between two (stream, buffer slot) pairs when there is more than one and profiling is off: a slot's buffers
+// are reused only by later chunks of the same stream, which orders them.
+int chunk_slots(const gpe_handle* h, long long nchunk) { return (nchunk > 1 && !h->prof_on) ? 2 : 1; }
+
+// body(ci, slot, stream) for the chunks ci = 0 .. nchunk - 1, forked from the handle's stream and joined back into it
+template <class Body>
+int for_chunks(gpe_handle* h, long long nchunk, Body body) {
+    const bool two = chunk_slots(h, nchunk) == 2;
+    if (two) {
+        CK(cudaEventRecord(h->ev_fork, h->st));
+        for (int k = 0; k < 2; k++) CK(cudaStreamWaitEvent(h->sub_st[k], h->ev_fork, 0));
+    }
+    for (long long ci = 0; ci < nchunk; ci++) {
+        const int k = two ? (int)(ci & 1) : 0;
+        if (int rc = body(ci, k, two ? h->sub_st[k] : h->st)) return rc;
+    }
+    if (two) {
+        for (int k = 0; k < 2; k++) {
+            CK(cudaEventRecord(h->ev_join[k], h->sub_st[k]));
+            CK(cudaStreamWaitEvent(h->st, h->ev_join[k], 0));
+        }
+    }
+    return 0;
+}
+
 // One chunk on stream `st` with the buffers of `sl`: points already in P_dev [mc, d] (rows >= count
 // arbitrary but finite).
 int predict_chunk(gpe_handle* h, gpe_handle::PredSlot& sl, cudaStream_t st, const double* P_dev, const double* Hs_dev,
                   long long count, int mc, double* mean_dev, double* var_dev, const GridXcov* gx = nullptr, const ImpFuse* imp = nullptr) {
-    const int np = h->npad;
-    {
-        ProfScope ps(h, gpe_handle::CAT_COV, st);
-        if (gx != nullptr) CK(launch_xcov_grid(h->family, gx->T, gx->sp, h->n, np, mc, gx->start, count, h->fit_c, sl.C, gx->smem, st));
-        else CK(launch_xcov(h->family, h->fXs, P_dev, h->fwinv, h->n, h->d, np, mc, count, h->fit_c, sl.C, mc, st));
-    }
-    h->launches++;
-    int rc;
-    // aux = [A^-1 H K^-T | e]^T C     (TN, skinny: the q + 1 live columns of the panel padded to 16 or 32 rows)
-    // rows / columns >= n of the padded matrices are identity padding and the slab's rows >= n are zero: the products need
-    // only the first kp = n rounded up to the k-tile (n = 2000: 2000 instead of 2048 -- the last, heaviest row tile of the
-    // triangular product has 80 live rows, not 128)
-    const int kp = std::min(np, (h->n + GEMM_BK - 1) / GEMM_BK * GEMM_BK);
-    const int maux = (h->q + 1 <= 16) ? 16 : NR;
-    if ((rc = gpe_gemm(h, st, {.A = h->fE, .B = sl.C, .C = sl.Aux, .lda = NR, .ldb = mc, .ldc = mc, .M = maux, .N = mc, .K = kp}, GEMM_TN)))
-        return rc;
-    int ntile = 0;
-    if (var_dev != nullptr || imp != nullptr) {
-        // column norms of Z = Linv C    (Linv lower: k <= i), reduced in the epilogue
-        GemmP z{.A = h->fLi, .B = sl.C, .C = sl.Part, .lda = np, .ldb = mc, .ldc = mc, .M = np, .N = mc, .K = np, .kmode = KM_LE_I};
-        OzHint hint;
-        bool one_row = false;
-        const bool int8 = gpe_int8_route(h, st, z, GEMM_NN, EPI_SUMSQ);      // decided once: the plan below is the route taken
-        if (int8) {
-            // INT8 tensor-core route (gpe_ozaki.cuh): the residue planes of L^-1 are made once per fit and stream (the tag is the
-            // generation of the fit state), the padded size is used (rows >= n of Z are zero).  Every entry of the slab is
-            // c exp(-D) or c R(D), in [0, c]: one scale for all points, no pass over the slab for its maxima.  (A point far from
-            // every training input then keeps fewer significant bits of its tiny column -- its variance is the prior's to the same
-            // absolute accuracy, which is what the subtraction prior - |Z|^2 needs.)
-            hint = OzHint{.reuse_a = true, .a_tag = h->fit_gen, .b_bound = h->fit_c};
-            one_row = oz_sumsq_swapped(z, EPI_SUMSQ);
-        } else {
-            z.M = z.K = kp;
-        }
-        if ((rc = gpe_gemm_routed(h, st, z, GEMM_NN, EPI_SUMSQ, int8, hint))) return rc;
-        ntile = one_row ? 1 : (z.M + 127) / 128;
-    }
+    int rc, ntile = 0;
+    if ((rc = posterior_cross(h, st, P_dev, gx, mc, count, sl.C, sl.Aux))) return rc;
+    if ((var_dev != nullptr || imp != nullptr) && (rc = fit_z_product(h, st, sl.C, mc, sl.Part, EPI_SUMSQ, &ntile))) return rc;
     {
         ProfScope ps(h, gpe_handle::CAT_OTHER, st);
         if (imp != nullptr)
@@ -793,7 +840,6 @@ __global__ void __launch_bounds__(128) sens_sample_finalize_kernel(const double*
         for (int a = 0; a < q; a++) s = fma(G[(size_t)a * cols + x], G[(size_t)a * cols + y], s);
         return s;
     };
-    auto prior = [&](double D) { return cscale * (FAM == FAMILY_MATERN52 ? gpe_matern52(D) : gpe_exp(-D)); };
     const size_t jA = i, jB = (size_t)Mc + i;
     const double* pa = P + jA * d;
     const double* pb = P + jB * d;
@@ -804,7 +850,7 @@ __global__ void __launch_bounds__(128) sens_sample_finalize_kernel(const double*
     }
     const double mA = mean(jA), mB = mean(jB);
     const double vA = sigma2 * (astar - psum(0) + gdot(jA, jA)), vB = sigma2 * (astar - psum(1) + gdot(jB, jB));
-    const double cAB = sigma2 * (prior(Dab) - psum(2) + gdot(jA, jB));
+    const double cAB = sigma2 * (cov_prior<FAM>(cscale, Dab) - psum(2) + gdot(jA, jB));
     double* col = terms + threadIdx.x;
     col[0] = mA;
     col[128] = cAB;
@@ -821,8 +867,8 @@ __global__ void __launch_bounds__(128) sens_sample_finalize_kernel(const double*
         const double dfw = (pa[w] - pb[w]) * winv[w];
         const double mX = mean(jX);
         const double vX = sigma2 * (astar - psum(3 + 3 * k) + gdot(jX, jX));
-        const double cBX = sigma2 * (prior(Dbx) - psum(4 + 3 * k) + gdot(jB, jX));
-        const double cAX = sigma2 * (prior(dfw * dfw) - psum(5 + 3 * k) + gdot(jA, jX));
+        const double cBX = sigma2 * (cov_prior<FAM>(cscale, Dbx) - psum(4 + 3 * k) + gdot(jB, jX));
+        const double cAX = sigma2 * (cov_prior<FAM>(cscale, dfw * dfw) - psum(5 + 3 * k) + gdot(jA, jX));
         col[(3 + k) * 128] = (mB - shift) * (mX - mA) + cBX - cAB;
         col[(3 + nw + k) * 128] = 0.5 * ((mA - mX) * (mA - mX) + vA + vX - 2.0 * cAX);
     }
@@ -911,15 +957,12 @@ int gpe_fit_state(gpe_handle* h, const double* delta, double nugget, double sigm
 
 static int predict_common(gpe_handle* h, const double* Xs, const double* Hs, const GridDesc* grid, long long start,
                           long long m, double* mean, double* var, const ImpFuse* imp_call = nullptr) {
-    if (!h->fitted) return h->fail_msg("gpe_fit_state has not succeeded on this handle");
-    if (!Hs && !h->has_basis) return h->fail_msg("no H* given and no device basis set (gpe_set_basis)");
+    int rc;
+    if ((rc = check_fit(h, Hs != nullptr))) return rc;
     NvtxRange nvtx(grid ? "gpe_predict_grid" : "gpe_predict");
     CK(cudaSetDevice(h->device));
     long long chunk = std::min<long long>(default_chunk(h), (m + 127) / 128 * 128);
-    int rc;
     if ((rc = ensure_predict_ws(h, chunk))) return rc;
-    // Chunks alternate between two (stream, buffer slot) pairs: a slot's staging buffers are reused only
-    // by later chunks of the same stream, which orders them.
     const bool x_dev = Xs && gpe_is_device_ptr(Xs), h_dev = Hs && gpe_is_device_ptr(Hs);
     const bool mean_dev = imp_call || gpe_is_device_ptr(mean), var_dev = var && gpe_is_device_ptr(var);
     const int d = h->d, q = h->q;
@@ -947,17 +990,10 @@ static int predict_common(gpe_handle* h, const double* Xs, const double* Hs, con
             use_sep = true;
         }
     }
-    const bool two = m > chunk && !h->prof_on;
-    if (two) {
-        CK(cudaEventRecord(h->ev_fork, h->st));
-        for (int k = 0; k < 2; k++) CK(cudaStreamWaitEvent(h->sub_st[k], h->ev_fork, 0));
-    }
-    int ci = 0;
-    for (long long s = 0; s < m; s += chunk, ci++) {
-        gpe_handle::PredSlot& sl = h->ps[two ? (ci & 1) : 0];
-        cudaStream_t st = two ? h->sub_st[ci & 1] : h->st;
-        long long cnt = std::min(chunk, m - s);
-        int mc = (int)((cnt + 127) / 128 * 128);
+    rc = for_chunks(h, (m + chunk - 1) / chunk, [&](long long ci, int k, cudaStream_t st) {
+        gpe_handle::PredSlot& sl = h->ps[k];
+        const long long s = ci * chunk, cnt = std::min(chunk, m - s);
+        const int mc = (int)((cnt + 127) / 128 * 128);
         const double* P = nullptr;
         if (grid) {
             grid_points_kernel<<<(mc + 255) / 256, 256, 0, st>>>(*grid, start + s, cnt, mc, sl.X);
@@ -966,8 +1002,7 @@ static int predict_common(gpe_handle* h, const double* Xs, const double* Hs, con
         } else if (x_dev && cnt == mc) {
             P = Xs + (size_t)s * d;
         } else {
-            if (cnt < mc) CK(cudaMemsetAsync(sl.X, 0, (size_t)mc * d * sizeof(double), st));
-            CK(cudaMemcpyAsync(sl.X, Xs + (size_t)s * d, (size_t)cnt * d * sizeof(double), cudaMemcpyDefault, st));
+            CK(stage_points(sl.X, Xs + (size_t)s * d, cnt, mc, d, st));
             P = sl.X;
         }
         const double* Hc = nullptr;
@@ -991,13 +1026,9 @@ static int predict_common(gpe_handle* h, const double* Xs, const double* Hs, con
         if ((rc = predict_chunk(h, sl, st, P, Hc, cnt, mc, mo, vo, use_sep ? &gx : nullptr, imp_call ? &ic : nullptr))) return rc;
         if (!mean_dev) CK(cudaMemcpyAsync(mean + s, sl.Mean, cnt * sizeof(double), cudaMemcpyDeviceToHost, st));
         if (var && !var_dev) CK(cudaMemcpyAsync(var + s, sl.Var, cnt * sizeof(double), cudaMemcpyDeviceToHost, st));
-    }
-    if (two) {
-        for (int k = 0; k < 2; k++) {
-            CK(cudaEventRecord(h->ev_join[k], h->sub_st[k]));
-            CK(cudaStreamWaitEvent(h->st, h->ev_join[k], 0));
-        }
-    }
+        return 0;
+    });
+    if (rc) return rc;
     // asynchronous mode (gpe_set_async): with device-resident points and outputs nothing on the host waits for this call
     const bool all_dev = mean_dev && (!var || var_dev) && (!Xs || x_dev) && (!Hs || h_dev) && !(imp_call && imp_call->last);
     if (!(h->async && all_dev)) CK(cudaStreamSynchronize(h->st));
@@ -1075,8 +1106,7 @@ int gpe_cross_cov(gpe_handle* h, const double* delta, double nugget, int kind, c
     CK(t_P.get(&P, (size_t)mc * d));
     CK(t_Cm.get(&Cm, (size_t)np * mc));
     CK(cudaMemcpyAsync(wd, w.data(), sizeof(double) * d, cudaMemcpyHostToDevice, h->st));
-    CK(cudaMemsetAsync(P, 0, sizeof(double) * (size_t)mc * d, h->st));
-    CK(cudaMemcpyAsync(P, Xs, sizeof(double) * (size_t)m * d, cudaMemcpyDefault, h->st));
+    CK(stage_points(P, Xs, m, mc, d, h->st));
     scale_train_kernel<<<(d * np + 255) / 256, 256, 0, h->st>>>(h->X, wd, h->n, d, np, xs);
     CK(launch_xcov(h->family, xs, P, wd, h->n, d, np, mc, m, kind ? 1.0 : 1.0 - nugget, Cm, mc, h->st));
     h->launches += 2;
@@ -1092,8 +1122,8 @@ int gpe_predict_fullcov(gpe_handle* h, const double* Xs, const double* Hs, int m
                         double* V) {
     if (h && m == 0) return 0;
     if (!h || !Xs || !mean || !V || m < 1) return h ? h->fail_msg("bad argument") : -2;
-    if (!h->fitted) return h->fail_msg("gpe_fit_state has not succeeded on this handle");
-    if (!Hs && !h->has_basis) return h->fail_msg("no H* given and no device basis set (gpe_set_basis)");
+    int rc;
+    if ((rc = check_fit(h, Hs != nullptr))) return rc;
     NvtxRange nvtx("gpe_predict_fullcov");
     CK(cudaSetDevice(h->device));
     const int np = h->npad, d = h->d, q = h->q;
@@ -1110,14 +1140,10 @@ int gpe_predict_fullcov(gpe_handle* h, const double* Xs, const double* Hs, int m
     CK(t_G.get(&G, (size_t)NR * mp));
     CK(md.stage(mean, (size_t)m));
     CK(Vd.stage(V, (size_t)m * m));
-    CK(cudaMemsetAsync(P, 0, sizeof(double) * (size_t)mp * d, h->st));
-    CK(cudaMemcpyAsync(P, Xs, sizeof(double) * (size_t)m * d, cudaMemcpyDefault, h->st));
+    CK(stage_points(P, Xs, m, mp, d, h->st));
     CK(Hd.stage(Hs, (size_t)m * q));
     CK(rn.stage(r_new, (size_t)m));
-    CK(launch_xcov(h->family, h->fXs, P, h->fwinv, h->n, d, np, mp, m, h->fit_c, Cm, mp, h->st));
-    h->launches++;
-    int rc = 0;
-    if (!rc) rc = gpe_gemm(h, h->st, {.A = h->fE, .B = Cm, .C = aux, .lda = NR, .ldb = mp, .ldc = mp, .M = NR, .N = mp, .K = np}, GEMM_TN);
+    rc = posterior_cross(h, h->st, P, nullptr, mp, m, Cm, aux);
     if (!rc)
         rc = gpe_gemm(h, h->st, {.A = h->fLi, .B = Cm, .C = Zm, .lda = np, .ldb = mp, .ldc = mp, .M = np, .N = mp, .K = np, .kmode = KM_LE_I},
                       GEMM_NN);
@@ -1181,8 +1207,8 @@ int gpe_sens_sample(gpe_handle* h, const double* XA, const double* XB, long long
     if (h && M == 0) return 0;
     if (!h || !XA || !XB || !which || !sums || M < 0) return h ? h->fail_msg("bad argument") : -2;
     if (nw < 1 || nw > SS_MAXW) return h->fail_msg("gpe_sens_sample takes 1 <= nw <= 16 inputs");
-    if (!h->fitted) return h->fail_msg("gpe_fit_state has not succeeded on this handle");
-    if (!h->has_basis) return h->fail_msg("no H* given and no device basis set (gpe_set_basis)");
+    int rc;
+    if ((rc = check_fit(h, false))) return rc;
     NvtxRange nvtx("gpe_sens_sample");
     CK(cudaSetDevice(h->device));
     std::vector<int> wv;
@@ -1199,7 +1225,6 @@ int gpe_sens_sample(gpe_handle* h, const double* XA, const double* XB, long long
     const int cols = (int)(nb * Mc);
     const int ntile = (h->n + 127) / 128;
     const long long nchunk = (M + Mc - 1) / Mc, nblk = nchunk * (Mc / 128);
-    int rc;
     if ((rc = ensure_predict_ws(h, cols))) return rc;
     DevIn<double> xa(h), xb(h);
     DevIn<int> wd(h);
@@ -1208,50 +1233,28 @@ int gpe_sens_sample(gpe_handle* h, const double* XA, const double* XB, long long
     CK(xb.stage(XB, (size_t)M * d));
     CK(wd.stage(which, (size_t)nw));
     CK(so.stage(sums, (size_t)2 * T));
-    const bool two = nchunk > 1 && !h->prof_on;
     TmpDev t_z[2] = {TmpDev(h), TmpDev(h)}, t_g[2] = {TmpDev(h), TmpDev(h)}, t_part[2] = {TmpDev(h), TmpDev(h)};
     TmpDev t_bp(h);
     double *Zs[2] = {nullptr, nullptr}, *Gs[2] = {nullptr, nullptr}, *Parts[2] = {nullptr, nullptr}, *bpart = nullptr;
-    for (int k = 0; k < (two ? 2 : 1); k++) {
+    for (int k = 0; k < chunk_slots(h, nchunk); k++) {
         CK(t_z[k].get(&Zs[k], (size_t)np * cols));
         CK(t_g[k].get(&Gs[k], (size_t)q * cols));
         CK(t_part[k].get(&Parts[k], (size_t)ntile * E * Mc));
     }
     CK(t_bp.get(&bpart, (size_t)nblk * 2 * T));
-    if (two) {
-        CK(cudaEventRecord(h->ev_fork, h->st));
-        for (int k = 0; k < 2; k++) CK(cudaStreamWaitEvent(h->sub_st[k], h->ev_fork, 0));
-    }
     const BasisDesc bd = basis_of(h);
     const double s2 = h->fit_sigma * h->fit_sigma;
-    const int kp = std::min(np, (h->n + GEMM_BK - 1) / GEMM_BK * GEMM_BK);
-    const int maux = (q + 1 <= 16) ? 16 : NR;
-    long long ci = 0;
-    for (long long s = 0; s < M; s += Mc, ci++) {
-        const int k = two ? (int)(ci & 1) : 0;
+    rc = for_chunks(h, nchunk, [&](long long ci, int k, cudaStream_t st) {
         gpe_handle::PredSlot& sl = h->ps[k];
-        cudaStream_t st = two ? h->sub_st[k] : h->st;
-        const long long cnt = std::min(Mc, M - s);
+        const long long s = ci * Mc, cnt = std::min(Mc, M - s);
         {
             ProfScope ps(h, gpe_handle::CAT_OTHER, st);
             sens_compose_kernel<<<(unsigned)((cols + 127) / 128), 128, 0, st>>>(xa.p + (size_t)s * d, xb.p + (size_t)s * d, cnt, (int)Mc,
                                                                                d, wd.p, nw, sl.X);
         }
-        {
-            ProfScope ps(h, gpe_handle::CAT_COV, st);
-            CK(launch_xcov(h->family, h->fXs, sl.X, h->fwinv, h->n, d, np, cols, cols, h->fit_c, sl.C, cols, st));
-        }
-        h->launches += 2;
-        // aux = [A^-1 H K^-T | e]^T C, as in predict_chunk
-        if ((rc = gpe_gemm(h, st, {.A = h->fE, .B = sl.C, .C = sl.Aux, .lda = NR, .ldb = cols, .ldc = cols, .M = maux, .N = cols, .K = kp},
-                           GEMM_TN)))
-            return rc;
-        // Z = L^-1 C stored; on the INT8 route the residue planes of L^-1 are converted once per stream and fit state (the key
-        // differs from the prediction's swapped product) and every entry of C lies in [0, c]
-        GemmP z{.A = h->fLi, .B = sl.C, .C = Zs[k], .lda = np, .ldb = cols, .ldc = cols, .M = np, .N = cols, .K = np, .kmode = KM_LE_I};
-        const bool int8 = gpe_int8_route(h, st, z, GEMM_NN, EPI_STORE);
-        const OzHint hint = int8 ? OzHint{.reuse_a = true, .a_tag = h->fit_gen, .b_bound = h->fit_c} : OzHint();
-        if ((rc = gpe_gemm_routed(h, st, z, GEMM_NN, EPI_STORE, int8, hint))) return rc;
+        h->launches++;
+        if ((rc = posterior_cross(h, st, sl.X, nullptr, cols, cols, sl.C, sl.Aux))) return rc;
+        if ((rc = fit_z_product(h, st, sl.C, cols, Zs[k], EPI_STORE))) return rc;
         {
             ProfScope ps(h, gpe_handle::CAT_OTHER, st);
             sens_pairdot_kernel<<<dim3((unsigned)(Mc / 128), ntile, (nw + SS_PG - 1) / SS_PG), 128, 0, st>>>(Zs[k], h->n, (int)Mc, nw, Parts[k]);
@@ -1263,13 +1266,9 @@ int gpe_sens_sample(gpe_handle* h, const double* XA, const double* XB, long long
                                                                                       shift, bpart, ci * (Mc / 128));
         }
         h->launches += 3;
-    }
-    if (two) {
-        for (int k = 0; k < 2; k++) {
-            CK(cudaEventRecord(h->ev_join[k], h->sub_st[k]));
-            CK(cudaStreamWaitEvent(h->st, h->ev_join[k], 0));
-        }
-    }
+        return 0;
+    });
+    if (rc) return rc;
     {
         ProfScope ps(h, gpe_handle::CAT_OTHER, h->st);
         sens_sample_reduce_kernel<<<1, 128, 0, h->st>>>(bpart, nblk, 2 * T, so.p);
