@@ -64,6 +64,7 @@ def load():
         "gpe_sens_contract": (i, [p, p, p, p, d, p, i, p, p]),
         "gpe_sens_main_effect": (i, [p, p, p, p, p, p, d, p, i, p, i, p]),
         "gpe_sens_sample": (i, [p, p, p, ll, p, i, d, p]),
+        "gpe_predict_grad": (i, [p, p, ll, p, p]),
         "gpe_dbg_gemm": (i, [p, p, p, p, i, i, i, ll, ll, ll, i, i, i, d, i, i, i, i, i]),
         "gpe_dbg_gemm_oz": (i, [p, p, p, p, i, i, i, ll, ll, ll, i, i, i, d, i, i, i, i, i, i, p, p, p, p, p]),
         "gpe_potrf": (i, [p, p, i, i, p, p, p, p]),
@@ -81,7 +82,7 @@ EXPORTS = ["gpe_version", "gpe_create", "gpe_destroy", "gpe_last_error", "gpe_la
            "gpe_get_stream", "gpe_set_streams", "gpe_set_async", "gpe_set_kernel", "gpe_synchronize", "gpe_profile_enable", "gpe_profile_read",
            "gpe_set_training", "gpe_set_basis", "gpe_cov_build", "gpe_cov_grad", "gpe_cross_cov", "gpe_llh_grad_batch",
            "gpe_fit_state", "gpe_loo", "gpe_predict", "gpe_predict_grid", "gpe_predict_fullcov", "gpe_implausibility", "gpe_predict_implaus",
-           "gpe_solve", "gpe_sens_contract", "gpe_sens_main_effect", "gpe_sens_sample", "gpe_potrf", "gpe_pdist_argmin",
+           "gpe_solve", "gpe_sens_contract", "gpe_sens_main_effect", "gpe_sens_sample", "gpe_predict_grad", "gpe_potrf", "gpe_pdist_argmin",
            "gpe_dbg_gemm", "gpe_dbg_gemm_oz", "gpe_dbg_potrf_inv", "gpe_dbg_int8_products"]
 
 
@@ -274,6 +275,21 @@ class Device:
             mean, var = out
         self._ck(self.L.gpe_predict(self.h, _ptr(Xs), _ptr(Hs), m, _ptr(mean), _ptr(var)))
         return mean, var
+
+    def predict_grad(self, Xs, want_var=True, out=None):
+        """Posterior gradient at the points Xs [m, d] (NumPy or torch CUDA tensor; see gpe_predict_grad): (dmean [m, d],
+        dvar [m, d] or None), derivatives with respect to the scaled training inputs.  ``out``: a (dmean, dvar) pair to fill
+        (dvar may be None)."""
+        if isinstance(Xs, np.ndarray) or not hasattr(Xs, "data_ptr"):
+            Xs = _f64(Xs).reshape(-1, self.d)
+        m = int(Xs.shape[0])
+        if out is None:
+            dmean = np.empty((m, self.d))
+            dvar = np.empty((m, self.d)) if want_var else None
+        else:
+            dmean, dvar = out
+        self._ck(self.L.gpe_predict_grad(self.h, _ptr(Xs), m, _ptr(dmean), _ptr(dvar)))
+        return dmean, dvar
 
     def predict_grid(self, levels, lo, hi, start, count, want_var=True, out=None):
         levels = np.ascontiguousarray(levels, dtype=np.int32)

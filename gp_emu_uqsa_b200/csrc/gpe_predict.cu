@@ -8,7 +8,7 @@
 // a flat grid index) and a skinny product [A^-1 H K^-T | e]^T C gives the mean and the regression-variance
 // term (posterior_cross), and Z = L^-1 C runs with the column norms |L^-1 c_j|^2 reduced in the GEMM
 // epilogue (fit_z_product).   v_j = sigma^2 (a*_jj - |L^-1 c_j|^2 + |K^-1 h_j - (Gm K^-T)^T c_j|^2).
-// gpe_predict_fullcov and gpe_sens_sample build on the same steps.
+// gpe_predict_fullcov, gpe_sens_sample and gpe_predict_grad (a derivative slab in place of C) build on the same steps.
 #include "gpe_handle.h"
 
 #include <algorithm>
@@ -329,6 +329,90 @@ static cudaError_t launch_xcov(int family, const double* Xs, const double* P, co
     return launch_xcov_fam<FAMILY_GAUSSIAN>(Xs, P, winv, n, d, npad, mc, count, cscale, Cm, ldc, st);
 }
 
+// K1g: the derivative slab of the cross-covariance, C[i][k mc + j] = delta_k d/dp_k [c R(D_ij)] = 2 c phi(D_ij) u_ijk with
+// u_ijk = (x_ik - p_jk) / delta_k and phi = -dR/dD (exp(-D); Matérn: G(D)).  |entry| <= c (DESIGN.md section 9e).  xcov_kernel's
+// tiling: D of the 8 x 4 entries in registers, then per row a second pass over the shared tiles, one input k at a time.  Two
+// CTAs per SM, not three: the second pass keeps more registers live than xcov_kernel's store loop and spills at 80.
+template <int FAM>
+__global__ void __launch_bounds__(256, 2) xcov_grad_kernel(const double* __restrict__ Xs /*[d][npad]*/, const double* __restrict__ P /*[mc][d]*/,
+                                                        const double* __restrict__ winv, int n, int d, int npad, int mc, long long count,
+                                                        double cscale, double* __restrict__ Cm /*[npad][d mc]*/) {
+    extern __shared__ __align__(16) double sm[];
+    double* Xt = sm;                   // [d][64]
+    double* Pt = sm + (size_t)d * 64;  // [d][128+2]
+    const int tid = threadIdx.x;
+    const int j0 = blockIdx.x * 128, k0 = blockIdx.y * 64;
+    const size_t ldc = (size_t)d * mc;
+    for (int e = tid; e < d * 64; e += 256) {
+        int k = e / 64, rr = e % 64;
+        Xt[k * 64 + rr] = Xs[(size_t)k * npad + k0 + rr];
+    }
+    {
+        const int jj = tid >> 1;
+        for (int k = tid & 1; k < d; k += 2) Pt[k * 130 + jj] = P[(size_t)(j0 + jj) * d + k] * winv[k];
+    }
+    __syncthreads();
+    const int ty = tid >> 5, tx = tid & 31;
+    double D[8][4];
+#pragma unroll
+    for (int a = 0; a < 8; a++)
+#pragma unroll
+        for (int c = 0; c < 4; c++) D[a][c] = 0.0;
+    for (int k = 0; k < d; k++) {
+        double xr[8], pj[4];
+#pragma unroll
+        for (int a = 0; a < 8; a++) xr[a] = Xt[k * 64 + ty + 8 * a];
+        double2 v0 = *reinterpret_cast<const double2*>(&Pt[k * 130 + 2 * tx]);
+        double2 v1 = *reinterpret_cast<const double2*>(&Pt[k * 130 + 64 + 2 * tx]);
+        pj[0] = v0.x; pj[1] = v0.y; pj[2] = v1.x; pj[3] = v1.y;
+#pragma unroll
+        for (int a = 0; a < 8; a++)
+#pragma unroll
+            for (int c = 0; c < 4; c++) {
+                double df = xr[a] - pj[c];
+                D[a][c] = fma(df, df, D[a][c]);
+            }
+    }
+    const double c2 = 2.0 * cscale;
+#pragma unroll
+    for (int a = 0; a < 8; a++) {
+        const int row = ty + 8 * a, gk = k0 + row;
+        const bool live = gk < n;
+        double s[4];
+#pragma unroll
+        for (int c = 0; c < 4; c++) {      // phi one row's four chains at a time (both families): 32 at once would spill
+            double phi;
+            if constexpr (FAM == FAMILY_MATERN52) gpe_matern52(D[a][c], phi);
+            else phi = gpe_exp(-D[a][c]);
+            const int gj = j0 + 64 * (c >> 1) + 2 * tx + (c & 1);
+            s[c] = (live && gj < count) ? c2 * phi : 0.0;
+        }
+        double* crow = Cm + (size_t)gk * ldc + j0 + 2 * tx;
+        for (int k = 0; k < d; k++) {
+            const double xr = Xt[k * 64 + row];
+            const double2 v0 = *reinterpret_cast<const double2*>(&Pt[k * 130 + 2 * tx]);
+            const double2 v1 = *reinterpret_cast<const double2*>(&Pt[k * 130 + 64 + 2 * tx]);
+            *reinterpret_cast<double2*>(crow + (size_t)k * mc) = make_double2(s[0] * (xr - v0.x), s[1] * (xr - v0.y));
+            *reinterpret_cast<double2*>(crow + (size_t)k * mc + 64) = make_double2(s[2] * (xr - v1.x), s[3] * (xr - v1.y));
+        }
+    }
+}
+
+template <int FAM>
+static cudaError_t launch_xcov_grad_fam(const double* Xs, const double* P, const double* winv, int n, int d, int npad, int mc,
+                                        long long count, double cscale, double* Cm, cudaStream_t st) {
+    static SmemOptIn optin;
+    const size_t smem = (size_t)d * (64 + 130) * sizeof(double);
+    if (cudaError_t e = optin.ensure(xcov_grad_kernel<FAM>, smem); e != cudaSuccess) return e;
+    xcov_grad_kernel<FAM><<<dim3(mc / 128, npad / 64), 256, smem, st>>>(Xs, P, winv, n, d, npad, mc, count, cscale, Cm);
+    return cudaGetLastError();
+}
+static cudaError_t launch_xcov_grad(int family, const double* Xs, const double* P, const double* winv, int n, int d, int npad, int mc,
+                                    long long count, double cscale, double* Cm, cudaStream_t st) {
+    if (family == FAMILY_MATERN52) return launch_xcov_grad_fam<FAMILY_MATERN52>(Xs, P, winv, n, d, npad, mc, count, cscale, Cm, st);
+    return launch_xcov_grad_fam<FAMILY_GAUSSIAN>(Xs, P, winv, n, d, npad, mc, count, cscale, Cm, st);
+}
+
 // K5 implausibility I = |mean - z| / sqrt(var + var_extra) of a point against each emulator's observation z, the per-point
 // ascending list of the maxno largest I over the emulators (history_match.py:96-132) and, on the finished lists, the keep mask,
 // the counts and the cell statistics.  Two routes share the update and the reduction below, so they give bit-identical results:
@@ -418,6 +502,15 @@ __device__ __forceinline__ double basis_value(const double* __restrict__ Hs, int
     return (pw == 1) ? x : pow(x, (double)pw);
 }
 
+// d h_a / d x_k at point j for the device polynomial basis
+__device__ __forceinline__ double basis_deriv(const double* __restrict__ P, int d, const BasisDesc& bd, long long j, int k, int a) {
+    const int pw = bd.pw[a];
+    if (a == 0 || bd.idx[a] != k || pw == 0) return 0.0;
+    if (pw == 1) return 1.0;
+    const double x = P[(size_t)j * d + k];
+    return (pw == 2) ? 2.0 * x : pw * pow(x, (double)(pw - 1));
+}
+
 // Row a of the forward substitution kv = K^-1 h with the lower-triangular K (leading dimension LD), from kv[0:a] and h_a.
 // One row at a time: the callers use kv[a] as soon as it is ready.
 template <int LD>
@@ -494,6 +587,53 @@ __global__ void __launch_bounds__(128) predict_finalize_kernel(const double* __r
         if (!imp.last) return;
         imp_finish(top, live, j, imp.first_index + j, imp.st);
     }
+}
+
+// per (point j, input k), one thread per column k mc + j of the derivative slab b (b = delta_k dc/dp_k): with a = aux of the
+// column and zn = |L^-1 b|^2 (tile partials),
+//   dmean = sum_a beta_a dh_a/dp_k + a[q] / delta_k,   dvar = sigma^2 ((c kappa - zn) / delta_k^2 + |K^-1 dh - a[0:q] / delta_k|^2),
+// written to dmean / dvar [count][d]
+__global__ void __launch_bounds__(128) predict_grad_finalize_kernel(const double* __restrict__ part, int ntile, const double* __restrict__ aux,
+                                                                    int mc, const double* __restrict__ P, BasisDesc bd, int d,
+                                                                    const double* __restrict__ winv, const double* __restrict__ Kf,
+                                                                    const double* __restrict__ beta, double sigma2, double ckappa,
+                                                                    long long count, double* __restrict__ dmean, double* __restrict__ dvar) {
+    __shared__ double Ks[NR][NR + 1];
+    __shared__ double bs[NR];
+    const int q = bd.q;
+    for (int e = threadIdx.x; e < NR * NR; e += blockDim.x) Ks[e / NR][e % NR] = Kf[e];
+    if (threadIdx.x < NR) bs[threadIdx.x] = beta[threadIdx.x];
+    __syncthreads();
+    const size_t ld = (size_t)d * mc;
+    const size_t col = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
+    const int k = (int)(col / mc);
+    const long long j = (long long)(col % mc);
+    if (k >= d || j >= count) return;
+    const double w = winv[k];
+    double dh[NR];
+#pragma unroll
+    for (int a = 0; a < NR; a++) dh[a] = (a < q) ? basis_deriv(P, d, bd, j, k, a) : 0.0;
+    double mu = aux[(size_t)q * ld + col] * w;
+#pragma unroll
+    for (int a = 0; a < NR; a++)
+        if (a < q) mu = fma(dh[a], bs[a], mu);
+    dmean[j * d + k] = mu;
+    if (dvar == nullptr) return;
+    double gn = 0.0;
+    double kv[NR];
+#pragma unroll
+    for (int a = 0; a < NR; a++) {
+        if (a < q) {
+            kv[a] = forward_subst_row<NR + 1>(&Ks[0][0], kv, dh[a], a);
+            const double g = fma(-aux[(size_t)a * ld + col], w, kv[a]);
+            gn = fma(g, g, gn);
+        } else {
+            kv[a] = 0.0;
+        }
+    }
+    double zn = 0.0;
+    for (int t = 0; t < ntile; t++) zn += part[(size_t)t * ld + col];
+    dvar[j * d + k] = sigma2 * fma(ckappa - zn, w * w, gn);
 }
 
 struct ImpDesc {
@@ -598,8 +738,15 @@ cudaError_t stage_points(double* P, const double* Xs, long long cnt, int mc, int
 // triangular product has 80 live rows, not 128)
 int live_k(const gpe_handle* h) { return std::min(h->npad, (h->n + GEMM_BK - 1) / GEMM_BK * GEMM_BK); }
 
+// aux = [A^-1 H K^-T | e]^T C of a slab C [npad][cols] (TN, skinny: the q + 1 live columns of the panel padded to 16 or 32 rows)
+int posterior_aux(gpe_handle* h, cudaStream_t st, const double* C, int cols, double* aux) {
+    const int maux = (h->q + 1 <= 16) ? 16 : NR;
+    return gpe_gemm(h, st, {.A = h->fE, .B = C, .C = aux, .lda = NR, .ldb = cols, .ldc = cols, .M = maux, .N = cols, .K = live_k(h)},
+                    GEMM_TN);
+}
+
 // The slab C [npad][cols] = c K(training, points) of the points P [cols][d] or of the grid chunk gx (columns >= count zero), and
-// aux = [A^-1 H K^-T | e]^T C (TN, skinny: the q + 1 live columns of the panel padded to 16 or 32 rows)
+// its aux
 int posterior_cross(gpe_handle* h, cudaStream_t st, const double* P, const GridXcov* gx, int cols, long long count, double* C,
                     double* aux) {
     {
@@ -608,9 +755,7 @@ int posterior_cross(gpe_handle* h, cudaStream_t st, const double* P, const GridX
         else CK(launch_xcov(h->family, h->fXs, P, h->fwinv, h->n, h->d, h->npad, cols, count, h->fit_c, C, cols, st));
     }
     h->launches++;
-    const int maux = (h->q + 1 <= 16) ? 16 : NR;
-    return gpe_gemm(h, st, {.A = h->fE, .B = C, .C = aux, .lda = NR, .ldb = cols, .ldc = cols, .M = maux, .N = cols, .K = live_k(h)},
-                    GEMM_TN);
+    return posterior_aux(h, st, C, cols, aux);
 }
 
 // Z = L^-1 C of the fit state (L^-1 lower: k <= i), stored into out (EPI_STORE) or reduced to column norms in the epilogue, tile
@@ -1275,6 +1420,55 @@ int gpe_sens_sample(gpe_handle* h, const double* XA, const double* XB, long long
     }
     h->launches++;
     CK(so.flush());
+    CK(cudaStreamSynchronize(h->st));
+    CK(cudaGetLastError());
+    return 0;
+}
+
+int gpe_predict_grad(gpe_handle* h, const double* Xs, long long m, double* dmean, double* dvar) {
+    if (h && m == 0) return 0;
+    if (!h || !Xs || !dmean || m < 0) return h ? h->fail_msg("gpe_predict_grad: Xs and dmean are required and m must be >= 0") : -2;
+    int rc;
+    if ((rc = check_fit(h, false))) return rc;
+    NvtxRange nvtx("gpe_predict_grad");
+    CK(cudaSetDevice(h->device));
+    const int d = h->d;
+    // points per chunk: a multiple of 256 (the INT8 route's column tile) with the chunk's d Mc columns at most the prediction
+    // chunk, but never fewer than 256 (the rule of gpe_sens_sample)
+    const long long Mc = std::min<long long>(std::max<long long>(256, default_chunk(h) / d / 256 * 256), (m + 255) / 256 * 256);
+    const int cols = (int)(d * Mc);
+    if ((rc = ensure_predict_ws(h, cols))) return rc;
+    const bool x_dev = gpe_is_device_ptr(Xs), mean_dev = gpe_is_device_ptr(dmean), var_dev = dvar && gpe_is_device_ptr(dvar);
+    const BasisDesc bd = basis_of(h);
+    const double s2 = h->fit_sigma * h->fit_sigma;
+    const double kappa = h->family == FAMILY_MATERN52 ? 5.0 / 3.0 : 2.0;     // -2 R'(0)
+    rc = for_chunks(h, (m + Mc - 1) / Mc, [&](long long ci, int k, cudaStream_t st) {
+        gpe_handle::PredSlot& sl = h->ps[k];
+        const long long s = ci * Mc, cnt = std::min(Mc, m - s);
+        const double* P = sl.X;
+        if (x_dev && cnt == Mc) P = Xs + (size_t)s * d;
+        else CK(stage_points(sl.X, Xs + (size_t)s * d, cnt, (int)Mc, d, st));
+        {
+            ProfScope ps(h, gpe_handle::CAT_COV, st);
+            CK(launch_xcov_grad(h->family, h->fXs, P, h->fwinv, h->n, d, h->npad, (int)Mc, cnt, h->fit_c, sl.C, st));
+        }
+        h->launches++;
+        int ntile = 0;
+        if ((rc = posterior_aux(h, st, sl.C, cols, sl.Aux))) return rc;
+        if (dvar != nullptr && (rc = fit_z_product(h, st, sl.C, cols, sl.Part, EPI_SUMSQ, &ntile))) return rc;
+        double* mo = mean_dev ? dmean + (size_t)s * d : sl.Mean;
+        double* vo = dvar ? (var_dev ? dvar + (size_t)s * d : sl.Var) : nullptr;
+        {
+            ProfScope ps(h, gpe_handle::CAT_OTHER, st);
+            predict_grad_finalize_kernel<<<(unsigned)((cols + 127) / 128), 128, 0, st>>>(sl.Part, ntile, sl.Aux, (int)Mc, P, bd, d, h->fwinv,
+                                                                                         h->fK, h->fbeta, s2, h->fit_c * kappa, cnt, mo, vo);
+        }
+        h->launches++;
+        if (!mean_dev) CK(cudaMemcpyAsync(dmean + (size_t)s * d, sl.Mean, (size_t)cnt * d * sizeof(double), cudaMemcpyDeviceToHost, st));
+        if (dvar && !var_dev) CK(cudaMemcpyAsync(dvar + (size_t)s * d, sl.Var, (size_t)cnt * d * sizeof(double), cudaMemcpyDeviceToHost, st));
+        return 0;
+    });
+    if (rc) return rc;
     CK(cudaStreamSynchronize(h->st));
     CK(cudaGetLastError());
     return 0;

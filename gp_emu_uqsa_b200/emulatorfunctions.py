@@ -10,7 +10,7 @@ from . import _emulatoroptimise as _emuo
 from . import _emulatorplotting as _emup
 from . import _lib
 
-__all__ = ["setup", "train", "plot", "posterior", "posterior_sample", "posterior_diag", "loo"]
+__all__ = ["setup", "train", "plot", "posterior", "posterior_sample", "posterior_diag", "posterior_grad", "loo"]
 
 
 def setup(config_file, datashuffle=True, scaleinputs=True):
@@ -147,6 +147,26 @@ def posterior_diag(E, x):
     xs = _emuc.Data(x, None, E.basis, E.par, E.beliefs, E.K)
     p = _emuc.Posterior(xs, E.training, E.par, E.beliefs, E.K, diag_only=True)
     return p.mean, p.var_diag
+
+
+def posterior_grad(E, x):
+    """(dmean [m,d], dvar [m,d]): the gradient of the posterior mean and the posterior variance of each component of the
+    gradient, at the points x (NumPy array or torch CUDA tensor), for the emulator's polynomial mean basis.  Derivatives of
+    the continuous part of the process (the nugget has none), taken in the scaled input units the emulator works in.  For
+    the units of the inputs file, divide column k of dmean by the span ``E.all_data.minmax[k, 1] - E.all_data.minmax[k, 0]``
+    and column k of dvar by its square."""
+    if E.basis.poly is None:
+        raise _lib.GpeError("the posterior gradient needs a polynomial mean basis ('1.0', 'x', 'x**k' terms)")
+    dev, _, _, st = E.training.fit(beta=E.par.beta, r_div=E.training._A_args[0])
+    if st != 0:
+        raise _lib.GpeError("training covariance matrix is not positive definite")
+    if hasattr(x, "data_ptr"):
+        import torch
+        m, d = int(x.shape[0]), E.training.inputs.shape[1]
+        dmean = torch.empty((m, d), dtype=torch.float64, device=x.device)
+        dvar = torch.empty((m, d), dtype=torch.float64, device=x.device)
+        return dev.predict_grad(x, out=(dmean, dvar))
+    return dev.predict_grad(_as_points(E, x))
 
 
 def posterior_sample(E, x, predict=True):

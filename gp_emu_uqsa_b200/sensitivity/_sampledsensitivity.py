@@ -9,12 +9,17 @@ main effects are means of the posterior mean over a sample with one input held a
 
 Unlike the closed-form class, ``EVTw`` here is the true total-effect variance E*[V_T,P] = E*[E[Var(f | x_~P)]], not the
 reference's ``uEV - E*[V_P]``.
+
+``dgsm()`` adds the derivative-based global sensitivity measures nu_P = E[(df/dx_P)^2] (Sobol' & Kucherenko 2009) from the
+posterior gradient (``gpe_predict_grad``) at sample A, and the Poincare bound C_P nu_P on the total-effect variance of the
+continuous part of the process (C_P = v_P for normal inputs, (hi - lo)^2 / pi^2 for uniform ones).
 """
 import numpy as np
 from scipy.special import ndtri
 from scipy.stats import qmc
 
 MAX_GROUP = 16      # inputs per device pass (gpe_sens_sample)
+DGSM_SLICE = 65536  # samples per gpe_predict_grad call of dgsm()
 
 
 def sample_points(d, samples, seed, m=None, v=None, bounds=None):
@@ -44,8 +49,8 @@ class SampledSensitivity:
     (``bounds``), one entry per active input, in the scaled training-input units ``Sensitivity`` takes.
 
     Attributes after the analyses: ``uE``, ``uV``, ``uEV``, ``senseindex`` (E*[V_P]), ``EVTw`` (the true total-effect
-    variance E*[V_T,P]), ``effect``, ``mean_effect``, and ``stderr``, a dict with the plain Monte Carlo standard error of
-    each under the same key (the Sobol points make the actual error smaller)."""
+    variance E*[V_T,P]), ``effect``, ``mean_effect``, ``dgsm_nu`` and ``dgsm_bound`` (``dgsm()``), and ``stderr``, a dict
+    with the plain Monte Carlo standard error of each under the same key (the Sobol points make the actual error smaller)."""
 
     def __init__(self, emul, m=None, v=None, bounds=None, samples=65536, seed=0):
         self._train = emul.training
@@ -63,7 +68,7 @@ class SampledSensitivity:
         self._est = None
         self._device()
         self.done_uncertainty = self.done_sensitivity = self.done_main_effect = False
-        self.done_interaction = self.done_totaleffectvar = False
+        self.done_interaction = self.done_totaleffectvar = self.done_dgsm = False
 
     def _device(self):
         """The handle with this emulator's fit state (re-factored only if another user of the training set changed it)."""
@@ -128,6 +133,30 @@ class SampledSensitivity:
         for P in range(self.d):
             print("E(V[T" + str(P) + "]):", self.EVTw[P])
 
+    def dgsm(self):
+        """dgsm_nu[P] = E*[nu_P] = E_x[(dm*/dx_P)^2 + Var*(df/dx_P)], the posterior mean of the derivative-based measure, from
+        the posterior gradient at sample A; dgsm_bound[P] = C_P dgsm_nu[P] bounds the total-effect variance of the continuous
+        part of the process, E*[V_T,P] - sigma^2 (a* - c) in the terms of ``EVTw`` (which includes the nugget's share)."""
+        print("\n*** Derivative-based global sensitivity measures ***")
+        A, _ = self._points(self.samples)
+        dev, M = self._device(), self.samples
+        s, s2 = np.zeros(self.d), np.zeros(self.d)
+        for i in range(0, M, DGSM_SLICE):
+            dm, dv = dev.predict_grad(A[i:i + DGSM_SLICE])
+            t = dm * dm + dv
+            s += t.sum(0)
+            s2 += (t * t).sum(0)
+        nu, err = _mean_err(s, s2, M)
+        if self.bounds is None:
+            C = self.v.copy()
+        else:
+            C = (self.bounds[:, 1] - self.bounds[:, 0]) ** 2 / np.pi ** 2
+        self.dgsm_nu, self.dgsm_bound = nu, C * nu
+        self.stderr.update(dgsm_nu=err, dgsm_bound=C * err)
+        self.done_dgsm = True
+        for P in range(self.d):
+            print("DGSM input " + str(P) + ": E*[nu] " + str(self.dgsm_nu[P]) + ", bound on E*[V_T] " + str(self.dgsm_bound[P]))
+
     def main_effect(self, plot=False, points=100, w=[], samples=4096):
         """effect[P, j] = mean_s [m*(B_s with x_P = xw_j) - m*(B_s)] and mean_effect[P, j] = mean_s m*(B_s with x_P = xw_j)
         on the x_w grid of ``Sensitivity.main_effect`` (``samples`` points B of the input distribution)."""
@@ -170,3 +199,6 @@ class SampledSensitivity:
                 f.write("xw " + ' '.join(map(str, [i for i in np.linspace(0.0, 1.0, self.effect[0].size)])) + "\n")
                 for i in range(0, self.d):
                     f.write("ME" + str(i) + " " + ' '.join(map(str, self.effect[i])) + "\n")
+            if self.done_dgsm:
+                f.write("DGSM " + ' '.join(map(str, self.dgsm_nu)) + "\n")
+                f.write("DGSMbound " + ' '.join(map(str, self.dgsm_bound)) + "\n")

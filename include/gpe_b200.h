@@ -234,6 +234,20 @@ int gpe_sens_main_effect(gpe_handle* h, const double* t1, const double* t2, cons
 int gpe_sens_sample(gpe_handle* h, const double* XA, const double* XB, long long M, const int* which, int nw,
                     double shift, double* sums);
 
+/* Posterior gradient of the emulator at m explicit points Xs [m,d] (scaled training-input units, as gpe_predict), for the
+ * state gpe_fit_state factored (either family, every nugget form, sigma and beta as given there); needs the device basis
+ * (gpe_set_basis) -- a caller's H* has no derivative, so there is no Hs argument.  Outputs [m,d], row-major, host or device:
+ *   dmean[j,k] = d m*(x_j) / dx_k = sum_a beta_a dh_a/dx_k + e^T dc_k
+ *   dvar[j,k]  = Var*(d f(x_j) / dx_k) = sigma^2 (c kappa / delta_k^2 - |L^-1 dc_k|^2 + |K^-1 dh_k - (A^-1 H K^-T)^T dc_k|^2)
+ * with dc_k = d/dx_k [c R(D(X, x_j))] = (2 / delta_k) c phi(D) u_k, u_k = (X_ik - x_jk) / delta_k, phi = -dR/dD (exp(-D) for the
+ * Gaussian kernel, (5/6)(1 + sqrt5 r) exp(-sqrt5 r) for Matern 5/2), c = 1 - nugget (or 1 for the alternative nugget) and
+ * kappa = -2 R'(0) = 2 (Gaussian) or 5/3 (Matern 5/2).  This is the derivative of the continuous part of the process: the
+ * nugget and the alternative nugget's r are white noise and have none (the off-diagonal prior c R that gpe_sens_sample uses for
+ * distinct points).  The derivative cross-covariance is formed as delta_k dc_k, whose entries are bounded by c like the
+ * cross-covariance itself, so it goes through the same products with the same scale.  dvar may be NULL (gradient of the mean
+ * only).  Cost: the posterior of d m columns, i.e. about one prediction of d m points. */
+int gpe_predict_grad(gpe_handle* h, const double* Xs, long long m, double* dmean, double* dvar);
+
 /* Maximin criterion of the optimised Latin hypercube (design_inputs/design_inputs.py:59-77):
  * argmin_out[k] = np.argmin(pdist(concat(designs[k], extra), 'sqeuclidean')) for N candidate designs
  * designs [N, n, dim] and shared extra points [ne, dim] (fextra; NULL / 0 if none).  Distances are
