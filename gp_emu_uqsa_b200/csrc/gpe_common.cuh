@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <cstdint>
 #include <cstdio>
+#include <type_traits>
 
 #if defined(__CUDA_ARCH__) && (__CUDA_ARCH__ < 1000)
 #error "gp_emu_uqsa_b200 kernels are written for sm_100a (B200) only"
@@ -127,10 +128,70 @@ __device__ __forceinline__ double gpe_matern52(double D) {
     double G;
     return gpe_matern52(D, G);   // (G is dead code here)
 }
+// kappa = -2 R'(0) of the family (R as a function of D): the prior variance of a scaled derivative of the process
+template <int FAM>
+constexpr double FAMILY_KAPPA = FAM == FAMILY_MATERN52 ? 5.0 / 3.0 : 2.0;
+
+// f(std::integral_constant<int, FAMILY_...>{}) for the run-time family: the one place where a family picks the kernel
+// instantiations a launch site runs.  A static inside the generic lambda f is one per family instantiation.
+template <class F>
+decltype(auto) with_family(int family, F&& f) {
+    if (family == FAMILY_MATERN52) return f(std::integral_constant<int, FAMILY_MATERN52>{});
+    return f(std::integral_constant<int, FAMILY_GAUSSIAN>{});
+}
 // Prior covariance c·k(D) of two distinct points at scaled squared distance D
 template <int FAM>
 __device__ __forceinline__ double cov_prior(double cscale, double D) {
     return cscale * (FAM == FAMILY_MATERN52 ? gpe_matern52(D) : gpe_exp(-D));
+}
+
+// ---- squared-distance tiles: the D of every covariance tile c k(D) ---------------------------------------------------------------
+// The inputs, scaled by 1/delta, are held k-major in shared memory: the row tile Xi [d][RA RS] and the column tile Xj [d][2 CH + 2].
+// A thread owns RA x 4 entries, rows ty + RS a and columns 2tx + {0, 1}, CH + 2tx + {0, 1}: the row operand is a broadcast, the
+// column operand a conflict-free double2.  Two shapes are in use: 4 x 4 (RS 16, CH 32: 64 x 64 entries, strides 64 / 66) and
+// 8 x 4 (RS 8, CH 64: 64 rows x 128 points, strides 64 / 130).  Direct differences (no |x|^2+|y|^2-2xy GEMM trick: it would lose
+// cond(A) digits and break the 1e-10 parity target).
+
+// the operands of input k: xi[a] = Xi[k][ty + RS a], xj = Xj[k][2tx, 2tx + 1, CH + 2tx, CH + 2tx + 1]
+template <int RA, int RS, int CH>
+__device__ __forceinline__ void tile_operands(const double* Xi, const double* Xj, int k, int ty, int tx, double (&xi)[RA],
+                                              double (&xj)[4]) {
+#pragma unroll
+    for (int a = 0; a < RA; a++) xi[a] = Xi[k * (RA * RS) + ty + RS * a];
+    const double2 v0 = *reinterpret_cast<const double2*>(&Xj[k * (2 * CH + 2) + 2 * tx]);
+    const double2 v1 = *reinterpret_cast<const double2*>(&Xj[k * (2 * CH + 2) + CH + 2 * tx]);
+    xj[0] = v0.x; xj[1] = v0.y; xj[2] = v1.x; xj[3] = v1.y;
+}
+
+// D[a][c] = sum_k (xi[a] - xj[c])^2, accumulated in input order
+template <int RA, int RS, int CH>
+__device__ __forceinline__ void sqdist_tile(const double* Xi, const double* Xj, int d, int ty, int tx, double (&D)[RA][4]) {
+#pragma unroll
+    for (int a = 0; a < RA; a++)
+#pragma unroll
+        for (int c = 0; c < 4; c++) D[a][c] = 0.0;
+    for (int k = 0; k < d; k++) {
+        double xi[RA], xj[4];
+        tile_operands<RA, RS, CH>(Xi, Xj, k, ty, tx, xi, xj);
+#pragma unroll
+        for (int a = 0; a < RA; a++)
+#pragma unroll
+            for (int c = 0; c < 4; c++) {
+                const double df = xi[a] - xj[c];
+                D[a][c] = fma(df, df, D[a][c]);
+            }
+    }
+}
+
+// The two tiles of the 4 x 4 shape from the rows i0 + r and j0 + r (r < 64) of X [n][d], scaled by w [d], zero for rows >= n.
+// 256 threads; no integer division: thread -> (row, k mod 4), 4 lanes read 32 contiguous bytes of a row.
+__device__ __forceinline__ void fill_scaled_tiles(const double* __restrict__ X, const double* __restrict__ w, int n, int d, int i0,
+                                                  int j0, double* Xi, double* Xj, int tid) {
+    const int row = tid >> 2, gi = i0 + row, gj = j0 + row;
+    for (int k = tid & 3; k < d; k += 4) {
+        Xi[k * 64 + row] = (gi < n) ? X[(size_t)gi * d + k] * w[k] : 0.0;
+        Xj[k * 66 + row] = (gj < n) ? X[(size_t)gj * d + k] * w[k] : 0.0;
+    }
 }
 
 __device__ __forceinline__ double warp_sum(double v) {

@@ -43,10 +43,7 @@ void launch_prep_theta(const double* theta, int B, int p, int d, int mode, doubl
 }
 
 // =========================================================================== K1 covariance build
-// 64x64 tile per CTA, 256 threads, 4x4 entries per thread.  X tiles are pre-scaled by 1/delta and
-// held k-major in shared memory so the row operand is a broadcast and the column operand a
-// conflict-free double2.  Direct differences (no |x|^2+|y|^2-2xy GEMM trick: it would lose
-// cond(A) digits and break the 1e-10 parity target).
+// 64x64 tile per CTA, 256 threads, 4x4 entries per thread (the 4 x 4 shape of sqdist_tile, gpe_common.cuh).
 constexpr int CT = 64;
 
 // lower-triangle tile index t = ti (ti + 1) / 2 + tj  ->  (ti, tj): 1-D grids launch no empty CTAs for the upper half
@@ -76,39 +73,21 @@ __global__ void __launch_bounds__(256, 3) cov_build_kernel(const double* __restr
     double* Xi = sm;                   // [d][CT]
     double* Xj = sm + (size_t)d * CT;  // [d][CT+2]
     const int tid = threadIdx.x;
-    const double* w = winv + (size_t)b * d;
-    {   // tile fill without integer division: thread -> (row, k mod 4); 4 lanes read 32 contiguous bytes of a row
-        const int row = tid >> 2, gi = ti * CT + row, gj = tj * CT + row;
-        for (int k = tid & 3; k < d; k += 4) {
-            Xi[k * CT + row] = (gi < n) ? X[(size_t)gi * d + k] * w[k] : 0.0;
-            Xj[k * (CT + 2) + row] = (gj < n) ? X[(size_t)gj * d + k] * w[k] : 0.0;
-        }
-    }
+    fill_scaled_tiles(X, winv + (size_t)b * d, n, d, ti * CT, tj * CT, Xi, Xj, tid);
     __syncthreads();
     const ItemPar ip = par[b];
     const int ty = tid >> 4, tx = tid & 15;
     double D[4][4], G[GMODE == 1 ? 4 : 1][4];
-#pragma unroll
-    for (int a = 0; a < 4; a++)
-#pragma unroll
-        for (int c = 0; c < 4; c++) {
-            D[a][c] = 0.0;
-            if constexpr (GMODE == 1) G[a][c] = 1.0;
-        }
-    for (int k = 0; k < d; k++) {
+    sqdist_tile<4, 16, 32>(Xi, Xj, d, ty, tx, D);
+    if constexpr (GMODE == 1) {      // Delta_gdim^2 of each entry (0 <= gdim < d)
         double xi[4], xj[4];
-#pragma unroll
-        for (int a = 0; a < 4; a++) xi[a] = Xi[k * CT + ty + 16 * a];
-        double2 v0 = *reinterpret_cast<const double2*>(&Xj[k * (CT + 2) + 2 * tx]);
-        double2 v1 = *reinterpret_cast<const double2*>(&Xj[k * (CT + 2) + 32 + 2 * tx]);
-        xj[0] = v0.x; xj[1] = v0.y; xj[2] = v1.x; xj[3] = v1.y;
+        tile_operands<4, 16, 32>(Xi, Xj, gdim, ty, tx, xi, xj);
 #pragma unroll
         for (int a = 0; a < 4; a++)
 #pragma unroll
             for (int c = 0; c < 4; c++) {
-                double df = xi[a] - xj[c];
-                D[a][c] = fma(df, df, D[a][c]);
-                if constexpr (GMODE == 1) { if (k == gdim) G[a][c] = df * df; }
+                const double df = xi[a] - xj[c];
+                G[a][c] = df * df;
             }
     }
     // all 16 exponentials first, outside the padding / diagonal case analysis: straight-line code whose 16 polynomial
@@ -149,34 +128,19 @@ __global__ void __launch_bounds__(256, 3) cov_build_kernel(const double* __restr
     }
 }
 
-template <int FAM>
-static cudaError_t launch_cov_build_fam(const double* X, const double* r, int n, int d, int npad, const ItemPar* par,
-                                       const double* winv, double* A, long long sA, dim3 grid, size_t smem, int full,
-                                       cudaStream_t st, int gmode, int gdim, double* Eout) {
-    static SmemOptIn opt0, opt1, opt2;
-    cudaError_t e;
-    if (gmode == 0) {
-        if ((e = opt0.ensure(cov_build_kernel<0, FAM>, smem)) != cudaSuccess) return e;
-        cov_build_kernel<0, FAM><<<grid, 256, smem, st>>>(X, r, n, d, npad, par, winv, A, sA, full, gdim, Eout);
-    } else if (gmode == 1) {
-        if ((e = opt1.ensure(cov_build_kernel<1, FAM>, smem)) != cudaSuccess) return e;
-        cov_build_kernel<1, FAM><<<grid, 256, smem, st>>>(X, r, n, d, npad, par, winv, A, sA, full, gdim, nullptr);
-    } else {
-        if ((e = opt2.ensure(cov_build_kernel<2, FAM>, smem)) != cudaSuccess) return e;
-        cov_build_kernel<2, FAM><<<grid, 256, smem, st>>>(X, r, n, d, npad, par, winv, A, sA, full, gdim, nullptr);
-    }
-    return cudaGetLastError();
-}
-
 cudaError_t launch_cov_build(const double* X, const double* r, int n, int d, int npad, const ItemPar* par,
                              const double* winv, double* A, long long sA, int B, int full, cudaStream_t st, int gmode, int gdim,
                              double* Eout, int family) {
     const int nt = npad / CT;
     dim3 grid = full ? dim3(nt, nt, B) : dim3(nt * (nt + 1) / 2, 1, B);
     size_t smem = (size_t)d * (CT + CT + 2) * sizeof(double);
-    if (family == FAMILY_MATERN52)
-        return launch_cov_build_fam<FAMILY_MATERN52>(X, r, n, d, npad, par, winv, A, sA, grid, smem, full, st, gmode, gdim, nullptr);
-    return launch_cov_build_fam<FAMILY_GAUSSIAN>(X, r, n, d, npad, par, winv, A, sA, grid, smem, full, st, gmode, gdim, Eout);
+    return with_family(family, [&](auto fam) {
+        static SmemOptIn opt[3];
+        auto kern = gmode == 0 ? cov_build_kernel<0, fam> : (gmode == 1 ? cov_build_kernel<1, fam> : cov_build_kernel<2, fam>);
+        if (cudaError_t e = opt[gmode].ensure(kern, smem); e != cudaSuccess) return e;
+        kern<<<grid, 256, smem, st>>>(X, r, n, d, npad, par, winv, A, sA, full, gdim, Eout);
+        return cudaGetLastError();
+    });
 }
 
 __global__ void unpad_sym_kernel(const double* __restrict__ A, int npad, int n, double* __restrict__ out, int mirror) {
@@ -767,14 +731,7 @@ __global__ void __launch_bounds__(256, 2) grad_partial_kernel(const double* __re
     double* Uj = Ui + (size_t)nu * CT;              // [nu][66]
     double* red = Uj + (size_t)nu * (CT + 2);       // [8][d+3]
     const int tid = threadIdx.x;
-    const double* w = winv + (size_t)b * d;
-    {   // tile fill without integer division: thread -> (row, k mod 4); 4 lanes read 32 contiguous bytes of a row
-        const int row = tid >> 2, gi = ti * CT + row, gj = tj * CT + row;
-        for (int k = tid & 3; k < d; k += 4) {
-            Xi[k * CT + row] = (gi < n) ? X[(size_t)gi * d + k] * w[k] : 0.0;
-            Xj[k * (CT + 2) + row] = (gj < n) ? X[(size_t)gj * d + k] * w[k] : 0.0;
-        }
-    }
+    fill_scaled_tiles(X, winv + (size_t)b * d, n, d, ti * CT, tj * CT, Xi, Xj, tid);
     const double* Ub = U + (size_t)b * npad * NR;
     {
         const int row = tid >> 2;
@@ -810,7 +767,7 @@ __global__ void __launch_bounds__(256, 2) grad_partial_kernel(const double* __re
 #pragma unroll
         for (int a = 0; a < 4; a++)
 #pragma unroll
-            for (int c = 0; c < 4; c++) D[a][c] = dot[a][c] = 0.0;
+            for (int c = 0; c < 4; c++) dot[a][c] = 0.0;
         for (int k = 0; k < nu; k++) {
             double ui[4], uj[4];
 #pragma unroll
@@ -837,21 +794,7 @@ __global__ void __launch_bounds__(256, 2) grad_partial_kernel(const double* __re
 #pragma unroll
                 for (int h = 0; h < 2; h++) { D[a][2 * h] = ev[a][h].x; D[a][2 * h + 1] = ev[a][h].y; }
         } else {
-            for (int k = 0; k < d; k++) {
-                double xi[4], xj[4];
-#pragma unroll
-                for (int a = 0; a < 4; a++) xi[a] = Xi[k * CT + ty + 16 * a];
-                double2 v0 = *reinterpret_cast<const double2*>(&Xj[k * (CT + 2) + 2 * tx]);
-                double2 v1 = *reinterpret_cast<const double2*>(&Xj[k * (CT + 2) + 32 + 2 * tx]);
-                xj[0] = v0.x; xj[1] = v0.y; xj[2] = v1.x; xj[3] = v1.y;
-#pragma unroll
-                for (int a = 0; a < 4; a++)
-#pragma unroll
-                    for (int c = 0; c < 4; c++) {
-                        double df = xi[a] - xj[c];
-                        D[a][c] = fma(df, df, D[a][c]);
-                    }
-            }
+            sqdist_tile<4, 16, 32>(Xi, Xj, d, ty, tx, D);
             if constexpr (FAM == FAMILY_GAUSSIAN) {
 #pragma unroll
                 for (int a = 0; a < 4; a++)
@@ -915,11 +858,7 @@ __global__ void __launch_bounds__(256, 2) grad_partial_kernel(const double* __re
             int k = k0 + kk;
             if (k < d) {
                 double xi[4], xj[4];
-#pragma unroll
-                for (int a = 0; a < 4; a++) xi[a] = Xi[k * CT + ty + 16 * a];
-                double2 v0 = *reinterpret_cast<const double2*>(&Xj[k * (CT + 2) + 2 * tx]);
-                double2 v1 = *reinterpret_cast<const double2*>(&Xj[k * (CT + 2) + 32 + 2 * tx]);
-                xj[0] = v0.x; xj[1] = v0.y; xj[2] = v1.x; xj[3] = v1.y;
+                tile_operands<4, 16, 32>(Xi, Xj, k, ty, tx, xi, xj);
 #pragma unroll
                 for (int a = 0; a < 4; a++)
 #pragma unroll
@@ -949,18 +888,16 @@ void launch_grad_partial(const double* X, const double* r, int n, int d, int npa
                          int B, cudaStream_t st, const double* E, int family) {
     int nt = npad / CT;
     size_t smem = ((size_t)(d + nu) * (CT + CT + 2) + 8 * (size_t)(d + 3)) * sizeof(double);
-    static SmemOptIn optin, optin_e, optin_m;
     const dim3 grid(nt * (nt + 1) / 2, 1, B);
-    if (family == FAMILY_MATERN52) {      // always recomputed: the covariance build keeps no copy of R or G
-        optin_m.ensure(grad_partial_kernel<false, FAMILY_MATERN52>, smem);
-        grad_partial_kernel<false, FAMILY_MATERN52><<<grid, 256, smem, st>>>(X, r, n, d, npad, winv, Ainv, sAinv, U, nu, part, nullptr);
-    } else if (E != nullptr) {         // (same layout and item stride as A^-1)
-        optin_e.ensure(grad_partial_kernel<true, FAMILY_GAUSSIAN>, smem);
-        grad_partial_kernel<true, FAMILY_GAUSSIAN><<<grid, 256, smem, st>>>(X, r, n, d, npad, winv, Ainv, sAinv, U, nu, part, E);
-    } else {
-        optin.ensure(grad_partial_kernel<false, FAMILY_GAUSSIAN>, smem);
-        grad_partial_kernel<false, FAMILY_GAUSSIAN><<<grid, 256, smem, st>>>(X, r, n, d, npad, winv, Ainv, sAinv, U, nu, part, nullptr);
-    }
+    with_family(family, [&](auto fam) {
+        static SmemOptIn optin, optin_e;
+        auto kern = grad_partial_kernel<false, fam>;
+        SmemOptIn* opt = &optin;
+        if constexpr (fam == FAMILY_GAUSSIAN)      // Matérn: always recomputed, the covariance build keeps no copy of R or G
+            if (E != nullptr) { kern = grad_partial_kernel<true, fam>; opt = &optin_e; }      // (same layout and item stride as A^-1)
+        opt->ensure(kern, smem);
+        kern<<<grid, 256, smem, st>>>(X, r, n, d, npad, winv, Ainv, sAinv, U, nu, part, E);
+    });
 }
 
 // Sum the tile partials in a fixed order and apply the per-parameter prefactors

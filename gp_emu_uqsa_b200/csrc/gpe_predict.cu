@@ -60,11 +60,15 @@ __global__ void grid_points_kernel(GridDesc g, long long start, long long count,
 }
 
 // K1x: C[k][j] = c * exp(-sum_dim ((x_k - p_j)/delta)^2) for a chunk of mc points (FAMILY_MATERN52: c * R(sum_dim ..)).
-// CTA = 64 training rows x 128 points, 256 threads, each thread 8 rows x 4 points.
-template <int FAM>
-__global__ void __launch_bounds__(256, 3) xcov_kernel(const double* __restrict__ Xs /*[d][npad]*/, const double* __restrict__ P /*[mc][d]*/,
-                                                   const double* __restrict__ winv, int n, int d, int npad, int mc, long long count,
-                                                   double cscale, double* __restrict__ Cm, int ldc) {
+// CTA = 64 training rows x 128 points, 256 threads, each thread 8 rows x 4 points (the 8 x 4 shape of sqdist_tile).
+// GRAD: the derivative slab instead, C[i][k mc + j] = delta_k d/dp_k [c R(D_ij)] = 2 c phi(D_ij) u_ijk with
+// u_ijk = (x_ik - p_jk) / delta_k and phi = -dR/dD (exp(-D); Matérn: G(D)); |entry| <= c (DESIGN.md section 9e).  After D, per
+// row a second pass over the shared tiles, one input k at a time.  Two CTAs per SM, not three: the second pass keeps more
+// registers live than the store loop of C and spills at 80.
+template <int FAM, bool GRAD>
+__global__ void __launch_bounds__(256, GRAD ? 2 : 3) xcov_kernel(const double* __restrict__ Xs /*[d][npad]*/, const double* __restrict__ P /*[mc][d]*/,
+                                                              const double* __restrict__ winv, int n, int d, int npad, int mc, long long count,
+                                                              double cscale, double* __restrict__ Cm, int ldc) {
     extern __shared__ __align__(16) double sm[];
     double* Xt = sm;                   // [d][64]
     double* Pt = sm + (size_t)d * 64;  // [d][128+2]
@@ -81,49 +85,56 @@ __global__ void __launch_bounds__(256, 3) xcov_kernel(const double* __restrict__
     __syncthreads();
     const int ty = tid >> 5, tx = tid & 31;   // rows ty + 8a (a<8); points 2tx+{0,1}, 64+2tx+{0,1}
     double D[8][4];
+    sqdist_tile<8, 8, 64>(Xt, Pt, d, ty, tx, D);
+    if constexpr (GRAD) {
+        const double c2 = 2.0 * cscale;
 #pragma unroll
-    for (int a = 0; a < 8; a++)
+        for (int a = 0; a < 8; a++) {
+            const int row = ty + 8 * a, gk = k0 + row;
+            const bool live = gk < n;
+            double s[4];
 #pragma unroll
-        for (int c = 0; c < 4; c++) D[a][c] = 0.0;
-    for (int k = 0; k < d; k++) {
-        double xr[8], pj[4];
-#pragma unroll
-        for (int a = 0; a < 8; a++) xr[a] = Xt[k * 64 + ty + 8 * a];
-        double2 v0 = *reinterpret_cast<const double2*>(&Pt[k * 130 + 2 * tx]);
-        double2 v1 = *reinterpret_cast<const double2*>(&Pt[k * 130 + 64 + 2 * tx]);
-        pj[0] = v0.x; pj[1] = v0.y; pj[2] = v1.x; pj[3] = v1.y;
+            for (int c = 0; c < 4; c++) {      // phi one row's four chains at a time (both families): 32 at once would spill
+                double phi;
+                if constexpr (FAM == FAMILY_MATERN52) gpe_matern52(D[a][c], phi);
+                else phi = gpe_exp(-D[a][c]);
+                const int gj = j0 + 64 * (c >> 1) + 2 * tx + (c & 1);
+                s[c] = (live && gj < count) ? c2 * phi : 0.0;
+            }
+            double* crow = Cm + (size_t)gk * d * mc + j0 + 2 * tx;      // row stride d mc (= ldc), formed in 64 bits
+            for (int k = 0; k < d; k++) {
+                const double xr = Xt[k * 64 + row];
+                const double2 v0 = *reinterpret_cast<const double2*>(&Pt[k * 130 + 2 * tx]);
+                const double2 v1 = *reinterpret_cast<const double2*>(&Pt[k * 130 + 64 + 2 * tx]);
+                *reinterpret_cast<double2*>(crow + (size_t)k * mc) = make_double2(s[0] * (xr - v0.x), s[1] * (xr - v0.y));
+                *reinterpret_cast<double2*>(crow + (size_t)k * mc + 64) = make_double2(s[2] * (xr - v1.x), s[3] * (xr - v1.y));
+            }
+        }
+    } else {
 #pragma unroll
         for (int a = 0; a < 8; a++)
 #pragma unroll
-            for (int c = 0; c < 4; c++) {
-                double df = xr[a] - pj[c];
-                D[a][c] = fma(df, df, D[a][c]);
+            for (int c = 0; c < 4; c++)      // straight-line: the chains interleave
+                if constexpr (FAM == FAMILY_GAUSSIAN) D[a][c] = gpe_exp(-D[a][c]);
+#pragma unroll
+        for (int a = 0; a < 8; a++) {
+            int gk = k0 + ty + 8 * a;
+            bool live = gk < n;
+            if constexpr (FAM == FAMILY_MATERN52) {      // one row's four chains at a time: 32 at once would spill
+#pragma unroll
+                for (int c = 0; c < 4; c++) D[a][c] = gpe_matern52(D[a][c]);
             }
-    }
 #pragma unroll
-    for (int a = 0; a < 8; a++)
-#pragma unroll
-        for (int c = 0; c < 4; c++)      // straight-line: the chains interleave
-            if constexpr (FAM == FAMILY_GAUSSIAN) D[a][c] = gpe_exp(-D[a][c]);
-#pragma unroll
-    for (int a = 0; a < 8; a++) {
-        int gk = k0 + ty + 8 * a;
-        bool live = gk < n;
-        if constexpr (FAM == FAMILY_MATERN52) {      // one row's four chains at a time: 32 at once would spill
-#pragma unroll
-            for (int c = 0; c < 4; c++) D[a][c] = gpe_matern52(D[a][c]);
-        }
-#pragma unroll
-        for (int hh = 0; hh < 2; hh++) {
-            int gj = j0 + 64 * hh + 2 * tx;
-            double2 v;
-            v.x = (live && gj < count) ? cscale * D[a][2 * hh] : 0.0;
-            v.y = (live && gj + 1 < count) ? cscale * D[a][2 * hh + 1] : 0.0;
-            *reinterpret_cast<double2*>(&Cm[(size_t)gk * ldc + gj]) = v;
+            for (int hh = 0; hh < 2; hh++) {
+                int gj = j0 + 64 * hh + 2 * tx;
+                double2 v;
+                v.x = (live && gj < count) ? cscale * D[a][2 * hh] : 0.0;
+                v.y = (live && gj + 1 < count) ? cscale * D[a][2 * hh + 1] : 0.0;
+                *reinterpret_cast<double2*>(&Cm[(size_t)gk * ldc + gj]) = v;
+            }
         }
     }
 }
-
 
 // ---- K1x for tensor-grid points: the Gaussian kernel factorises over the input dimensions,
 //     exp(-sum_k ((x_ik - g_k)/delta_k)^2) = prod_k exp(-((x_ik - g_k)/delta_k)^2),
@@ -285,19 +296,20 @@ static cudaError_t launch_xcov_grid_nf(const double* T, const GridSep& sp, int n
     return cudaGetLastError();
 }
 
-template <int FAM>
-static cudaError_t launch_xcov_grid(const double* T, const GridSep& sp, int n, int npad, int mc, long long start, long long count,
-                                    double cscale, double* Cm, size_t smem, cudaStream_t st) {
-    switch (sp.nf) {
-        case 1: return launch_xcov_grid_nf<1, FAM>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
-        case 2: return launch_xcov_grid_nf<2, FAM>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
-        case 3: return launch_xcov_grid_nf<3, FAM>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
-        case 4: return launch_xcov_grid_nf<4, FAM>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
-        case 5: return launch_xcov_grid_nf<5, FAM>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
-        case 6: return launch_xcov_grid_nf<6, FAM>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
-        case 7: return launch_xcov_grid_nf<7, FAM>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
-        default: return cudaErrorInvalidValue;
-    }
+static cudaError_t launch_xcov_grid(int family, const double* T, const GridSep& sp, int n, int npad, int mc, long long start,
+                                    long long count, double cscale, double* Cm, size_t smem, cudaStream_t st) {
+    return with_family(family, [&](auto fam) {
+        switch (sp.nf) {
+            case 1: return launch_xcov_grid_nf<1, fam>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
+            case 2: return launch_xcov_grid_nf<2, fam>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
+            case 3: return launch_xcov_grid_nf<3, fam>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
+            case 4: return launch_xcov_grid_nf<4, fam>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
+            case 5: return launch_xcov_grid_nf<5, fam>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
+            case 6: return launch_xcov_grid_nf<6, fam>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
+            case 7: return launch_xcov_grid_nf<7, fam>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
+            default: return cudaErrorInvalidValue;
+        }
+    });
 }
 
 struct GridXcov {        // what predict_chunk needs to build a chunk's cross-covariance from the tables
@@ -307,110 +319,18 @@ struct GridXcov {        // what predict_chunk needs to build a chunk's cross-co
     long long start;     // flat index of the chunk's first point
 };
 
-static cudaError_t launch_xcov_grid(int family, const double* T, const GridSep& sp, int n, int npad, int mc, long long start,
-                                    long long count, double cscale, double* Cm, size_t smem, cudaStream_t st) {
-    if (family == FAMILY_MATERN52) return launch_xcov_grid<FAMILY_MATERN52>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
-    return launch_xcov_grid<FAMILY_GAUSSIAN>(T, sp, n, npad, mc, start, count, cscale, Cm, smem, st);
-}
-
-// C [n rows of npad, ldc] = cscale * K(training, P) for the mc points P [mc, d] (columns >= count zero)
-template <int FAM>
-static cudaError_t launch_xcov_fam(const double* Xs, const double* P, const double* winv, int n, int d, int npad, int mc,
-                                   long long count, double cscale, double* Cm, int ldc, cudaStream_t st) {
-    static SmemOptIn optin;      // d >= 32 needs more than 48 KB for the two k-major tiles
-    const size_t smem = (size_t)d * (64 + 130) * sizeof(double);
-    if (cudaError_t e = optin.ensure(xcov_kernel<FAM>, smem); e != cudaSuccess) return e;
-    xcov_kernel<FAM><<<dim3(mc / 128, npad / 64), 256, smem, st>>>(Xs, P, winv, n, d, npad, mc, count, cscale, Cm, ldc);
-    return cudaGetLastError();
-}
+// C [n rows of npad, ldc] = cscale * K(training, P) for the mc points P [mc, d] (columns >= count zero); GRAD: the derivative
+// slab, input k's mc columns at k mc (ldc = d mc)
+template <bool GRAD>
 static cudaError_t launch_xcov(int family, const double* Xs, const double* P, const double* winv, int n, int d, int npad, int mc,
                                long long count, double cscale, double* Cm, int ldc, cudaStream_t st) {
-    if (family == FAMILY_MATERN52) return launch_xcov_fam<FAMILY_MATERN52>(Xs, P, winv, n, d, npad, mc, count, cscale, Cm, ldc, st);
-    return launch_xcov_fam<FAMILY_GAUSSIAN>(Xs, P, winv, n, d, npad, mc, count, cscale, Cm, ldc, st);
-}
-
-// K1g: the derivative slab of the cross-covariance, C[i][k mc + j] = delta_k d/dp_k [c R(D_ij)] = 2 c phi(D_ij) u_ijk with
-// u_ijk = (x_ik - p_jk) / delta_k and phi = -dR/dD (exp(-D); Matérn: G(D)).  |entry| <= c (DESIGN.md section 9e).  xcov_kernel's
-// tiling: D of the 8 x 4 entries in registers, then per row a second pass over the shared tiles, one input k at a time.  Two
-// CTAs per SM, not three: the second pass keeps more registers live than xcov_kernel's store loop and spills at 80.
-template <int FAM>
-__global__ void __launch_bounds__(256, 2) xcov_grad_kernel(const double* __restrict__ Xs /*[d][npad]*/, const double* __restrict__ P /*[mc][d]*/,
-                                                        const double* __restrict__ winv, int n, int d, int npad, int mc, long long count,
-                                                        double cscale, double* __restrict__ Cm /*[npad][d mc]*/) {
-    extern __shared__ __align__(16) double sm[];
-    double* Xt = sm;                   // [d][64]
-    double* Pt = sm + (size_t)d * 64;  // [d][128+2]
-    const int tid = threadIdx.x;
-    const int j0 = blockIdx.x * 128, k0 = blockIdx.y * 64;
-    const size_t ldc = (size_t)d * mc;
-    for (int e = tid; e < d * 64; e += 256) {
-        int k = e / 64, rr = e % 64;
-        Xt[k * 64 + rr] = Xs[(size_t)k * npad + k0 + rr];
-    }
-    {
-        const int jj = tid >> 1;
-        for (int k = tid & 1; k < d; k += 2) Pt[k * 130 + jj] = P[(size_t)(j0 + jj) * d + k] * winv[k];
-    }
-    __syncthreads();
-    const int ty = tid >> 5, tx = tid & 31;
-    double D[8][4];
-#pragma unroll
-    for (int a = 0; a < 8; a++)
-#pragma unroll
-        for (int c = 0; c < 4; c++) D[a][c] = 0.0;
-    for (int k = 0; k < d; k++) {
-        double xr[8], pj[4];
-#pragma unroll
-        for (int a = 0; a < 8; a++) xr[a] = Xt[k * 64 + ty + 8 * a];
-        double2 v0 = *reinterpret_cast<const double2*>(&Pt[k * 130 + 2 * tx]);
-        double2 v1 = *reinterpret_cast<const double2*>(&Pt[k * 130 + 64 + 2 * tx]);
-        pj[0] = v0.x; pj[1] = v0.y; pj[2] = v1.x; pj[3] = v1.y;
-#pragma unroll
-        for (int a = 0; a < 8; a++)
-#pragma unroll
-            for (int c = 0; c < 4; c++) {
-                double df = xr[a] - pj[c];
-                D[a][c] = fma(df, df, D[a][c]);
-            }
-    }
-    const double c2 = 2.0 * cscale;
-#pragma unroll
-    for (int a = 0; a < 8; a++) {
-        const int row = ty + 8 * a, gk = k0 + row;
-        const bool live = gk < n;
-        double s[4];
-#pragma unroll
-        for (int c = 0; c < 4; c++) {      // phi one row's four chains at a time (both families): 32 at once would spill
-            double phi;
-            if constexpr (FAM == FAMILY_MATERN52) gpe_matern52(D[a][c], phi);
-            else phi = gpe_exp(-D[a][c]);
-            const int gj = j0 + 64 * (c >> 1) + 2 * tx + (c & 1);
-            s[c] = (live && gj < count) ? c2 * phi : 0.0;
-        }
-        double* crow = Cm + (size_t)gk * ldc + j0 + 2 * tx;
-        for (int k = 0; k < d; k++) {
-            const double xr = Xt[k * 64 + row];
-            const double2 v0 = *reinterpret_cast<const double2*>(&Pt[k * 130 + 2 * tx]);
-            const double2 v1 = *reinterpret_cast<const double2*>(&Pt[k * 130 + 64 + 2 * tx]);
-            *reinterpret_cast<double2*>(crow + (size_t)k * mc) = make_double2(s[0] * (xr - v0.x), s[1] * (xr - v0.y));
-            *reinterpret_cast<double2*>(crow + (size_t)k * mc + 64) = make_double2(s[2] * (xr - v1.x), s[3] * (xr - v1.y));
-        }
-    }
-}
-
-template <int FAM>
-static cudaError_t launch_xcov_grad_fam(const double* Xs, const double* P, const double* winv, int n, int d, int npad, int mc,
-                                        long long count, double cscale, double* Cm, cudaStream_t st) {
-    static SmemOptIn optin;
-    const size_t smem = (size_t)d * (64 + 130) * sizeof(double);
-    if (cudaError_t e = optin.ensure(xcov_grad_kernel<FAM>, smem); e != cudaSuccess) return e;
-    xcov_grad_kernel<FAM><<<dim3(mc / 128, npad / 64), 256, smem, st>>>(Xs, P, winv, n, d, npad, mc, count, cscale, Cm);
-    return cudaGetLastError();
-}
-static cudaError_t launch_xcov_grad(int family, const double* Xs, const double* P, const double* winv, int n, int d, int npad, int mc,
-                                    long long count, double cscale, double* Cm, cudaStream_t st) {
-    if (family == FAMILY_MATERN52) return launch_xcov_grad_fam<FAMILY_MATERN52>(Xs, P, winv, n, d, npad, mc, count, cscale, Cm, st);
-    return launch_xcov_grad_fam<FAMILY_GAUSSIAN>(Xs, P, winv, n, d, npad, mc, count, cscale, Cm, st);
+    return with_family(family, [&](auto fam) {
+        static SmemOptIn optin;      // d >= 32 needs more than 48 KB for the two k-major tiles
+        const size_t smem = (size_t)d * (64 + 130) * sizeof(double);
+        if (cudaError_t e = optin.ensure(xcov_kernel<fam, GRAD>, smem); e != cudaSuccess) return e;
+        xcov_kernel<fam, GRAD><<<dim3(mc / 128, npad / 64), 256, smem, st>>>(Xs, P, winv, n, d, npad, mc, count, cscale, Cm, ldc);
+        return cudaGetLastError();
+    });
 }
 
 // K5 implausibility I = |mean - z| / sqrt(var + var_extra) of a point against each emulator's observation z, the per-point
@@ -752,7 +672,7 @@ int posterior_cross(gpe_handle* h, cudaStream_t st, const double* P, const GridX
     {
         ProfScope ps(h, gpe_handle::CAT_COV, st);
         if (gx != nullptr) CK(launch_xcov_grid(h->family, gx->T, gx->sp, h->n, h->npad, cols, gx->start, count, h->fit_c, C, gx->smem, st));
-        else CK(launch_xcov(h->family, h->fXs, P, h->fwinv, h->n, h->d, h->npad, cols, count, h->fit_c, C, cols, st));
+        else CK(launch_xcov<false>(h->family, h->fXs, P, h->fwinv, h->n, h->d, h->npad, cols, count, h->fit_c, C, cols, st));
     }
     h->launches++;
     return posterior_aux(h, st, C, cols, aux);
@@ -1111,25 +1031,19 @@ static int predict_common(gpe_handle* h, const double* Xs, const double* Hs, con
     const bool x_dev = Xs && gpe_is_device_ptr(Xs), h_dev = Hs && gpe_is_device_ptr(Hs);
     const bool mean_dev = imp_call || gpe_is_device_ptr(mean), var_dev = var && gpe_is_device_ptr(var);
     const int d = h->d, q = h->q;
-    // tensor grid: tabulate the one-dimensional kernel factors once (GPE_GRID_SEP=0 keeps the direct kernel)
+    // tensor grid: tabulate the one-dimensional kernel factors once (the direct kernel when the tables do not fit)
     GridXcov gx;
     bool use_sep = false;
     TmpDev t_tab(h);
     if (grid) {
-        static int sep_on = -1;
-        if (sep_on < 0) {
-            const char* e = getenv("GPE_GRID_SEP");
-            sep_on = (e && e[0] == '0') ? 0 : 1;
-        }
         int ltot = 0;
-        if (sep_on && plan_grid_sep(*grid, gx.sp, gx.smem, ltot)) {
+        if (plan_grid_sep(*grid, gx.sp, gx.smem, ltot)) {
             double* T = nullptr;
             CK(t_tab.get(&T, (size_t)ltot * h->npad));
             const long long tot = (long long)ltot * h->npad;
-            if (h->family == FAMILY_MATERN52)
-                grid_table_kernel<FAMILY_MATERN52><<<(unsigned)((tot + 255) / 256), 256, 0, h->st>>>(h->fXs, h->fwinv, *grid, gx.sp, h->npad, ltot, T);
-            else
-                grid_table_kernel<FAMILY_GAUSSIAN><<<(unsigned)((tot + 255) / 256), 256, 0, h->st>>>(h->fXs, h->fwinv, *grid, gx.sp, h->npad, ltot, T);
+            with_family(h->family, [&](auto fam) {
+                grid_table_kernel<fam><<<(unsigned)((tot + 255) / 256), 256, 0, h->st>>>(h->fXs, h->fwinv, *grid, gx.sp, h->npad, ltot, T);
+            });
             h->launches++;
             gx.T = T;
             use_sep = true;
@@ -1253,7 +1167,7 @@ int gpe_cross_cov(gpe_handle* h, const double* delta, double nugget, int kind, c
     CK(cudaMemcpyAsync(wd, w.data(), sizeof(double) * d, cudaMemcpyHostToDevice, h->st));
     CK(stage_points(P, Xs, m, mc, d, h->st));
     scale_train_kernel<<<(d * np + 255) / 256, 256, 0, h->st>>>(h->X, wd, h->n, d, np, xs);
-    CK(launch_xcov(h->family, xs, P, wd, h->n, d, np, mc, m, kind ? 1.0 : 1.0 - nugget, Cm, mc, h->st));
+    CK(launch_xcov<false>(h->family, xs, P, wd, h->n, d, np, mc, m, kind ? 1.0 : 1.0 - nugget, Cm, mc, h->st));
     h->launches += 2;
     bool dev = gpe_is_device_ptr(C_out);
     CK(cudaMemcpy2DAsync(C_out, sizeof(double) * m, Cm, sizeof(double) * mc, sizeof(double) * m, h->n,
@@ -1299,11 +1213,13 @@ int gpe_predict_fullcov(gpe_handle* h, const double* Xs, const double* Hs, int m
         // mean via the diagonal finalize (var == nullptr)
         predict_finalize_kernel<false><<<(m + 127) / 128, 128, 0, h->st>>>(nullptr, 0, aux, mp, P, Hd.p, bd, d, h->fK, h->fbeta, s2,
                                                                             h->fit_astar, m, md.p, nullptr, ImpFuse{});
-        auto fin = h->family == FAMILY_MATERN52 ? fullcov_finalize_kernel<FAMILY_MATERN52> : fullcov_finalize_kernel<FAMILY_GAUSSIAN>;
-        fin<<<(m + 127) / 128, 128, 0, h->st>>>(ZtZ, mp, aux, mp, P, Hd.p, bd, d, h->fwinv, h->fK, s2, h->fit_c, h->fit_astar, rn.p, m, G, Vd.p, 0);
-        size_t tot = (size_t)m * m;
-        fin<<<(unsigned)((tot + 255) / 256), 256, 0, h->st>>>(ZtZ, mp, aux, mp, P, Hd.p, bd, d, h->fwinv, h->fK, s2, h->fit_c, h->fit_astar,
-                                                            rn.p, m, G, Vd.p, 1);
+        const size_t tot = (size_t)m * m;
+        with_family(h->family, [&](auto fam) {
+            fullcov_finalize_kernel<fam><<<(m + 127) / 128, 128, 0, h->st>>>(ZtZ, mp, aux, mp, P, Hd.p, bd, d, h->fwinv, h->fK, s2, h->fit_c,
+                                                                             h->fit_astar, rn.p, m, G, Vd.p, 0);
+            fullcov_finalize_kernel<fam><<<(unsigned)((tot + 255) / 256), 256, 0, h->st>>>(ZtZ, mp, aux, mp, P, Hd.p, bd, d, h->fwinv, h->fK, s2,
+                                                                                          h->fit_c, h->fit_astar, rn.p, m, G, Vd.p, 1);
+        });
         h->launches += 3;
         CK(md.flush());
         CK(Vd.flush());
@@ -1405,10 +1321,11 @@ int gpe_sens_sample(gpe_handle* h, const double* XA, const double* XB, long long
             sens_pairdot_kernel<<<dim3((unsigned)(Mc / 128), ntile, (nw + SS_PG - 1) / SS_PG), 128, 0, st>>>(Zs[k], h->n, (int)Mc, nw, Parts[k]);
             fullcov_finalize_kernel<FAMILY_GAUSSIAN><<<(unsigned)((cols + 127) / 128), 128, 0, st>>>(
                 nullptr, cols, sl.Aux, cols, sl.X, nullptr, bd, d, h->fwinv, h->fK, s2, h->fit_c, h->fit_astar, nullptr, cols, Gs[k], nullptr, 0);
-            auto fin = h->family == FAMILY_MATERN52 ? sens_sample_finalize_kernel<FAMILY_MATERN52> : sens_sample_finalize_kernel<FAMILY_GAUSSIAN>;
-            fin<<<(unsigned)(Mc / 128), 128, (size_t)T * 128 * sizeof(double), st>>>(Parts[k], ntile, sl.Aux, Gs[k], sl.X, bd, d, h->fwinv,
-                                                                                      h->fbeta, wd.p, nw, (int)Mc, cnt, s2, h->fit_c, h->fit_astar,
-                                                                                      shift, bpart, ci * (Mc / 128));
+            with_family(h->family, [&](auto fam) {
+                sens_sample_finalize_kernel<fam><<<(unsigned)(Mc / 128), 128, (size_t)T * 128 * sizeof(double), st>>>(
+                    Parts[k], ntile, sl.Aux, Gs[k], sl.X, bd, d, h->fwinv, h->fbeta, wd.p, nw, (int)Mc, cnt, s2, h->fit_c, h->fit_astar, shift,
+                    bpart, ci * (Mc / 128));
+            });
         }
         h->launches += 3;
         return 0;
@@ -1441,7 +1358,7 @@ int gpe_predict_grad(gpe_handle* h, const double* Xs, long long m, double* dmean
     const bool x_dev = gpe_is_device_ptr(Xs), mean_dev = gpe_is_device_ptr(dmean), var_dev = dvar && gpe_is_device_ptr(dvar);
     const BasisDesc bd = basis_of(h);
     const double s2 = h->fit_sigma * h->fit_sigma;
-    const double kappa = h->family == FAMILY_MATERN52 ? 5.0 / 3.0 : 2.0;     // -2 R'(0)
+    const double kappa = with_family(h->family, [](auto fam) { return FAMILY_KAPPA<fam>; });
     rc = for_chunks(h, (m + Mc - 1) / Mc, [&](long long ci, int k, cudaStream_t st) {
         gpe_handle::PredSlot& sl = h->ps[k];
         const long long s = ci * Mc, cnt = std::min(Mc, m - s);
@@ -1450,7 +1367,7 @@ int gpe_predict_grad(gpe_handle* h, const double* Xs, long long m, double* dmean
         else CK(stage_points(sl.X, Xs + (size_t)s * d, cnt, (int)Mc, d, st));
         {
             ProfScope ps(h, gpe_handle::CAT_COV, st);
-            CK(launch_xcov_grad(h->family, h->fXs, P, h->fwinv, h->n, d, h->npad, (int)Mc, cnt, h->fit_c, sl.C, st));
+            CK(launch_xcov<true>(h->family, h->fXs, P, h->fwinv, h->n, d, h->npad, (int)Mc, cnt, h->fit_c, sl.C, cols, st));
         }
         h->launches++;
         int ntile = 0;

@@ -50,12 +50,7 @@ __global__ void __launch_bounds__(256) sens_pw_kernel(const double* __restrict__
     double* uj = ui + ST;                   // [64]
     __shared__ double red[32];
     const int tj = blockIdx.x, ti = blockIdx.y, tid = threadIdx.x;
-    for (int e = tid; e < ST * d; e += 256) {
-        int row = e / d, k = e % d;
-        int gi = ti * ST + row, gj = tj * ST + row;
-        Xi[k * ST + row] = (gi < n) ? X[(size_t)gi * d + k] * sg[k] : 0.0;
-        Xj[k * (ST + 2) + row] = (gj < n) ? X[(size_t)gj * d + k] * sg[k] : 0.0;
-    }
+    fill_scaled_tiles(X, sg, n, d, ti * ST, tj * ST, Xi, Xj, tid);
     if (tid < 2 * ST) {
         int row = tid & (ST - 1);
         int g = (tid < ST ? ti : tj) * ST + row;
@@ -72,25 +67,7 @@ __global__ void __launch_bounds__(256) sens_pw_kernel(const double* __restrict__
     __syncthreads();
     const int ty = tid >> 4, tx = tid & 15;
     double D[4][4];
-#pragma unroll
-    for (int a = 0; a < 4; a++)
-#pragma unroll
-        for (int c = 0; c < 4; c++) D[a][c] = 0.0;
-    for (int k = 0; k < d; k++) {
-        double xi[4], xj[4];
-#pragma unroll
-        for (int a = 0; a < 4; a++) xi[a] = Xi[k * ST + ty + 16 * a];
-        double2 v0 = *reinterpret_cast<const double2*>(&Xj[k * (ST + 2) + 2 * tx]);
-        double2 v1 = *reinterpret_cast<const double2*>(&Xj[k * (ST + 2) + 32 + 2 * tx]);
-        xj[0] = v0.x; xj[1] = v0.y; xj[2] = v1.x; xj[3] = v1.y;
-#pragma unroll
-        for (int a = 0; a < 4; a++)
-#pragma unroll
-            for (int c = 0; c < 4; c++) {
-                double df = xi[a] - xj[c];
-                D[a][c] = fma(df, df, D[a][c]);
-            }
-    }
+    sqdist_tile<4, 16, 32>(Xi, Xj, d, ty, tx, D);
     const bool lower = tj <= ti;
     double acc = 0.0;
 #pragma unroll

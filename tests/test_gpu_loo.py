@@ -209,7 +209,7 @@ def test_loo_of_trained_toy_sim_emulator(golden_dir, tmp_path):
     import shutil
     import gp_emu_uqsa_b200 as g
     for f in os.listdir(os.path.join(golden_dir, "toy-sim")):
-        shutil.copy(os.path.join(golden_dir, "toy-sim", f), tmp_path)
+        shutil.copyfile(os.path.join(golden_dir, "toy-sim", f), os.path.join(str(tmp_path), f))
     path = os.path.join(str(tmp_path), "toy-sim_beliefs")
     text = open(path).read().rstrip("\n")
     with open(path, "w") as f:

@@ -4,8 +4,6 @@ history matching, the multistart optimiser end to end, and the switch back to th
 import contextlib
 import io
 import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -13,7 +11,6 @@ import pytest
 from oracle import matern_oracle as M
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 MAT = 1
 MODES = [1, 5, 0, 4, 2, 6]          # MUCM, MUCM + free nugget, gp4ml, + free nugget, alt nugget, alt + free nugget
 
@@ -167,34 +164,29 @@ def test_posterior_mean_and_variance(kind):
     assert np.max(np.abs(V2 - Vref[:300, :300])) <= 1e-8 * scale
 
 
-_GRID_SCRIPT = r"""
-import sys, numpy as np
-sys.path.insert(0, %r)
-from gp_emu_uqsa_b200 import _lib
-rng = np.random.default_rng(5)
-X = rng.random((500, 3)); y = np.sin(X.sum(1)); H = np.column_stack([np.ones(500), X])
-dev = _lib.Device(0); dev.set_training(X, y, H); dev.set_basis([0, 1, 2], [1, 1, 1]); dev.set_kernel(1)
-assert dev.fit_state(np.array([0.3, 0.5, 0.7]), 1e-3, 1.2, 0)[2] == 0
-lv, lo, hi = np.array([9, 8, 7]), np.array([-0.1, 0.0, 0.2]), np.array([1.1, 1.0, 0.9])
-gm, gv = dev.predict_grid(lv, lo, hi, 3, 500)
-idx = np.arange(3, 503)
-dig = np.stack([idx // 56, (idx // 7) %% 8, idx %% 7], 1).astype(float)
-P = lo + (dig + 0.5) * ((hi - lo) / lv)
-pm, pv = dev.predict(P)
-np.save(sys.argv[1], np.stack([gm, gv, pm, pv]))
-"""
-
-
-def test_grid_matches_explicit_points_both_paths(tmp_path):
-    """Tensor grid through the additive table and through the direct kernel (GPE_GRID_SEP=0, read once per process,
-    hence the subprocesses) against the same points given explicitly."""
-    for sep in ("1", "0"):
-        out = str(tmp_path / ("g%s.npy" % sep))
-        env = dict(os.environ, GPE_GRID_SEP=sep)
-        subprocess.run([sys.executable, "-c", _GRID_SCRIPT % ROOT, out], check=True, env=env)
-        gm, gv, pm, pv = np.load(out)
-        assert np.max(np.abs(gm - pm)) <= 1e-10 * np.abs(pm).max()
-        assert np.max(np.abs(gv - pv)) <= 1e-9 * np.abs(pv).max()
+def test_grid_matches_explicit_points_both_paths():
+    """Tensor grid through the table kernel and through the direct kernel against the same points given explicitly, for both
+    families.  Levels (4100, 3, 3) sum to more than the tables hold (4096), so that grid takes the direct kernel; at one chunk the
+    table path launches exactly one kernel more (grid_table_kernel)."""
+    rng = np.random.default_rng(5)
+    X = rng.random((500, 3))
+    y = np.sin(X.sum(1))
+    lo, hi = np.array([-0.1, 0.0, 0.2]), np.array([1.1, 1.0, 0.9])
+    idx = np.arange(3, 503)
+    for family in (0, MAT):
+        dev = _device(X, y, np.column_stack([np.ones(500), X]), family=family)
+        assert dev.fit_state(np.array([0.3, 0.5, 0.7]), 1e-3, 1.2, 0)[2] == 0
+        launches = []
+        for lv in (np.array([9, 8, 7]), np.array([4100, 3, 3])):
+            before = dev.launches
+            gm, gv = dev.predict_grid(lv, lo, hi, 3, 500)
+            launches.append(dev.launches - before)
+            dig = np.stack([idx // (lv[1] * lv[2]), (idx // lv[2]) % lv[1], idx % lv[2]], 1).astype(float)
+            pm, pv = dev.predict(lo + (dig + 0.5) * ((hi - lo) / lv))
+            assert np.max(np.abs(gm - pm)) <= 1e-10 * np.abs(pm).max(), (family, lv)
+            assert np.max(np.abs(gv - pv)) <= 1e-9 * np.abs(pv).max(), (family, lv)
+        assert launches[0] == launches[1] + 1, (family, launches)
+        dev.close()
 
 
 def test_predict_implaus_bit_identical_to_predict_and_implausibility():

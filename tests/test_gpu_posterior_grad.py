@@ -164,7 +164,7 @@ def _golden_emulator(golden_dir, tmp, basis_str=None, train=True):
     import gp_emu_uqsa_b200 as g
     os.makedirs(tmp, exist_ok=True)
     for f in os.listdir(os.path.join(golden_dir, "toy-sim")):
-        shutil.copy(os.path.join(golden_dir, "toy-sim", f), tmp)
+        shutil.copyfile(os.path.join(golden_dir, "toy-sim", f), os.path.join(str(tmp), f))
     if basis_str is not None:
         path = os.path.join(str(tmp), "toy-sim_beliefs")
         txt = open(path).read().split("\n")
